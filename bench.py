@@ -6,6 +6,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W          # N > 1, one rank per GPU
     python bench.py --impl reference ...                                # the reference's CPU path
+    python bench.py ... --dump-outputs DIR                              # + x of the last timed step
 
 Workload (config.workload): BASELINE.json configs[2] -- generate_lap2d_matrix N = 40000, dense
 fp64, fixed 200 CG iterations, A row-sharded over the N GPUs by the reference's
@@ -293,27 +294,33 @@ def product_arm(args):
     variant_name = cgb.gemv_variants()[ctx.get_option("gemv_variant")]
 
     # ---- value: device-resident steps
-    def step():
+    def step(x_out=None):
         ctx.solve_begin(None, iters, 1e-10, False)   # x0 = 0 set on the device; not timed
         ms = ctx.iterate(iters)
-        info = ctx.solve_end(None, None)
+        info = ctx.solve_end(x_out, None)
         return ms, info
 
     for _ in range(args.warmup):
         step()
+    # --dump-outputs: the last timed step also downloads x (after its timed device region)
+    x_last = np.empty(n) if args.dump_outputs and rank == 0 else None
     sampler = ClockSampler(local) if rank == 0 else None
-    barrier()
-    l0 = ctx.launch_count()
-    t_wall0 = time.perf_counter()
-    dev_ms = 0.0
-    info = None
-    for _ in range(args.steps):
-        ms, info = step()
-        dev_ms += ms
-    barrier()
-    wall_s = time.perf_counter() - t_wall0
-    launches = ctx.launch_count() - l0
-    clocks = sampler.stop() if sampler else None
+    try:
+        barrier()
+        l0 = ctx.launch_count()
+        t_wall0 = time.perf_counter()
+        dev_ms = 0.0
+        info = None
+        for s in range(args.steps):
+            ms, info = step(x_last if s == args.steps - 1 else None)
+            dev_ms += ms
+        barrier()
+        wall_s = time.perf_counter() - t_wall0
+        launches = ctx.launch_count() - l0
+    finally:
+        clocks = sampler.stop() if sampler else None   # never leave nvidia-smi running
+    if x_last is not None:
+        dump_outputs(args.dump_outputs, x_last, info)
     dev_ms = allmax(dev_ms)
     launches_all = int(allsum(float(launches)))
     done_iters = int(info.iterations)
@@ -490,6 +497,17 @@ def product_arm(args):
     return 0
 
 
+def dump_outputs(out_dir, x, info):
+    """Writes what the last timed step returns to its caller -- x (every rank holds all of it) and
+    the solve info -- as float64 out_dir/<name>.npy.  The inputs are generated from N alone, so two
+    builds run with the same arguments can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"x": x, "k": info.k, "iterations": info.iterations, "converged": info.converged,
+              "rsold": info.rsold, "rsnew": info.rsnew}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 GOLDEN = {20000: "full_n20000_it200.npz", 28284: "full_n28284_it200.npz", 40000: "full_n40000_it200.npz"}
 
 
@@ -567,7 +585,11 @@ def main():
     ap.add_argument("--cpu-ranks", dest="cpu_ranks", type=int, default=1,
                     help="MPI ranks of the CPU reference (forked on this host; default 1 rank x all threads)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write x and the solve info of the last one as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "b200":
         print("bench.py: note: fewer than 3 warm-up steps requested", file=sys.stderr)
     if args.impl == "reference":

@@ -6,6 +6,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 pytestmark = [pytest.mark.gpu, pytest.mark.timeout(600)]
@@ -21,8 +22,10 @@ def _bench(*extra):
     return json.loads(lines[0])
 
 
-def test_bench_line_small_system():
-    d = _bench("--size", "4096", "--iters", "50", "--steps", "3", "--warmup", "3", "--cpu-iters", "10")
+def test_bench_line_small_system(O, tmp_path):
+    dump = tmp_path / "out"
+    d = _bench("--size", "4096", "--iters", "50", "--steps", "3", "--warmup", "3", "--cpu-iters", "10",
+               "--dump-outputs", str(dump))
     for key in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better",
                 "scaling", "vs_baseline", "dtype", "data", "config", "roofline", "cpu_baseline", "e2e",
                 "gpu_launches", "clocks"):
@@ -48,6 +51,14 @@ def test_bench_line_small_system():
     if os.path.exists(os.path.join(ROOT, "oracle", "_ref", "cgsolver_ref")):
         assert cb["kind"] == "reference" and cb["cores"] >= 1 and cb["value"] > 0
     assert "sm_mhz" in d["clocks"] and "reasons" in d["clocks"]
+    # --dump-outputs: what the last timed step returned, bit for bit the oracle's 50 iterations
+    ref = O.solve(O.generate_lap2d(4096), O.init_source_term(4096), max_iter=50, nranks=1, nblk=148)
+    out = {f.stem: np.load(f) for f in dump.glob("*.npy")}
+    assert sorted(out) == ["converged", "iterations", "k", "rsnew", "rsold", "x"]
+    assert all(a.dtype == np.float64 for a in out.values())
+    assert np.array_equal(out["x"], ref.x)
+    assert (out["k"], out["iterations"], out["converged"]) == (ref.k, len(ref.hist), ref.converged)
+    assert (out["rsold"], out["rsnew"]) == (ref.rsold, ref.rsnew)
 
 
 def test_bench_line_graph_schedule():

@@ -93,6 +93,40 @@ def test_form2_compat_kernel_mode(O, tmp_path):
     assert [row.split(",")[:2] for row in out.read_text().splitlines()] == [["64", "16"], ["8", "900"]]
 
 
+def test_cli_prints_what_the_reference_printed(O, tmp_path, golden_dir):
+    """Both command-line forms against the stored stdout of the unmodified reference's own cgsolver on
+    the same command line (tests/golden/, make_golden.py): a run capped above the rounding floor prints
+    its [STEP k] and, to the 7 printed digits, its three numbers; converged runs stop within +-1 of an
+    iteration count the reference itself produces for the system."""
+    from parity_util import reference_k_set
+
+    def numbers(line):
+        m = LINE.match(line if line.startswith("\t") else "\t" + line)
+        assert m, line
+        return int(m.group(1)), [float(m.group(i)) for i in (2, 3, 4)]
+
+    out = tmp_path / "res.txt"
+    g = np.load(os.path.join(golden_dir, "gen_n1000_it50.npz"))
+    r = _run(["1000", str(out), "50"])
+    assert r.returncode == 0, r.stderr
+    (k, mine), (k_ref, ref) = numbers(_step_line(r.stdout)), numbers(str(g["openblas_stdout_line"]))
+    assert k == k_ref == 50
+    for a, b in zip(mine, ref):
+        assert abs(a - b) <= 2e-6 * abs(b), (mine, ref)
+    mtx = str(tmp_path / "lap30.mtx")
+    O.write_lap2d_5pt_mtx(mtx, 30)
+    for name, args in (("gen_n1024.npz", ["1024", str(out)]),
+                       ("mtx_lap2d_5pt_n30.npz", [mtx, "64", "16", "true", str(out)])):
+        g = np.load(os.path.join(golden_dir, name))
+        r = _run(args)
+        assert r.returncode == 0, r.stderr
+        k, (_, nx, _) = numbers(_step_line(r.stdout))
+        assert min(abs(k - kr) for kr in reference_k_set(golden_dir, g)) <= 1, (name, k)
+        assert abs(nx - float(g["openblas_norm_x"])) <= 2e-6 * nx, name
+    rows = out.read_text().splitlines()
+    assert [row.split(",")[:2] for row in rows] == [["1000", "1"], ["1024", "1"], ["64", "16"]]
+
+
 def test_multi_gpu_cli_psize_column(O, tmp_path, cgb):
     if cgb.device_count() < 2:
         pytest.skip("needs 2 GPUs")
