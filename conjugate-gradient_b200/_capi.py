@@ -45,6 +45,7 @@ SIGNATURES = [
     ("cgb_device_count", C.c_int, [C.POINTER(C.c_int)]),
     ("cgb_partition", C.c_int, [C.c_int64, C.c_int, _i64p, _i64p]),
     ("cgb_create", C.c_int, [C.c_int64, C.c_int, C.c_int, C.c_int, C.POINTER(_CTX)]),
+    ("cgb_create_csr", C.c_int, [C.c_int64, C.c_int, C.c_int, C.c_int, C.POINTER(_CTX)]),
     ("cgb_destroy", C.c_int, [_CTX]),
     ("cgb_comm_unique_id", C.c_int, [C.c_void_p]),
     ("cgb_comm_init", C.c_int, [_CTX, C.c_void_p]),
@@ -140,13 +141,21 @@ def gemv_variants():
 
 
 class Context:
-    """One rank (= one GPU, one row shard).  Thin object wrapper over cgb_ctx*."""
+    """One rank (= one GPU, one row shard).  Thin object wrapper over cgb_ctx*.
 
-    def __init__(self, n: int, rank: int = 0, world: int = 1, device: int = 0):
+    storage="dense" holds the shard as rows x ld doubles (cgb_create), storage="csr" as CSR
+    (cgb_create_csr): bitwise the same results, memory bounded by the non-zeros."""
+
+    _CREATE = {"dense": "cgb_create", "csr": "cgb_create_csr"}
+
+    def __init__(self, n: int, rank: int = 0, world: int = 1, device: int = 0, storage: str = "dense"):
+        if storage not in self._CREATE:
+            raise ValueError(f"storage must be 'dense' or 'csr', not {storage!r}")
         self._lib = load()
         self._h = _CTX()
-        _check(self._lib.cgb_create(n, rank, world, device, C.byref(self._h)))
+        _check(getattr(self._lib, self._CREATE[storage])(n, rank, world, device, C.byref(self._h)))
         self.n = n
+        self.storage = storage
 
     def close(self):
         if getattr(self, "_h", None):
@@ -194,6 +203,10 @@ class Context:
         v = C.c_int64()
         _check(self._lib.cgb_get_option(self._h, key.encode(), C.byref(v)))
         return v.value
+
+    def nnz(self) -> int:
+        """Entries stored in this rank's shard (CSR storage; 0 for a dense context)."""
+        return self.get_option("nnz")
 
     def autotune(self, iters: int = 0) -> dict:
         """One-off tile-shape selection (cgb_autotune); returns the choice and every candidate's time."""

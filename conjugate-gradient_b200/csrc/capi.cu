@@ -134,6 +134,9 @@ struct cgb_ctx {
     int trace_blocks[3] = {0, 0, 0}; // capacity in blocks per launch
     int trace_cap = 0;
 
+    int storage = 0;               // 0: dense rows x ld shard `A`, 1: CSR shard `csr` (cgb_create_csr)
+    CsrShard csr;
+    unsigned int *arrive = nullptr; // CSR: arrival counters of the once-per-iteration vector phase
     double *A = nullptr, *p = nullptr, *r = nullptr, *x = nullptr, *b = nullptr;
     double *apx = nullptr, *rrpart = nullptr, *papart = nullptr, *scratch = nullptr, *hist = nullptr, *sink = nullptr;
     // apx: plain gather buffer [world][slot_cap] doubles.  ll: fused-mode LL buffers
@@ -218,6 +221,9 @@ GemvArgs make_gemv_args(const cgb_ctx *c, const double *v, int advance)
     GemvArgs a;
     memset(&a, 0, sizeof a);
     a.A = c->A;
+    a.csr_rp = c->csr.rp;
+    a.csr_col = c->csr.col;
+    a.csr_val = c->csr.val;
     a.v = v;
     a.base = c->apx;
     a.ctl = c->ctl;
@@ -262,6 +268,7 @@ VecArgs make_vec_args(const cgb_ctx *c)
     a.n = c->n;
     a.tol = c->tol;
     a.pdl = (c->opt_pdl && !c->opt_profile) ? 1 : 0;
+    a.arrive = c->arrive;
     if (c->trace_cap > 0) {
         a.trace_xr = make_trace(c, 1, (int)c->nchunks);
         a.trace_p = make_trace(c, 2, (int)c->nchunks);
@@ -308,7 +315,8 @@ int launch_matvec(cgb_ctx *c, const double *v, int advance, int variant)
         return CGB_OK;
     }
     const GemvArgs a = make_gemv_args(c, v, advance);
-    CK(gemv_variant(variant).launch(a, c->sm_count * gemv_variant(variant).ctas_per_sm, c->stream));
+    if (c->storage == 1) CK(launch_spmv(a, c->sm_count, c->stream));
+    else CK(gemv_variant(variant).launch(a, c->sm_count * gemv_variant(variant).ctas_per_sm, c->stream));
     c->kernel_launches += 1;
     return CGB_OK;
 }
@@ -323,17 +331,29 @@ int launch_gather(cgb_ctx *c)
     return CGB_OK;
 }
 
+// the three vector kernels of one iteration; CSR contexts compute every scalar once per iteration
+int launch_vector_phase(cgb_ctx *c)
+{
+    const VecArgs va = make_vec_args(c);
+    if (c->storage == 1) {
+        CK(launch_pap_alpha(va, c->stream));
+        CK(launch_update_xr_once(va, c->stream));
+        CK(launch_update_p_once(va, c->stream));
+    } else {
+        CK(launch_pap_partials(va, c->stream));                             // cg.cc:105
+        CK(launch_update_xr(va, c->stream));                                // cg.cc:106-117
+        CK(launch_update_p(va, c->stream));                                 // cg.cc:120-132
+    }
+    c->kernel_launches += 3;
+    return CGB_OK;
+}
+
 int launch_iteration(cgb_ctx *c)
 {
     int rc = launch_matvec(c, c->p, 1, c->variant);                        // cg.cc:100-102
     if (rc) return rc;
     if ((rc = launch_gather(c))) return rc;                                 // cg.cc:135-136 (moved)
-    const VecArgs va = make_vec_args(c);
-    CK(launch_pap_partials(va, c->stream));                                 // cg.cc:105
-    CK(launch_update_xr(va, c->stream));                                    // cg.cc:106-117
-    CK(launch_update_p(va, c->stream));                                     // cg.cc:120-132
-    c->kernel_launches += 3;
-    return CGB_OK;
+    return launch_vector_phase(c);
 }
 
 int build_graph(cgb_ctx *c)
@@ -380,6 +400,7 @@ void persist_scratch(const cgb_ctx *c, int *scr_n)
 // nullptr when the persistent schedule can run this context as configured, else the reason
 const char *persist_unusable(const cgb_ctx *c)
 {
+    if (c->storage == 1) return "CSR storage";
     if (c->opt_compat) return "compat mat-vec";
     if (c->opt_profile) return "profile mode (per-launch events)";
     if (c->world > 1 && c->opt_exchange != 1) return "ncclAllGather exchange";
@@ -503,7 +524,8 @@ extern "C" const char *cgb_gemv_variant_name(int v)
 }
 
 // ------------------------------------------------------------------ context
-extern "C" int cgb_create(int64_t n, int rank, int world, int device, cgb_ctx **out)
+// cgb_create / cgb_create_csr: everything but the shard is the same
+static int create_ctx(int64_t n, int rank, int world, int device, int storage, cgb_ctx **out)
 {
     if (!out) return fail(CGB_ERR_INVALID, "null out");
     *out = nullptr;
@@ -511,6 +533,8 @@ extern "C" int cgb_create(int64_t n, int rank, int world, int device, cgb_ctx **
     if (world < 1 || world > kMaxWorld || rank < 0 || rank >= world)
         return fail(CGB_ERR_INVALID, "bad rank/world %d/%d (world <= %d)", rank, world, kMaxWorld);
     if (n < world) return fail(CGB_ERR_INVALID, "n (%lld) < world (%d)", (long long)n, world);
+    if (storage == 1 && n > INT32_MAX)
+        return fail(CGB_ERR_INVALID, "CSR storage keeps 32-bit column indices: n must be <= %d", INT32_MAX);
     int ndev = 0;
     CK(cudaGetDeviceCount(&ndev));
     if (ndev == 0) return fail(CGB_ERR_NO_DEVICE, "no CUDA device");
@@ -529,6 +553,7 @@ extern "C" int cgb_create(int64_t n, int rank, int world, int device, cgb_ctx **
     c->rank = rank;
     c->world = world;
     c->device = device;
+    c->storage = storage;
     c->sm_count = prop.multiProcessorCount;
     if (const char *e = getenv("CGB_SPIN_TIMEOUT_MS")) { // default of the option "spin_timeout_ms"
         const long long v = atoll(e);
@@ -565,7 +590,15 @@ extern "C" int cgb_create(int64_t n, int rank, int world, int device, cgb_ctx **
     CKB(cudaEventCreateWithFlags(&c->ev_batch[0], cudaEventDisableTiming));
     CKB(cudaEventCreateWithFlags(&c->ev_batch[1], cudaEventDisableTiming));
     const size_t vec_bytes = (size_t)c->ld * sizeof(double);
-    CKB(cudaMalloc(&c->A, (size_t)c->rows * c->ld * sizeof(double)));
+    if (storage == 1) {
+        CKB(cudaMalloc(&c->csr.rp, (size_t)(c->rows + 1) * sizeof(long long)));
+        CKB(cudaMemsetAsync(c->csr.rp, 0, (size_t)(c->rows + 1) * sizeof(long long), c->stream));
+        CKB(cudaMalloc(&c->arrive, 2 * sizeof(unsigned int)));
+        CKB(cudaMemsetAsync(c->arrive, 0, 2 * sizeof(unsigned int), c->stream));
+    } else {
+        CKB(cudaMalloc(&c->A, (size_t)c->rows * c->ld * sizeof(double)));
+        CKB(cudaMemsetAsync(c->A, 0, (size_t)c->rows * c->ld * sizeof(double), c->stream));
+    }
     CKB(cudaMalloc(&c->p, vec_bytes));
     CKB(cudaMalloc(&c->r, vec_bytes));
     CKB(cudaMalloc(&c->x, vec_bytes));
@@ -596,7 +629,6 @@ extern "C" int cgb_create(int64_t n, int rank, int world, int device, cgb_ctx **
     CKB(cudaHostGetDevicePointer(&c->d_hdone, c->h_done, 0));
     CKB(cudaHostAlloc(&c->h_pin, 64 * sizeof(double), cudaHostAllocDefault));
     *c->h_done = 0;
-    CKB(cudaMemsetAsync(c->A, 0, (size_t)c->rows * c->ld * sizeof(double), c->stream));
     CKB(cudaMemsetAsync(c->p, 0, vec_bytes, c->stream));
     CKB(cudaMemsetAsync(c->r, 0, vec_bytes, c->stream));
     CKB(cudaMemsetAsync(c->x, 0, vec_bytes, c->stream));
@@ -606,11 +638,25 @@ extern "C" int cgb_create(int64_t n, int rank, int world, int device, cgb_ctx **
     CKB(cudaMemsetAsync(c->st, 0, sizeof(State), c->stream));
     CKB(cudaStreamSynchronize(c->stream));
     CKB(preload_vec_kernels());
-    CKB(gemv_variant(c->variant).preload());
-    if (persist_index(c) >= 0) CKB(persist_variant(persist_index(c)).preload());
+    if (storage == 1) {
+        CKB(preload_spmv_kernels());
+    } else {
+        CKB(gemv_variant(c->variant).preload());
+        if (persist_index(c) >= 0) CKB(persist_variant(persist_index(c)).preload());
+    }
 #undef CKB
     *out = c;
     return CGB_OK;
+}
+
+extern "C" int cgb_create(int64_t n, int rank, int world, int device, cgb_ctx **out)
+{
+    return create_ctx(n, rank, world, device, 0, out);
+}
+
+extern "C" int cgb_create_csr(int64_t n, int rank, int world, int device, cgb_ctx **out)
+{
+    return create_ctx(n, rank, world, device, 1, out);
 }
 
 extern "C" int cgb_destroy(cgb_ctx *c)
@@ -627,6 +673,10 @@ extern "C" int cgb_destroy(cgb_ctx *c)
     for (double *p : bufs)
         if (p) cudaFree(p);
     if (c->st) cudaFree(c->st);
+    if (c->csr.rp) cudaFree(c->csr.rp);
+    if (c->csr.col) cudaFree(c->csr.col);
+    if (c->csr.val) cudaFree(c->csr.val);
+    if (c->arrive) cudaFree(c->arrive);
     if (c->compat_part) cudaFree(c->compat_part);
     free_trace(c);
     if (c->ll) cudaFree(c->ll);
@@ -746,9 +796,15 @@ extern "C" int cgb_generate_lap2d(cgb_ctx *c)
     int rc = use_device(c);
     if (rc) return rc;
     if (c->in_solve) return fail(CGB_ERR_STATE, "solve in progress");
-    CK(launch_generate_lap2d(c->A, c->n, c->ld, c->row0, c->rows, c->stream));
-    c->kernel_launches += 1;
-    CK(cudaStreamSynchronize(c->stream));
+    if (c->storage == 1) {
+        c->matrix_set = false;
+        CK(csr_generate_lap2d(&c->csr, c->n, c->row0, c->rows, c->stream));
+        c->kernel_launches += 3;
+    } else {
+        CK(launch_generate_lap2d(c->A, c->n, c->ld, c->row0, c->rows, c->stream));
+        c->kernel_launches += 1;
+        CK(cudaStreamSynchronize(c->stream));
+    }
     c->matrix_set = true;
     return CGB_OK;
 }
@@ -759,6 +815,7 @@ extern "C" int cgb_set_matrix_rows(cgb_ctx *c, const double *rows_host, int64_t 
     int rc = use_device(c);
     if (rc) return rc;
     if (c->in_solve) return fail(CGB_ERR_STATE, "solve in progress");
+    if (c->storage == 1) return fail(CGB_ERR_STATE, "dense rows cannot be set on a CSR context (use cgb_set_matrix_coo)");
     if (!rows_host || nrows < 0 || first_row < 0 || first_row + nrows > c->n || ld_host < c->n)
         return fail(CGB_ERR_INVALID, "bad row block [%lld, +%lld) ld %lld", (long long)first_row,
                     (long long)nrows, (long long)ld_host);
@@ -800,6 +857,24 @@ extern "C" int cgb_set_matrix_coo(cgb_ctx *c, int64_t nz, const int32_t *irn, co
             cudaFree(bad);
         }
     } t;
+    if (c->storage == 1) {
+        // CSR: the writes as sequence 2z (direct) / 2z+1 (mirror), stable-sorted by (row, column),
+        // the last of every run kept (spmv.cu)
+        if (nz > 0) {
+            CK(cudaMalloc(&t.i, (size_t)nz * sizeof(int)));
+            CK(cudaMalloc(&t.j, (size_t)nz * sizeof(int)));
+            CK(cudaMalloc(&t.v, (size_t)nz * sizeof(double)));
+            CK(cudaMemcpyAsync(t.i, irn, (size_t)nz * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+            CK(cudaMemcpyAsync(t.j, jcn, (size_t)nz * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+            CK(cudaMemcpyAsync(t.v, val, (size_t)nz * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+        }
+        int bad = 0;
+        c->matrix_set = false;
+        CK(csr_from_coo(&c->csr, c->n, c->row0, c->rows, t.i, t.j, t.v, nz, symmetric ? 1 : 0, &bad, c->stream));
+        if (bad) return fail(CGB_ERR_INVALID, "a COO entry lies outside %lld x %lld", (long long)c->n, (long long)c->n);
+        c->matrix_set = true;
+        return CGB_OK;
+    }
     CK(cudaMemsetAsync(c->A, 0, (size_t)c->rows * c->ld * sizeof(double), c->stream));
     if (nz > 0) {
         CK(cudaMalloc(&t.i, (size_t)nz * sizeof(int)));
@@ -837,7 +912,17 @@ extern "C" int cgb_get_matrix_rows(cgb_ctx *c, double *rows_host, int64_t first_
         ld_host < c->n)
         return fail(CGB_ERR_INVALID, "rows [%lld, +%lld) are not inside this rank's shard",
                     (long long)first_row, (long long)nrows);
-    if (nrows > 0) {
+    if (nrows > 0 && c->storage == 1) { // densified through a device buffer (a test hook)
+        double *dense = nullptr;
+        CK(cudaMalloc(&dense, (size_t)nrows * c->n * sizeof(double)));
+        cudaError_t e = csr_densify(c->csr, first_row - c->row0, nrows, c->n, dense, c->stream);
+        if (e == cudaSuccess)
+            e = cudaMemcpy2DAsync(rows_host, (size_t)ld_host * 8, dense, (size_t)c->n * 8, (size_t)c->n * 8,
+                                  (size_t)nrows, cudaMemcpyDeviceToHost, c->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+        cudaFree(dense);
+        CK(e);
+    } else if (nrows > 0) {
         CK(cudaMemcpy2DAsync(rows_host, (size_t)ld_host * 8, c->A + (first_row - c->row0) * c->ld,
                              (size_t)c->ld * 8, (size_t)c->n * 8, (size_t)nrows,
                              cudaMemcpyDeviceToHost, c->stream));
@@ -875,6 +960,10 @@ extern "C" int cgb_set_option(cgb_ctx *c, const char *key, int64_t value)
     const std::string k(key);
     // the schedules hand the complete state over between launches, so this one may change mid-solve
     if (c->in_solve && k != "schedule") return fail(CGB_ERR_STATE, "options cannot change during a solve");
+    // CSR contexts have one mat-vec: the dense-only modes are refused, the launch-shape knobs
+    // (set by the CUDA-form command line) are kept but change nothing
+    if (c->storage == 1 && ((k == "compat" && value == 1) || ((k == "loopback" || k == "trace") && value > 0)))
+        return fail(CGB_ERR_STATE, "option '%s' = %lld is not available with CSR storage", key, (long long)value);
     if (k == "gemv_variant") {
         if (value < 0 || value >= gemv_variant_count())
             return fail(CGB_ERR_INVALID, "gemv_variant %lld out of range", (long long)value);
@@ -1023,6 +1112,8 @@ extern "C" int cgb_get_option(cgb_ctx *c, const char *key, int64_t *value)
     else if (k == "num_threads") *value = c->opt_num_threads;
     else if (k == "block_width") *value = c->opt_block_width;
     else if (k == "transposed") *value = c->opt_transposed;
+    else if (k == "storage") *value = c->storage;
+    else if (k == "nnz") *value = c->storage == 1 ? c->csr.nnz : 0;
     else return fail(CGB_ERR_INVALID, "unknown option '%s'", key);
     return CGB_OK;
 }
@@ -1167,11 +1258,7 @@ extern "C" int cgb_iterate(cgb_ctx *c, int64_t iters, float *ms)
                 if ((rc = launch_matvec(c, c->p, 1, c->variant))) return rc;
                 CK(cudaEventRecord(c->prof_ev[slot + 1], c->stream));
                 if ((rc = launch_gather(c))) return rc;
-                const VecArgs va = make_vec_args(c);
-                CK(launch_pap_partials(va, c->stream));
-                CK(launch_update_xr(va, c->stream));
-                CK(launch_update_p(va, c->stream));
-                c->kernel_launches += 3;
+                if ((rc = launch_vector_phase(c))) return rc;
                 i += 1;
             } else {
                 if ((rc = launch_iteration(c))) return rc;
@@ -1335,7 +1422,7 @@ extern "C" int cgb_bench_gemv(cgb_ctx *c, int variant, int reps, float *ms_avg)
     // A rank of a world > 1 without a configured exchange times its shard with local stores
     // only (shape tuning on one GPU).  The gather geometry follows the timed variant.
     const int keep_variant = c->variant;
-    if (variant != keep_variant) {
+    if (variant != keep_variant && c->storage == 0) {
         set_variant(c, variant);
         drop_graph(c);
         CK(gemv_variant(variant).preload()); // loads the kernel and sets its shared-memory limit
@@ -1364,9 +1451,13 @@ extern "C" int cgb_bench_read(cgb_ctx *c, int reps, float *ms_avg)
     if (rc) return rc;
     if (reps < 1) return fail(CGB_ERR_INVALID, "reps < 1");
     const long long nd = c->rows * c->ld;
-    CK(launch_read_stream(c->A, nd, c->sink, c->sm_count, c->stream));
+    auto read_once = [&]() {
+        return c->storage == 1 ? launch_read_csr(c->csr, c->rows, c->sink, c->sm_count, c->stream)
+                               : launch_read_stream(c->A, nd, c->sink, c->sm_count, c->stream);
+    };
+    CK(read_once());
     CK(cudaEventRecord(c->ev0, c->stream));
-    for (int i = 0; i < reps; ++i) CK(launch_read_stream(c->A, nd, c->sink, c->sm_count, c->stream));
+    for (int i = 0; i < reps; ++i) CK(read_once());
     CK(cudaEventRecord(c->ev1, c->stream));
     CK(cudaEventSynchronize(c->ev1));
     c->kernel_launches += reps + 1;
@@ -1427,6 +1518,10 @@ extern "C" int cgb_autotune(cgb_ctx *c, int iters, int *chosen, float *us_per_it
     const int nv = gemv_variant_count();
     if (us_per_iter)
         for (int v = 0; v < nv; ++v) us_per_iter[v] = -1.f;
+    if (c->storage == 1) { // one CSR mat-vec: nothing to choose
+        if (chosen) *chosen = c->variant;
+        return CGB_OK;
+    }
     const int keep_variant = c->variant, keep_loopback = c->opt_loopback, keep_exchange = c->opt_exchange;
     const bool keep_ready = c->p2p_ready;
     const double keep_tol = c->tol;

@@ -92,6 +92,11 @@ struct GemvArgs {
     int pdl;              // host side: launch with the programmatic-dependent-launch attribute
     int l2_prefetch;      // pipeline steps of A prefetched into L2 before the dependency wait
     Trace trace;          // diagnostic timeline (option "trace"); buf == nullptr: off
+    // CSR storage (spmv.cu; A is then nullptr): rows + 1 row pointers, global column indices
+    // ascending and unique within a row, values
+    const long long *csr_rp;
+    const int *csr_col;
+    const double *csr_val;
 };
 
 // ---- persistent schedule (persist.cu): the whole CG loop in one cooperative launch ----
@@ -289,6 +294,22 @@ __device__ __forceinline__ void advance_state(const GemvArgs &a, int lane)
         st->rsold = s;                          // cg.cc:132 rsold = rsnew (cg.cc:91 when it == -1)
         st->rsnew = s;
         st->iter = it + 1;
+    }
+}
+
+// One result (a row of Ap) into the gather buffer: locally, or --
+// fused exchange -- as a self-flagging LL entry straight into every rank's buffer over NVLink
+// (peer stores).  That store IS the all-gather: no fence, no flag, no collective kernel.
+// Called by ALL lanes of a warp with the same value: in fused mode lane g stores to rank g -- one
+// store instruction with `world` transactions in flight (a loop in one lane serialises the
+// strong.sys stores: ~0.35 us each on the local GPU, a NVLink round trip each to a peer).
+__device__ __forceinline__ void store_out(const GemvArgs &a, long long plain_off, long long ll_off,
+                                          unsigned tag, double v, int lane)
+{
+    if (!a.p2p) {
+        if (lane == 0) a.base[plain_off] = v;
+    } else if (lane < a.world) {
+        ll_store(a.peer_ll[lane] + ll_off, v, tag);
     }
 }
 

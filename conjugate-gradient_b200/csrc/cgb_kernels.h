@@ -1,4 +1,4 @@
-// cgb_kernels.h -- host-callable launchers of the sm_100a kernels (gemv.cu, vec.cu).
+// cgb_kernels.h -- host-callable launchers of the sm_100a kernels (gemv.cu, spmv.cu, vec.cu).
 #pragma once
 
 #include "cgb_device.cuh"
@@ -16,8 +16,7 @@ template <class... KArgs, class... Args>
 inline cudaError_t launch_kernel(void (*kernel)(KArgs...), int grid, int block, size_t smem,
                                  cudaStream_t stream, bool pdl, Args &&...args)
 {
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof cfg);
+    cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid, 1, 1);
     cfg.blockDim = dim3((unsigned)block, 1, 1);
     cfg.dynamicSmemBytes = smem;
@@ -76,6 +75,7 @@ struct VecArgs {
     double tol;
     int pdl;                 // host side: chain update_xr / update_p with programmatic dependent launch
     Trace trace_xr, trace_p; // diagnostic timelines of update_xr / update_p (buf == nullptr: off)
+    unsigned int *arrive;    // 2 zeroed arrival counters of the once-per-iteration phase (CSR contexts)
 };
 // r = b - A x0 ; p = r ; rrpart = chunk partials of r.p             (cg.cc:77-92)
 cudaError_t launch_init_residual(const VecArgs &a, cudaStream_t s);
@@ -98,6 +98,15 @@ cudaError_t launch_dot(const double *a, const double *b, long long n, double *sc
 cudaError_t launch_pap_plain(const double *v, const double *apx, const Gather &g, long long n, double *papart,
                              double *out, cudaStream_t s);
 
+// The same three steps with every scalar computed ONCE per iteration (CSR contexts): the last
+// block of pap_alpha reduces the p'Ap partials into alpha (st->conj, st->alpha), the last block of
+// update_xr_once reduces the r'r partials into st->rsnew and takes the stop test, update_p_once
+// reads both.  Per-iteration traffic is O(N) and nothing is sized by the chunk count; every State
+// transition and every bit equals the kernels above.
+cudaError_t launch_pap_alpha(const VecArgs &a, cudaStream_t s);
+cudaError_t launch_update_xr_once(const VecArgs &a, cudaStream_t s);
+cudaError_t launch_update_p_once(const VecArgs &a, cudaStream_t s);
+
 // fused mode, hooks only: consume the running exchange into the plain gather buffer `apx`
 // (the kernels of the iteration read the LL entries directly)
 cudaError_t launch_exchange_collect(double *apx, const Gather &g, cudaStream_t s);
@@ -111,5 +120,27 @@ cudaError_t launch_generate_lap2d(double *A, long long n, long long ld, long lon
 cudaError_t launch_scatter_coo(double *A, long long n, long long ld, long long row0, long long rows,
                                const int *irn, const int *jcn, const double *val, long long nz,
                                int symmetric, unsigned char *win, int *bad, cudaStream_t s);
+
+// ---- CSR storage (spmv.cu) ----------------------------------------------------------
+// The shard: rp[rows + 1] (allocated with the context), col[nnz] / val[nnz] (sized by the builders)
+struct CsrShard {
+    long long *rp = nullptr;
+    int *col = nullptr;
+    double *val = nullptr;
+    long long nnz = 0;
+};
+cudaError_t preload_spmv_kernels();
+// the CSR mat-vec, lane order (bitwise the dense mat-vec); a.csr_* set
+cudaError_t launch_spmv(const GemvArgs &a, int sm_count, cudaStream_t s);
+// generate_lap2d_matrix's non-zeros of rows [row0, row0 + rows); synchronises
+cudaError_t csr_generate_lap2d(CsrShard *m, long long n, long long row0, long long rows, cudaStream_t s);
+// Matrix::read semantics from device COO triples (file order, mirror when symmetric, later writes
+// win); *bad_host = 1 (and the shard unchanged) when an entry lies outside n x n; synchronises
+cudaError_t csr_from_coo(CsrShard *m, long long n, long long row0, long long rows, const int *irn, const int *jcn,
+                         const double *val, long long nz, int symmetric, int *bad_host, cudaStream_t s);
+// local rows [lr0, lr0 + nrows) as a dense nrows x n device buffer
+cudaError_t csr_densify(const CsrShard &m, long long lr0, long long nrows, long long n, double *dst, cudaStream_t s);
+// streams the three CSR arrays once (the read ceiling of the CSR mat-vec)
+cudaError_t launch_read_csr(const CsrShard &m, long long rows, double *sink, int sm_count, cudaStream_t s);
 
 } // namespace cgb

@@ -28,22 +28,6 @@
 
 namespace cgb {
 
-// One result (a row of Ap) into the gather buffer: locally, or --
-// fused exchange -- as a self-flagging LL entry straight into every rank's buffer over NVLink
-// (peer stores).  That store IS the all-gather: no fence, no flag, no collective kernel.
-// Called by ALL lanes of a warp with the same value: in fused mode lane g stores to rank g -- one
-// store instruction with `world` transactions in flight (a loop in one lane serialises the
-// strong.sys stores: ~0.35 us each on the local GPU, a NVLink round trip each to a peer).
-__device__ __forceinline__ void store_out(const GemvArgs &a, long long plain_off, long long ll_off,
-                                          unsigned tag, double v, int lane)
-{
-    if (!a.p2p) {
-        if (lane == 0) a.base[plain_off] = v;
-    } else if (lane < a.world) {
-        ll_store(a.peer_ll[lane] + ll_off, v, tag);
-    }
-}
-
 // ------------------------------------------------------------------------------- TMA
 // POL 0: 1-D bulk copies (one per tile row) with L2 hints -- the product path.
 // POL 1: the same without hints.

@@ -1,0 +1,380 @@
+// spmv.cu -- CSR storage of the row shard: the mat-vec in lane order and the builders of the shard
+// (generate_lap2d_matrix, Matrix::read's COO semantics) on the device.
+//
+// Exactness.  The dense mat-vec (gemv.cu, oracle/cg_oracle.h "lane order") keeps 64 accumulators
+// acc[c % 64] = fma(A[i][c], p[c], acc[c % 64]) over ascending c from +0, adds acc[2l] + acc[2l+1]
+// per lane and finishes with the butterfly ^16, ^8, ^4, ^2, ^1.  An accumulator is never -0 (it
+// starts at +0 and an exactly-zero sum rounds to +0 unless both operands are -0), so for a finite
+// p[c] an entry A[i][c] = +-0 leaves it unchanged, and so does adding an all-zero partner in the
+// lane sum or the butterfly.  Touching the stored entries only -- each bucket's fma chain over its
+// entries in ascending column order, absent buckets and partners skipped -- therefore gives the
+// dense result bit for bit.  (A NaN / Inf of p at a column where A is zero makes the dense row
+// NaN and leaves this one alone; only a solve that has already diverged gets there.)
+//
+// Layout: one warp per 32 consecutive rows.  A row of at most kShortRow entries (the 2-D stencil
+// has 3 to 5) is done by its own lane: bucket sums, then the merge tree above with absent
+// entries skipped.  Longer rows are taken by the whole warp one after the other, lane l owning
+// buckets 2l and 2l+1 exactly like the dense consumers; entries reach their owner in column order
+// in 32-entry slabs broadcast by shuffle.
+#include "cgb_device.cuh"
+#include "cgb_kernels.h"
+
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
+#include <cub/device/device_select.cuh>
+
+namespace cgb {
+
+namespace {
+
+constexpr int kShortRow = 8;    // entries a single lane handles (the merge tree is kShortRow^2 / 2 per level)
+constexpr int kSpmvThreads = 256;
+
+// lane order for a row of at most kShortRow entries, by one thread
+__device__ __forceinline__ double row_short(const int *col, const double *val, int len, const double *v)
+{
+    double s[kShortRow];
+    int key[kShortRow];
+    bool live[kShortRow];
+#pragma unroll
+    for (int e = 0; e < kShortRow; ++e) {
+        live[e] = false;
+        key[e] = 0;
+        s[e] = 0.0;
+        if (e < len) {
+            const int c = __ldcs(col + e);
+            const double prod_a = __ldcs(val + e), pv = __ldg(v + c);
+            const int b = c & 63;
+            bool merged = false;
+#pragma unroll
+            for (int f = 0; f < e; ++f)
+                if (live[f] && key[f] == b) { // same bucket, earlier column: continue its chain
+                    s[f] = __fma_rn(prod_a, pv, s[f]);
+                    merged = true;
+                }
+            key[e] = b;
+            live[e] = !merged;
+            s[e] = merged ? 0.0 : __fma_rn(prod_a, pv, 0.0);
+        }
+    }
+    // bucket 2l + j: lane sum (bit 0), then the butterfly over the lane index l = bits 5..1
+    const int bits[6] = {1, 32, 16, 8, 4, 2};
+#pragma unroll
+    for (int lv = 0; lv < 6; ++lv) {
+#pragma unroll
+        for (int e = 0; e < kShortRow; ++e) key[e] &= ~bits[lv];
+#pragma unroll
+        for (int e = 1; e < kShortRow; ++e)
+#pragma unroll
+            for (int f = 0; f < e; ++f)
+                if (live[f] && live[e] && key[f] == key[e]) {
+                    s[f] = __dadd_rn(s[f], s[e]);
+                    live[e] = false;
+                }
+    }
+    double y = 0.0;
+#pragma unroll
+    for (int e = 0; e < kShortRow; ++e)
+        if (live[e]) y = s[e];
+    return y;
+}
+
+// lane order for a row of any length, by the whole warp (every lane returns the row's value)
+__device__ __forceinline__ double row_warp(const int *col, const double *val, long long len, const double *v, int lane)
+{
+    double acc0 = 0.0, acc1 = 0.0;
+    for (long long k0 = 0; k0 < len; k0 += 32) {
+        const long long k = k0 + lane;
+        int c = 0;
+        double av = 0.0, pv = 0.0;
+        if (k < len) {
+            c = __ldcs(col + k);
+            av = __ldcs(val + k);
+            pv = __ldg(v + c);
+        }
+        const int m = (len - k0 < 32) ? (int)(len - k0) : 32;
+        for (int j = 0; j < m; ++j) {
+            const int cj = __shfl_sync(0xffffffffu, c, j);
+            const double aj = __shfl_sync(0xffffffffu, av, j);
+            const double pj = __shfl_sync(0xffffffffu, pv, j);
+            if (((cj & 63) >> 1) == lane) {
+                if (cj & 1) acc1 = __fma_rn(aj, pj, acc1);
+                else acc0 = __fma_rn(aj, pj, acc0);
+            }
+        }
+    }
+    return warp_butterfly(__dadd_rn(acc0, acc1));
+}
+
+__global__ void __launch_bounds__(kSpmvThreads) spmv_csr_kernel(const GemvArgs a)
+{
+    griddep_launch_dependents();
+    griddep_wait();
+    if (a.st->done) return;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    if (a.advance && blockIdx.x == 0 && warp == 0) advance_state(a, lane);
+    const unsigned tag = a.p2p ? exchange_tag(a.ctl) : 0u;
+    const long long obase = a.slot_off;
+    const long long lbase = (long long)(tag & 1u) * a.bufstride + a.slot_off;
+    const long long nwarps = (long long)gridDim.x * (kSpmvThreads / 32);
+    for (long long w = (long long)blockIdx.x * (kSpmvThreads / 32) + warp; w * 32 < a.rows; w += nwarps) {
+        const long long li = w * 32 + lane;
+        long long beg = 0, len = 0;
+        if (li < a.rows) {
+            beg = __ldcs(a.csr_rp + li);
+            len = __ldcs(a.csr_rp + li + 1) - beg;
+        }
+        const bool is_long = len > kShortRow;
+        if (li < a.rows && !is_long) {
+            const double y = row_short(a.csr_col + beg, a.csr_val + beg, (int)len, a.v);
+            if (!a.p2p) {
+                a.base[obase + li] = y;
+            } else {
+                for (int g = 0; g < a.world; ++g) ll_store(a.peer_ll[g] + lbase + li, y, tag);
+            }
+        }
+        unsigned todo = __ballot_sync(0xffffffffu, is_long);
+        while (todo) {
+            const int src = __ffs(todo) - 1;
+            todo &= todo - 1;
+            const long long b = __shfl_sync(0xffffffffu, beg, src), l = __shfl_sync(0xffffffffu, len, src);
+            const double y = row_warp(a.csr_col + b, a.csr_val + b, l, a.v, lane);
+            store_out(a, obase + w * 32 + src, lbase + w * 32 + src, tag, y, lane);
+        }
+    }
+}
+
+// ---- builders ---------------------------------------------------------------------------
+// generate_lap2d_matrix (cg.cc:159-188): the non-zeros of generate_lap2d_kernel, per row in
+// ascending column order: i-1-inc, i-1, i, i+1, i+1+inc; emit(column, value) for each
+template <class Emit>
+__device__ __forceinline__ void lap2d_row(long long n, long long inc, long long i, Emit emit)
+{
+    if (i > inc) emit(i - 1 - inc, -1.0);
+    if (i > 0) emit(i - 1, -1.0);
+    emit(i, 4.0);
+    if (i < n - 1) emit(i + 1, -1.0);
+    if (i < n - 1 - inc) emit(i + 1 + inc, -1.0);
+}
+
+__global__ void lap2d_count_kernel(long long n, long long inc, long long row0, long long rows, long long *cnt)
+{
+    const long long li = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (li >= rows) return;
+    long long k = 0;
+    lap2d_row(n, inc, row0 + li, [&](long long, double) { ++k; });
+    cnt[li] = k;
+}
+
+__global__ void lap2d_fill_kernel(long long n, long long inc, long long row0, long long rows, const long long *rp,
+                                  int *col, double *val)
+{
+    const long long li = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (li >= rows) return;
+    long long o = rp[li];
+    lap2d_row(n, inc, row0 + li, [&](long long c, double v) {
+        col[o] = (int)c;
+        val[o++] = v;
+    });
+}
+
+// Matrix::read (matrix.cc:12-21) as write sequence 2z (A(i,j)) and 2z+1 (A(j,i), symmetric only);
+// a write outside this shard's rows gets the key that sorts last
+constexpr unsigned long long kNoKey = ~0ULL;
+__global__ void coo_keys_kernel(long long n, long long row0, long long rows, const int *irn, const int *jcn,
+                                const double *val, long long nz, int symmetric, unsigned long long *key,
+                                double *kval, int *bad)
+{
+    const long long z = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (z >= nz) return;
+    const long long i = irn[z], j = jcn[z];
+    const double a = val[z];
+    unsigned long long k0 = kNoKey, k1 = kNoKey;
+    if (i < 0 || j < 0 || i >= n || j >= n) {
+        *bad = 1;
+    } else {
+        if (i >= row0 && i < row0 + rows) k0 = ((unsigned long long)(i - row0) << 32) | (unsigned long long)j;
+        if (symmetric && j >= row0 && j < row0 + rows) k1 = ((unsigned long long)(j - row0) << 32) | (unsigned long long)i;
+    }
+    key[2 * z] = k0;
+    key[2 * z + 1] = k1;
+    kval[2 * z] = a;
+    kval[2 * z + 1] = a;
+}
+
+// after the stable sort: the last write of every (row, column) run survives
+__global__ void coo_last_kernel(const unsigned long long *key, long long m, unsigned char *keep)
+{
+    const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= m) return;
+    keep[k] = (key[k] != kNoKey && (k == m - 1 || key[k + 1] != key[k])) ? 1 : 0;
+}
+
+// row pointers and columns from the surviving keys (sorted by row, then column)
+__global__ void csr_rows_kernel(const unsigned long long *key, long long nnz, long long rows, long long *rp)
+{
+    const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r > rows) return;
+    const unsigned long long want = (unsigned long long)r << 32;
+    long long lo = 0, hi = nnz; // first key >= want
+    while (lo < hi) {
+        const long long mid = (lo + hi) >> 1;
+        if (key[mid] < want) lo = mid + 1;
+        else hi = mid;
+    }
+    rp[r] = lo;
+}
+__global__ void csr_cols_kernel(const unsigned long long *key, long long nnz, int *col)
+{
+    const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k < nnz) col[k] = (int)(key[k] & 0xffffffffULL);
+}
+
+// rows [lr0, lr0 + nrows) of the shard into a dense nrows x n buffer (zeroed by the caller)
+__global__ void csr_densify_kernel(const long long *rp, const int *col, const double *val, long long lr0,
+                                   long long nrows, long long n, double *dst)
+{
+    const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= nrows) return;
+    for (long long k = rp[lr0 + r]; k < rp[lr0 + r + 1]; ++k) dst[r * n + col[k]] = val[k];
+}
+
+inline unsigned blocks_for(long long n, int t) { return (unsigned)((n + t - 1) / t > 0 ? (n + t - 1) / t : 1); }
+
+// device scratch freed on every path
+struct DevBuf {
+    void *p = nullptr;
+    ~DevBuf() { cudaFree(p); }
+    cudaError_t alloc(size_t bytes) { return cudaMalloc(&p, bytes > 0 ? bytes : 1); }
+    template <class T> T *as() const { return static_cast<T *>(p); }
+};
+
+#define CU(call)                                                                                   \
+    do {                                                                                           \
+        cudaError_t e_ = (call);                                                                   \
+        if (e_ != cudaSuccess) return e_;                                                          \
+    } while (0)
+
+// replace the value / column arrays of the shard by fresh ones of `nnz` entries
+cudaError_t csr_resize(CsrShard *m, long long nnz)
+{
+    cudaFree(m->col);
+    cudaFree(m->val);
+    m->col = nullptr;
+    m->val = nullptr;
+    m->nnz = 0;
+    CU(cudaMalloc(&m->col, (size_t)(nnz > 0 ? nnz : 1) * sizeof(int)));
+    CU(cudaMalloc(&m->val, (size_t)(nnz > 0 ? nnz : 1) * sizeof(double)));
+    m->nnz = nnz;
+    return cudaSuccess;
+}
+
+} // namespace
+
+cudaError_t preload_spmv_kernels()
+{
+    cudaFuncAttributes fa;
+    return cudaFuncGetAttributes(&fa, spmv_csr_kernel);
+}
+
+cudaError_t launch_spmv(const GemvArgs &a, int sm_count, cudaStream_t s)
+{
+    // enough warps to cover every row once, capped at 32 resident blocks per SM (grid-stride beyond)
+    long long blocks = (a.rows + kSpmvThreads - 1) / kSpmvThreads;
+    if (blocks > 32LL * sm_count) blocks = 32LL * sm_count;
+    if (blocks < 1) blocks = 1;
+    return launch_kernel(spmv_csr_kernel, (int)blocks, kSpmvThreads, 0, s, a.pdl != 0, a);
+}
+
+cudaError_t csr_generate_lap2d(CsrShard *m, long long n, long long row0, long long rows, cudaStream_t s)
+{
+    const long long inc = (long long)floor(sqrt((double)n)); // cg.cc:175
+    DevBuf cnt, tmp;
+    CU(cnt.alloc((size_t)rows * sizeof(long long)));
+    lap2d_count_kernel<<<blocks_for(rows, 256), 256, 0, s>>>(n, inc, row0, rows, cnt.as<long long>());
+    CU(cudaGetLastError());
+    size_t tmp_bytes = 0;
+    CU(cub::DeviceScan::InclusiveSum(nullptr, tmp_bytes, cnt.as<long long>(), m->rp + 1, rows, s));
+    CU(tmp.alloc(tmp_bytes));
+    CU(cudaMemsetAsync(m->rp, 0, sizeof(long long), s));
+    CU(cub::DeviceScan::InclusiveSum(tmp.p, tmp_bytes, cnt.as<long long>(), m->rp + 1, rows, s));
+    long long nnz = 0;
+    CU(cudaMemcpyAsync(&nnz, m->rp + rows, sizeof nnz, cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    CU(csr_resize(m, nnz));
+    lap2d_fill_kernel<<<blocks_for(rows, 256), 256, 0, s>>>(n, inc, row0, rows, m->rp, m->col, m->val);
+    CU(cudaGetLastError());
+    return cudaStreamSynchronize(s);
+}
+
+cudaError_t csr_from_coo(CsrShard *m, long long n, long long row0, long long rows, const int *irn, const int *jcn,
+                         const double *val, long long nz, int symmetric, int *bad_host, cudaStream_t s)
+{
+    *bad_host = 0;
+    const long long m2 = 2 * nz;
+    DevBuf key, kval, key_s, kval_s, keep, key_k, kval_k, nsel, bad, tmp;
+    CU(key.alloc((size_t)m2 * 8));
+    CU(kval.alloc((size_t)m2 * 8));
+    CU(key_s.alloc((size_t)m2 * 8));
+    CU(kval_s.alloc((size_t)m2 * 8));
+    CU(keep.alloc((size_t)m2));
+    CU(key_k.alloc((size_t)m2 * 8));
+    CU(kval_k.alloc((size_t)m2 * 8));
+    CU(nsel.alloc(sizeof(long long)));
+    CU(bad.alloc(sizeof(int)));
+    CU(cudaMemsetAsync(bad.p, 0, sizeof(int), s));
+    CU(cudaMemsetAsync(nsel.p, 0, sizeof(long long), s));
+    if (nz > 0) {
+        coo_keys_kernel<<<blocks_for(nz, 256), 256, 0, s>>>(n, row0, rows, irn, jcn, val, nz, symmetric,
+                                                            key.as<unsigned long long>(), kval.as<double>(), bad.as<int>());
+        CU(cudaGetLastError());
+        // radix sort is stable: equal (row, column) keys keep their write order
+        size_t b_sort = 0, b_sel = 0, b_sel2 = 0;
+        CU(cub::DeviceRadixSort::SortPairs(nullptr, b_sort, key.as<unsigned long long>(), key_s.as<unsigned long long>(),
+                                           kval.as<double>(), kval_s.as<double>(), m2, 0, 64, s));
+        CU(cub::DeviceSelect::Flagged(nullptr, b_sel, key_s.as<unsigned long long>(), keep.as<unsigned char>(),
+                                      key_k.as<unsigned long long>(), nsel.as<long long>(), m2, s));
+        CU(cub::DeviceSelect::Flagged(nullptr, b_sel2, kval_s.as<double>(), keep.as<unsigned char>(),
+                                      kval_k.as<double>(), nsel.as<long long>(), m2, s));
+        size_t b = b_sort > b_sel ? b_sort : b_sel;
+        if (b_sel2 > b) b = b_sel2;
+        CU(tmp.alloc(b));
+        CU(cub::DeviceRadixSort::SortPairs(tmp.p, b_sort, key.as<unsigned long long>(), key_s.as<unsigned long long>(),
+                                           kval.as<double>(), kval_s.as<double>(), m2, 0, 64, s));
+        coo_last_kernel<<<blocks_for(m2, 256), 256, 0, s>>>(key_s.as<unsigned long long>(), m2, keep.as<unsigned char>());
+        CU(cudaGetLastError());
+        CU(cub::DeviceSelect::Flagged(tmp.p, b_sel, key_s.as<unsigned long long>(), keep.as<unsigned char>(),
+                                      key_k.as<unsigned long long>(), nsel.as<long long>(), m2, s));
+        CU(cub::DeviceSelect::Flagged(tmp.p, b_sel2, kval_s.as<double>(), keep.as<unsigned char>(),
+                                      kval_k.as<double>(), nsel.as<long long>(), m2, s));
+    }
+    long long nnz = 0;
+    CU(cudaMemcpyAsync(&nnz, nsel.p, sizeof nnz, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(bad_host, bad.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    if (*bad_host) return cudaSuccess;
+    CU(csr_resize(m, nnz));
+    csr_rows_kernel<<<blocks_for(rows + 1, 256), 256, 0, s>>>(key_k.as<unsigned long long>(), nnz, rows, m->rp);
+    csr_cols_kernel<<<blocks_for(nnz, 256), 256, 0, s>>>(key_k.as<unsigned long long>(), nnz, m->col);
+    CU(cudaGetLastError());
+    if (nnz > 0) CU(cudaMemcpyAsync(m->val, kval_k.p, (size_t)nnz * 8, cudaMemcpyDeviceToDevice, s));
+    return cudaStreamSynchronize(s);
+}
+
+cudaError_t csr_densify(const CsrShard &m, long long lr0, long long nrows, long long n, double *dst, cudaStream_t s)
+{
+    CU(cudaMemsetAsync(dst, 0, (size_t)nrows * n * sizeof(double), s));
+    csr_densify_kernel<<<blocks_for(nrows, 256), 256, 0, s>>>(m.rp, m.col, m.val, lr0, nrows, n, dst);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_read_csr(const CsrShard &m, long long rows, double *sink, int sm_count, cudaStream_t s)
+{
+    CU(launch_read_stream(m.val, m.nnz, sink, sm_count, s));
+    CU(launch_read_stream(reinterpret_cast<const double *>(m.col), m.nnz / 2, sink, sm_count, s));
+    return launch_read_stream(reinterpret_cast<const double *>(m.rp), rows + 1, sink, sm_count, s);
+}
+
+#undef CU
+
+} // namespace cgb

@@ -153,6 +153,98 @@ __global__ void __launch_bounds__(kChunk) update_p_kernel(const VecArgs a, long 
     trace_stamp(rec, 3);
 }
 
+// ---- the once-per-iteration vector phase (CSR contexts) ----------------------------------
+// Every block publishes its chunk partial; the last block to arrive (threadfence + arrival
+// counter, reset by that block) reduces all of them with the same warp_det_sum as the kernels
+// above.  Returns true in warp 0 of the last block, after which the partials are visible.
+__device__ __forceinline__ bool publish_partial(double *part, double t, unsigned int *arrive, int tid)
+{
+    __shared__ int sh_last;
+    if (tid == 0) {
+        part[blockIdx.x] = t;
+        __threadfence();
+        sh_last = atomicAdd(arrive, 1u) == gridDim.x - 1;
+    }
+    __syncthreads();
+    if (!sh_last || tid >= 32) return false;
+    __threadfence();
+    return true;
+}
+// warp_det_sum over partials other blocks wrote during this launch (read from L2)
+__device__ __forceinline__ double warp_det_sum_l2(const double *v, long long n, int lane)
+{
+    double s = 0.0;
+    for (long long t = lane; t < n; t += 32) s = __dadd_rn(s, __ldcg(v + t));
+    return warp_butterfly(s);
+}
+
+__global__ void __launch_bounds__(kChunk) pap_alpha_kernel(const VecArgs a)
+{
+    __shared__ double wsum[8];
+    const int tid = threadIdx.x;
+    griddep_launch_dependents();
+    griddep_wait();
+    if (a.st->done) return;
+    const GatherView gv = gather_view(a.apx, a.g);
+    const long long i = (long long)blockIdx.x * kChunk + tid;
+    const double v = (i < a.n) ? __dmul_rn(a.p[i], gather_read(gv, gather_index(a.g, i))) : 0.0;
+    const double t = block_chunk256(v, wsum, tid);
+    if (!publish_partial(a.papart, t, &a.arrive[0], tid)) return;
+    const double conj = warp_det_sum_l2(a.papart, gridDim.x, tid);        // p'Ap     cg.cc:105-106
+    if (tid == 0) {
+        const double rsold = a.st->rsold;
+        const double clamp = __dmul_rn(rsold, kNearZero);
+        a.st->conj = conj;
+        a.st->alpha = __ddiv_rn(rsold, (conj < clamp) ? clamp : conj);   // cg.cc:107
+        a.arrive[0] = 0;
+    }
+}
+
+__global__ void __launch_bounds__(kChunk) update_xr_once_kernel(const VecArgs a)
+{
+    __shared__ double wsum[8];
+    const int tid = threadIdx.x;
+    griddep_launch_dependents();
+    griddep_wait();                      // pap_alpha has completed: st->alpha is final
+    if (a.st->done) return;
+    const double alpha = a.st->alpha;
+    const GatherView gv = gather_view(a.apx, a.g);
+    const long long i = (long long)blockIdx.x * kChunk + tid;
+    double v = 0.0;
+    if (i < a.n) {
+        const double pi = a.p[i];
+        a.x[i] = __fma_rn(alpha, pi, a.x[i]);                          // cg.cc:110
+        const double rn = __fma_rn(-alpha, gather_read(gv, gather_index(a.g, i)), a.r[i]); // cg.cc:113
+        a.r[i] = rn;
+        v = __dmul_rn(rn, rn);                                         // cg.cc:116
+    }
+    const double t = block_chunk256(v, wsum, tid);
+    exchange_consumed(a.g, tid);
+    if (!publish_partial(a.rrpart, t, &a.arrive[1], tid)) return;
+    const double rsnew = warp_det_sum_l2(a.rrpart, gridDim.x, tid);      // cg.cc:116-117
+    if (tid == 0) {
+        a.st->rsnew = rsnew;
+        if (sqrt(rsnew) < a.tol) {                                      // cg.cc:120-121
+            // break BEFORE p / rsold are updated: rsold stays stale, x stops here
+            if (a.hist) a.hist[a.st->iter] = rsnew;
+            a.st->done = 1;
+            if (a.host_done) *a.host_done = 1;
+            __threadfence_system();
+        }
+        a.arrive[1] = 0;
+    }
+}
+
+__global__ void __launch_bounds__(kChunk) update_p_once_kernel(const VecArgs a)
+{
+    griddep_launch_dependents(); // the next mat-vec may start now
+    griddep_wait();              // update_xr_once has completed: r, st->rsnew and the stop test are final
+    if (a.st->done) return;
+    const double beta = __ddiv_rn(a.st->rsnew, a.st->rsold);                      // cg.cc:124
+    const long long i = (long long)blockIdx.x * kChunk + threadIdx.x;
+    if (i < a.n) a.p[i] = __fma_rn(beta, a.p[i], a.r[i]);                         // cg.cc:127-129
+}
+
 __global__ void __launch_bounds__(32) finalize_kernel(const VecArgs a, long long nchunks)
 {
     if (a.st->done) return;
@@ -349,6 +441,9 @@ cudaError_t preload_vec_kernels()
     if ((e = cudaFuncGetAttributes(&fa, pap_partials_kernel)) != cudaSuccess) return e;
     if ((e = cudaFuncGetAttributes(&fa, update_xr_kernel)) != cudaSuccess) return e;
     if ((e = cudaFuncGetAttributes(&fa, update_p_kernel)) != cudaSuccess) return e;
+    if ((e = cudaFuncGetAttributes(&fa, pap_alpha_kernel)) != cudaSuccess) return e;
+    if ((e = cudaFuncGetAttributes(&fa, update_xr_once_kernel)) != cudaSuccess) return e;
+    if ((e = cudaFuncGetAttributes(&fa, update_p_once_kernel)) != cudaSuccess) return e;
     if ((e = cudaFuncGetAttributes(&fa, finalize_kernel)) != cudaSuccess) return e;
     if ((e = cudaFuncGetAttributes(&fa, debug_partials_kernel)) != cudaSuccess) return e;
     if ((e = cudaFuncGetAttributes(&fa, debug_final_kernel)) != cudaSuccess) return e;
@@ -378,6 +473,21 @@ cudaError_t launch_update_p(const VecArgs &a, cudaStream_t s)
     const long long nchunks = grid_for(a.n);
     return launch_kernel(update_p_kernel, (int)nchunks, kChunk, (size_t)nchunks * sizeof(double), s,
                          a.pdl != 0, a, nchunks);
+}
+
+cudaError_t launch_pap_alpha(const VecArgs &a, cudaStream_t s)
+{
+    return launch_kernel(pap_alpha_kernel, grid_for(a.n), kChunk, 0, s, a.pdl != 0, a);
+}
+
+cudaError_t launch_update_xr_once(const VecArgs &a, cudaStream_t s)
+{
+    return launch_kernel(update_xr_once_kernel, grid_for(a.n), kChunk, 0, s, a.pdl != 0, a);
+}
+
+cudaError_t launch_update_p_once(const VecArgs &a, cudaStream_t s)
+{
+    return launch_kernel(update_p_once_kernel, grid_for(a.n), kChunk, 0, s, a.pdl != 0, a);
 }
 
 cudaError_t launch_finalize(const VecArgs &a, cudaStream_t s)

@@ -67,11 +67,21 @@ void CGSolver::ensure_contexts(int64_t n)
 {
     if (!m_ctx.empty() && m_ctx_n == n) return;
     destroy_contexts();
+    // CGB_STORAGE=csr holds the shards in CSR storage (bitwise the same solve, memory bounded by
+    // the non-zeros); unset or "dense" keeps the dense shards
+    const char *storage = std::getenv("CGB_STORAGE");
+    const std::string st = storage ? storage : "dense";
+    if (st != "dense" && st != "csr") throw std::runtime_error("CGB_STORAGE must be 'dense' or 'csr', not '" + st + "'");
+    m_csr = st == "csr";
+    const char *kernel = std::getenv("CGB_KERNEL");
+    if (m_csr && kernel && std::string(kernel) == "compat")
+        throw std::runtime_error("CGB_KERNEL=compat runs the reference's dense mat-vec topologies and cannot be "
+                                 "combined with CGB_STORAGE=csr");
     const int G = psize();
     m_ctx.assign(G, nullptr);
     for (int r = 0; r < G; ++r) {
-        const int rc = cgb_create(n, r, G, m_devices[r], &m_ctx[r]);
-        if (rc) raise("cgb_create", rc);
+        const int rc = m_csr ? cgb_create_csr(n, r, G, m_devices[r], &m_ctx[r]) : cgb_create(n, r, G, m_devices[r], &m_ctx[r]);
+        if (rc) raise(m_csr ? "cgb_create_csr" : "cgb_create", rc);
     }
     m_ctx_n = n;
     if (G > 1) { // replaces MPI_Init / MPI_COMM_WORLD (cg_main.cc:15-20)

@@ -66,6 +66,8 @@ public:
     /// direct choice of the mat-vec variant (index or -1 = default)
     void set_gemv_variant(int v) { m_variant = v; }
     void set_quiet(bool q) { m_quiet = q; }
+    /// the shards are held in CSR storage (environment CGB_STORAGE=csr at context creation)
+    bool csr_storage() const { return m_csr; }
 
 private:
     void ensure_contexts(int64_t n);
@@ -86,6 +88,7 @@ private:
     bool m_rhs_uploaded{false};
     int m_variant{-1};
     bool m_quiet{false};
+    bool m_csr{false};
     Stats m_stats;
 };
 

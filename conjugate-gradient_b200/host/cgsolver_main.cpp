@@ -10,6 +10,7 @@
 // The reference ships these as two binaries; here argv[1] decides: an integer selects the
 // first form.  The MPI launcher's rank count (`srun -n P`) becomes the environment variable
 // CGB_GPUS (number of GPUs, default 1) or CGB_DEVICES (comma-separated device list).
+// CGB_STORAGE=csr holds the matrix in CSR storage instead of dense shards (same output).
 #include "cg_solver.hpp"
 
 #include <chrono>
@@ -61,7 +62,8 @@ static void write_json(const CGSolver &solver, double elapsed)
        << ", \"solve_seconds\": " << elapsed << ", \"loop_seconds\": " << s.loop_seconds
        << ", \"it_per_s\": " << (s.loop_seconds > 0 ? s.iterations / s.loop_seconds : 0.0)
        << ", \"gemv_variant\": \"" << s.gemv_variant << "\", \"norm_x\": " << s.norm_x
-       << ", \"rel_resid\": " << s.rel_resid << ", \"rsold\": " << s.rsold << "}" << std::endl;
+       << ", \"rel_resid\": " << s.rel_resid << ", \"rsold\": " << s.rsold
+       << (solver.csr_storage() ? ", \"storage\": \"csr\"" : "") << "}" << std::endl;
 }
 
 // cgsolver N outfile [max_iter]

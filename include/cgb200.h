@@ -55,6 +55,23 @@ int cgb_partition(int64_t n, int psize, int64_t *start_rows, int64_t *num_rows);
  * (rows x ld doubles, ld = n rounded up to 16) and the work vectors -- the
  * std::vector / cudaMallocManaged temporaries of solve (cg.cc:55-75, cg.cu:179-193). */
 int cgb_create(int64_t n, int rank, int world, int device, cgb_ctx **out);
+
+/* The same rank with the shard held in CSR storage: no dense shard is allocated, so the system
+ * size is bounded by the non-zeros, not by n^2 (n <= INT32_MAX: column indices are int32_t,
+ * global; row pointers int64_t; values double; columns ascending and unique within a row).
+ * The matrix comes from cgb_generate_lap2d or cgb_set_matrix_coo (built on the device);
+ * cgb_set_matrix_rows returns CGB_ERR_STATE.  Vectors, exchange wiring and cgb_get_layout are
+ * those of cgb_create; the solve runs on the graph schedule ("schedule_in_use" reads 0).
+ * Exactness: the CSR mat-vec keeps the lane order of the dense one over the stored entries, and
+ * a zero entry never changes a lane-order sum, so every result -- k, the r'r history, x, the
+ * DEBUG numbers, the hooks -- is bitwise that of a dense context holding the same matrix as long
+ * as the vector multiplied stays finite.  (A NaN / Inf of p at a column where A is zero makes the
+ * dense row NaN and leaves the CSR row alone; only an already diverged solve gets there.)
+ * Options: "compat" = 1, "loopback" > 0 and "trace" > 0 return CGB_ERR_STATE; "gemv_variant",
+ * "num_threads", "block_width" and "transposed" are accepted and change nothing; cgb_autotune
+ * changes nothing and reports every candidate as not run.  Read-only: "storage" (0 dense,
+ * 1 CSR), "nnz" (entries stored in this rank's shard). */
+int cgb_create_csr(int64_t n, int rank, int world, int device, cgb_ctx **out);
 int cgb_destroy(cgb_ctx *ctx);
 
 /* Replaces MPI_Init_thread / MPI_COMM_WORLD (code/MPI/cg_main.cc:15-20): rank 0 obtains an
@@ -93,7 +110,7 @@ int cgb_set_matrix_rows(cgb_ctx *ctx, const double *rows_host, int64_t first_row
 int cgb_set_matrix_coo(cgb_ctx *ctx, int64_t nz, const int32_t *irn, const int32_t *jcn,
                        const double *val, int symmetric);
 
-/* Read rows of the shard back (tests). */
+/* Read rows of the shard back (tests); a CSR shard is densified. */
 int cgb_get_matrix_rows(cgb_ctx *ctx, double *rows_host, int64_t first_row, int64_t nrows,
                         int64_t ld_host);
 
