@@ -138,6 +138,8 @@ struct cgb_ctx {
     CsrShard csr;
     unsigned int *arrive = nullptr; // CSR: arrival counters of the once-per-iteration vector phase
     double *A = nullptr, *p = nullptr, *r = nullptr, *x = nullptr, *b = nullptr;
+    int2 *env = nullptr;           // dense: [first, last + 1) of the non-zero columns of every local row,
+                                   // rebuilt after every write of A (the mat-vecs stream only these windows)
     double *apx = nullptr, *rrpart = nullptr, *papart = nullptr, *scratch = nullptr, *hist = nullptr, *sink = nullptr;
     // apx: plain gather buffer [world][slot_cap] doubles.  ll: fused-mode LL buffers
     // [2][world][slot_cap] x 16 B, the allocation peers map; ctl: local control words.
@@ -221,6 +223,7 @@ GemvArgs make_gemv_args(const cgb_ctx *c, const double *v, int advance)
     GemvArgs a;
     memset(&a, 0, sizeof a);
     a.A = c->A;
+    a.env = c->env;
     a.csr_rp = c->csr.rp;
     a.csr_col = c->csr.col;
     a.csr_val = c->csr.val;
@@ -420,6 +423,7 @@ int launch_persist(cgb_ctx *c, long long iters)
     PersistArgs a;
     memset(&a, 0, sizeof a);
     a.A = c->A;
+    a.env = c->env;
     a.x = c->x;
     a.r = c->r;
     a.p = c->p;
@@ -598,6 +602,8 @@ static int create_ctx(int64_t n, int rank, int world, int device, int storage, c
     } else {
         CKB(cudaMalloc(&c->A, (size_t)c->rows * c->ld * sizeof(double)));
         CKB(cudaMemsetAsync(c->A, 0, (size_t)c->rows * c->ld * sizeof(double), c->stream));
+        CKB(cudaMalloc(&c->env, (size_t)(c->rows > 0 ? c->rows : 1) * sizeof(int2)));
+        CKB(cudaMemsetAsync(c->env, 0, (size_t)(c->rows > 0 ? c->rows : 1) * sizeof(int2), c->stream)); // all rows empty
     }
     CKB(cudaMalloc(&c->p, vec_bytes));
     CKB(cudaMalloc(&c->r, vec_bytes));
@@ -673,6 +679,7 @@ extern "C" int cgb_destroy(cgb_ctx *c)
     for (double *p : bufs)
         if (p) cudaFree(p);
     if (c->st) cudaFree(c->st);
+    if (c->env) cudaFree(c->env);
     if (c->csr.rp) cudaFree(c->csr.rp);
     if (c->csr.col) cudaFree(c->csr.col);
     if (c->csr.val) cudaFree(c->csr.val);
@@ -802,7 +809,8 @@ extern "C" int cgb_generate_lap2d(cgb_ctx *c)
         c->kernel_launches += 3;
     } else {
         CK(launch_generate_lap2d(c->A, c->n, c->ld, c->row0, c->rows, c->stream));
-        c->kernel_launches += 1;
+        CK(launch_row_envelope(c->A, c->ld, 0, c->rows, c->env, c->stream));
+        c->kernel_launches += 2;
         CK(cudaStreamSynchronize(c->stream));
     }
     c->matrix_set = true;
@@ -825,6 +833,8 @@ extern "C" int cgb_set_matrix_rows(cgb_ctx *c, const double *rows_host, int64_t 
         CK(cudaMemcpy2DAsync(c->A + (lo - c->row0) * c->ld, (size_t)c->ld * 8,
                              rows_host + (lo - first_row) * ld_host, (size_t)ld_host * 8,
                              (size_t)c->n * 8, (size_t)(hi - lo), cudaMemcpyHostToDevice, c->stream));
+        CK(launch_row_envelope(c->A, c->ld, lo - c->row0, hi - lo, c->env, c->stream)); // the rows written
+        c->kernel_launches += 1;
         CK(cudaStreamSynchronize(c->stream));
     }
     c->matrix_set = true;
@@ -888,7 +898,8 @@ extern "C" int cgb_set_matrix_coo(cgb_ctx *c, int64_t nz, const int32_t *irn, co
         CK(cudaMemcpyAsync(t.v, val, (size_t)nz * sizeof(double), cudaMemcpyHostToDevice, c->stream));
         CK(launch_scatter_coo(c->A, c->n, c->ld, c->row0, c->rows, t.i, t.j, t.v, nz, symmetric ? 1 : 0, t.win,
                               t.bad, c->stream));
-        c->kernel_launches += 3;
+        CK(launch_row_envelope(c->A, c->ld, 0, c->rows, c->env, c->stream));
+        c->kernel_launches += 4;
         int bad = 0;
         CK(cudaMemcpyAsync(&bad, t.bad, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
         CK(cudaStreamSynchronize(c->stream));
@@ -897,6 +908,7 @@ extern "C" int cgb_set_matrix_coo(cgb_ctx *c, int64_t nz, const int32_t *irn, co
             return fail(CGB_ERR_INVALID, "a COO entry lies outside %lld x %lld", (long long)c->n, (long long)c->n);
         }
     } else {
+        CK(cudaMemsetAsync(c->env, 0, (size_t)c->rows * sizeof(int2), c->stream)); // the zeroed shard: every row empty
         CK(cudaStreamSynchronize(c->stream));
     }
     c->matrix_set = true;
@@ -1114,6 +1126,17 @@ extern "C" int cgb_get_option(cgb_ctx *c, const char *key, int64_t *value)
     else if (k == "transposed") *value = c->opt_transposed;
     else if (k == "storage") *value = c->storage;
     else if (k == "nnz") *value = c->storage == 1 ? c->csr.nnz : 0;
+    else if (k == "envelope_doubles") { // sum over this rank's rows of (last + 1 - first); 0 on a CSR context
+        *value = 0;
+        if (c->storage == 0 && c->rows > 0) {
+            CK(cudaSetDevice(c->device));
+            std::vector<int2> env((size_t)c->rows);
+            CK(cudaMemcpyAsync(env.data(), c->env, (size_t)c->rows * sizeof(int2), cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaStreamSynchronize(c->stream));
+            for (const int2 &e : env)
+                if (e.y > e.x) *value += e.y - e.x;
+        }
+    }
     else return fail(CGB_ERR_INVALID, "unknown option '%s'", key);
     return CGB_OK;
 }
@@ -1215,7 +1238,7 @@ extern "C" int cgb_iterate(cgb_ctx *c, int64_t iters, float *ms)
             if (code < 0)
                 return fail(CGB_ERR_TIMEOUT, "a device-side wait (kind %d: 1 = an LL entry -- a peer rank's mat-vec rows or a chunk "
                             "partial, 4 = p chunks, 5 = tile for the consumers, 6 / 9 = row partition hand-over, 7 = free "
-                            "pipeline stage, 8 = drain) exceeded spin_timeout_ms = %lld: a rank is "
+                            "pipeline stage, 8 = drain, 10 = column-window table) exceeded spin_timeout_ms = %lld: a rank is "
                             "missing or stuck (%s) [cta %d thread %d: %d %d %d %d]", -code, c->spin_timeout_ms,
                             cudaGetErrorString(e), c->h_done[1], c->h_done[2], c->h_done[3], c->h_done[4], c->h_done[5],
                             c->h_done[6]);

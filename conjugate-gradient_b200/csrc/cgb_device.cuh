@@ -68,8 +68,57 @@ struct Trace {
     int nblk;                // CTAs per launch
 };
 
+// ---- column windows of the dense mat-vec --------------------------------------------------
+// env[i] = [first, last + 1) of the non-zero (not +-0) columns of local row i; first >= end: the row
+// is all zero (the zeroed shard of a new context is {0, 0} everywhere).  A row block is streamed over
+// the hull of its rows' envelopes only: every column outside it holds +-0 in every row of the block,
+// and a lane-order accumulator (which starts at +0 and is never -0) is unchanged by fma(+-0, p, acc)
+// for finite p -- the result is the full-row stream's, bit for bit.
+//   c_begin is rounded DOWN to a multiple of 64: lane l owns the columns c % 64 = 2l, 2l + 1 of every
+//           tile, which holds only if every tile starts at a multiple of 64
+//   c_end   is rounded up to a multiple of 16 and clipped to ld: every bulk copy stays a whole number
+//           of 16-byte units at a 16-byte-aligned address
+// A block table entry packs (c_begin / 16) | (c_end / 16) << 16, which covers ld <= kWinMaxLd (a dense
+// shard that wide holds 8 TB per 1000 rows); a wider ld streams full rows.
+constexpr int kWinBlocks = 128;                  // blocks of a CTA with a table entry; later ones stream full rows
+constexpr long long kWinMaxLd = 16LL * 0xffff;
+__device__ __forceinline__ unsigned block_window(const int2 *env, long long rb0, int nr, long long ld)
+{
+    int lo = 0x7fffffff, hi = 0;
+#pragma unroll 4
+    for (int j = 0; j < nr; ++j) {
+        const int2 e = env[rb0 + j];
+        if (e.x < e.y) {
+            lo = e.x < lo ? e.x : lo;
+            hi = e.y > hi ? e.y : hi;
+        }
+    }
+    if (lo >= hi) return 0u; // no non-zero in the block: an empty window
+    const long long cb = (long long)(lo & ~63), ce0 = ((long long)hi + 15) & ~15LL;
+    const long long ce = ce0 < ld ? ce0 : ld;
+    return (unsigned)(cb >> 4) | ((unsigned)(ce >> 4) << 16);
+}
+// the window of block b from a CTA's table `tab` (filled with block_window for b < kWinBlocks)
+__device__ __forceinline__ void window_of(const unsigned *tab, int b, long long ld, long long &cb, long long &ce)
+{
+    if (b < kWinBlocks && ld <= kWinMaxLd) {
+        const unsigned w = tab[b];
+        cb = (long long)(w & 0xffffu) << 4;
+        ce = (long long)(w >> 16) << 4;
+    } else {
+        cb = 0;
+        ce = ld;
+    }
+}
+// tiles of width wd (a multiple of 64) that cover [cb, ce)
+__device__ __forceinline__ int window_tiles(long long cb, long long ce, int wd)
+{
+    return ce > cb ? (int)((ce - cb + wd - 1) / wd) : 0;
+}
+
 struct GemvArgs {
     const double *A;      // rows x ld shard, zero-padded columns
+    const int2 *env;      // rows envelopes of A (see block_window)
     const double *v;      // input vector, ld doubles, zero-padded
     double *base;         // local plain gather buffer
     uint4 *peer_ll[kMaxWorld]; // fused mode: every rank's LL buffers (self included), peer-mapped
@@ -107,6 +156,7 @@ struct PersistSync {
 };
 struct PersistArgs {
     const double *A;           // rows x ld shard
+    const int2 *env;           // rows envelopes of A (see block_window)
     double *x, *r, *p;         // full-length replicated vectors (ld doubles)
     double *rrpart;            // nchunks chunk partials of r'r (also the hand-over to the next launch)
     uint4 *peer_ll[kMaxWorld]; // every rank's LL gather buffers (self included)

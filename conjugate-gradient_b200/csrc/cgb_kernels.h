@@ -115,6 +115,9 @@ cudaError_t launch_exchange_collect(double *apx, const Gather &g, cudaStream_t s
 // generate_lap2d_matrix (cg.cc:159-188) into the shard
 cudaError_t launch_generate_lap2d(double *A, long long n, long long ld, long long row0,
                                   long long rows, cudaStream_t s);
+// non-zero envelope of local rows [lr0, lr0 + nrows) of the shard into env (see block_window)
+cudaError_t launch_row_envelope(const double *A, long long ld, long long lr0, long long nrows, int2 *env,
+                                cudaStream_t s);
 // Matrix::read's densification (matrix.cc:12-21) on the device, "later entries overwrite" resolved
 // with an atomicMax of the entry index per cell (win: nz bytes of scratch, bad: 1 int, both device)
 cudaError_t launch_scatter_coo(double *A, long long n, long long ld, long long row0, long long rows,

@@ -3,7 +3,7 @@
 // MatVec / MatVecT atomicAdd kernels (code/CUDA/cg.cu:14-110).
 //
 // HBM-bound (0.25 flop/byte): CUDA cores, never tensor cores.  A is read exactly once per
-// launch.  Two families share ONE summation order (oracle/cg_oracle.h, "lane order"), so any
+// launch -- by the tma_* variants only the column window of each row block (block_window).  Two families share ONE summation order (oracle/cg_oracle.h, "lane order"), so any
 // variant is bitwise interchangeable:
 //
 //   tma_*  one persistent CTA per SM owns a contiguous row range.  A producer warp streams
@@ -73,9 +73,21 @@ __device__ __forceinline__ void gemv_tma_body(const GemvArgs &a, const void *tma
     const long long r1 = (long long)(c + 1) * a.rows / nblk;
     const int nrows = (int)(r1 - r0);
     const int nb = (nrows + TR - 1) / TR;          // row blocks, balanced below
-    const int ntc = (int)((a.ld + TC - 1) / TC);   // column tiles
+
+    // Programmatic dependent launch: this grid may become resident while the previous kernels of
+    // the iteration (update_xr / update_p, even the tail of the previous mat-vec) still run.
+    // A (and with it the column windows) never changes, so the block table is built and the
+    // producer fills the whole ring with A tiles BEFORE waiting for them; only p, the scalars and
+    // the exchange tag are read after the wait.
+    griddep_launch_dependents();
 
     __shared__ unsigned long long *s_rec; // diagnostic timeline record of this CTA (nullptr: off)
+    __shared__ unsigned s_win[kWinBlocks]; // column window of every row block (POL 0 / 1)
+    if (POL != 2 && a.ld <= kWinMaxLd)
+        for (int b = tid; b < nb && b < kWinBlocks; b += blockDim.x) {
+            const long long rb0 = r0 + (long long)b * nrows / nb;
+            s_win[b] = block_window(a.env, rb0, (int)(r0 + (long long)(b + 1) * nrows / nb - rb0), a.ld);
+        }
     if (tid == 0) {
         for (int s = 0; s < STAGES; ++s) {
             mbar_init(&full[s], 1);
@@ -90,26 +102,43 @@ __device__ __forceinline__ void gemv_tma_body(const GemvArgs &a, const void *tma
     }
     __syncthreads();
     unsigned long long *const rec = s_rec;
-
-    // Programmatic dependent launch: this grid may become resident while the previous kernels of
-    // the iteration (update_xr / update_p, even the tail of the previous mat-vec) still run.
-    // A never changes, so the producer fills the whole ring with A tiles BEFORE waiting for
-    // them; only p, the scalars and the exchange tag are read after the wait.
-    griddep_launch_dependents();
+    // columns [cb, ce) of block b are streamed; the tensor-map variant keeps full rows
+    auto window = [&](int b, long long &cb, long long &ce) {
+        if (POL == 2) {
+            cb = 0;
+            ce = a.ld;
+        } else {
+            window_of(s_win, b, a.ld, cb, ce);
+        }
+    };
 
     if (warp == CW) {
         // ===== producer: keeps the ring full, runs ahead across row blocks =====
         const uint64_t pol_a = l2_policy_evict_first();
         const uint64_t pol_p = l2_policy_evict_last();
-        const unsigned total = (unsigned)nb * (unsigned)ntc;
-        // pipeline step `it` = (row block b, column tile t); part 1 = A rows, part 2 = p slice
-        auto issue = [&](unsigned it, bool partA, bool partP) {
-            const int b = (int)(it / (unsigned)ntc), t = (int)(it - (unsigned)b * (unsigned)ntc);
-            const long long rb0 = r0 + (long long)b * nrows / nb;
-            const int nr = (int)(r0 + (long long)(b + 1) * nrows / nb - rb0);
+        // cursor over the pipeline steps: column tile t of row block b (blocks without tiles skipped)
+        struct Cur {
+            int b, t, nr, ntb;
+            long long rb0, cb, ce;
+        };
+        auto seek = [&](Cur &k, int b) {
+            for (k.b = b; k.b < nb; ++k.b) {
+                k.t = 0;
+                k.rb0 = r0 + (long long)k.b * nrows / nb;
+                k.nr = (int)(r0 + (long long)(k.b + 1) * nrows / nb - k.rb0);
+                window(k.b, k.cb, k.ce);
+                k.ntb = window_tiles(k.cb, k.ce, TC);
+                if (k.ntb > 0) return;
+            }
+        };
+        auto next = [&](Cur &k) {
+            if (++k.t >= k.ntb) seek(k, k.b + 1);
+        };
+        // pipeline step `it` at cursor k; part 1 = A rows, part 2 = p slice
+        auto issue = [&](unsigned it, const Cur &k, bool partA, bool partP) {
             const int stage = it % STAGES;
-            const long long c0 = (long long)t * TC;
-            const int w = (int)((a.ld - c0 < TC) ? (a.ld - c0) : TC);
+            const long long c0 = k.cb + (long long)k.t * TC;
+            const int w = (int)((k.ce - c0 < TC) ? (k.ce - c0) : TC);
             if (partA && POL == 2) {
                 // whole boxes: rows past nr belong to the next row block (or are zero-filled past
                 // the shard), columns past ld are zero-filled; the barrier counts full boxes
@@ -121,53 +150,53 @@ __device__ __forceinline__ void gemv_tma_body(const GemvArgs &a, const void *tma
                 if (lane == 0) // the descriptor path is warp-uniform: one elected lane issues the boxes
                     for (int j = 0; j < nbox; ++j)
                         tensor_g2s_2d(dstA + (size_t)j * TR * kBoxCols, tmap, (int)(c0 + (long long)j * kBoxCols),
-                                      (int)rb0, &full[stage], pol_a);
+                                      (int)k.rb0, &full[stage], pol_a);
             } else if (partA) {
-                if (lane == 0) mbar_arrive_expect_tx(&full[stage], (unsigned)((nr + 1) * w * 8));
+                if (lane == 0) mbar_arrive_expect_tx(&full[stage], (unsigned)((k.nr + 1) * w * 8));
                 __syncwarp();
                 double *dstA = sA + (size_t)stage * TR * TC;
-                for (int j = lane; j < nr; j += 32) {
+                for (int j = lane; j < k.nr; j += 32) {
                     if (POL == 0)
-                        bulk_g2s(dstA + (size_t)j * TC, a.A + (rb0 + j) * a.ld + c0, (unsigned)(w * 8),
+                        bulk_g2s(dstA + (size_t)j * TC, a.A + (k.rb0 + j) * a.ld + c0, (unsigned)(w * 8),
                                  &full[stage], pol_a);
                     else
-                        bulk_g2s_nohint(dstA + (size_t)j * TC, a.A + (rb0 + j) * a.ld + c0,
+                        bulk_g2s_nohint(dstA + (size_t)j * TC, a.A + (k.rb0 + j) * a.ld + c0,
                                         (unsigned)(w * 8), &full[stage]);
                 }
             }
             if (partP && lane == 31)
                 bulk_g2s(sP + (size_t)stage * TC, a.v + c0, (unsigned)(w * 8), &full[stage], pol_p);
         };
-        const unsigned npro = total < (unsigned)STAGES ? total : (unsigned)STAGES;
-        for (unsigned it = 0; it < npro; ++it) issue(it, true, false);   // A only: no dependency
+        Cur k0;
+        seek(k0, 0);
+        Cur ka = k0;
+        unsigned npro = 0;
+        for (; npro < (unsigned)STAGES && ka.b < nb; ++npro, next(ka)) issue(npro, ka, true, false); // A only: no dependency
         // While the vector updates (and, multi-GPU, the exchange) of the previous iteration
         // finish, HBM would idle once the ring is full: pull the next steps of A into L2.
-        if (a.l2_prefetch > 0) {
-            const unsigned npf = (total - npro < (unsigned)a.l2_prefetch) ? total : npro + (unsigned)a.l2_prefetch;
-            for (unsigned it = npro; it < npf; ++it) {
-                const int b = (int)(it / (unsigned)ntc), t = (int)(it - (unsigned)b * (unsigned)ntc);
-                const long long rb0 = r0 + (long long)b * nrows / nb;
-                const int nr = (int)(r0 + (long long)(b + 1) * nrows / nb - rb0);
-                const long long c0 = (long long)t * TC;
-                const int w = (int)((a.ld - c0 < TC) ? (a.ld - c0) : TC);
-                for (int j = lane; j < nr; j += 32)
-                    bulk_prefetch_l2(a.A + (rb0 + j) * a.ld + c0, (unsigned)(w * 8));
+        {
+            Cur pf = ka;
+            for (int q = 0; q < a.l2_prefetch && pf.b < nb; ++q, next(pf)) {
+                const long long c0 = pf.cb + (long long)pf.t * TC;
+                const int w = (int)((pf.ce - c0 < TC) ? (pf.ce - c0) : TC);
+                for (int j = lane; j < pf.nr; j += 32)
+                    bulk_prefetch_l2(a.A + (pf.rb0 + j) * a.ld + c0, (unsigned)(w * 8));
             }
         }
         if (lane == 0) trace_stamp(rec, 1);
         griddep_wait();                                                    // p is final from here on
         if (lane == 0) trace_stamp(rec, 2);
         const int done = a.st->done;
-        for (unsigned it = 0; it < npro; ++it) issue(it, false, true);
+        for (unsigned it = 0; it < npro; ++it, next(k0)) issue(it, k0, false, true);
         if (done) {
             // converged earlier: the launch is a no-op, but the copies in flight must land
             // before the CTA may exit
             for (unsigned it = 0; it < npro; ++it) mbar_wait(&full[it % STAGES], 0u);
             return;
         }
-        for (unsigned it = npro; it < total; ++it) {
+        for (unsigned it = npro; ka.b < nb; ++it, next(ka)) {
             mbar_wait(&empty[it % STAGES], ((it / STAGES) & 1u) ^ 1u);
-            issue(it, true, true);
+            issue(it, ka, true, true);
         }
         if (lane == 0) trace_stamp(rec, 4);
     } else {
@@ -184,6 +213,9 @@ __device__ __forceinline__ void gemv_tma_body(const GemvArgs &a, const void *tma
             const int nr = (int)(r0 + (long long)(b + 1) * nrows / nb - rb0);
             // rows of this warp inside the block: warp, warp + CW, ...
             const int nv = (nr > warp) ? ((nr - warp + CW - 1) / CW) : 0;
+            long long cb, ce;
+            window(b, cb, ce);
+            const int ntc = window_tiles(cb, ce, TC);
             double acc0[RPW], acc1[RPW];
 #pragma unroll
             for (int s = 0; s < RPW; ++s) {
@@ -193,8 +225,8 @@ __device__ __forceinline__ void gemv_tma_body(const GemvArgs &a, const void *tma
             for (int t = 0; t < ntc; ++t, ++it) {
                 const int stage = it % STAGES;
                 const unsigned ph = (it / STAGES) & 1u;
-                const long long c0 = (long long)t * TC;
-                const int w = (int)((a.ld - c0 < TC) ? (a.ld - c0) : TC);
+                const long long c0 = cb + (long long)t * TC;
+                const int w = (int)((ce - c0 < TC) ? (ce - c0) : TC);
                 mbar_wait(&full[stage], ph);
                 if (rec && it == 0 && tid == 0) trace_stamp(rec, 3);
                 const double2 *sa2 = reinterpret_cast<const double2 *>(sA + (size_t)stage * TR * TC);
@@ -239,6 +271,7 @@ __device__ __forceinline__ void gemv_tma_body(const GemvArgs &a, const void *tma
             }
         }
         if (tid == 0) {
+            if (rec && it == 0 && nb > 0) trace_stamp(rec, 3); // no block had a column to stream
             trace_stamp(rec, 5);
             trace_stamp(rec, 6);
         }

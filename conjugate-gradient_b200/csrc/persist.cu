@@ -161,16 +161,20 @@ __device__ __forceinline__ void mbar_wait_ns(const PersistArgs &a, uint64_t *bar
 // Geometry of one CTA's mat-vec for a given row range: balanced row blocks of at most TR rows,
 // tile width per block as wide as the stage allows (a full stage keeps the bytes in flight -- and
 // with them this SM's share of the saturated HBM stream -- independent of the rows-per-CTA ratio).
+// Block b streams the columns of its window (block_window) from the table s_win[par][b] in tiles of
+// that width; T, the pipeline steps of the mat-vec, is summed from the table by the producer.
 struct Geo {
     long long r0;
-    int nrows, nb, lo, n_hi, w_lo, w_hi, ntc_lo, ntc_hi;
-    unsigned T; // pipeline steps of the mat-vec
+    int nrows, nb, lo, n_hi, w_lo, w_hi, par;
+    unsigned T;
 };
 template <int TR, int SLOT, int PMAX>
-__device__ __forceinline__ Geo make_geo(long long r0, long long r1, long long ld)
+__device__ __forceinline__ Geo make_geo(long long r0, long long r1, int par)
 {
     Geo g;
     g.r0 = r0;
+    g.par = par;
+    g.T = 0;
     g.nrows = (int)(r1 - r0);
     g.nb = (g.nrows + TR - 1) / TR;
     g.lo = g.nb ? g.nrows / g.nb : 1; // the balanced split gives blocks of lo or lo + 1 rows
@@ -179,9 +183,6 @@ __device__ __forceinline__ Geo make_geo(long long r0, long long r1, long long ld
     g.w_lo = w > PMAX ? PMAX : w;
     w = (SLOT / (g.lo + 1)) & ~63;
     g.w_hi = w > PMAX ? PMAX : w;
-    g.ntc_lo = (int)((ld + g.w_lo - 1) / g.w_lo);
-    g.ntc_hi = (int)((ld + g.w_hi - 1) / g.w_hi);
-    g.T = (unsigned)(g.nb - g.n_hi) * (unsigned)g.ntc_lo + (unsigned)g.n_hi * (unsigned)g.ntc_hi;
     return g;
 }
 
@@ -209,6 +210,8 @@ __global__ void __launch_bounds__((CW + 1) * 32, 1) cg_persist_kernel(const Pers
     __shared__ volatile int s_stop;          // consumers -> producer: loop left
     __shared__ volatile int s_part_seq;      // highest iteration whose row partition is in s_bnd
     __shared__ volatile int s_prod_geo;      // highest iteration whose row partition the producer has read
+                                             // and whose window table it has written
+    __shared__ unsigned s_win[2][kWinBlocks]; // column window of every row block, iteration parity
     __shared__ int s_bnd[2][kMaxGrid + 1];   // row boundaries of all CTAs, iteration parity
     __shared__ double s_tm[kMaxGrid];        // mat-vec-phase times of all CTAs (re-balancing)
     __shared__ long long s_c0[8];            // per stage: first column and width of the tile in flight
@@ -227,8 +230,8 @@ __global__ void __launch_bounds__((CW + 1) * 32, 1) cg_persist_kernel(const Pers
         }
         fence_mbar_init();
         s_stop = 0;
-        s_part_seq = balance ? 1 : 0x7fffffff;
-        s_prod_geo = 0;
+        s_part_seq = 1;
+        s_prod_geo = -1;
     }
     if (nblk <= kMaxGrid)
         for (int k = tid; k <= nblk; k += blockDim.x) { // static start: the balanced split of gemv.cu
@@ -241,37 +244,60 @@ __global__ void __launch_bounds__((CW + 1) * 32, 1) cg_persist_kernel(const Pers
 
     const unsigned nchunks = (unsigned)a.nchunks;
     auto geo_of = [&](int m) {
-        if (nblk <= kMaxGrid) return make_geo<TR, SLOT, PMAX>(s_bnd[m & 1][c], s_bnd[m & 1][c + 1], a.ld);
-        return make_geo<TR, SLOT, PMAX>((long long)c * a.rows / nblk, (long long)(c + 1) * a.rows / nblk, a.ld);
+        if (nblk <= kMaxGrid) return make_geo<TR, SLOT, PMAX>(s_bnd[m & 1][c], s_bnd[m & 1][c + 1], m & 1);
+        return make_geo<TR, SLOT, PMAX>((long long)c * a.rows / nblk, (long long)(c + 1) * a.rows / nblk, m & 1);
     };
 
     if (warp == CW) {
         // ================= producer: streams A, never waits for the vector phases =================
         const uint64_t pol_a = l2_policy_evict_first();
         const uint64_t pol_p = l2_policy_evict_last();
+        // the window table of a mat-vec (its slot is free: see the wait for s_part_seq) and its steps T
+        auto take_windows = [&](Geo &ge) {
+            unsigned T = 0;
+            for (int b = lane; b < ge.nb; b += 32) {
+                const long long rb0 = ge.r0 + (long long)b * ge.nrows / ge.nb;
+                const int nr = (int)(ge.r0 + (long long)(b + 1) * ge.nrows / ge.nb - rb0);
+                if (b < kWinBlocks && a.ld <= kWinMaxLd) s_win[ge.par][b] = block_window(a.env, rb0, nr, a.ld);
+                long long cb, ce;
+                window_of(s_win[ge.par], b, a.ld, cb, ce);
+                T += (unsigned)window_tiles(cb, ce, (nr == ge.lo) ? ge.w_lo : ge.w_hi);
+            }
+            ge.T = __reduce_add_sync(0xffffffffu, T);
+            __syncwarp(); // the table is read by every lane from here on
+        };
         // cursor over the pipeline steps (row block b, column tile t) of one mat-vec
         struct Cur {
             int b, t, nr, wdb, ntb;
-            long long rb0;
+            long long rb0, cb, ce;
         };
+        // the first block from b on (wrapping around) with a tile to stream; none (T == 0): ntb = 0
         auto cur_block = [&](Cur &k, const Geo &ge, int b) {
-            k.b = b;
             k.t = 0;
-            if (ge.nb == 0) {
-                k.nr = 0; k.wdb = 64; k.ntb = 1; k.rb0 = ge.r0;
-                return;
+            k.nr = 0; k.wdb = 64; k.ntb = 0; k.rb0 = ge.r0; k.cb = 0; k.ce = 0; k.b = 0;
+            for (int n = 0; n < ge.nb; ++n, ++b) {
+                if (b >= ge.nb) b = 0;
+                k.b = b;
+                k.rb0 = ge.r0 + (long long)b * ge.nrows / ge.nb;
+                k.nr = (int)(ge.r0 + (long long)(b + 1) * ge.nrows / ge.nb - k.rb0);
+                k.wdb = (k.nr == ge.lo) ? ge.w_lo : ge.w_hi;
+                window_of(s_win[ge.par], b, a.ld, k.cb, k.ce);
+                k.ntb = window_tiles(k.cb, k.ce, k.wdb);
+                if (k.ntb > 0) return;
             }
-            k.rb0 = ge.r0 + (long long)b * ge.nrows / ge.nb;
-            k.nr = (int)(ge.r0 + (long long)(b + 1) * ge.nrows / ge.nb - k.rb0);
-            k.wdb = (k.nr == ge.lo) ? ge.w_lo : ge.w_hi;
-            k.ntb = (k.nr == ge.lo) ? ge.ntc_lo : ge.ntc_hi;
         };
         auto cur_next = [&](Cur &k, const Geo &ge) {
-            if (++k.t == k.ntb) cur_block(k, ge, (k.b + 1 >= ge.nb) ? 0 : k.b + 1);
+            if (++k.t >= k.ntb) cur_block(k, ge, k.b + 1);
+        };
+        // first column and width of the tile under the cursor
+        auto cur_tile = [&](const Cur &k, long long &c0, int &w) {
+            c0 = k.cb + (long long)k.t * k.wdb;
+            w = (int)((k.ce - c0 < k.wdb) ? (k.ce - c0) : k.wdb);
         };
         auto issueA = [&](unsigned g, const Cur &k) {
-            const long long c0 = (long long)k.t * k.wdb;
-            const int w = (int)((a.ld - c0 < k.wdb) ? (a.ld - c0) : k.wdb);
+            long long c0;
+            int w;
+            cur_tile(k, c0, w);
             const int stage = g % STAGES;
             if (lane == 0) {
                 s_c0[stage] = c0;
@@ -292,8 +318,13 @@ __global__ void __launch_bounds__((CW + 1) * 32, 1) cg_persist_kernel(const Pers
             if (g >= (unsigned)STAGES) mbar_wait_ns(a, &empty[g % STAGES], ((g / STAGES) & 1u) ^ 1u, 7, (int)g);
         };
         Geo ge = geo_of(0);
+        take_windows(ge);
         Cur cur;
         cur_block(cur, ge, 0);
+        if (lane == 0) {
+            __threadfence_block();
+            s_prod_geo = 0;
+        }
         unsigned gbase = 0; // global step index of the first tile of mat-vec m
         unsigned pre = 0;   // steps of the coming mat-vec whose A part is already in flight
         for (int m = 0; m < a.iters; ++m) {
@@ -330,8 +361,9 @@ __global__ void __launch_bounds__((CW + 1) * 32, 1) cg_persist_kernel(const Pers
                 unsigned u = pre;
                 for (int q = 0; q < a.l2_prefetch && u < ge.T; ++q, ++u) cur_next(pf, ge);
                 for (int q = 0; q < a.l2_ramp && u < ge.T; ++q, ++u) {
-                    const long long c0 = (long long)pf.t * pf.wdb;
-                    const int w = (int)((a.ld - c0 < pf.wdb) ? (a.ld - c0) : pf.wdb);
+                    long long c0;
+                    int w;
+                    cur_tile(pf, c0, w);
                     for (int j = lane; j < pf.nr; j += 32)
                         bulk_prefetch_l2(a.A + (pf.rb0 + j) * a.ld + c0, (unsigned)(w * 8));
                     cur_next(pf, ge);
@@ -346,7 +378,9 @@ __global__ void __launch_bounds__((CW + 1) * 32, 1) cg_persist_kernel(const Pers
             gbase += ge.T;
             pre = 0;
             if (m + 1 < a.iters) {
-                // the row range of the next mat-vec (re-balanced two iterations ago) ...
+                // the row range of the next mat-vec (re-balanced two iterations ago; s_part_seq is also
+                // raised without re-balancing: the consumers are then past mat-vec m - 1, so the slot
+                // of its window table can take the next one) ...
                 int stop = 0;
                 if (lane == 0) {
                     const unsigned long long t0 = globaltimer_ns();
@@ -363,6 +397,7 @@ __global__ void __launch_bounds__((CW + 1) * 32, 1) cg_persist_kernel(const Pers
                 __threadfence_block();
                 if (stop) return; // nothing in flight: all steps of mat-vec m were consumed or the loop never reached it
                 ge = geo_of(m + 1);
+                take_windows(ge);
                 cur_block(cur, ge, 0);
                 __syncwarp();
                 if (lane == 0) {
@@ -379,8 +414,9 @@ __global__ void __launch_bounds__((CW + 1) * 32, 1) cg_persist_kernel(const Pers
                 }
                 Cur pf = cur;
                 for (int u = 0; u < a.l2_prefetch && (unsigned)u + pre < ge.T; ++u) {
-                    const long long c0 = (long long)pf.t * pf.wdb;
-                    const int w = (int)((a.ld - c0 < pf.wdb) ? (a.ld - c0) : pf.wdb);
+                    long long c0;
+                    int w;
+                    cur_tile(pf, c0, w);
                     for (int j = lane; j < pf.nr; j += 32)
                         bulk_prefetch_l2(a.A + (pf.rb0 + j) * a.ld + c0, (unsigned)(w * 8));
                     cur_next(pf, ge);
@@ -498,6 +534,12 @@ __global__ void __launch_bounds__((CW + 1) * 32, 1) cg_persist_kernel(const Pers
         uint4 *const aux = a.rr_ll + (long long)(tag & 1u) * a.rr_stride; // [r'r | p'Ap | times]
         uint4 *const rrview = aux, *const papview = aux + a.nchunks, *const tmview = aux + 2 * a.nchunks;
         const Geo ge = geo_of(m);
+        if (s_prod_geo < m) { // the window table of this mat-vec (normally written an iteration ago)
+            const unsigned long long t0 = globaltimer_ns();
+            while (s_prod_geo < m)
+                if (globaltimer_ns() - t0 > a.spin_ns) spin_timeout(a, 10, m);
+        }
+        __threadfence_block();
         // the two parities of the partition are re-balanced in turn, two iterations out of eight
         const bool rebalance_now = balance && (m & 7) < 2 && m + 2 < a.iters;
         unsigned long long *rec = nullptr;
@@ -509,12 +551,15 @@ __global__ void __launch_bounds__((CW + 1) * 32, 1) cg_persist_kernel(const Pers
 
         // ------------------------------------------------ phase M: Ap rows of this CTA (cg.cc:100-102)
         unsigned long long tm0 = 0;
+        const unsigned g_mv = g; // first step of this mat-vec
         for (int b = 0; b < ge.nb; ++b) {
             const long long rb0 = ge.r0 + (long long)b * ge.nrows / ge.nb;
             const int nr = (int)(ge.r0 + (long long)(b + 1) * ge.nrows / ge.nb - rb0);
             const int nv = (nr > warp) ? ((nr - warp + CW - 1) / CW) : 0;
             const int wd = (nr == ge.lo) ? ge.w_lo : ge.w_hi;
-            const int ntc = (nr == ge.lo) ? ge.ntc_lo : ge.ntc_hi;
+            long long cb, ce;
+            window_of(s_win[ge.par], b, a.ld, cb, ce);
+            const int ntc = window_tiles(cb, ce, wd); // 0: the block's rows are +0
             double acc0[RPW], acc1[RPW];
 #pragma unroll
             for (int s = 0; s < RPW; ++s) {
@@ -524,10 +569,10 @@ __global__ void __launch_bounds__((CW + 1) * 32, 1) cg_persist_kernel(const Pers
             for (int t = 0; t < ntc; ++t, ++g) {
                 const int stage = g % STAGES;
                 const unsigned ph = (g / STAGES) & 1u;
-                const long long c0 = (long long)t * wd;
-                const int w = (int)((a.ld - c0 < wd) ? (a.ld - c0) : wd);
+                const long long c0 = cb + (long long)t * wd;
+                const int w = (int)((ce - c0 < wd) ? (ce - c0) : wd);
                 mbar_wait_ns(a, &full[stage], ph, 5, m, (int)g, b, t);
-                if (tid == 0 && b == 0 && t == 0) {
+                if (tid == 0 && g == g_mv) {
                     tm0 = globaltimer_ns();
                     if (rec) rec[3] = tm0;
                 }
@@ -585,13 +630,19 @@ __global__ void __launch_bounds__((CW + 1) * 32, 1) cg_persist_kernel(const Pers
                 }
             }
         }
+        const bool streamed = g != g_mv;
+        if (tid == 0 && !streamed && ge.nb > 0) { // rows, but no block had a column to stream
+            tm0 = globaltimer_ns();
+            if (rec) rec[3] = tm0;
+        }
         if (rebalance_now || trace) { // uniform over the CTA
             named_bar_sync(1, NCT); // all rows of this CTA are stored
             if (tid == 0) {
                 const unsigned long long t1 = globaltimer_ns();
                 if (rec) rec[5] = t1;
-                // the time this CTA streamed its rows in: the input of the re-balancing
-                if (rebalance_now) ll_store(tmview + c, ge.nrows > 0 ? (double)(t1 - tm0) : 0.0, tag);
+                // the time this CTA streamed its rows in: the input of the re-balancing (no reading
+                // without a streamed tile: such a CTA gets the mean speed)
+                if (rebalance_now) ll_store(tmview + c, streamed ? (double)(t1 - tm0) : 0.0, tag);
             }
         }
 
@@ -655,7 +706,7 @@ __global__ void __launch_bounds__((CW + 1) * 32, 1) cg_persist_kernel(const Pers
         // ---- re-balancing (off the critical path: the r'r partials of the other CTAs are still on
         // their way): rows for mat-vec m + 2 in proportion to the speed every CTA showed in this one.
         // Every CTA computes the same boundaries from the same 148 numbers; no result bit depends on them.
-        if (balance && warp == CW - 1) {
+        if (warp == CW - 1) {
             const int par = m & 1;
             if (rebalance_now) {
                 // this parity's slot still holds the partition of mat-vec m: the producer must have

@@ -379,6 +379,41 @@ __global__ void __launch_bounds__(256) generate_lap2d_kernel(double *A, long lon
     }
 }
 
+// Envelope of every row of [lr0, lr0 + nrows) (see block_window): one warp per row, 128-bit loads,
+// lane l sees the columns 2(l + 32 i), +1; "non-zero" is any bit pattern but +-0 (NaN and Inf count).
+__global__ void __launch_bounds__(256) row_envelope_kernel(const double *A, long long ld, long long lr0,
+                                                            long long nrows, int2 *env)
+{
+    const long long row = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (row >= nrows) return;
+    const unsigned long long *a = reinterpret_cast<const unsigned long long *>(A + (lr0 + row) * ld);
+    const long long nq = ld >> 1;
+    constexpr unsigned long long kMag = 0x7fffffffffffffffULL;
+    int first = 0x7fffffff, last = -1;
+    long long q = lane;
+    for (; q + 3 * 32 < nq; q += 4 * 32) {
+        ulonglong2 v[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) v[u] = __ldcs(reinterpret_cast<const ulonglong2 *>(a) + q + 32 * u);
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int j = (int)(2 * (q + 32 * u));
+            if (v[u].x & kMag) { first = min(first, j); last = j; }
+            if (v[u].y & kMag) { first = min(first, j + 1); last = j + 1; }
+        }
+    }
+    for (; q < nq; q += 32) {
+        const ulonglong2 v = __ldcs(reinterpret_cast<const ulonglong2 *>(a) + q);
+        const int j = (int)(2 * q);
+        if (v.x & kMag) { first = min(first, j); last = j; }
+        if (v.y & kMag) { first = min(first, j + 1); last = j + 1; }
+    }
+    first = __reduce_min_sync(0xffffffffu, first);
+    last = __reduce_max_sync(0xffffffffu, last);
+    if (lane == 0) env[lr0 + row] = last >= 0 ? make_int2(first, last + 1) : make_int2(0, 0);
+}
+
 // Matrix::read's densification (matrix.cc:12-21: A(i,j) = a, and A(j,i) = a when symmetric, in file
 // order, later entries overwriting) as three parallel passes.  The shard's own 8-byte cells hold
 // "index of the last writer + 1" between pass 1 and pass 3 (0 = untouched = the value 0.0).
@@ -432,6 +467,14 @@ __global__ void __launch_bounds__(256) coo_store_kernel(double *A, long long ld,
 inline int grid_for(long long n) { return (int)((n + kChunk - 1) / kChunk); }
 
 } // namespace
+
+cudaError_t launch_row_envelope(const double *A, long long ld, long long lr0, long long nrows, int2 *env,
+                                cudaStream_t s)
+{
+    if (nrows <= 0) return cudaSuccess;
+    row_envelope_kernel<<<(unsigned)((nrows + 7) / 8), 256, 0, s>>>(A, ld, lr0, nrows, env);
+    return cudaGetLastError();
+}
 
 cudaError_t preload_vec_kernels()
 {

@@ -70,7 +70,9 @@ int cgb_create(int64_t n, int rank, int world, int device, cgb_ctx **out);
  * Options: "compat" = 1, "loopback" > 0 and "trace" > 0 return CGB_ERR_STATE; "gemv_variant",
  * "num_threads", "block_width" and "transposed" are accepted and change nothing; cgb_autotune
  * changes nothing and reports every candidate as not run.  Read-only: "storage" (0 dense,
- * 1 CSR), "nnz" (entries stored in this rank's shard). */
+ * 1 CSR), "nnz" (entries stored in this rank's shard), "envelope_doubles" (dense: the sum over
+ * this rank's rows of last + 1 - first non-zero column, the part of each row the mat-vecs stream;
+ * 0 on a CSR context). */
 int cgb_create_csr(int64_t n, int rank, int world, int device, cgb_ctx **out);
 int cgb_destroy(cgb_ctx *ctx);
 
