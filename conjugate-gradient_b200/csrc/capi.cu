@@ -1580,6 +1580,9 @@ extern "C" int cgb_autotune(cgb_ctx *c, int iters, int *chosen, float *us_per_it
     for (int v = 0; v < nv && rc == CGB_OK; ++v) {
         if (strncmp(gemv_variant(v).name, "tma", 3) != 0 || strstr(gemv_variant(v).name, "nohint")) continue;
         set_variant(c, v);
+        // only shapes with a persistent instantiation, on either schedule (DESIGN.md 3.3): the
+        // choice stays a shape both schedules run when the schedule is switched after tuning
+        if (persist_index(c) < 0) continue;
         const bool persist = want_persist && !persist_unusable(c);
         if (want_persist && !persist) continue; // compare like with like
         if (gemv_variant(v).preload() != cudaSuccess) { cudaGetLastError(); continue; }
