@@ -570,11 +570,7 @@ static int create_ctx(int64_t n, int rank, int world, int device, int storage, c
     c->n_loc = n / world;
     c->maxrows = num[world - 1];
     c->nchunks = (n + kChunk - 1) / kChunk;
-    int max_cps = 1;
-    for (int v = 0; v < gemv_variant_count(); ++v)
-        if (gemv_variant(v).ctas_per_sm > max_cps) max_cps = gemv_variant(v).ctas_per_sm;
     c->slot_cap = (c->maxrows + 1) & ~1LL;
-    (void)max_cps;
     set_variant(c, 0);
 
     auto bail = [&](int code) {

@@ -9,8 +9,8 @@ The parent's libcgb200.so is cross-compiled from the parent commit into profiles
 Every measurement runs in a process of its own (the library is bound once per process through
 _capi.LIB_PATH); the builds alternate, case by case, round by round, so both see the same machine.
 
-Cases (default persistent schedule, tol = 0 so no batch stops early, device-timed cgb_iterate
-batches with the solve state resident, as bench.py's `value`):
+Cases (the persistent schedule unless --schedule 0 selects the graph schedule, tol = 0 so no batch
+stops early, device-timed cgb_iterate batches with the solve state resident, as bench.py's `value`):
   lap40k / lap20k : generate_lap2d at N = 40 000 / 20 000 (bench.py's system and --workload weak)
   dense20k        : a seeded, diagonally dominant, symmetric matrix with every entry non-zero at
                     N = 20 000 through set_matrix_rows: every window is [0, ld), the windowed stream
@@ -20,7 +20,7 @@ geometry of the static partition (A rows + p slice per block, tma_w8r2c512s3, 14
 persistent kernel re-balances rows, which moves these by a few blocks' worth), that over the time,
 and a digest of x + r'r history of a 200-iteration (dense: 50) solve, to show both builds agree.
 
-    python profiles/envelope_bench.py [--rounds 3] [--out DIR]
+    python profiles/envelope_bench.py [--rounds 3] [--schedule 1] [--out DIR]
 """
 import argparse
 import hashlib
@@ -95,11 +95,13 @@ def setup(cgb, ctx, case, n):
     ctx.set_rhs(cgb.init_source_term(n))
 
 
-def worker(case, batch, min_ms):
+def worker(case, batch, min_ms, schedule):
     cgb = importlib.import_module("conjugate-gradient_b200")
     n = CASES[case]
     with cgb.Context(n, 0, 1, 0) as ctx:
         setup(cgb, ctx, case, n)
+        ctx.set_option("schedule", schedule)
+        ctx_schedule = ctx.get_option("schedule_in_use")
         try:
             envd = ctx.get_option("envelope_doubles")
         except cgb.CgbError:                            # the parent build has no such option
@@ -119,7 +121,7 @@ def worker(case, batch, min_ms):
             "it_per_s": round(it / (sum(ms) * 1e-3), 1),
             "us_per_iter": round(1e3 * sum(ms) / it, 3),
             "batch_it_per_s": [round(batch / (m * 1e-3), 1) for m in ms],
-            "envelope_doubles": envd, "digest": dg}
+            "envelope_doubles": envd, "schedule_in_use": ctx_schedule, "digest": dg}
 
 
 def main():
@@ -128,6 +130,7 @@ def main():
     ap.add_argument("--cases", default=",".join(CASES))
     ap.add_argument("--batch", type=int, default=200)
     ap.add_argument("--min-ms", type=float, default=1000.0)
+    ap.add_argument("--schedule", type=int, default=1, help="1 persistent kernel, 0 CUDA graph of 4 kernels per iteration")
     ap.add_argument("--out", default=None, help="also write DIR/envelope_bench.jsonl")
     ap.add_argument("--worker", default=None, help=argparse.SUPPRESS)
     ap.add_argument("--lib", default=None, help=argparse.SUPPRESS)
@@ -136,7 +139,7 @@ def main():
         sys.path.insert(0, ROOT)
         if a.lib:
             importlib.import_module("conjugate-gradient_b200._capi").LIB_PATH = a.lib
-        print(json.dumps(worker(a.worker, a.batch, a.min_ms)), flush=True)
+        print(json.dumps(worker(a.worker, a.batch, a.min_ms, a.schedule)), flush=True)
         return
     if not os.path.exists(PARENT_LIB):
         sys.exit(f"{PARENT_LIB} is missing (see the docstring)")
@@ -147,7 +150,7 @@ def main():
         for c in cases:
             for build in (("parent", "new") if rnd % 2 == 0 else ("new", "parent")):
                 cmd = [sys.executable, os.path.abspath(__file__), "--worker", c, "--batch", str(a.batch),
-                       "--min-ms", str(a.min_ms)] + (["--lib", PARENT_LIB] if build == "parent" else [])
+                       "--min-ms", str(a.min_ms), "--schedule", str(a.schedule)] + (["--lib", PARENT_LIB] if build == "parent" else [])
                 out = subprocess.run(cmd, capture_output=True, text=True, timeout=1800, check=True)
                 r = json.loads(out.stdout.strip().splitlines()[-1])
                 r.update(build=build, round=rnd)
@@ -164,7 +167,7 @@ def main():
             wb = windowed_bytes(n, lambda i: lap2d_env(i, n))
         dense_b = 8 * n * ((n + 15) // 16 * 16)
         us = 1e6 / statistics.median(rn)
-        s = {"case": c, "n": n, **info,
+        s = {"case": c, "n": n, "schedule": a.schedule, **info,
              "new_it_per_s": rn, "parent_it_per_s": rp,
              "new_median": statistics.median(rn), "parent_median": statistics.median(rp),
              "speedup_median": round(statistics.median(rn) / statistics.median(rp), 3),

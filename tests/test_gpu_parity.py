@@ -238,15 +238,14 @@ def test_persistent_schedule_ragged_sizes_every_shape(cgb, O, n):
         assert np.array_equal([nx, rr], [ref.norm_x, ref.rel_resid], equal_nan=True), name
 
 
-def test_schedules_interleave_bitwise(cgb, O):
-    """cgb_iterate in pieces, alternating the persistent kernel and the graph schedule on the
-    same solve: the state handed over between launches (x, r, p, r'r partials, k) is complete,
-    so any split gives the bits of one uninterrupted solve."""
+def _interleave_schedules(cgb, O, graph, profile):
     n = 3000
     b = O.init_source_term(n)
     with _ctx(cgb, n) as ctx:
         ctx.generate_lap2d()
         ctx.set_rhs(b)
+        ctx.set_option("graph", graph)
+        ctx.set_option("profile", profile)
         nblk = ctx.layout().nblk
         ctx.solve_begin(np.zeros(n), 150, 1e-10, True)
         for sched, iters in ((1, 7), (0, 20), (1, 1), (1, 40), (0, 3), (1, 79)):
@@ -257,6 +256,88 @@ def test_schedules_interleave_bitwise(cgb, O):
     ref = O.solve(O.generate_lap2d(n), b, max_iter=150, nranks=1, nblk=nblk)
     assert info.k == ref.k == 150 and info.iterations == 150
     assert np.array_equal(hist, ref.hist) and np.array_equal(x, ref.x)
+
+
+def test_schedules_interleave_bitwise(cgb, O):
+    """cgb_iterate in pieces, alternating the persistent kernel and the graph schedule on the
+    same solve: the state handed over between launches (x, r, p, r'r partials, k) is complete,
+    so any split gives the bits of one uninterrupted solve."""
+    _interleave_schedules(cgb, O, graph=1, profile=0)
+
+
+@pytest.mark.parametrize("graph,profile", [(0, 0), (1, 1), (0, 1)])
+def test_schedules_interleave_launch_modes(cgb, O, graph, profile):
+    """The same split when the graph-schedule pieces run as plain launches (graph = 0) or in
+    profile mode, which launches without programmatic dependent launch and, since the persistent
+    kernel cannot run there, keeps the whole solve on the graph schedule's kernels."""
+    _interleave_schedules(cgb, O, graph=graph, profile=profile)
+
+
+def test_vector_kernel_timelines(cgb, O):
+    """Option "trace" on the graph schedule: thread 0 of every block of update_xr stamps entry <=
+    dependency met <= alpha known <= exit, of update_p entry <= dependency met <= exit, in each of
+    the last 8 launches, and each kernel counts one launch per iteration.  Every update_p block
+    passes its dependency after every update_xr block of the same iteration has exited, and every
+    update_xr block of the next iteration after every update_p block: a block that skipped a launch
+    would leave a stale slot out of this order."""
+    n, iters, cap = 3000, 40, 8
+    with _ctx(cgb, n) as ctx:
+        ctx.generate_lap2d()
+        ctx.set_rhs(O.init_source_term(n))
+        ctx.set_option("schedule", 0)
+        ctx.set_option("trace", cap)
+        info, _ = ctx.solve(np.zeros(n), max_iter=iters, tol=1e-10, history=True)
+        nchunks = ctx.layout().nchunks
+        xr, n_xr = ctx.trace_read(1)
+        p, n_p = ctx.trace_read(2)
+    assert info.iterations == iters and not info.converged
+    assert n_xr == n_p == iters
+    assert xr.shape == p.shape == (cap, nchunks, 8)
+    xr, p = xr.astype(np.int64), p.astype(np.int64)
+    assert np.all(xr[:, :, 0] > 0) and np.all(np.diff(xr[:, :, :4], axis=2) >= 0)
+    assert np.all(p[:, :, 0] > 0) and np.all(p[:, :, 1] >= p[:, :, 0]) and np.all(p[:, :, 3] >= p[:, :, 1])
+    assert np.all(p[:, :, 1].min(axis=1) >= xr[:, :, 3].max(axis=1))
+    assert np.all(xr[1:, :, 1].min(axis=1) >= p[:-1, :, 3].max(axis=1))
+
+
+@pytest.mark.parametrize("case", list(SCHEDULES) + ["csr"])
+def test_nearzero_clamp_bitwise_vs_oracle(cgb, O, case):
+    """alpha = rsold / max(p'Ap, rsold * NEARZERO) (cg.cc:107).  On -lap2d every p'Ap is negative,
+    so the clamp fires in every iteration: alpha = rsold / (rsold * 1e-14) and r'r grows by ~1e57 per
+    iteration (it overflows in the fourth, so three keep every number finite).  Dense storage under
+    every schedule (one-iteration graphs, so the graph is replayed) and CSR storage, bit for bit
+    against the oracle."""
+    n, iters = 1000, 3
+    A = -O.generate_lap2d(n)
+    b = O.init_source_term(n)
+    schedule, graph = SCHEDULES.get(case, (0, 1))
+    with cgb.Context(n, storage="csr" if case == "csr" else "dense") as ctx:
+        if case == "csr":
+            i, j = np.nonzero(A)
+            ctx.set_matrix_coo(i.astype(np.int32), j.astype(np.int32), A[i, j], symmetric=False)
+        else:
+            ctx.set_matrix_rows(A)
+        ctx.set_rhs(b)
+        ctx.set_option("schedule", schedule)
+        ctx.set_option("graph", graph)
+        ctx.set_option("graph_unroll", 1)
+        assert ctx.get_option("schedule_in_use") == schedule
+        x = np.zeros(n)
+        info, hist = ctx.solve(x, max_iter=iters, tol=1e-10, history=True)
+        nx, rr = ctx.residual_check()
+        nblk = ctx.layout().nblk
+    ref = O.solve(A, b, max_iter=iters, nranks=1, nblk=nblk)
+    assert np.all(np.isfinite(ref.hist)) and np.all(np.isfinite(ref.x))
+    assert info.k == ref.k == iters and info.iterations == iters
+    assert np.array_equal(hist, ref.hist, equal_nan=True)
+    assert np.array_equal(x, ref.x, equal_nan=True)
+    assert np.array_equal([info.rsold, info.rsnew, nx, rr],
+                          [ref.rsold, ref.rsnew, ref.norm_x, ref.rel_resid], equal_nan=True)
+    # the first iteration (p = r = b) took the clamped step, not rsold / p'Ap
+    rs = O.dot(b, b)
+    assert O.dot(b, A @ b) < rs * 1e-14
+    r1 = b - rs / (rs * 1e-14) * (A @ b)
+    assert abs(hist[0] - r1 @ r1) <= 1e-12 * hist[0]
 
 
 def test_solve_mtx_bitwise_vs_oracle(cgb, O, tmp_path):
