@@ -67,6 +67,9 @@ SIGNATURES = [
     ("cgb_solve_begin", C.c_int, [_CTX, _dp, C.c_int64, C.c_double, C.c_int]),
     ("cgb_iterate", C.c_int, [_CTX, C.c_int64, C.POINTER(C.c_float)]),
     ("cgb_solve_end", C.c_int, [_CTX, _dp, _dp, C.POINTER(SolveInfo)]),
+    ("cgb_solve_block_begin", C.c_int, [_CTX, C.c_int, _dp, _dp, C.c_int64, C.c_double, C.c_int]),
+    ("cgb_solve_block_end", C.c_int, [_CTX, _dp, _dp, C.POINTER(SolveInfo)]),
+    ("cgb_solve_block", C.c_int, [_CTX, C.c_int, _dp, _dp, C.c_int64, C.c_double, _dp, C.POINTER(SolveInfo)]),
     ("cgb_residual_check", C.c_int, [_CTX, _dp, _dp]),
     ("cgb_gemv", C.c_int, [_CTX, _dp, _dp, _dp, _dp]),
     ("cgb_dot", C.c_int, [_CTX, _dp, _dp, _dp]),
@@ -262,6 +265,42 @@ class Context:
         info = SolveInfo()
         _check(self._lib.cgb_solve_end(self._h, _p(x), _p(hist), C.byref(info)))
         return info
+
+    # -- block solve (CSR, one rank): column j bit for bit the single solve of A x = B[j] from X0[j]
+    def _block_inputs(self, B, X0):
+        B = np.ascontiguousarray(B, dtype=np.float64)
+        assert B.ndim == 2 and B.shape[1] == self.n, "B must be (nrhs, n)"
+        X = np.zeros_like(B) if X0 is None else np.array(X0, dtype=np.float64, order="C")
+        assert X.shape == B.shape
+        return B, X
+
+    def solve_block(self, B, X0=None, max_iter: int = 0, tol: float = 1e-10, history: bool = False):
+        """B: (nrhs, n) right-hand sides; returns (X, infos, hist) -- X (nrhs, n), one SolveInfo per
+        column, and (history=True) a list of each column's r'r history, else None."""
+        B, X = self._block_inputs(B, X0)
+        nrhs = B.shape[0]
+        hist = np.zeros((nrhs, max(max_iter, 1)), dtype=np.float64) if history else None
+        infos = (SolveInfo * nrhs)()
+        _check(self._lib.cgb_solve_block(self._h, nrhs, _p(B), _p(X), max_iter, tol, _p(hist), infos))
+        return X, list(infos), self._block_hist(hist, infos)
+
+    def solve_block_begin(self, B, X0=None, max_iter: int = 0, tol: float = 1e-10, history: bool = False):
+        B, X0 = self._block_inputs(B, X0)
+        self._block = (B.shape[0], max_iter, history)
+        _check(self._lib.cgb_solve_block_begin(self._h, B.shape[0], _p(B), _p(X0), max_iter, tol, int(history)))
+
+    def solve_block_end(self):
+        """(X, infos, hist) of the block solve begun with solve_block_begin (advanced by iterate)."""
+        nrhs, max_iter, history = self._block
+        X = np.empty((nrhs, self.n), dtype=np.float64)
+        hist = np.zeros((nrhs, max(max_iter, 1)), dtype=np.float64) if history else None
+        infos = (SolveInfo * nrhs)()
+        _check(self._lib.cgb_solve_block_end(self._h, _p(X), _p(hist), infos))
+        return X, list(infos), self._block_hist(hist, infos)
+
+    @staticmethod
+    def _block_hist(hist, infos):
+        return None if hist is None else [hist[j, :infos[j].iterations].copy() for j in range(len(infos))]
 
     def residual_check(self):
         nx, rr = C.c_double(), C.c_double()

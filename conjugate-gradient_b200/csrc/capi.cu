@@ -107,6 +107,31 @@ int load_nccl()
     } while (0)
 
 // ------------------------------------------------------------------ context
+// Block solve (cgb_solve_block_begin): its own buffers, States, flag and graph, allocated on the
+// first block solve and never shared with the single solve.
+static_assert(kMaxRhs == CGB_MAX_RHS, "one limit of columns");
+struct BlockSolve {
+    int cap = 0;                    // columns the vector buffers hold
+    int nrhs = 0;                   // columns of the solve in progress
+    double *x = nullptr, *r = nullptr, *p = nullptr, *b = nullptr; // [cap][ld]
+    double *ap = nullptr;           // [cap][slot]
+    double *rrpart = nullptr, *papart = nullptr; // [cap][nchunks]
+    State *st = nullptr;            // [cap]
+    unsigned int *arrive = nullptr; // [cap][2] arrival counters, then the count of converged columns
+    double *hist = nullptr;         // [cap][hist_ld]
+    long long hist_ld = 0;
+    int *h_done = nullptr, *d_hdone = nullptr; // mapped pinned flag: every column has converged
+    cudaGraph_t graph = nullptr;
+    cudaGraphExec_t graph_exec = nullptr;
+    // what the captured arguments bake in
+    int graph_len = 0, graph_nrhs = 0, graph_pdl = 0;
+    double graph_tol = 0.0;
+    const double *graph_hist = nullptr;
+    bool active = false, keep_history = false;
+    long long max_iter = 0, launched = 0;
+    double tol = 0.0, loop_ms = 0.0;
+};
+
 struct cgb_ctx {
     long long n = 0, ld = 0, rows = 0, row0 = 0, n_loc = 0, maxrows = 0, nchunks = 0;
     int rank = 0, world = 1, device = 0, sm_count = 0;
@@ -163,12 +188,14 @@ struct cgb_ctx {
     cudaGraphExec_t graph_exec = nullptr;
     ncclComm_t comm = nullptr;
 
-    bool matrix_set = false, rhs_set = false, in_solve = false;
+    bool matrix_set = false, rhs_set = false;
+    bool in_solve = false;         // a single or (blk.active) a block solve is between begin and end
     long long max_iter = 0, launched = 0, kernel_launches = 0;
     double tol = 1e-10, graph_tol = -1.0;
     double loop_ms = 0.0;
     double prof_gemv_ms = 0.0;
     long long prof_gemv_n = 0;
+    BlockSolve blk;
 };
 
 namespace {
@@ -491,6 +518,214 @@ int read_state(cgb_ctx *c, State *out)
     return CGB_OK;
 }
 
+// ---- block solve ---------------------------------------------------------------------------
+void drop_block_graph(cgb_ctx *c)
+{
+    BlockSolve &k = c->blk;
+    if (k.graph_exec) cudaGraphExecDestroy(k.graph_exec);
+    if (k.graph) cudaGraphDestroy(k.graph);
+    k.graph_exec = nullptr;
+    k.graph = nullptr;
+}
+
+void free_block_vectors(cgb_ctx *c)
+{
+    BlockSolve &k = c->blk;
+    double *bufs[] = {k.x, k.r, k.p, k.b, k.ap, k.rrpart, k.papart};
+    for (double *p : bufs)
+        if (p) cudaFree(p);
+    if (k.st) cudaFree(k.st);
+    if (k.arrive) cudaFree(k.arrive);
+    k.x = k.r = k.p = k.b = k.ap = k.rrpart = k.papart = nullptr;
+    k.st = nullptr;
+    k.arrive = nullptr;
+    k.cap = 0;
+}
+
+void free_block(cgb_ctx *c)
+{
+    BlockSolve &k = c->blk;
+    drop_block_graph(c);
+    free_block_vectors(c);
+    if (k.hist) cudaFree(k.hist);
+    k.hist = nullptr;
+    k.hist_ld = 0;
+    if (k.h_done) cudaFreeHost(k.h_done);
+    k.h_done = k.d_hdone = nullptr;
+}
+
+// buffers for nrhs columns and, with a history, max(max_iter, 1) entries per column; grows only
+int size_block(cgb_ctx *c, int nrhs, long long max_iter, bool history)
+{
+    BlockSolve &k = c->blk;
+    auto alloc = [&](void **p, size_t bytes) -> int {
+        cudaError_t e = cudaMalloc(p, bytes);
+        if (e == cudaSuccess) e = cudaMemsetAsync(*p, 0, bytes, c->stream);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            return fail(e == cudaErrorMemoryAllocation ? CGB_ERR_NOMEM : CGB_ERR_CUDA, "block solve buffers: %s",
+                        cudaGetErrorString(e));
+        }
+        return CGB_OK;
+    };
+    int rc = CGB_OK;
+    if (!k.h_done) { // first block solve of this context
+        CK(preload_spmv_block_kernels());
+        CK(preload_vec_block_kernels());
+        CK(cudaHostAlloc(&k.h_done, sizeof(int), cudaHostAllocMapped));
+        CK(cudaHostGetDevicePointer(&k.d_hdone, k.h_done, 0));
+    }
+    const long long hist_need = max_iter > 0 ? max_iter : 1;
+    if (nrhs > k.cap) {
+        drop_block_graph(c);
+        free_block_vectors(c);
+        const size_t vec = (size_t)nrhs * c->ld * sizeof(double);
+        const size_t part = (size_t)nrhs * c->nchunks * sizeof(double);
+        if ((rc = alloc((void **)&k.x, vec)) || (rc = alloc((void **)&k.r, vec)) || (rc = alloc((void **)&k.p, vec)) ||
+            (rc = alloc((void **)&k.b, vec)) || (rc = alloc((void **)&k.ap, (size_t)nrhs * c->slot_cap * sizeof(double))) ||
+            (rc = alloc((void **)&k.rrpart, part)) || (rc = alloc((void **)&k.papart, part)) ||
+            (rc = alloc((void **)&k.st, (size_t)nrhs * sizeof(State))) ||
+            (rc = alloc((void **)&k.arrive, (size_t)(2 * nrhs + 1) * sizeof(unsigned int)))) {
+            free_block_vectors(c);
+            return rc;
+        }
+        k.cap = nrhs;
+        if (k.hist) cudaFree(k.hist); // its column stride follows from the new capacity
+        k.hist = nullptr;
+        k.hist_ld = 0;
+    }
+    if (history && hist_need > k.hist_ld) {
+        drop_block_graph(c);
+        if (k.hist) cudaFree(k.hist);
+        k.hist = nullptr;
+        k.hist_ld = 0;
+        if ((rc = alloc((void **)&k.hist, (size_t)k.cap * hist_need * sizeof(double)))) return rc;
+        k.hist_ld = hist_need;
+    }
+    return CGB_OK;
+}
+
+BlockArgs make_block_args(const cgb_ctx *c, const double *v, int advance)
+{
+    const BlockSolve &k = c->blk;
+    BlockArgs a;
+    memset(&a, 0, sizeof a);
+    a.rp = c->csr.rp;
+    a.col = c->csr.col;
+    a.val = c->csr.val;
+    a.v = v;
+    a.x = k.x;
+    a.r = k.r;
+    a.p = k.p;
+    a.b = k.b;
+    a.ap = k.ap;
+    a.rrpart = k.rrpart;
+    a.papart = k.papart;
+    a.st = k.st;
+    a.arrive = k.arrive;
+    a.ndone = k.arrive + 2 * k.cap;
+    a.host_done = k.d_hdone;
+    a.hist = k.keep_history ? k.hist : nullptr;
+    a.n = c->n;
+    a.ld = c->ld;
+    a.rows = c->rows;
+    a.slot = c->slot_cap;
+    a.nchunks = c->nchunks;
+    a.hist_ld = k.hist_ld;
+    a.nrhs = k.nrhs;
+    a.advance = advance;
+    a.pdl = (advance && c->opt_pdl) ? 1 : 0; // only inside the CG loop
+    a.tol = k.tol;
+    return a;
+}
+
+// mat-vec + the three vector kernels of one block iteration
+int launch_block_iteration(cgb_ctx *c)
+{
+    const BlockArgs a = make_block_args(c, c->blk.p, 1);
+    CK(launch_spmv_block(a, c->sm_count, c->stream));
+    CK(launch_pap_alpha_block(a, c->stream));
+    CK(launch_update_xr_block(a, c->stream));
+    CK(launch_update_p_block(a, c->stream));
+    c->kernel_launches += 4;
+    return CGB_OK;
+}
+
+int build_block_graph(cgb_ctx *c, int len)
+{
+    BlockSolve &k = c->blk;
+    drop_block_graph(c);
+    CK(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
+    int rc = CGB_OK;
+    const long long before = c->kernel_launches;
+    for (int u = 0; u < len && rc == CGB_OK; ++u) rc = launch_block_iteration(c);
+    c->kernel_launches = before; // capture launches nothing
+    cudaGraph_t g = nullptr;
+    cudaError_t e = cudaStreamEndCapture(c->stream, &g);
+    if (rc != CGB_OK) {
+        if (g) cudaGraphDestroy(g);
+        return rc;
+    }
+    CK(e);
+    k.graph = g;
+    CK(cudaGraphInstantiate(&k.graph_exec, k.graph, 0));
+    k.graph_len = len;
+    k.graph_nrhs = k.nrhs;
+    k.graph_tol = k.tol;
+    k.graph_hist = make_block_args(c, k.p, 1).hist;
+    k.graph_pdl = c->opt_pdl;
+    return CGB_OK;
+}
+
+// cgb_iterate of a block solve: the graph schedule of a CSR single solve, with the block's own graph
+int block_iterate(cgb_ctx *c, int64_t iters, float *ms)
+{
+    BlockSolve &k = c->blk;
+    int rc;
+    long long todo = std::min<long long>(iters, k.max_iter - k.launched);
+    if (todo < 0) todo = 0;
+    const bool graph = c->opt_graph != 0;
+    const int want_len = c->graph_unroll < c->poll_every ? c->graph_unroll : c->poll_every;
+    if (k.graph_exec && (k.graph_len != want_len || k.graph_nrhs != k.nrhs || k.graph_tol != k.tol ||
+                         k.graph_hist != make_block_args(c, k.p, 1).hist || k.graph_pdl != c->opt_pdl))
+        drop_block_graph(c);
+    if (graph && !k.graph_exec && todo >= want_len) {
+        if ((rc = build_block_graph(c, want_len))) return rc;
+    }
+    CK(cudaEventRecord(c->ev0, c->stream));
+    long long issued = 0;
+    int batch_idx = 0;
+    while (issued < todo) {
+        if (*(volatile int *)k.h_done) break; // every column converged: later launches would be no-ops
+        const long long batch = std::min<long long>(c->poll_every, todo - issued);
+        long long i = 0;
+        while (i < batch) {
+            if (graph && k.graph_exec && batch - i >= k.graph_len) {
+                CK(cudaGraphLaunch(k.graph_exec, c->stream));
+                c->kernel_launches += 4LL * k.graph_len;
+                c->graph_replays += 1;
+                i += k.graph_len;
+            } else {
+                if ((rc = launch_block_iteration(c))) return rc;
+                i += 1;
+            }
+        }
+        issued += batch;
+        // at most two batches in flight, as in cgb_iterate
+        CK(cudaEventRecord(c->ev_batch[batch_idx & 1], c->stream));
+        if (batch_idx >= 1) CK(cudaEventSynchronize(c->ev_batch[(batch_idx - 1) & 1]));
+        ++batch_idx;
+    }
+    CK(cudaEventRecord(c->ev1, c->stream));
+    CK(cudaEventSynchronize(c->ev1));
+    float t = 0.f;
+    CK(cudaEventElapsedTime(&t, c->ev0, c->ev1));
+    k.loop_ms += t;
+    k.launched += issued;
+    if (ms) *ms = t;
+    return CGB_OK;
+}
+
 } // namespace
 
 // ------------------------------------------------------------------ library
@@ -688,6 +923,7 @@ extern "C" int cgb_destroy(cgb_ctx *c)
     if (c->ctl) cudaFree(c->ctl);
     if (c->h_done) cudaFreeHost(c->h_done);
     if (c->h_pin) cudaFreeHost(c->h_pin);
+    free_block(c);
     if (c->ev0) cudaEventDestroy(c->ev0);
     if (c->ev1) cudaEventDestroy(c->ev1);
     for (cudaEvent_t e : c->ev_batch)
@@ -1212,6 +1448,7 @@ extern "C" int cgb_iterate(cgb_ctx *c, int64_t iters, float *ms)
     if (rc) return rc;
     if (!c->in_solve) return fail(CGB_ERR_STATE, "cgb_solve_begin was not called");
     if (iters < 0) return fail(CGB_ERR_INVALID, "iters < 0");
+    if (c->blk.active) return block_iterate(c, iters, ms);
     long long todo = std::min<long long>(iters, c->max_iter - c->launched);
     if (todo < 0) todo = 0;
     const bool profile = c->opt_profile != 0;
@@ -1324,6 +1561,7 @@ extern "C" int cgb_solve_end(cgb_ctx *c, double *x_host, double *resid_hist, cgb
     int rc = use_device(c);
     if (rc) return rc;
     if (!c->in_solve) return fail(CGB_ERR_STATE, "no solve in progress");
+    if (c->blk.active) return fail(CGB_ERR_STATE, "a block solve is in progress (cgb_solve_block_end)");
     CK(launch_finalize(make_vec_args(c), c->stream));
     c->kernel_launches += 1;
     State s;
@@ -1360,6 +1598,116 @@ extern "C" int cgb_solve(cgb_ctx *c, double *x_host, int64_t max_iter, double to
         return rc;
     }
     return cgb_solve_end(c, x_host, resid_hist, info);
+}
+
+// ------------------------------------------------------------------ block solve
+// A null context on a machine without a device is reported as the missing device, like the
+// context creation it stands for.
+static int null_context()
+{
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+        cudaGetLastError();
+        return fail(CGB_ERR_NO_DEVICE, "no CUDA device");
+    }
+    return fail(CGB_ERR_INVALID, "null context");
+}
+
+extern "C" int cgb_solve_block_begin(cgb_ctx *c, int nrhs, const double *b_host, const double *x0_host,
+                                     int64_t max_iter, double tol, int keep_history)
+{
+    if (!c) return null_context();
+    if (nrhs < 1 || nrhs > CGB_MAX_RHS) return fail(CGB_ERR_INVALID, "nrhs must be in [1, %d] (got %d)", CGB_MAX_RHS, nrhs);
+    if (!b_host) return fail(CGB_ERR_INVALID, "null b");
+    if (max_iter < 0) return fail(CGB_ERR_INVALID, "max_iter < 0");
+    int rc = use_device(c);
+    if (rc) return rc;
+    if (c->storage != 1)
+        return fail(CGB_ERR_STATE, "block solves need CSR storage: the dense mat-vec streams one p per tile pipeline");
+    if (c->world > 1)
+        return fail(CGB_ERR_STATE, "block solves run on one rank: the exchange carries one vector per row");
+    if (!c->matrix_set) return fail(CGB_ERR_STATE, "matrix not set");
+    if (c->in_solve) return fail(CGB_ERR_STATE, c->blk.active ? "block solve already in progress" : "a single solve is in progress");
+    BlockSolve &k = c->blk;
+    if ((rc = size_block(c, nrhs, max_iter, keep_history != 0))) return rc;
+    k.nrhs = nrhs;
+    k.max_iter = max_iter;
+    k.tol = tol;
+    k.keep_history = keep_history != 0;
+    k.launched = 0;
+    k.loop_ms = 0.0;
+    if (k.keep_history) CK(cudaMemsetAsync(k.hist, 0, (size_t)k.cap * k.hist_ld * sizeof(double), c->stream));
+    std::vector<State> s0((size_t)nrhs);
+    memset(s0.data(), 0, s0.size() * sizeof(State));
+    for (State &s : s0) s.iter = -1;
+    *k.h_done = 0;
+    CK(cudaMemcpyAsync(k.st, s0.data(), s0.size() * sizeof(State), cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemsetAsync(k.arrive, 0, (size_t)(2 * k.cap + 1) * sizeof(unsigned int), c->stream));
+    const size_t row = (size_t)c->n * 8, pitch = (size_t)c->ld * 8;
+    CK(cudaMemcpy2DAsync(k.b, pitch, b_host, row, row, (size_t)nrhs, cudaMemcpyHostToDevice, c->stream));
+    if (x0_host) CK(cudaMemcpy2DAsync(k.x, pitch, x0_host, row, row, (size_t)nrhs, cudaMemcpyHostToDevice, c->stream));
+    else CK(cudaMemsetAsync(k.x, 0, (size_t)nrhs * pitch, c->stream));
+    // r = b - A x0 ; p = r ; partials of r.p, per column                cg.cc:77-92
+    const BlockArgs a = make_block_args(c, k.x, 0);
+    CK(launch_spmv_block(a, c->sm_count, c->stream));
+    CK(launch_init_residual_block(a, c->stream));
+    c->kernel_launches += 2;
+    CK(cudaStreamSynchronize(c->stream));
+    k.active = true;
+    c->in_solve = true;
+    return CGB_OK;
+}
+
+extern "C" int cgb_solve_block_end(cgb_ctx *c, double *x_host, double *resid_hist, cgb_solve_info *info)
+{
+    if (!c) return null_context();
+    int rc = use_device(c);
+    if (rc) return rc;
+    BlockSolve &k = c->blk;
+    if (!k.active) return fail(CGB_ERR_STATE, "no block solve in progress");
+    if (resid_hist && !k.keep_history) return fail(CGB_ERR_STATE, "history was not requested in cgb_solve_block_begin");
+    const BlockArgs a = make_block_args(c, k.p, 0);
+    CK(launch_finalize_block(a, c->stream));
+    c->kernel_launches += 1;
+    std::vector<State> s((size_t)k.nrhs);
+    CK(cudaMemcpyAsync(s.data(), k.st, s.size() * sizeof(State), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    const size_t row = (size_t)c->n * 8, pitch = (size_t)c->ld * 8;
+    if (x_host) CK(cudaMemcpy2DAsync(x_host, row, k.x, pitch, row, (size_t)k.nrhs, cudaMemcpyDeviceToHost, c->stream));
+    for (int j = 0; j < k.nrhs; ++j) {
+        const long long executed = s[j].done ? s[j].iter + 1 : s[j].iter;
+        if (resid_hist && executed > 0)
+            CK(cudaMemcpyAsync(resid_hist + (size_t)j * k.max_iter, k.hist + (size_t)j * k.hist_ld,
+                               (size_t)executed * 8, cudaMemcpyDeviceToHost, c->stream));
+        if (info) {
+            info[j].k = s[j].iter;
+            info[j].converged = s[j].done;
+            info[j].rsold = s[j].rsold;
+            info[j].rsnew = s[j].rsnew;
+            info[j].seconds = k.loop_ms * 1e-3;
+            info[j].iterations = executed;
+        }
+    }
+    CK(cudaStreamSynchronize(c->stream));
+    k.active = false;
+    c->in_solve = false;
+    return CGB_OK;
+}
+
+extern "C" int cgb_solve_block(cgb_ctx *c, int nrhs, const double *b_host, double *x_host, int64_t max_iter,
+                               double tol, double *resid_hist, cgb_solve_info *info)
+{
+    if (!c) return null_context();
+    if (!x_host) return fail(CGB_ERR_INVALID, "null x");
+    int rc = cgb_solve_block_begin(c, nrhs, b_host, x_host, max_iter, tol, resid_hist != nullptr);
+    if (rc) return rc;
+    rc = cgb_iterate(c, max_iter, nullptr);
+    if (rc) {
+        c->blk.active = false;
+        c->in_solve = false;
+        return rc;
+    }
+    return cgb_solve_block_end(c, x_host, resid_hist, info);
 }
 
 extern "C" int cgb_residual_check(cgb_ctx *c, double *norm_x, double *rel_resid)

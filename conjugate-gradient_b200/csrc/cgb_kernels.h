@@ -28,6 +28,22 @@ inline cudaError_t launch_kernel(void (*kernel)(KArgs...), int grid, int block, 
     cfg.numAttrs = pdl ? 1 : 0;
     return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
+// the same with a 2-D grid (block solve: x = chunk, y = column)
+template <class... KArgs, class... Args>
+inline cudaError_t launch_kernel_xy(void (*kernel)(KArgs...), dim3 grid, int block, cudaStream_t stream, bool pdl,
+                                    Args &&...args)
+{
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid;
+    cfg.blockDim = dim3((unsigned)block, 1, 1);
+    cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = pdl ? 1 : 0;
+    return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
+}
 
 // ---- mat-vec (gemv.cu) --------------------------------------------------------------
 struct GemvVariant {
@@ -145,5 +161,43 @@ cudaError_t csr_from_coo(CsrShard *m, long long n, long long row0, long long row
 cudaError_t csr_densify(const CsrShard &m, long long lr0, long long nrows, long long n, double *dst, cudaStream_t s);
 // streams the three CSR arrays once (the read ceiling of the CSR mat-vec)
 cudaError_t launch_read_csr(const CsrShard &m, long long rows, double *sink, int sm_count, cudaStream_t s);
+
+// ---- block solve (CSR, one rank): nrhs right-hand sides against one matrix (spmv.cu, vec.cu) ----
+// Column j of x, r, p, b starts at j * ld, of ap at j * slot, of the chunk partials at j * nchunks,
+// of the history at j * hist_ld; st[j] is its State.  Every column runs the kernels of a single CSR
+// solve with its own scalars and arrival counters, so its bits are that solve's; a column whose
+// st[j].done is set is skipped by every kernel, like a single solve after its break.
+constexpr int kMaxRhs = 8;
+struct BlockArgs {
+    const long long *rp;      // the CSR shard
+    const int *col;
+    const double *val;
+    const double *v;          // mat-vec input: x (init) or p (loop)
+    double *x, *r, *p;
+    const double *b;
+    double *ap;               // mat-vec result, [nrhs][slot]
+    double *rrpart, *papart;  // [nrhs][nchunks]
+    State *st;                // [nrhs]
+    unsigned int *arrive;     // [nrhs][2] zeroed arrival counters of pap_alpha / update_xr
+    unsigned int *ndone;      // columns that have converged
+    int *host_done;           // mapped pinned flag, raised when ndone reaches nrhs
+    double *hist;             // nullable, [nrhs][hist_ld]
+    long long n, ld, rows, slot, nchunks, hist_ld;
+    int nrhs;
+    int advance;              // mat-vec: 1 inside the CG loop (block 0 advances every live State)
+    int pdl;
+    double tol;
+};
+cudaError_t preload_spmv_block_kernels();
+cudaError_t preload_vec_block_kernels();
+// ap[j] = A v[j] for the live columns: rp / col / val read once per row for all of them
+cudaError_t launch_spmv_block(const BlockArgs &a, int sm_count, cudaStream_t s);
+// r = b - A x0 ; p = r ; r'r chunk partials, per column
+cudaError_t launch_init_residual_block(const BlockArgs &a, cudaStream_t s);
+// pap_alpha / update_xr_once / update_p_once / finalize per column (grid y = column)
+cudaError_t launch_pap_alpha_block(const BlockArgs &a, cudaStream_t s);
+cudaError_t launch_update_xr_block(const BlockArgs &a, cudaStream_t s);
+cudaError_t launch_update_p_block(const BlockArgs &a, cudaStream_t s);
+cudaError_t launch_finalize_block(const BlockArgs &a, cudaStream_t s);
 
 } // namespace cgb

@@ -144,6 +144,168 @@ __global__ void __launch_bounds__(kSpmvThreads) spmv_csr_kernel(const GemvArgs a
     }
 }
 
+// ---- block mat-vec (block solve) ----------------------------------------------------------
+// Every column is spmv_csr_kernel's arithmetic on that column alone: row_short's bucket chains and
+// merge tree over the row's entries, row_warp's lane-owned accumulators and butterfly.  Only the
+// loads are shared: a row's rp / col / val come from memory once for all columns.
+
+// row_short for one column, the row's (at most kShortRow) entries already in registers
+__device__ __forceinline__ double row_short_regs(const int (&col)[kShortRow], const double (&val)[kShortRow], int len,
+                                                 const double *v)
+{
+    double s[kShortRow];
+    int key[kShortRow];
+    bool live[kShortRow];
+#pragma unroll
+    for (int e = 0; e < kShortRow; ++e) {
+        live[e] = false;
+        key[e] = 0;
+        s[e] = 0.0;
+        if (e < len) {
+            const double prod_a = val[e], pv = __ldg(v + col[e]);
+            const int b = col[e] & 63;
+            bool merged = false;
+#pragma unroll
+            for (int f = 0; f < e; ++f)
+                if (live[f] && key[f] == b) {
+                    s[f] = __fma_rn(prod_a, pv, s[f]);
+                    merged = true;
+                }
+            key[e] = b;
+            live[e] = !merged;
+            s[e] = merged ? 0.0 : __fma_rn(prod_a, pv, 0.0);
+        }
+    }
+    const int bits[6] = {1, 32, 16, 8, 4, 2};
+#pragma unroll
+    for (int lv = 0; lv < 6; ++lv) {
+#pragma unroll
+        for (int e = 0; e < kShortRow; ++e) key[e] &= ~bits[lv];
+#pragma unroll
+        for (int e = 1; e < kShortRow; ++e)
+#pragma unroll
+            for (int f = 0; f < e; ++f)
+                if (live[f] && live[e] && key[f] == key[e]) {
+                    s[f] = __dadd_rn(s[f], s[e]);
+                    live[e] = false;
+                }
+    }
+    double y = 0.0;
+#pragma unroll
+    for (int e = 0; e < kShortRow; ++e)
+        if (live[e]) y = s[e];
+    return y;
+}
+
+// row_warp for the live columns of `mask` (y[j] in every lane); each 32-entry slab is loaded once
+template <int NC>
+__device__ __forceinline__ void row_warp_block(const int *col, const double *val, long long len, const double *v,
+                                               long long ld, unsigned mask, int lane, double (&y)[NC])
+{
+    double acc0[NC], acc1[NC];
+#pragma unroll
+    for (int j = 0; j < NC; ++j) acc0[j] = acc1[j] = 0.0;
+    for (long long k0 = 0; k0 < len; k0 += 32) {
+        const long long k = k0 + lane;
+        int c = 0;
+        double av = 0.0, pv[NC];
+#pragma unroll
+        for (int j = 0; j < NC; ++j) pv[j] = 0.0;
+        if (k < len) {
+            c = __ldcs(col + k);
+            av = __ldcs(val + k);
+#pragma unroll
+            for (int j = 0; j < NC; ++j)
+                if (mask >> j & 1u) pv[j] = __ldg(v + j * ld + c);
+        }
+        const int m = (len - k0 < 32) ? (int)(len - k0) : 32;
+        for (int i = 0; i < m; ++i) {
+            const int ci = __shfl_sync(0xffffffffu, c, i);
+            const double ai = __shfl_sync(0xffffffffu, av, i);
+            const bool mine = ((ci & 63) >> 1) == lane;
+#pragma unroll
+            for (int j = 0; j < NC; ++j) {
+                if (!(mask >> j & 1u)) continue; // warp-uniform
+                const double pj = __shfl_sync(0xffffffffu, pv[j], i);
+                if (mine) {
+                    if (ci & 1) acc1[j] = __fma_rn(ai, pj, acc1[j]);
+                    else acc0[j] = __fma_rn(ai, pj, acc0[j]);
+                }
+            }
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < NC; ++j) y[j] = (mask >> j & 1u) ? warp_butterfly(__dadd_rn(acc0[j], acc1[j])) : 0.0;
+}
+
+// advance_state of column j (one full warp)
+__device__ __forceinline__ void advance_column(const BlockArgs &a, int j, int lane)
+{
+    const double s = warp_det_sum(a.rrpart + j * a.nchunks, a.nchunks, lane);
+    if (lane == 0) {
+        State *st = a.st + j;
+        const long long it = st->iter;
+        if (it >= 0 && a.hist) a.hist[j * a.hist_ld + it] = s;
+        st->rsold = s;
+        st->rsnew = s;
+        st->iter = it + 1;
+    }
+}
+
+template <int NC>
+__global__ void __launch_bounds__(kSpmvThreads) spmv_csr_block_kernel(const BlockArgs a)
+{
+    griddep_launch_dependents();
+    griddep_wait();
+    unsigned mask = 0; // live columns; no kernel of this iteration changes a `done` before this one ends
+#pragma unroll
+    for (int j = 0; j < NC; ++j)
+        if (!a.st[j].done) mask |= 1u << j;
+    if (!mask) return;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    if (a.advance && blockIdx.x == 0 && warp == 0)
+        for (int j = 0; j < NC; ++j)
+            if (mask >> j & 1u) advance_column(a, j, lane);
+    const long long nwarps = (long long)gridDim.x * (kSpmvThreads / 32);
+    for (long long w = (long long)blockIdx.x * (kSpmvThreads / 32) + warp; w * 32 < a.rows; w += nwarps) {
+        const long long li = w * 32 + lane;
+        long long beg = 0, len = 0;
+        if (li < a.rows) {
+            beg = __ldcs(a.rp + li);
+            len = __ldcs(a.rp + li + 1) - beg;
+        }
+        const bool is_long = len > kShortRow;
+        if (li < a.rows && !is_long) {
+            int c[kShortRow];
+            double av[kShortRow];
+#pragma unroll
+            for (int e = 0; e < kShortRow; ++e) {
+                c[e] = 0;
+                av[e] = 0.0;
+                if (e < len) {
+                    c[e] = __ldcs(a.col + beg + e);
+                    av[e] = __ldcs(a.val + beg + e);
+                }
+            }
+#pragma unroll
+            for (int j = 0; j < NC; ++j)
+                if (mask >> j & 1u) a.ap[j * a.slot + li] = row_short_regs(c, av, (int)len, a.v + j * a.ld);
+        }
+        unsigned todo = __ballot_sync(0xffffffffu, is_long);
+        while (todo) {
+            const int src = __ffs(todo) - 1;
+            todo &= todo - 1;
+            const long long b = __shfl_sync(0xffffffffu, beg, src), l = __shfl_sync(0xffffffffu, len, src);
+            double y[NC];
+            row_warp_block<NC>(a.col + b, a.val + b, l, a.v, a.ld, mask, lane, y);
+            if (lane == 0)
+#pragma unroll
+                for (int j = 0; j < NC; ++j)
+                    if (mask >> j & 1u) a.ap[j * a.slot + w * 32 + src] = y[j];
+        }
+    }
+}
+
 // ---- builders ---------------------------------------------------------------------------
 // generate_lap2d_matrix (cg.cc:159-188): the non-zeros of generate_lap2d_kernel, per row in
 // ascending column order: i-1-inc, i-1, i, i+1, i+1+inc; emit(column, value) for each
@@ -284,6 +446,50 @@ cudaError_t launch_spmv(const GemvArgs &a, int sm_count, cudaStream_t s)
     if (blocks > 32LL * sm_count) blocks = 32LL * sm_count;
     if (blocks < 1) blocks = 1;
     return launch_kernel(spmv_csr_kernel, (int)blocks, kSpmvThreads, 0, s, a.pdl != 0, a);
+}
+
+namespace {
+template <int NC> cudaError_t launch_spmv_block_nc(const BlockArgs &a, int sm_count, cudaStream_t s)
+{
+    long long blocks = (a.rows + kSpmvThreads - 1) / kSpmvThreads; // the grid of launch_spmv
+    if (blocks > 32LL * sm_count) blocks = 32LL * sm_count;
+    if (blocks < 1) blocks = 1;
+    return launch_kernel(spmv_csr_block_kernel<NC>, (int)blocks, kSpmvThreads, 0, s, a.pdl != 0, a);
+}
+template <int NC> cudaError_t preload_spmv_block_nc()
+{
+    cudaFuncAttributes fa;
+    return cudaFuncGetAttributes(&fa, spmv_csr_block_kernel<NC>);
+}
+} // namespace
+
+cudaError_t launch_spmv_block(const BlockArgs &a, int sm_count, cudaStream_t s)
+{
+    static_assert(kMaxRhs == 8, "one instantiation per column count");
+    switch (a.nrhs) {
+    case 1: return launch_spmv_block_nc<1>(a, sm_count, s);
+    case 2: return launch_spmv_block_nc<2>(a, sm_count, s);
+    case 3: return launch_spmv_block_nc<3>(a, sm_count, s);
+    case 4: return launch_spmv_block_nc<4>(a, sm_count, s);
+    case 5: return launch_spmv_block_nc<5>(a, sm_count, s);
+    case 6: return launch_spmv_block_nc<6>(a, sm_count, s);
+    case 7: return launch_spmv_block_nc<7>(a, sm_count, s);
+    case 8: return launch_spmv_block_nc<8>(a, sm_count, s);
+    default: return cudaErrorInvalidValue;
+    }
+}
+
+cudaError_t preload_spmv_block_kernels()
+{
+    cudaError_t e;
+    if ((e = preload_spmv_block_nc<1>()) != cudaSuccess) return e;
+    if ((e = preload_spmv_block_nc<2>()) != cudaSuccess) return e;
+    if ((e = preload_spmv_block_nc<3>()) != cudaSuccess) return e;
+    if ((e = preload_spmv_block_nc<4>()) != cudaSuccess) return e;
+    if ((e = preload_spmv_block_nc<5>()) != cudaSuccess) return e;
+    if ((e = preload_spmv_block_nc<6>()) != cudaSuccess) return e;
+    if ((e = preload_spmv_block_nc<7>()) != cudaSuccess) return e;
+    return preload_spmv_block_nc<8>();
 }
 
 cudaError_t csr_generate_lap2d(CsrShard *m, long long n, long long row0, long long rows, cudaStream_t s)

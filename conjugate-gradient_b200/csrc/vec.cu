@@ -245,6 +245,111 @@ __global__ void __launch_bounds__(kChunk) update_p_once_kernel(const VecArgs a)
     if (i < a.n) a.p[i] = __fma_rn(beta, a.p[i], a.r[i]);                         // cg.cc:127-129
 }
 
+// ---- block solve: the kernels above per column (blockIdx.y = column j) ---------------------------
+// Same chunks, same last-block reductions, same FMAs as the CSR single solve; column j has its own
+// State and arrival counters, and a column that is done returns like a single solve after its break.
+__global__ void __launch_bounds__(kChunk) init_residual_block_kernel(const BlockArgs a)
+{
+    __shared__ double wsum[8];
+    const int tid = threadIdx.x, j = blockIdx.y;
+    const long long i = (long long)blockIdx.x * kChunk + tid, o = j * a.ld + i;
+    double v = 0.0;
+    if (i < a.n) {
+        const double rr = __fma_rn(-1.0, a.ap[j * a.slot + i], a.b[o]); // cg.cc:82
+        a.r[o] = rr;
+        a.p[o] = rr;                                                    // cg.cc:85
+        v = __dmul_rn(rr, rr);                                          // cg.cc:91
+    }
+    const double t = block_chunk256(v, wsum, tid);
+    if (tid == 0) a.rrpart[j * a.nchunks + blockIdx.x] = t;
+}
+
+__global__ void __launch_bounds__(kChunk) pap_alpha_block_kernel(const BlockArgs a)
+{
+    __shared__ double wsum[8];
+    const int tid = threadIdx.x, j = blockIdx.y;
+    griddep_launch_dependents();
+    griddep_wait();
+    State *st = a.st + j;
+    if (st->done) return;
+    const long long i = (long long)blockIdx.x * kChunk + tid;
+    const double v = (i < a.n) ? __dmul_rn(a.p[j * a.ld + i], a.ap[j * a.slot + i]) : 0.0;
+    const double t = block_chunk256(v, wsum, tid);
+    double *part = a.papart + j * a.nchunks;
+    if (!publish_partial(part, t, &a.arrive[2 * j], tid)) return;
+    const double conj = warp_det_sum_l2(part, gridDim.x, tid);        // p'Ap     cg.cc:105-106
+    if (tid == 0) {
+        const double rsold = st->rsold;
+        const double clamp = __dmul_rn(rsold, kNearZero);
+        st->conj = conj;
+        st->alpha = __ddiv_rn(rsold, (conj < clamp) ? clamp : conj);   // cg.cc:107
+        a.arrive[2 * j] = 0;
+    }
+}
+
+__global__ void __launch_bounds__(kChunk) update_xr_block_kernel(const BlockArgs a)
+{
+    __shared__ double wsum[8];
+    const int tid = threadIdx.x, j = blockIdx.y;
+    griddep_launch_dependents();
+    griddep_wait();
+    State *st = a.st + j;
+    if (st->done) return;
+    const double alpha = st->alpha;
+    const long long i = (long long)blockIdx.x * kChunk + tid, o = j * a.ld + i;
+    double v = 0.0;
+    if (i < a.n) {
+        const double pi = a.p[o];
+        a.x[o] = __fma_rn(alpha, pi, a.x[o]);                                   // cg.cc:110
+        const double rn = __fma_rn(-alpha, a.ap[j * a.slot + i], a.r[o]);       // cg.cc:113
+        a.r[o] = rn;
+        v = __dmul_rn(rn, rn);                                                  // cg.cc:116
+    }
+    const double t = block_chunk256(v, wsum, tid);
+    double *part = a.rrpart + j * a.nchunks;
+    if (!publish_partial(part, t, &a.arrive[2 * j + 1], tid)) return;
+    const double rsnew = warp_det_sum_l2(part, gridDim.x, tid);        // cg.cc:116-117
+    if (tid == 0) {
+        st->rsnew = rsnew;
+        if (sqrt(rsnew) < a.tol) {                                      // cg.cc:120-121
+            if (a.hist) a.hist[j * a.hist_ld + st->iter] = rsnew;
+            st->done = 1;
+            // the last column to converge tells the host that every later launch is a no-op
+            if (atomicAdd(a.ndone, 1u) == (unsigned)a.nrhs - 1u && a.host_done) *a.host_done = 1;
+            __threadfence_system();
+        }
+        a.arrive[2 * j + 1] = 0;
+    }
+}
+
+__global__ void __launch_bounds__(kChunk) update_p_block_kernel(const BlockArgs a)
+{
+    const int j = blockIdx.y;
+    griddep_launch_dependents();
+    griddep_wait();
+    const State *st = a.st + j;
+    if (st->done) return;
+    const double beta = __ddiv_rn(st->rsnew, st->rsold);                          // cg.cc:124
+    const long long i = (long long)blockIdx.x * kChunk + threadIdx.x, o = j * a.ld + i;
+    if (i < a.n) a.p[o] = __fma_rn(beta, a.p[o], a.r[o]);                         // cg.cc:127-129
+}
+
+// one warp per column
+__global__ void __launch_bounds__(32) finalize_block_kernel(const BlockArgs a)
+{
+    const int j = blockIdx.x, lane = threadIdx.x;
+    State *st = a.st + j;
+    if (st->done) return;
+    const double s = warp_det_sum(a.rrpart + j * a.nchunks, a.nchunks, lane);
+    if (lane == 0) {
+        const long long it = st->iter;
+        if (it >= 0 && a.hist) a.hist[j * a.hist_ld + it] = s;
+        st->rsold = s; // cg.cc:132
+        st->rsnew = s;
+        st->iter = it + 1;
+    }
+}
+
 __global__ void __launch_bounds__(32) finalize_kernel(const VecArgs a, long long nchunks)
 {
     if (a.st->done) return;
@@ -531,6 +636,44 @@ cudaError_t launch_update_xr_once(const VecArgs &a, cudaStream_t s)
 cudaError_t launch_update_p_once(const VecArgs &a, cudaStream_t s)
 {
     return launch_kernel(update_p_once_kernel, grid_for(a.n), kChunk, 0, s, a.pdl != 0, a);
+}
+
+cudaError_t preload_vec_block_kernels()
+{
+    cudaFuncAttributes fa;
+    cudaError_t e;
+    if ((e = cudaFuncGetAttributes(&fa, init_residual_block_kernel)) != cudaSuccess) return e;
+    if ((e = cudaFuncGetAttributes(&fa, pap_alpha_block_kernel)) != cudaSuccess) return e;
+    if ((e = cudaFuncGetAttributes(&fa, update_xr_block_kernel)) != cudaSuccess) return e;
+    if ((e = cudaFuncGetAttributes(&fa, update_p_block_kernel)) != cudaSuccess) return e;
+    return cudaFuncGetAttributes(&fa, finalize_block_kernel);
+}
+
+cudaError_t launch_init_residual_block(const BlockArgs &a, cudaStream_t s)
+{
+    init_residual_block_kernel<<<dim3((unsigned)a.nchunks, (unsigned)a.nrhs), kChunk, 0, s>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_pap_alpha_block(const BlockArgs &a, cudaStream_t s)
+{
+    return launch_kernel_xy(pap_alpha_block_kernel, dim3((unsigned)a.nchunks, (unsigned)a.nrhs), kChunk, s, a.pdl != 0, a);
+}
+
+cudaError_t launch_update_xr_block(const BlockArgs &a, cudaStream_t s)
+{
+    return launch_kernel_xy(update_xr_block_kernel, dim3((unsigned)a.nchunks, (unsigned)a.nrhs), kChunk, s, a.pdl != 0, a);
+}
+
+cudaError_t launch_update_p_block(const BlockArgs &a, cudaStream_t s)
+{
+    return launch_kernel_xy(update_p_block_kernel, dim3((unsigned)a.nchunks, (unsigned)a.nrhs), kChunk, s, a.pdl != 0, a);
+}
+
+cudaError_t launch_finalize_block(const BlockArgs &a, cudaStream_t s)
+{
+    finalize_block_kernel<<<a.nrhs, 32, 0, s>>>(a);
+    return cudaGetLastError();
 }
 
 cudaError_t launch_finalize(const VecArgs &a, cudaStream_t s)

@@ -133,7 +133,7 @@ int cgb_set_rhs(cgb_ctx *ctx, const double *b_host);
  * column-tile width of the mat-vec; "graph": 0/1 CUDA-graph replay of the iteration;
  * "poll_every" / "graph_unroll": graph schedule only -- iterations between two looks at the stop flag and
  * iterations per graph (the instantiated graph holds min of the two; "graph_replays", read-only,
- * counts its launches);
+ * counts its launches, and those of the block solve's graph);
  * "pdl": 0/1 programmatic dependent launch between the kernels of the iteration (the next
  * mat-vec prefetches A while the vector updates still run); "l2_prefetch": pipeline steps of A
  * the mat-vec additionally pulls into L2 before that wait (0 = off); "l2_ramp": persistent
@@ -209,6 +209,38 @@ int cgb_solve_begin(cgb_ctx *ctx, const double *x0_host, int64_t max_iter, doubl
                     int keep_history);
 int cgb_iterate(cgb_ctx *ctx, int64_t iters, float *ms);
 int cgb_solve_end(cgb_ctx *ctx, double *x_host, double *resid_hist, cgb_solve_info *info);
+
+/* ---- block solve: up to CGB_MAX_RHS right-hand sides against one matrix ------------------
+ * Column j of a block solve is, bit for bit, a single solve of A x = b_j from x0_j with the same
+ * max_iter and tol: k, converged, rsold, rsnew, the r'r history and x.  The columns share every
+ * read of the matrix (each row's CSR entries are loaded once per iteration for all of them) and
+ * every launch, but no arithmetic.  A column that converges is frozen -- its x, r, p, scalars and
+ * history stop changing -- while the others go on; the loop ends when every column has converged
+ * or after max_iter loop bodies.
+ * Layout: column j of b_host, x0_host and x_host is n contiguous doubles at offset j * n;
+ * x0_host == NULL means zeros.  resid_hist (nullable) holds nrhs * max_iter doubles, column j's
+ * r'r history at j * max_iter, filled like cgb_solve's for that column.  info is an array of
+ * nrhs entries; `seconds` is the loop time all columns share.
+ * Needs a CSR context of world == 1 with its matrix set (no cgb_set_rhs: the right-hand sides are
+ * arguments).  CGB_ERR_STATE for a dense context (the tile pipeline of the dense mat-vec carries
+ * one p), for world > 1 (the exchange carries one vector per row), before the matrix is set, and
+ * while a single solve is in progress -- as cgb_solve_begin is refused during a block solve.
+ * CGB_ERR_INVALID for nrhs outside [1, CGB_MAX_RHS] or a null b_host / x_host.
+ * cgb_solve_block, like cgb_solve, takes the x0 columns in x_host and returns the solutions there.
+ * Begin / iterate / end work as for the single solve; cgb_iterate advances whichever solve is in
+ * progress and stops issuing launches once every column has converged.  The block solve has its
+ * own device buffers (allocated on a context's first block solve, grown for a larger nrhs, freed
+ * by cgb_destroy) and its own CUDA graph: it leaves the single solve's x, r, p, b, state, history
+ * and graph untouched, so cgb_residual_check still reports the last single solve.
+ * Options: "graph", "pdl", "poll_every" and "graph_unroll" apply as to a CSR single solve;
+ * "profile" does not apply (the block loop runs as if it were 0), and cgb_last_gemv_timing keeps
+ * describing single solves.  Block launches count in cgb_launch_count. */
+#define CGB_MAX_RHS 8
+int cgb_solve_block_begin(cgb_ctx *ctx, int nrhs, const double *b_host, const double *x0_host,
+                          int64_t max_iter, double tol, int keep_history);
+int cgb_solve_block_end(cgb_ctx *ctx, double *x_host, double *resid_hist, cgb_solve_info *info);
+int cgb_solve_block(cgb_ctx *ctx, int nrhs, const double *b_host, double *x_host, int64_t max_iter,
+                    double tol, double *resid_hist, cgb_solve_info *info);
 
 /* The DEBUG block at the end of solve (cg.cc:144-154, cg.cu:272-296): ||x|| and
  * ||A x - b|| / ||b|| for the x held on the device after a solve. */
