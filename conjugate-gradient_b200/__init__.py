@@ -8,8 +8,8 @@ tests and bench.py; it never computes anything itself and has no CPU fallback.
 The directory name contains a hyphen, so import it with
     importlib.import_module("conjugate-gradient_b200")
 """
-from ._capi import (CgbError, Context, Layout, SolveInfo, SIGNATURES, LIB_PATH, UNIQUE_ID_BYTES, EXCHANGE_BLOB_BYTES,
+from ._capi import (CgbError, Context, DeviceSolve, Layout, SolveInfo, SIGNATURES, LIB_PATH, UNIQUE_ID_BYTES, EXCHANGE_BLOB_BYTES,
                     device_count, gemv_variants, init_source_term, load, partition, unique_id)
 
-__all__ = ["CgbError", "Context", "Layout", "SolveInfo", "SIGNATURES", "LIB_PATH",
+__all__ = ["CgbError", "Context", "DeviceSolve", "Layout", "SolveInfo", "SIGNATURES", "LIB_PATH",
            "UNIQUE_ID_BYTES", "EXCHANGE_BLOB_BYTES", "device_count", "gemv_variants", "init_source_term", "load", "partition", "unique_id"]

@@ -70,6 +70,10 @@ SIGNATURES = [
     ("cgb_solve_block_begin", C.c_int, [_CTX, C.c_int, _dp, _dp, C.c_int64, C.c_double, C.c_int]),
     ("cgb_solve_block_end", C.c_int, [_CTX, _dp, _dp, C.POINTER(SolveInfo)]),
     ("cgb_solve_block", C.c_int, [_CTX, C.c_int, _dp, _dp, C.c_int64, C.c_double, _dp, C.POINTER(SolveInfo)]),
+    ("cgb_solve_device", C.c_int, [_CTX, C.c_void_p, C.c_void_p, C.c_int64, C.c_double, C.c_void_p, C.c_void_p,
+                                   C.c_void_p]),
+    ("cgb_solve_block_device", C.c_int, [_CTX, C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_double, C.c_void_p,
+                                         C.c_void_p, C.c_void_p]),
     ("cgb_residual_check", C.c_int, [_CTX, _dp, _dp]),
     ("cgb_gemv", C.c_int, [_CTX, _dp, _dp, _dp, _dp]),
     ("cgb_dot", C.c_int, [_CTX, _dp, _dp, _dp]),
@@ -141,6 +145,32 @@ def unique_id() -> bytes:
 def gemv_variants():
     lib = load()
     return [lib.cgb_gemv_variant_name(i).decode() for i in range(lib.cgb_gemv_variant_count())]
+
+
+class DeviceSolve:
+    """A solve enqueued by Context.solve_device / solve_block_device.  The caller's x (X) tensor
+    receives the solution when `stream` gets there; result() waits for that and decodes the device
+    info (and history) the way the host methods return them."""
+
+    def __init__(self, stream, info, hist, nrhs, block, keep):
+        self.stream = stream
+        self.info = info        # device tensor: nrhs cgb_solve_info records (uint8)
+        self.hist = hist        # device tensor (nrhs, max(max_iter, 1)) or None
+        self._nrhs, self._block = nrhs, block
+        self._keep = keep       # the caller's tensors stay alive until result()
+
+    def result(self):
+        """single: (SolveInfo, hist or None); block: (list of SolveInfo, list of histories or None)"""
+        self.stream.synchronize()
+        infos = list((SolveInfo * self._nrhs).from_buffer_copy(self.info.cpu().numpy().tobytes()))
+        hist = None
+        if self.hist is not None:
+            h = self.hist.cpu().numpy()
+            hist = [h[j, :infos[j].iterations].copy() for j in range(self._nrhs)]
+        self._keep = None
+        if self._block:
+            return infos, hist
+        return infos[0], (hist[0] if hist is not None else None)
 
 
 class Context:
@@ -301,6 +331,43 @@ class Context:
     @staticmethod
     def _block_hist(hist, infos):
         return None if hist is None else [hist[j, :infos[j].iterations].copy() for j in range(len(infos))]
+
+    # -- device solves: CUDA tensors in and out, ordered on a torch stream, no host round trip
+    def _device_args(self, tensors, stream):
+        import torch
+        dev = self.layout().device
+        for nm, t in tensors:
+            if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float64 and t.is_contiguous()):
+                raise TypeError(f"{nm} must be a contiguous float64 CUDA tensor")
+            if t.device.index != dev:
+                raise ValueError(f"{nm} is on cuda:{t.device.index}, the context on cuda:{dev}")
+        stream = torch.cuda.current_stream(dev) if stream is None else stream
+        return torch, dev, stream
+
+    def solve_device(self, x, b, max_iter: int, tol: float = 1e-10, history: bool = False, stream=None):
+        """cgb_solve_device: x (x0 in, the solution out) and b are (n,) float64 CUDA tensors; the solve
+        is enqueued on `stream` (default: the current torch stream) and the call returns at once."""
+        torch, dev, stream = self._device_args([("x", x), ("b", b)], stream)
+        assert x.numel() == self.n and b.numel() == self.n
+        info = torch.zeros(C.sizeof(SolveInfo), dtype=torch.uint8, device=f"cuda:{dev}")
+        hist = torch.zeros((1, max(max_iter, 1)), dtype=torch.float64, device=f"cuda:{dev}") if history else None
+        _check(self._lib.cgb_solve_device(self._h, b.data_ptr(), x.data_ptr(), max_iter, tol,
+                                          hist.data_ptr() if history else None, info.data_ptr(),
+                                          stream.cuda_stream))
+        return DeviceSolve(stream, info, hist, 1, False, (x, b))
+
+    def solve_block_device(self, X, B, max_iter: int = 0, tol: float = 1e-10, history: bool = False, stream=None):
+        """cgb_solve_block_device: X (X0 in, the solutions out) and B are (nrhs, n) float64 CUDA tensors."""
+        torch, dev, stream = self._device_args([("X", X), ("B", B)], stream)
+        assert B.ndim == 2 and B.shape[1] == self.n and X.shape == B.shape, "B and X must be (nrhs, n)"
+        nrhs = B.shape[0]
+        info = torch.zeros(max(nrhs, 1) * C.sizeof(SolveInfo), dtype=torch.uint8, device=f"cuda:{dev}")
+        hist = torch.zeros((max(nrhs, 1), max(max_iter, 1)), dtype=torch.float64, device=f"cuda:{dev}") \
+            if history else None
+        _check(self._lib.cgb_solve_block_device(self._h, nrhs, B.data_ptr(), X.data_ptr(), max_iter, tol,
+                                                hist.data_ptr() if history else None, info.data_ptr(),
+                                                stream.cuda_stream))
+        return DeviceSolve(stream, info, hist, nrhs, True, (X, B))
 
     def residual_check(self):
         nx, rr = C.c_double(), C.c_double()

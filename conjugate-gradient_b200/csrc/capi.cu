@@ -110,6 +110,22 @@ int load_nccl()
 // Block solve (cgb_solve_block_begin): its own buffers, States, flag and graph, allocated on the
 // first block solve and never shared with the single solve.
 static_assert(kMaxRhs == CGB_MAX_RHS, "one limit of columns");
+
+// The loop of a device solve on the graph schedule (cgb_solve_device, cgb_solve_block_device): one
+// CUDA graph whose WHILE nodes run the loop bodies until the stop test fires or max_iter is reached.
+// Keyed like the host graphs, plus `gen` (drop_graph / drop_block_graph calls since creation) and the
+// matrix arrays it reads.
+struct DeviceLoop {
+    cudaGraph_t graph = nullptr;
+    cudaGraphExec_t exec = nullptr;
+    int len = 0, nrhs = 0, pdl = 0;
+    int pdl_used = -1;              // 1: the bodies keep the programmatic dependent launches, 0: they do not
+    double tol = 0.0;
+    const double *hist = nullptr;
+    long long gen = -1;
+    const void *mat0 = nullptr, *mat1 = nullptr;
+};
+
 struct BlockSolve {
     int cap = 0;                    // columns the vector buffers hold
     int nrhs = 0;                   // columns of the solve in progress
@@ -130,6 +146,8 @@ struct BlockSolve {
     bool active = false, keep_history = false;
     long long max_iter = 0, launched = 0;
     double tol = 0.0, loop_ms = 0.0;
+    long long gen = 0;              // drop_block_graph calls: the buffers the block graphs bake in may have moved
+    DeviceLoop dloop;               // cgb_solve_block_device's graph
 };
 
 struct cgb_ctx {
@@ -196,6 +214,16 @@ struct cgb_ctx {
     double prof_gemv_ms = 0.0;
     long long prof_gemv_n = 0;
     BlockSolve blk;
+
+    // device solves (cgb_solve_device, cgb_solve_block_device); allocated on the first one
+    long long graph_gen = 0;       // drop_graph calls: what the graphs of the single solve bake in has changed
+    DeviceLoop dloop;              // cgb_solve_device's graph
+    LoopCtl *loopctl = nullptr;    // the loop's body limit, bodies issued, start stamp
+    double *dev_hist = nullptr;    // cgb_solve_device's r'r history (the host solve's `hist` stays its own)
+    long long dev_hist_cap = 0;
+    cudaEvent_t ev_dev[2] = {nullptr, nullptr}; // caller's stream -> ctx stream, and back
+    bool device_loop = false;      // kernels being enqueued belong to a device solve (see DeviceLaunch)
+    double *dloop_hist = nullptr;  // ... and write this history (nullable)
 };
 
 namespace {
@@ -270,7 +298,7 @@ GemvArgs make_gemv_args(const cgb_ctx *c, const double *v, int advance)
     a.st = c->st;
     a.rrpart = c->rrpart;
     a.nchunks = c->nchunks;
-    a.hist = c->hist;
+    a.hist = c->device_loop ? c->dloop_hist : c->hist;
     a.advance = advance;
     a.pdl = (advance && c->opt_pdl && !c->opt_profile) ? 1 : 0; // only inside the CG loop
     a.l2_prefetch = a.pdl ? c->opt_l2_prefetch : 0;
@@ -292,8 +320,8 @@ VecArgs make_vec_args(const cgb_ctx *c)
     a.rrpart = c->rrpart;
     a.papart = c->papart;
     a.st = c->st;
-    a.host_done = c->d_hdone;
-    a.hist = c->hist;
+    a.host_done = c->device_loop ? nullptr : c->d_hdone;
+    a.hist = c->device_loop ? c->dloop_hist : c->hist;
     a.g = make_gather(c);
     a.n = c->n;
     a.tol = c->tol;
@@ -331,6 +359,15 @@ void drop_graph(cgb_ctx *c)
     if (c->graph) cudaGraphDestroy(c->graph);
     c->graph_exec = nullptr;
     c->graph = nullptr;
+    c->graph_gen += 1; // cgb_solve_device's graph bakes in the same arguments
+}
+
+void drop_loop(DeviceLoop &d)
+{
+    if (d.exec) cudaGraphExecDestroy(d.exec);
+    if (d.graph) cudaGraphDestroy(d.graph);
+    d.exec = nullptr;
+    d.graph = nullptr;
 }
 
 // the mat-vec and, for world > 1, the gather of its result
@@ -464,8 +501,8 @@ int launch_persist(cgb_ctx *c, long long iters)
     a.sync = c->psync;
     a.st = c->st;
     a.ctl = c->ctl;
-    a.hist = c->hist;
-    a.host_done = c->d_hdone;
+    a.hist = c->device_loop ? c->dloop_hist : c->hist;
+    a.host_done = c->device_loop ? nullptr : c->d_hdone;
     a.ld = c->ld;
     a.rows = c->rows;
     a.row0 = c->row0;
@@ -526,6 +563,7 @@ void drop_block_graph(cgb_ctx *c)
     if (k.graph) cudaGraphDestroy(k.graph);
     k.graph_exec = nullptr;
     k.graph = nullptr;
+    k.gen += 1; // and so does cgb_solve_block_device's
 }
 
 void free_block_vectors(cgb_ctx *c)
@@ -546,6 +584,7 @@ void free_block(cgb_ctx *c)
 {
     BlockSolve &k = c->blk;
     drop_block_graph(c);
+    drop_loop(k.dloop);
     free_block_vectors(c);
     if (k.hist) cudaFree(k.hist);
     k.hist = nullptr;
@@ -624,7 +663,7 @@ BlockArgs make_block_args(const cgb_ctx *c, const double *v, int advance)
     a.st = k.st;
     a.arrive = k.arrive;
     a.ndone = k.arrive + 2 * k.cap;
-    a.host_done = k.d_hdone;
+    a.host_done = c->device_loop ? nullptr : k.d_hdone;
     a.hist = k.keep_history ? k.hist : nullptr;
     a.n = c->n;
     a.ld = c->ld;
@@ -724,6 +763,170 @@ int block_iterate(cgb_ctx *c, int64_t iters, float *ms)
     k.launched += issued;
     if (ms) *ms = t;
     return CGB_OK;
+}
+
+// ---- device solves -------------------------------------------------------------------------
+// While a device solve enqueues its kernels: "profile" reads 0 (as for a block solve), no kernel
+// raises the mapped host flag (nobody polls it, and a host solve queued behind this one resets it from
+// the host), and the history goes to the device solve's own buffer.
+struct DeviceLaunch {
+    cgb_ctx *c;
+    int keep_profile, keep_pdl;
+    DeviceLaunch(cgb_ctx *c_, double *hist) : c(c_), keep_profile(c_->opt_profile), keep_pdl(c_->opt_pdl)
+    {
+        c->opt_profile = 0;
+        c->device_loop = true;
+        c->dloop_hist = hist;
+    }
+    ~DeviceLaunch()
+    {
+        c->opt_profile = keep_profile;
+        c->opt_pdl = keep_pdl;
+        c->device_loop = false;
+        c->dloop_hist = nullptr;
+    }
+};
+
+// Pointers a device solve takes: device memory of the context's GPU (or managed memory)
+int check_device_ptr(const cgb_ctx *c, const void *p, const char *what)
+{
+    if (!p) return fail(CGB_ERR_INVALID, "null %s", what);
+    cudaPointerAttributes a;
+    cudaError_t e = cudaPointerGetAttributes(&a, p);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(CGB_ERR_INVALID, "%s is not a pointer CUDA knows (%s)", what, cudaGetErrorString(e));
+    }
+    if (a.type == cudaMemoryTypeManaged) return CGB_OK;
+    if (a.type != cudaMemoryTypeDevice)
+        return fail(CGB_ERR_INVALID, "%s is host memory: a device solve takes device pointers", what);
+    if (a.device != c->device)
+        return fail(CGB_ERR_INVALID, "%s lives on device %d, the context on device %d", what, a.device, c->device);
+    return CGB_OK;
+}
+
+// what a context's first device solve allocates
+int prepare_device_solve(cgb_ctx *c)
+{
+    if (c->loopctl) return CGB_OK;
+    CK(preload_loop_kernels());
+    for (cudaEvent_t &e : c->ev_dev)
+        if (!e) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    CK(cudaMalloc(&c->loopctl, sizeof(LoopCtl)));
+    CK(cudaMemsetAsync(c->loopctl, 0, sizeof(LoopCtl), c->stream));
+    return CGB_OK;
+}
+
+// Captures into `g` the launches `enqueue` makes on c->stream, after the node `dep` (nullable);
+// *tail = the last node captured.  The capture always ends, whatever fails.
+template <class F>
+int capture_into(cgb_ctx *c, cudaGraph_t g, cudaGraphNode_t dep, F enqueue, cudaGraphNode_t *tail)
+{
+    CK(cudaStreamBeginCaptureToGraph(c->stream, g, dep ? &dep : nullptr, nullptr, dep ? 1 : 0,
+                                     cudaStreamCaptureModeThreadLocal));
+    int rc = enqueue();
+    if (rc == CGB_OK && tail) {
+        cudaStreamCaptureStatus cs;
+        const cudaGraphNode_t *deps = nullptr;
+        size_t nd = 0;
+        cudaError_t e = cudaStreamGetCaptureInfo(c->stream, &cs, nullptr, nullptr, &deps, &nd);
+        if (e != cudaSuccess) rc = fail(CGB_ERR_CUDA, "cudaStreamGetCaptureInfo: %s", cudaGetErrorString(e));
+        else if (nd != 1) rc = fail(CGB_ERR_CUDA, "a captured loop control kernel left %zu tail nodes", nd);
+        else *tail = deps[0];
+    }
+    cudaGraph_t out = nullptr;
+    cudaError_t e = cudaStreamEndCapture(c->stream, &out);
+    if (rc) return rc;
+    CK(e);
+    return CGB_OK;
+}
+
+// The loop of a device solve as one graph (DESIGN 3.9):
+//   head -> WHILE { len loop bodies ; ctl } -> mid -> WHILE { 1 loop body ; ctl }
+// head, mid and ctl are loop_ctl_kernel: each sets the condition of the WHILE node it precedes or
+// runs in -- the stop test has not fired and the bodies issued so far leave room for the next
+// body under max_iter.  So no loop body starts past max_iter, and the count of bodies issued is the
+// host loop's (whole graphs of `len`, then single iterations), short of the no-op bodies the host
+// issues after the stop test fired.  `body` enqueues one loop body on c->stream.
+int build_loop(cgb_ctx *c, DeviceLoop &d, int len, const int *done, const unsigned int *ndone, int nrhs,
+               int (*body)(cgb_ctx *))
+{
+    drop_loop(d);
+    CK(cudaGraphCreate(&d.graph, 0));
+    const long long before = c->kernel_launches;
+    int rc = CGB_OK;
+    cudaGraphNode_t tail = nullptr;
+    for (int part = 0; part < 2 && rc == CGB_OK; ++part) {
+        const int step = part == 0 ? len : 1;
+        cudaGraphConditionalHandle h;
+        CK(cudaGraphConditionalHandleCreate(&h, d.graph, 0, cudaGraphCondAssignDefault));
+        cudaGraphNode_t ctl = nullptr;
+        rc = capture_into(c, d.graph, tail, [&]() -> int {
+            CK(launch_loop_ctl(c->loopctl, done, ndone, nrhs, h, 1, step, 0, part == 0 ? 1 : 0, c->stream));
+            return CGB_OK;
+        }, &ctl);
+        if (rc) break;
+        cudaGraphNodeParams p = {cudaGraphNodeTypeConditional};
+        p.conditional.handle = h;
+        p.conditional.type = cudaGraphCondTypeWhile;
+        p.conditional.size = 1;
+        CK(cudaGraphAddNode(&tail, d.graph, &ctl, 1, &p));
+        rc = capture_into(c, p.conditional.phGraph_out[0], nullptr, [&]() -> int {
+            int r = CGB_OK;
+            for (int u = 0; u < step && r == CGB_OK; ++u) r = body(c);
+            if (r == CGB_OK) CK(launch_loop_ctl(c->loopctl, done, ndone, nrhs, h, 1, step, step, 0, c->stream));
+            return r;
+        }, nullptr);
+    }
+    c->kernel_launches = before; // capture launches nothing
+    if (rc) return rc;
+    CK(cudaGraphInstantiate(&d.exec, d.graph, 0));
+    d.len = len;
+    d.pdl = c->opt_pdl;
+    return CGB_OK;
+}
+
+// The cached loop graph when its key still holds, else a new one.  The bodies are captured with
+// programmatic dependent launches when "pdl" asks for them; should the driver refuse them inside a
+// conditional body, they are captured without (DeviceLoop::pdl_used, option "device_loop_pdl").
+int ensure_loop(cgb_ctx *c, DeviceLoop &d, int len, int nrhs, double tol, const double *hist, long long gen,
+                const int *done, const unsigned int *ndone, int (*body)(cgb_ctx *))
+{
+    const void *m0 = c->storage == 1 ? (const void *)c->csr.col : (const void *)c->A;
+    const void *m1 = c->storage == 1 ? (const void *)c->csr.val : (const void *)c->env;
+    if (d.exec && d.len == len && d.nrhs == nrhs && d.tol == tol && d.hist == hist && d.gen == gen &&
+        d.pdl == c->opt_pdl && d.mat0 == m0 && d.mat1 == m1)
+        return CGB_OK;
+    const int want_pdl = c->opt_pdl;
+    int rc = build_loop(c, d, len, done, ndone, nrhs, body);
+    d.pdl_used = want_pdl;
+    if (rc && want_pdl) {
+        cudaGetLastError();
+        c->opt_pdl = 0; // DeviceLaunch restores it
+        rc = build_loop(c, d, len, done, ndone, nrhs, body);
+        d.pdl_used = 0;
+    }
+    if (rc) {
+        drop_loop(d);
+        return rc;
+    }
+    d.pdl = want_pdl;
+    d.nrhs = nrhs;
+    d.tol = tol;
+    d.hist = hist;
+    d.gen = gen;
+    d.mat0 = m0;
+    d.mat1 = m1;
+    return CGB_OK;
+}
+
+int single_body(cgb_ctx *c) { return launch_iteration(c); }
+int block_body(cgb_ctx *c) { return launch_block_iteration(c); }
+
+// kernels of the loop graph when it runs to max_iter (the host does not learn where it stops)
+long long loop_kernels(long long max_iter, int len, int per_body)
+{
+    return per_body * max_iter + 2 + max_iter / len + max_iter % len;
 }
 
 } // namespace
@@ -924,6 +1127,11 @@ extern "C" int cgb_destroy(cgb_ctx *c)
     if (c->h_done) cudaFreeHost(c->h_done);
     if (c->h_pin) cudaFreeHost(c->h_pin);
     free_block(c);
+    drop_loop(c->dloop);
+    if (c->loopctl) cudaFree(c->loopctl);
+    if (c->dev_hist) cudaFree(c->dev_hist);
+    for (cudaEvent_t e : c->ev_dev)
+        if (e) cudaEventDestroy(e);
     if (c->ev0) cudaEventDestroy(c->ev0);
     if (c->ev1) cudaEventDestroy(c->ev1);
     for (cudaEvent_t e : c->ev_batch)
@@ -1342,6 +1550,7 @@ extern "C" int cgb_get_option(cgb_ctx *c, const char *key, int64_t *value)
     else if (k == "poll_every") *value = c->poll_every;
     else if (k == "graph_unroll") *value = c->graph_unroll;
     else if (k == "graph_replays") *value = c->graph_replays;
+    else if (k == "device_loop_pdl") *value = c->dloop.pdl_used >= 0 ? c->dloop.pdl_used : c->blk.dloop.pdl_used;
     else if (k == "compat") *value = c->opt_compat;
     else if (k == "pdl") *value = c->opt_pdl;
     else if (k == "l2_prefetch") *value = c->opt_l2_prefetch;
@@ -1708,6 +1917,143 @@ extern "C" int cgb_solve_block(cgb_ctx *c, int nrhs, const double *b_host, doubl
         return rc;
     }
     return cgb_solve_block_end(c, x_host, resid_hist, info);
+}
+
+// ------------------------------------------------------------------ device solves
+// Refusals every device solve shares
+static int device_solve_state(cgb_ctx *c)
+{
+    if (c->world > 1)
+        return fail(CGB_ERR_STATE, "device solves run on one rank: the exchange of a world > 1 needs the host in lockstep");
+    if (c->in_solve)
+        return fail(CGB_ERR_STATE, c->blk.active ? "a block solve is in progress" : "a single solve is in progress");
+    if (!c->matrix_set) return fail(CGB_ERR_STATE, "matrix not set");
+    return CGB_OK;
+}
+
+// caller's stream -> context stream: the solve sees everything enqueued on `us` before the call
+static int device_solve_enter(cgb_ctx *c, cudaStream_t us)
+{
+    CK(cudaEventRecord(c->ev_dev[0], us));
+    CK(cudaStreamWaitEvent(c->stream, c->ev_dev[0], 0));
+    return CGB_OK;
+}
+
+// ... and back: work enqueued on `us` after the call sees x, the history and the info
+static int device_solve_leave(cgb_ctx *c, cudaStream_t us)
+{
+    CK(cudaEventRecord(c->ev_dev[1], c->stream));
+    CK(cudaStreamWaitEvent(us, c->ev_dev[1], 0));
+    return CGB_OK;
+}
+
+extern "C" int cgb_solve_device(cgb_ctx *c, const double *b_dev, double *x_dev, int64_t max_iter, double tol,
+                                double *hist_dev, cgb_solve_info *info_dev, void *stream)
+{
+    if (!c) return null_context();
+    int rc = use_device(c);
+    if (rc) return rc;
+    if ((rc = device_solve_state(c))) return rc;
+    if (max_iter < 0) return fail(CGB_ERR_INVALID, "max_iter < 0");
+    if ((rc = check_device_ptr(c, b_dev, "b")) || (rc = check_device_ptr(c, x_dev, "x")) ||
+        (rc = check_device_ptr(c, info_dev, "info")) || (hist_dev && (rc = check_device_ptr(c, hist_dev, "history"))))
+        return rc;
+    if ((rc = prepare_device_solve(c))) return rc;
+    const long long hist_need = max_iter > 0 ? max_iter : 1;
+    if (hist_dev && hist_need > c->dev_hist_cap) { // grows only; the loop graph is keyed on the pointer
+        CK(cudaStreamSynchronize(c->stream));
+        if (c->dev_hist) cudaFree(c->dev_hist);
+        c->dev_hist = nullptr;
+        c->dev_hist_cap = 0;
+        CK(cudaMalloc(&c->dev_hist, (size_t)hist_need * sizeof(double)));
+        c->dev_hist_cap = hist_need;
+    }
+    const cudaStream_t us = static_cast<cudaStream_t>(stream);
+    DeviceLaunch guard(c, hist_dev ? c->dev_hist : nullptr);
+    c->tol = tol;
+    const size_t bytes = (size_t)c->n * 8;
+    if ((rc = device_solve_enter(c, us))) return rc;
+    // cgb_set_rhs + cgb_solve_begin, stream-ordered: b, x0, State; r = b - A x0 ; p = r ; rsold = r.p
+    CK(cudaMemcpyAsync(c->b, b_dev, bytes, cudaMemcpyDeviceToDevice, c->stream));
+    CK(cudaMemcpyAsync(c->x, x_dev, bytes, cudaMemcpyDeviceToDevice, c->stream));
+    CK(launch_device_begin(c->st, 1, c->loopctl, max_iter, c->stream));
+    c->kernel_launches += 1;
+    if ((rc = launch_matvec(c, c->x, 0, c->variant))) return rc;
+    CK(launch_init_residual(make_vec_args(c), c->stream));
+    c->kernel_launches += 1;
+    if (c->opt_schedule == 1 && !persist_unusable(c)) {
+        // cgb_iterate's persistent launch: it leaves the loop on convergence by itself
+        if (max_iter > 0) {
+            CK(launch_loop_ctl(c->loopctl, nullptr, nullptr, 0, 0, 0, 1, 0, 1, c->stream)); // start stamp
+            c->kernel_launches += 1;
+        }
+        for (long long todo = max_iter; todo > 0;) {
+            const long long part = std::min<long long>(todo, 1 << 30);
+            if ((rc = launch_persist(c, part))) return rc;
+            todo -= part;
+        }
+    } else {
+        const int len = c->graph_unroll < c->poll_every ? c->graph_unroll : c->poll_every;
+        if ((rc = ensure_loop(c, c->dloop, len, 1, tol, c->dloop_hist, c->graph_gen, &c->st->done, nullptr, single_body)))
+            return rc;
+        CK(cudaGraphLaunch(c->dloop.exec, c->stream));
+        c->graph_replays += 1;
+        c->kernel_launches += loop_kernels(max_iter, len, c->opt_compat ? 5 : 4);
+    }
+    CK(launch_finalize(make_vec_args(c), c->stream));
+    CK(launch_device_info(c->st, 1, c->loopctl, info_dev, c->dloop_hist, 0, hist_dev, 0, c->stream));
+    c->kernel_launches += 2;
+    CK(cudaMemcpyAsync(x_dev, c->x, bytes, cudaMemcpyDeviceToDevice, c->stream));
+    if ((rc = device_solve_leave(c, us))) return rc;
+    c->rhs_set = true;
+    return CGB_OK;
+}
+
+extern "C" int cgb_solve_block_device(cgb_ctx *c, int nrhs, const double *B_dev, double *X_dev, int64_t max_iter,
+                                      double tol, double *hist_dev, cgb_solve_info *info_dev, void *stream)
+{
+    if (!c) return null_context();
+    if (nrhs < 1 || nrhs > CGB_MAX_RHS) return fail(CGB_ERR_INVALID, "nrhs must be in [1, %d] (got %d)", CGB_MAX_RHS, nrhs);
+    if (max_iter < 0) return fail(CGB_ERR_INVALID, "max_iter < 0");
+    int rc = use_device(c);
+    if (rc) return rc;
+    if (c->storage != 1)
+        return fail(CGB_ERR_STATE, "block solves need CSR storage: the dense mat-vec streams one p per tile pipeline");
+    if ((rc = device_solve_state(c))) return rc;
+    if ((rc = check_device_ptr(c, B_dev, "B")) || (rc = check_device_ptr(c, X_dev, "X")) ||
+        (rc = check_device_ptr(c, info_dev, "info")) || (hist_dev && (rc = check_device_ptr(c, hist_dev, "history"))))
+        return rc;
+    if ((rc = prepare_device_solve(c))) return rc;
+    BlockSolve &k = c->blk;
+    if ((rc = size_block(c, nrhs, max_iter, hist_dev != nullptr))) return rc;
+    k.nrhs = nrhs;
+    k.max_iter = max_iter;
+    k.tol = tol;
+    k.keep_history = hist_dev != nullptr;
+    const cudaStream_t us = static_cast<cudaStream_t>(stream);
+    DeviceLaunch guard(c, nullptr);
+    if ((rc = device_solve_enter(c, us))) return rc;
+    // cgb_solve_block_begin, stream-ordered
+    const size_t row = (size_t)c->n * 8, pitch = (size_t)c->ld * 8;
+    CK(cudaMemsetAsync(k.arrive, 0, (size_t)(2 * k.cap + 1) * sizeof(unsigned int), c->stream));
+    CK(cudaMemcpy2DAsync(k.b, pitch, B_dev, row, row, (size_t)nrhs, cudaMemcpyDeviceToDevice, c->stream));
+    CK(cudaMemcpy2DAsync(k.x, pitch, X_dev, row, row, (size_t)nrhs, cudaMemcpyDeviceToDevice, c->stream));
+    CK(launch_device_begin(k.st, nrhs, c->loopctl, max_iter, c->stream));
+    const BlockArgs a = make_block_args(c, k.x, 0);
+    CK(launch_spmv_block(a, c->sm_count, c->stream));
+    CK(launch_init_residual_block(a, c->stream));
+    c->kernel_launches += 3;
+    const int len = c->graph_unroll < c->poll_every ? c->graph_unroll : c->poll_every;
+    if ((rc = ensure_loop(c, k.dloop, len, nrhs, tol, a.hist, k.gen, nullptr, k.arrive + 2 * k.cap, block_body)))
+        return rc;
+    CK(cudaGraphLaunch(k.dloop.exec, c->stream));
+    c->graph_replays += 1;
+    c->kernel_launches += loop_kernels(max_iter, len, 4);
+    CK(launch_finalize_block(make_block_args(c, k.p, 0), c->stream));
+    CK(launch_device_info(k.st, nrhs, c->loopctl, info_dev, a.hist, k.hist_ld, hist_dev, max_iter, c->stream));
+    c->kernel_launches += 2;
+    CK(cudaMemcpy2DAsync(X_dev, row, k.x, pitch, row, (size_t)nrhs, cudaMemcpyDeviceToDevice, c->stream));
+    return device_solve_leave(c, us);
 }
 
 extern "C" int cgb_residual_check(cgb_ctx *c, double *norm_x, double *rel_resid)

@@ -7,6 +7,8 @@
 
 #include <utility>
 
+struct cgb_solve_info; // include/cgb200.h
+
 namespace cgb {
 
 // Launch with (pdl = true) or without the programmatic-stream-serialization attribute: the
@@ -199,5 +201,24 @@ cudaError_t launch_pap_alpha_block(const BlockArgs &a, cudaStream_t s);
 cudaError_t launch_update_xr_block(const BlockArgs &a, cudaStream_t s);
 cudaError_t launch_update_p_block(const BlockArgs &a, cudaStream_t s);
 cudaError_t launch_finalize_block(const BlockArgs &a, cudaStream_t s);
+
+// ---- device solves (loop.cu): the loop's bookkeeping without the host --------------------------
+// `limit` = max_iter of the solve, `bodies` = loop bodies issued so far, `t0` = %globaltimer at the
+// loop's start (0: no loop ran)
+struct LoopCtl {
+    long long limit, bodies;
+    unsigned long long t0, pad;
+};
+cudaError_t preload_loop_kernels();
+// st[0 .. nst) = the State cgb_solve_begin uploads; ctl = {max_iter, 0, 0}
+cudaError_t launch_device_begin(State *st, int nst, LoopCtl *ctl, long long max_iter, cudaStream_t s);
+// bodies = reset ? 0 : bodies + add (reset also stamps t0); with `set`, the WHILE condition h = the stop
+// test has not fired (*done, or *ndone == nrhs when done is null) and limit - bodies >= len
+cudaError_t launch_loop_ctl(LoopCtl *ctl, const int *done, const unsigned int *ndone, int nrhs,
+                            cudaGraphConditionalHandle h, int set, int len, int add, int reset, cudaStream_t s);
+// info[j] from st[j] (as cgb_solve_end) and, hist_out non-null, the executed r'r history of column j
+// from hist + j * hist_ld to hist_out + j * out_ld; seconds = %globaltimer now - ctl->t0
+cudaError_t launch_device_info(const State *st, int nrhs, const LoopCtl *ctl, cgb_solve_info *info, const double *hist,
+                               long long hist_ld, double *hist_out, long long out_ld, cudaStream_t s);
 
 } // namespace cgb

@@ -242,6 +242,43 @@ int cgb_solve_block_end(cgb_ctx *ctx, double *x_host, double *resid_hist, cgb_so
 int cgb_solve_block(cgb_ctx *ctx, int nrhs, const double *b_host, double *x_host, int64_t max_iter,
                     double tol, double *resid_hist, cgb_solve_info *info);
 
+/* ---- device solves: device memory in and out, ordered on the caller's stream ----------------
+ * cgb_solve_device is cgb_set_rhs + cgb_solve on buffers that live on the context's GPU:
+ *   b_dev     n doubles, the right-hand side
+ *   x_dev     n doubles, x0 on entry, the solution once the stream reaches the end of the solve
+ *   hist_dev  (nullable) max(max_iter, 1) doubles, receives r'r of every executed loop index
+ *   info_dev  one cgb_solve_info in device memory
+ *   stream    a cudaStream_t passed as void * (NULL = the legacy default stream)
+ * Stream-ordered and asynchronous: the solve sees all work enqueued on `stream` before the call, and
+ * work enqueued on `stream` after the call sees the finished x, history and info (an event recorded on
+ * `stream` is waited on by the context's own stream, and the reverse at the end).  Nothing waits for
+ * the host in between: the loop's stop test and its max_iter cap are decided on the device, and the
+ * whole loop is one launch -- the persistent kernel, or on the graph schedule one CUDA graph whose
+ * conditional WHILE nodes repeat the loop bodies.  Repeated solves of the same shape and options
+ * return without any host synchronisation; the first device solve of a context, and one that needs
+ * a larger history or block buffer than any before, allocate and may synchronise.
+ * Bits: k, converged, rsold, rsnew, iterations, the r'r history and x equal those of cgb_set_rhs +
+ * cgb_solve on the same context, on every schedule and storage.  info_dev->seconds is the device time
+ * of the loop from %globaltimer stamps of its first and last kernel.  Like cgb_set_rhs + cgb_solve,
+ * the solve leaves b and x in the context, so cgb_residual_check reports it.
+ * cgb_solve_block_device is cgb_solve_block likewise: column j of B_dev / X_dev at j * n, hist_dev
+ * (nullable) nrhs * max_iter doubles with column j at j * max_iter, info_dev nrhs entries; it keeps to
+ * the block buffers and leaves the single solve alone, as cgb_solve_block does.
+ * CGB_ERR_STATE: world > 1 (the fused exchange cannot be validated on one GPU, and the ncclAllGather
+ * exchange needs the ranks in host lockstep), a host solve or block solve between begin and end, the
+ * matrix not set, and for the block form whatever cgb_solve_block_begin refuses.
+ * CGB_ERR_INVALID: a null pointer, a host pointer or one on another device (cudaPointerGetAttributes),
+ * max_iter < 0, nrhs outside [1, CGB_MAX_RHS].
+ * Options: the solve runs as if "profile" were 0, as the block solve does; its graph launches count in
+ * "graph_replays" (one per solve on the graph schedule) and its kernels in cgb_launch_count, the loop
+ * counted as if it ran to max_iter.  "device_loop_pdl" (read-only): 1 when the loop graph's bodies
+ * keep the programmatic dependent launches, 0 when they are captured without, -1 before the first.
+ * A device fault surfaces as CGB_ERR_CUDA at the next call on the context that synchronises. */
+int cgb_solve_device(cgb_ctx *ctx, const double *b_dev, double *x_dev, int64_t max_iter, double tol,
+                     double *hist_dev, cgb_solve_info *info_dev, void *stream);
+int cgb_solve_block_device(cgb_ctx *ctx, int nrhs, const double *B_dev, double *X_dev, int64_t max_iter,
+                           double tol, double *hist_dev, cgb_solve_info *info_dev, void *stream);
+
 /* The DEBUG block at the end of solve (cg.cc:144-154, cg.cu:272-296): ||x|| and
  * ||A x - b|| / ||b|| for the x held on the device after a solve. */
 int cgb_residual_check(cgb_ctx *ctx, double *norm_x, double *rel_resid);
