@@ -107,47 +107,46 @@ int load_nccl()
     } while (0)
 
 // ------------------------------------------------------------------ context
-// Block solve (cgb_solve_block_begin): its own buffers, States, flag and graph, allocated on the
-// first block solve and never shared with the single solve.
 static_assert(kMaxRhs == CGB_MAX_RHS, "one limit of columns");
 
-// The loop of a device solve on the graph schedule (cgb_solve_device, cgb_solve_block_device): one
-// CUDA graph whose WHILE nodes run the loop bodies until the stop test fires or max_iter is reached.
-// Keyed like the host graphs, plus `gen` (drop_graph / drop_block_graph calls since creation) and the
-// matrix arrays it reads.
-struct DeviceLoop {
-    cudaGraph_t graph = nullptr;
-    cudaGraphExec_t exec = nullptr;
+// One solve in progress: the single solve's (cgb_ctx::run) or the block solve's (BlockSolve::run)
+struct SolveRun {
+    int nrhs = 1;
+    long long max_iter = 0, launched = 0;
+    double tol = 1e-10, loop_ms = 0.0;
+    State *st = nullptr;            // [nrhs]
+    double *hist = nullptr;         // column j's r'r history at hist + j * hist_ld; null: not kept
+    long long hist_ld = 0;
+};
+
+// A loop graph and what its captured kernel arguments bake in.  A context caches four: the host loops
+// of the single and the block solve (cgb_iterate) and the device loops of both (cgb_solve_device,
+// cgb_solve_block_device).  `gen` is cgb_ctx::graph_gen at capture.
+struct GraphKey {
     int len = 0, nrhs = 0, pdl = 0;
-    int pdl_used = -1;              // 1: the bodies keep the programmatic dependent launches, 0: they do not
     double tol = 0.0;
     const double *hist = nullptr;
     long long gen = -1;
-    const void *mat0 = nullptr, *mat1 = nullptr;
+};
+struct CachedGraph {
+    cudaGraph_t graph = nullptr;
+    cudaGraphExec_t exec = nullptr;
+    GraphKey key;
+    int pdl_used = -1;              // device loops: 1 the bodies keep the programmatic dependent launches, 0 not
 };
 
+// Block solve (cgb_solve_block_begin): its own buffers and States, allocated on the first block solve
+// and never shared with the single solve.
 struct BlockSolve {
     int cap = 0;                    // columns the vector buffers hold
-    int nrhs = 0;                   // columns of the solve in progress
     double *x = nullptr, *r = nullptr, *p = nullptr, *b = nullptr; // [cap][ld]
     double *ap = nullptr;           // [cap][slot]
     double *rrpart = nullptr, *papart = nullptr; // [cap][nchunks]
-    State *st = nullptr;            // [cap]
     unsigned int *arrive = nullptr; // [cap][2] arrival counters, then the count of converged columns
-    double *hist = nullptr;         // [cap][hist_ld]
-    long long hist_ld = 0;
-    int *h_done = nullptr, *d_hdone = nullptr; // mapped pinned flag: every column has converged
-    cudaGraph_t graph = nullptr;
-    cudaGraphExec_t graph_exec = nullptr;
-    // what the captured arguments bake in
-    int graph_len = 0, graph_nrhs = 0, graph_pdl = 0;
-    double graph_tol = 0.0;
-    const double *graph_hist = nullptr;
-    bool active = false, keep_history = false;
-    long long max_iter = 0, launched = 0;
-    double tol = 0.0, loop_ms = 0.0;
-    long long gen = 0;              // drop_block_graph calls: the buffers the block graphs bake in may have moved
-    DeviceLoop dloop;               // cgb_solve_block_device's graph
+    double *hist_buf = nullptr;     // [cap][hist_cap]
+    long long hist_cap = 0;
+    bool active = false;
+    SolveRun run;                   // st: [cap]
 };
 
 struct cgb_ctx {
@@ -160,7 +159,6 @@ struct cgb_ctx {
     double *compat_part = nullptr; // chunk partials of the compat mat-vec
     size_t compat_part_cap = 0;
     int poll_every = 16, graph_unroll = 16, opt_pdl = 1, opt_l2_prefetch = 4, opt_l2_ramp = 2;
-    int graph_len = 0;             // iterations in the instantiated graph (min(graph_unroll, poll_every))
     long long graph_replays = 0;   // graph launches since creation ("graph_replays", read-only option)
     int opt_balance = 1;           // persistent kernel: re-balance the rows between the CTAs from measured speeds
     long long aux_stride = 0;      // entries of one parity of the local LL side buffer
@@ -183,7 +181,7 @@ struct cgb_ctx {
     double *A = nullptr, *p = nullptr, *r = nullptr, *x = nullptr, *b = nullptr;
     int2 *env = nullptr;           // dense: [first, last + 1) of the non-zero columns of every local row,
                                    // rebuilt after every write of A (the mat-vecs stream only these windows)
-    double *apx = nullptr, *rrpart = nullptr, *papart = nullptr, *scratch = nullptr, *hist = nullptr, *sink = nullptr;
+    double *apx = nullptr, *rrpart = nullptr, *papart = nullptr, *scratch = nullptr, *sink = nullptr;
     // apx: plain gather buffer [world][slot_cap] doubles.  ll: fused-mode LL buffers
     // [2][world][slot_cap] x 16 B, the allocation peers map; ctl: local control words.
     long long bufstride = 0;
@@ -194,39 +192,50 @@ struct cgb_ctx {
     void *ipc_opened[kMaxWorld] = {};
     bool p2p_ready = false;
     int opt_exchange = 0; // 0 = ncclAllGather, 1 = fused peer stores
-    long long hist_cap = 0;
-    State *st = nullptr;
-    int *h_done = nullptr, *d_hdone = nullptr; // mapped pinned flag
+    long long hist_cap = 0;        // doubles at run.hist
+    // mapped pinned flag: [0] the stop test fired (raised by the solve in progress, single or block) or,
+    // negative, a device-side wait timed out; [1..6] context of a timeout report
+    int *h_done = nullptr, *d_hdone = nullptr;
     double *h_pin = nullptr;                   // pinned staging for small D2H reads
 
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_batch[2] = {nullptr, nullptr};
     std::vector<cudaEvent_t> prof_ev;
-    cudaGraph_t graph = nullptr;
-    cudaGraphExec_t graph_exec = nullptr;
     ncclComm_t comm = nullptr;
 
     bool matrix_set = false, rhs_set = false;
     bool in_solve = false;         // a single or (blk.active) a block solve is between begin and end
-    long long max_iter = 0, launched = 0, kernel_launches = 0;
-    double tol = 1e-10, graph_tol = -1.0;
-    double loop_ms = 0.0;
+    long long kernel_launches = 0;
+    SolveRun run;                  // the single solve; run.hist is the host API's history (null: not kept)
     double prof_gemv_ms = 0.0;
     long long prof_gemv_n = 0;
     BlockSolve blk;
 
+    // Bumped whenever something a captured loop graph bakes in, other than its key's own fields, may have
+    // changed: an option, a buffer that moved, a CSR matrix build (it reallocates col / val)
+    long long graph_gen = 0;
+    CachedGraph graph_single, graph_block, loop_single, loop_block; // host loops, device loops
+
     // device solves (cgb_solve_device, cgb_solve_block_device); allocated on the first one
-    long long graph_gen = 0;       // drop_graph calls: what the graphs of the single solve bake in has changed
-    DeviceLoop dloop;              // cgb_solve_device's graph
     LoopCtl *loopctl = nullptr;    // the loop's body limit, bodies issued, start stamp
-    double *dev_hist = nullptr;    // cgb_solve_device's r'r history (the host solve's `hist` stays its own)
+    double *dev_hist = nullptr;    // cgb_solve_device's r'r history (the host solve's stays its own)
     long long dev_hist_cap = 0;
     cudaEvent_t ev_dev[2] = {nullptr, nullptr}; // caller's stream -> ctx stream, and back
-    bool device_loop = false;      // kernels being enqueued belong to a device solve (see DeviceLaunch)
-    double *dloop_hist = nullptr;  // ... and write this history (nullable)
 };
 
 namespace {
+
+// How a solve's loop kernels launch: the r'r history they write (nullable), the mapped host flag they
+// raise when the stop test fires (null in a device solve: nobody polls it, and a host solve queued
+// behind it resets it from the host) and whether they chain by programmatic dependent launch.
+struct Mode {
+    double *hist;
+    int *host_done;
+    int pdl;
+};
+
+// the host API's single solve ("profile" times each mat-vec between events: no PDL)
+Mode host_mode(const cgb_ctx *c) { return {c->run.hist, c->d_hdone, (c->opt_pdl && !c->opt_profile) ? 1 : 0}; }
 
 int use_device(cgb_ctx *c)
 {
@@ -242,6 +251,15 @@ long long loopback_cap(const cgb_ctx *c)
 {
     if (!c->opt_loopback) return c->maxrows > 0 ? c->maxrows : 1;
     return c->rows > 0 ? c->rows : 1;
+}
+
+// the fused exchange's peer buffers; in "loopback" every "peer" is this rank's own buffer, shifted so
+// that slot g is hit
+void peer_pointers(const cgb_ctx *c, uint4 **peer)
+{
+    for (int g = 0; g < kMaxWorld; ++g) peer[g] = c->peer_ll[g];
+    if (c->opt_loopback)
+        for (int g = 0; g < c->world; ++g) peer[g] = c->ll + ((long long)g - c->rank) * c->slot;
 }
 
 Gather make_gather(const cgb_ctx *c)
@@ -273,7 +291,7 @@ Trace make_trace(const cgb_ctx *c, int which, int blocks)
     return t;
 }
 
-GemvArgs make_gemv_args(const cgb_ctx *c, const double *v, int advance)
+GemvArgs make_gemv_args(const cgb_ctx *c, const double *v, int advance, const Mode &m)
 {
     GemvArgs a;
     memset(&a, 0, sizeof a);
@@ -290,25 +308,23 @@ GemvArgs make_gemv_args(const cgb_ctx *c, const double *v, int advance)
     a.rank = c->rank;
     a.world = c->world;
     a.p2p = (c->world > 1 && c->opt_exchange == 1) ? 1 : 0;
-    for (int g = 0; g < kMaxWorld; ++g) a.peer_ll[g] = c->peer_ll[g];
+    peer_pointers(c, a.peer_ll);
     a.ld = c->ld;
     a.rows = c->rows;
     a.row0 = c->row0;
     a.maxrows = c->maxrows;
-    a.st = c->st;
+    a.st = c->run.st;
     a.rrpart = c->rrpart;
     a.nchunks = c->nchunks;
-    a.hist = c->device_loop ? c->dloop_hist : c->hist;
+    a.hist = m.hist;
     a.advance = advance;
-    a.pdl = (advance && c->opt_pdl && !c->opt_profile) ? 1 : 0; // only inside the CG loop
+    a.pdl = (advance && m.pdl) ? 1 : 0; // only inside the CG loop
     a.l2_prefetch = a.pdl ? c->opt_l2_prefetch : 0;
-    if (c->opt_loopback) // every "peer" is this rank's own buffer, shifted so that slot g is hit
-        for (int g = 0; g < c->world; ++g) a.peer_ll[g] = c->ll + ((long long)g - c->rank) * c->slot;
     if (c->trace_cap > 0 && advance) a.trace = make_trace(c, 0, c->nblk);
     return a;
 }
 
-VecArgs make_vec_args(const cgb_ctx *c)
+VecArgs make_vec_args(const cgb_ctx *c, const Mode &m)
 {
     VecArgs a;
     memset(&a, 0, sizeof a);
@@ -319,13 +335,13 @@ VecArgs make_vec_args(const cgb_ctx *c)
     a.apx = c->apx;
     a.rrpart = c->rrpart;
     a.papart = c->papart;
-    a.st = c->st;
-    a.host_done = c->device_loop ? nullptr : c->d_hdone;
-    a.hist = c->device_loop ? c->dloop_hist : c->hist;
+    a.st = c->run.st;
+    a.host_done = m.host_done;
+    a.hist = m.hist;
     a.g = make_gather(c);
     a.n = c->n;
-    a.tol = c->tol;
-    a.pdl = (c->opt_pdl && !c->opt_profile) ? 1 : 0;
+    a.tol = c->run.tol;
+    a.pdl = m.pdl;
     a.arrive = c->arrive;
     if (c->trace_cap > 0) {
         a.trace_xr = make_trace(c, 1, (int)c->nchunks);
@@ -353,472 +369,47 @@ void free_trace(cgb_ctx *c)
     c->trace_cap = 0;
 }
 
-void drop_graph(cgb_ctx *c)
+// `n` States as a solve starts them: zero, iter = -1
+int reset_states(cgb_ctx *c, State *st, int n)
 {
-    if (c->graph_exec) cudaGraphExecDestroy(c->graph_exec);
-    if (c->graph) cudaGraphDestroy(c->graph);
-    c->graph_exec = nullptr;
-    c->graph = nullptr;
-    c->graph_gen += 1; // cgb_solve_device's graph bakes in the same arguments
-}
-
-void drop_loop(DeviceLoop &d)
-{
-    if (d.exec) cudaGraphExecDestroy(d.exec);
-    if (d.graph) cudaGraphDestroy(d.graph);
-    d.exec = nullptr;
-    d.graph = nullptr;
-}
-
-// the mat-vec and, for world > 1, the gather of its result
-int launch_matvec(cgb_ctx *c, const double *v, int advance, int variant)
-{
-    if (c->opt_compat) { // reference topologies, NUM_THREADS / BLOCK_WIDTH literal (single GPU)
-        GemvArgs a = make_gemv_args(c, v, advance);
-        a.pdl = 0;
-        CK(launch_compat_matvec(a, c->nblk, c->opt_num_threads, c->opt_block_width, c->opt_transposed,
-                                c->compat_part, c->stream));
-        c->kernel_launches += 2;
-        return CGB_OK;
-    }
-    const GemvArgs a = make_gemv_args(c, v, advance);
-    if (c->storage == 1) CK(launch_spmv(a, c->sm_count, c->stream));
-    else CK(gemv_variant(variant).launch(a, c->sm_count * gemv_variant(variant).ctas_per_sm, c->stream));
-    c->kernel_launches += 1;
+    State s0[kMaxRhs];
+    memset(s0, 0, sizeof s0);
+    for (State &s : s0) s.iter = -1;
+    CK(cudaMemcpyAsync(st, s0, (size_t)n * sizeof(State), cudaMemcpyHostToDevice, c->stream));
     return CGB_OK;
 }
 
-int launch_gather(cgb_ctx *c)
+// ---- cached loop graphs ---------------------------------------------------------------------
+// Loop bodies in a loop graph: a batch between two looks at the stop flag is poll_every bodies, and a
+// longer graph could never be replayed
+int graph_len_wanted(const cgb_ctx *c) { return c->graph_unroll < c->poll_every ? c->graph_unroll : c->poll_every; }
+
+GraphKey graph_key(const cgb_ctx *c, int nrhs, double tol, const double *hist)
 {
-    if (c->world == 1) return CGB_OK;
-    if (c->opt_exchange == 1) return CGB_OK; // fused into the mat-vec kernel (peer stores + flags)
-    if (!c->comm) return fail(CGB_ERR_STATE, "world > 1 but neither cgb_comm_init nor cgb_exchange_import was called");
-    NK(g_nccl.AllGather(c->apx + (long long)c->rank * c->slot, c->apx, (size_t)c->slot, kNcclDouble,
-                        c->comm, c->stream));
-    return CGB_OK;
+    return GraphKey{graph_len_wanted(c), nrhs, c->opt_pdl, tol, hist, c->graph_gen};
 }
 
-// the three vector kernels of one iteration; CSR contexts compute every scalar once per iteration
-int launch_vector_phase(cgb_ctx *c)
+bool holds(const CachedGraph &g, const GraphKey &k)
 {
-    const VecArgs va = make_vec_args(c);
-    if (c->storage == 1) {
-        CK(launch_pap_alpha(va, c->stream));
-        CK(launch_update_xr_once(va, c->stream));
-        CK(launch_update_p_once(va, c->stream));
-    } else {
-        CK(launch_pap_partials(va, c->stream));                             // cg.cc:105
-        CK(launch_update_xr(va, c->stream));                                // cg.cc:106-117
-        CK(launch_update_p(va, c->stream));                                 // cg.cc:120-132
-    }
-    c->kernel_launches += 3;
-    return CGB_OK;
+    return g.exec && g.key.len == k.len && g.key.nrhs == k.nrhs && g.key.pdl == k.pdl && g.key.tol == k.tol &&
+           g.key.hist == k.hist && g.key.gen == k.gen;
 }
 
-int launch_iteration(cgb_ctx *c)
+void drop(CachedGraph &g)
 {
-    int rc = launch_matvec(c, c->p, 1, c->variant);                        // cg.cc:100-102
-    if (rc) return rc;
-    if ((rc = launch_gather(c))) return rc;                                 // cg.cc:135-136 (moved)
-    return launch_vector_phase(c);
+    if (g.exec) cudaGraphExecDestroy(g.exec);
+    if (g.graph) cudaGraphDestroy(g.graph);
+    g.exec = nullptr;
+    g.graph = nullptr;
 }
 
-int build_graph(cgb_ctx *c)
+void drop_graphs(cgb_ctx *c)
 {
-    drop_graph(c);
-    CK(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
-    int rc = CGB_OK;
-    const long long before = c->kernel_launches;
-    // a batch between two looks at the stop flag is poll_every iterations: a longer graph could never be replayed
-    c->graph_len = c->graph_unroll < c->poll_every ? c->graph_unroll : c->poll_every;
-    for (int u = 0; u < c->graph_len && rc == CGB_OK; ++u) rc = launch_iteration(c);
-    c->kernel_launches = before; // capture launches nothing
-    cudaGraph_t g = nullptr;
-    cudaError_t e = cudaStreamEndCapture(c->stream, &g);
-    if (rc != CGB_OK) {
-        if (g) cudaGraphDestroy(g);
-        return rc;
-    }
-    CK(e);
-    c->graph = g;
-    CK(cudaGraphInstantiate(&c->graph_exec, c->graph, 0));
-    c->graph_tol = c->tol; // tol and the history pointer are baked into the captured arguments
-    return CGB_OK;
-}
-
-// ---- persistent schedule (persist.cu) ------------------------------------------------
-// The persistent kernel exists for the tile shapes listed in persist.cu; it needs one CTA per SM,
-// the fused exchange (or one rank), at most persist_max_chunks() vector chunks per CTA and the
-// scratch for the block / chunk partials next to the tile ring in shared memory.
-int persist_index(const cgb_ctx *c)
-{
-    const char *name = gemv_variant(c->variant).name;
-    for (int i = 0; i < persist_variant_count(); ++i)
-        if (strcmp(persist_variant(i).name, name) == 0) return i;
-    return -1;
-}
-
-void persist_scratch(const cgb_ctx *c, int *scr_n)
-{
-    const long long scr = c->nchunks > c->nblk ? c->nchunks : c->nblk; // chunk partials / per-CTA timings
-    *scr_n = (int)((scr + 1) & ~1LL);
-}
-
-// nullptr when the persistent schedule can run this context as configured, else the reason
-const char *persist_unusable(const cgb_ctx *c)
-{
-    if (c->storage == 1) return "CSR storage";
-    if (c->opt_compat) return "compat mat-vec";
-    if (c->opt_profile) return "profile mode (per-launch events)";
-    if (c->world > 1 && c->opt_exchange != 1) return "ncclAllGather exchange";
-    if (gemv_variant(c->variant).ctas_per_sm != 1) return "variant runs 2 CTAs per SM";
-    const int pi = persist_index(c);
-    if (pi < 0) return "no persistent instantiation of this tile shape";
-    if (c->nchunks > (long long)persist_max_chunks() * c->nblk) return "N too large for the per-CTA vector chunks";
-    int scr_n;
-    persist_scratch(c, &scr_n);
-    if (persist_variant(pi).smem_fixed() + (size_t)scr_n * 8 + 4096 > (size_t)c->smem_optin) // + static
-        return "tile ring + scratch exceed shared memory";
-    return nullptr;
-}
-
-int launch_persist(cgb_ctx *c, long long iters)
-{
-    PersistArgs a;
-    memset(&a, 0, sizeof a);
-    a.A = c->A;
-    a.env = c->env;
-    a.x = c->x;
-    a.r = c->r;
-    a.p = c->p;
-    a.rrpart = c->rrpart;
-    for (int g = 0; g < kMaxWorld; ++g) a.peer_ll[g] = c->peer_ll[g];
-    if (c->opt_loopback)
-        for (int g = 0; g < c->world; ++g) a.peer_ll[g] = c->ll + ((long long)g - c->rank) * c->slot;
-    a.ll = c->ll;
-    a.rr_ll = c->rr_ll;
-    a.rr_stride = c->aux_stride;
-    a.sync = c->psync;
-    a.st = c->st;
-    a.ctl = c->ctl;
-    a.hist = c->device_loop ? c->dloop_hist : c->hist;
-    a.host_done = c->device_loop ? nullptr : c->d_hdone;
-    a.ld = c->ld;
-    a.rows = c->rows;
-    a.row0 = c->row0;
-    a.n = c->n;
-    a.maxrows = c->maxrows;
-    a.n_loc = c->n_loc > 0 ? c->n_loc : 1;
-    a.loc_cap = loopback_cap(c);
-    a.slot = c->slot;
-    a.bufstride = c->bufstride;
-    a.slot_off = (long long)c->rank * c->slot;
-    a.nchunks = c->nchunks;
-    a.rank = c->rank;
-    a.world = c->world;
-    a.iters = (int)iters;
-    a.l2_prefetch = c->opt_l2_prefetch;
-    a.l2_ramp = c->opt_l2_ramp;
-    a.balance = c->opt_balance;
-    persist_scratch(c, &a.scr_n);
-    a.tol = c->tol;
-    a.spin_ns = (unsigned long long)c->spin_timeout_ms * 1000000ULL;
-    if (c->trace_cap > 0) a.trace = make_trace(c, 0, c->nblk);
-    CK(cudaMemsetAsync(c->psync, 0, sizeof(PersistSync), c->stream));
-    CK(persist_variant(persist_index(c)).launch(a, c->nblk, c->stream));
-    c->kernel_launches += 1;
-    c->persist_launches += 1;
-    return CGB_OK;
-}
-
-bool exchange_configured(const cgb_ctx *c)
-{
-    return c->world == 1 || (c->opt_exchange == 1 ? c->p2p_ready : c->comm != nullptr);
-}
-
-// Hooks that read the gathered result with memcpys: in fused mode first consume the running
-// exchange into the plain buffer (this also advances the epoch, like every consumer kernel).
-int collect_for_host(cgb_ctx *c)
-{
-    const Gather g = make_gather(c);
-    if (g.p2p) {
-        CK(launch_exchange_collect(c->apx, g, c->stream));
-        c->kernel_launches += 1;
-    }
-    return CGB_OK;
-}
-
-int read_state(cgb_ctx *c, State *out)
-{
-    CK(cudaMemcpyAsync(out, c->st, sizeof(State), cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaStreamSynchronize(c->stream));
-    return CGB_OK;
-}
-
-// ---- block solve ---------------------------------------------------------------------------
-void drop_block_graph(cgb_ctx *c)
-{
-    BlockSolve &k = c->blk;
-    if (k.graph_exec) cudaGraphExecDestroy(k.graph_exec);
-    if (k.graph) cudaGraphDestroy(k.graph);
-    k.graph_exec = nullptr;
-    k.graph = nullptr;
-    k.gen += 1; // and so does cgb_solve_block_device's
-}
-
-void free_block_vectors(cgb_ctx *c)
-{
-    BlockSolve &k = c->blk;
-    double *bufs[] = {k.x, k.r, k.p, k.b, k.ap, k.rrpart, k.papart};
-    for (double *p : bufs)
-        if (p) cudaFree(p);
-    if (k.st) cudaFree(k.st);
-    if (k.arrive) cudaFree(k.arrive);
-    k.x = k.r = k.p = k.b = k.ap = k.rrpart = k.papart = nullptr;
-    k.st = nullptr;
-    k.arrive = nullptr;
-    k.cap = 0;
-}
-
-void free_block(cgb_ctx *c)
-{
-    BlockSolve &k = c->blk;
-    drop_block_graph(c);
-    drop_loop(k.dloop);
-    free_block_vectors(c);
-    if (k.hist) cudaFree(k.hist);
-    k.hist = nullptr;
-    k.hist_ld = 0;
-    if (k.h_done) cudaFreeHost(k.h_done);
-    k.h_done = k.d_hdone = nullptr;
-}
-
-// buffers for nrhs columns and, with a history, max(max_iter, 1) entries per column; grows only
-int size_block(cgb_ctx *c, int nrhs, long long max_iter, bool history)
-{
-    BlockSolve &k = c->blk;
-    auto alloc = [&](void **p, size_t bytes) -> int {
-        cudaError_t e = cudaMalloc(p, bytes);
-        if (e == cudaSuccess) e = cudaMemsetAsync(*p, 0, bytes, c->stream);
-        if (e != cudaSuccess) {
-            cudaGetLastError();
-            return fail(e == cudaErrorMemoryAllocation ? CGB_ERR_NOMEM : CGB_ERR_CUDA, "block solve buffers: %s",
-                        cudaGetErrorString(e));
-        }
-        return CGB_OK;
-    };
-    int rc = CGB_OK;
-    if (!k.h_done) { // first block solve of this context
-        CK(preload_spmv_block_kernels());
-        CK(preload_vec_block_kernels());
-        CK(cudaHostAlloc(&k.h_done, sizeof(int), cudaHostAllocMapped));
-        CK(cudaHostGetDevicePointer(&k.d_hdone, k.h_done, 0));
-    }
-    const long long hist_need = max_iter > 0 ? max_iter : 1;
-    if (nrhs > k.cap) {
-        drop_block_graph(c);
-        free_block_vectors(c);
-        const size_t vec = (size_t)nrhs * c->ld * sizeof(double);
-        const size_t part = (size_t)nrhs * c->nchunks * sizeof(double);
-        if ((rc = alloc((void **)&k.x, vec)) || (rc = alloc((void **)&k.r, vec)) || (rc = alloc((void **)&k.p, vec)) ||
-            (rc = alloc((void **)&k.b, vec)) || (rc = alloc((void **)&k.ap, (size_t)nrhs * c->slot_cap * sizeof(double))) ||
-            (rc = alloc((void **)&k.rrpart, part)) || (rc = alloc((void **)&k.papart, part)) ||
-            (rc = alloc((void **)&k.st, (size_t)nrhs * sizeof(State))) ||
-            (rc = alloc((void **)&k.arrive, (size_t)(2 * nrhs + 1) * sizeof(unsigned int)))) {
-            free_block_vectors(c);
-            return rc;
-        }
-        k.cap = nrhs;
-        if (k.hist) cudaFree(k.hist); // its column stride follows from the new capacity
-        k.hist = nullptr;
-        k.hist_ld = 0;
-    }
-    if (history && hist_need > k.hist_ld) {
-        drop_block_graph(c);
-        if (k.hist) cudaFree(k.hist);
-        k.hist = nullptr;
-        k.hist_ld = 0;
-        if ((rc = alloc((void **)&k.hist, (size_t)k.cap * hist_need * sizeof(double)))) return rc;
-        k.hist_ld = hist_need;
-    }
-    return CGB_OK;
-}
-
-BlockArgs make_block_args(const cgb_ctx *c, const double *v, int advance)
-{
-    const BlockSolve &k = c->blk;
-    BlockArgs a;
-    memset(&a, 0, sizeof a);
-    a.rp = c->csr.rp;
-    a.col = c->csr.col;
-    a.val = c->csr.val;
-    a.v = v;
-    a.x = k.x;
-    a.r = k.r;
-    a.p = k.p;
-    a.b = k.b;
-    a.ap = k.ap;
-    a.rrpart = k.rrpart;
-    a.papart = k.papart;
-    a.st = k.st;
-    a.arrive = k.arrive;
-    a.ndone = k.arrive + 2 * k.cap;
-    a.host_done = c->device_loop ? nullptr : k.d_hdone;
-    a.hist = k.keep_history ? k.hist : nullptr;
-    a.n = c->n;
-    a.ld = c->ld;
-    a.rows = c->rows;
-    a.slot = c->slot_cap;
-    a.nchunks = c->nchunks;
-    a.hist_ld = k.hist_ld;
-    a.nrhs = k.nrhs;
-    a.advance = advance;
-    a.pdl = (advance && c->opt_pdl) ? 1 : 0; // only inside the CG loop
-    a.tol = k.tol;
-    return a;
-}
-
-// mat-vec + the three vector kernels of one block iteration
-int launch_block_iteration(cgb_ctx *c)
-{
-    const BlockArgs a = make_block_args(c, c->blk.p, 1);
-    CK(launch_spmv_block(a, c->sm_count, c->stream));
-    CK(launch_pap_alpha_block(a, c->stream));
-    CK(launch_update_xr_block(a, c->stream));
-    CK(launch_update_p_block(a, c->stream));
-    c->kernel_launches += 4;
-    return CGB_OK;
-}
-
-int build_block_graph(cgb_ctx *c, int len)
-{
-    BlockSolve &k = c->blk;
-    drop_block_graph(c);
-    CK(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
-    int rc = CGB_OK;
-    const long long before = c->kernel_launches;
-    for (int u = 0; u < len && rc == CGB_OK; ++u) rc = launch_block_iteration(c);
-    c->kernel_launches = before; // capture launches nothing
-    cudaGraph_t g = nullptr;
-    cudaError_t e = cudaStreamEndCapture(c->stream, &g);
-    if (rc != CGB_OK) {
-        if (g) cudaGraphDestroy(g);
-        return rc;
-    }
-    CK(e);
-    k.graph = g;
-    CK(cudaGraphInstantiate(&k.graph_exec, k.graph, 0));
-    k.graph_len = len;
-    k.graph_nrhs = k.nrhs;
-    k.graph_tol = k.tol;
-    k.graph_hist = make_block_args(c, k.p, 1).hist;
-    k.graph_pdl = c->opt_pdl;
-    return CGB_OK;
-}
-
-// cgb_iterate of a block solve: the graph schedule of a CSR single solve, with the block's own graph
-int block_iterate(cgb_ctx *c, int64_t iters, float *ms)
-{
-    BlockSolve &k = c->blk;
-    int rc;
-    long long todo = std::min<long long>(iters, k.max_iter - k.launched);
-    if (todo < 0) todo = 0;
-    const bool graph = c->opt_graph != 0;
-    const int want_len = c->graph_unroll < c->poll_every ? c->graph_unroll : c->poll_every;
-    if (k.graph_exec && (k.graph_len != want_len || k.graph_nrhs != k.nrhs || k.graph_tol != k.tol ||
-                         k.graph_hist != make_block_args(c, k.p, 1).hist || k.graph_pdl != c->opt_pdl))
-        drop_block_graph(c);
-    if (graph && !k.graph_exec && todo >= want_len) {
-        if ((rc = build_block_graph(c, want_len))) return rc;
-    }
-    CK(cudaEventRecord(c->ev0, c->stream));
-    long long issued = 0;
-    int batch_idx = 0;
-    while (issued < todo) {
-        if (*(volatile int *)k.h_done) break; // every column converged: later launches would be no-ops
-        const long long batch = std::min<long long>(c->poll_every, todo - issued);
-        long long i = 0;
-        while (i < batch) {
-            if (graph && k.graph_exec && batch - i >= k.graph_len) {
-                CK(cudaGraphLaunch(k.graph_exec, c->stream));
-                c->kernel_launches += 4LL * k.graph_len;
-                c->graph_replays += 1;
-                i += k.graph_len;
-            } else {
-                if ((rc = launch_block_iteration(c))) return rc;
-                i += 1;
-            }
-        }
-        issued += batch;
-        // at most two batches in flight, as in cgb_iterate
-        CK(cudaEventRecord(c->ev_batch[batch_idx & 1], c->stream));
-        if (batch_idx >= 1) CK(cudaEventSynchronize(c->ev_batch[(batch_idx - 1) & 1]));
-        ++batch_idx;
-    }
-    CK(cudaEventRecord(c->ev1, c->stream));
-    CK(cudaEventSynchronize(c->ev1));
-    float t = 0.f;
-    CK(cudaEventElapsedTime(&t, c->ev0, c->ev1));
-    k.loop_ms += t;
-    k.launched += issued;
-    if (ms) *ms = t;
-    return CGB_OK;
-}
-
-// ---- device solves -------------------------------------------------------------------------
-// While a device solve enqueues its kernels: "profile" reads 0 (as for a block solve), no kernel
-// raises the mapped host flag (nobody polls it, and a host solve queued behind this one resets it from
-// the host), and the history goes to the device solve's own buffer.
-struct DeviceLaunch {
-    cgb_ctx *c;
-    int keep_profile, keep_pdl;
-    DeviceLaunch(cgb_ctx *c_, double *hist) : c(c_), keep_profile(c_->opt_profile), keep_pdl(c_->opt_pdl)
-    {
-        c->opt_profile = 0;
-        c->device_loop = true;
-        c->dloop_hist = hist;
-    }
-    ~DeviceLaunch()
-    {
-        c->opt_profile = keep_profile;
-        c->opt_pdl = keep_pdl;
-        c->device_loop = false;
-        c->dloop_hist = nullptr;
-    }
-};
-
-// Pointers a device solve takes: device memory of the context's GPU (or managed memory)
-int check_device_ptr(const cgb_ctx *c, const void *p, const char *what)
-{
-    if (!p) return fail(CGB_ERR_INVALID, "null %s", what);
-    cudaPointerAttributes a;
-    cudaError_t e = cudaPointerGetAttributes(&a, p);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        return fail(CGB_ERR_INVALID, "%s is not a pointer CUDA knows (%s)", what, cudaGetErrorString(e));
-    }
-    if (a.type == cudaMemoryTypeManaged) return CGB_OK;
-    if (a.type != cudaMemoryTypeDevice)
-        return fail(CGB_ERR_INVALID, "%s is host memory: a device solve takes device pointers", what);
-    if (a.device != c->device)
-        return fail(CGB_ERR_INVALID, "%s lives on device %d, the context on device %d", what, a.device, c->device);
-    return CGB_OK;
-}
-
-// what a context's first device solve allocates
-int prepare_device_solve(cgb_ctx *c)
-{
-    if (c->loopctl) return CGB_OK;
-    CK(preload_loop_kernels());
-    for (cudaEvent_t &e : c->ev_dev)
-        if (!e) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    CK(cudaMalloc(&c->loopctl, sizeof(LoopCtl)));
-    CK(cudaMemsetAsync(c->loopctl, 0, sizeof(LoopCtl), c->stream));
-    return CGB_OK;
+    for (CachedGraph *g : {&c->graph_single, &c->graph_block, &c->loop_single, &c->loop_block}) drop(*g);
 }
 
 // Captures into `g` the launches `enqueue` makes on c->stream, after the node `dep` (nullable);
-// *tail = the last node captured.  The capture always ends, whatever fails.
+// *tail (nullable) = the last node captured.  The capture always ends, whatever fails.
 template <class F>
 int capture_into(cgb_ctx *c, cudaGraph_t g, cudaGraphNode_t dep, F enqueue, cudaGraphNode_t *tail)
 {
@@ -841,27 +432,456 @@ int capture_into(cgb_ctx *c, cudaGraph_t g, cudaGraphNode_t dep, F enqueue, cuda
     return CGB_OK;
 }
 
-// The loop of a device solve as one graph (DESIGN 3.9):
+// `g` captured anew by `build(graph)` into a created graph, instantiated, and keyed with `key`
+template <class F>
+int rebuild(cgb_ctx *c, CachedGraph &g, const GraphKey &key, F build)
+{
+    drop(g);
+    CK(cudaGraphCreate(&g.graph, 0));
+    const long long before = c->kernel_launches;
+    int rc = build(g.graph);
+    c->kernel_launches = before; // capture launches nothing
+    if (rc == CGB_OK) {
+        const cudaError_t e = cudaGraphInstantiate(&g.exec, g.graph, 0);
+        if (e != cudaSuccess) rc = fail(CGB_ERR_CUDA, "instantiating a loop graph failed: %s", cudaGetErrorString(e));
+    }
+    if (rc) {
+        drop(g);
+        return rc;
+    }
+    g.key = key;
+    return CGB_OK;
+}
+
+// the mat-vec and, for world > 1, the gather of its result
+int launch_matvec(cgb_ctx *c, const double *v, int advance, int variant, const Mode &m)
+{
+    if (c->opt_compat) { // reference topologies, NUM_THREADS / BLOCK_WIDTH literal (single GPU)
+        GemvArgs a = make_gemv_args(c, v, advance, m);
+        a.pdl = 0;
+        CK(launch_compat_matvec(a, c->nblk, c->opt_num_threads, c->opt_block_width, c->opt_transposed,
+                                c->compat_part, c->stream));
+        c->kernel_launches += 2;
+        return CGB_OK;
+    }
+    const GemvArgs a = make_gemv_args(c, v, advance, m);
+    if (c->storage == 1) CK(launch_spmv(a, c->sm_count, c->stream));
+    else CK(gemv_variant(variant).launch(a, c->sm_count * gemv_variant(variant).ctas_per_sm, c->stream));
+    c->kernel_launches += 1;
+    return CGB_OK;
+}
+
+int launch_gather(cgb_ctx *c)
+{
+    if (c->world == 1) return CGB_OK;
+    if (c->opt_exchange == 1) return CGB_OK; // fused into the mat-vec kernel (peer stores + flags)
+    if (!c->comm) return fail(CGB_ERR_STATE, "world > 1 but neither cgb_comm_init nor cgb_exchange_import was called");
+    NK(g_nccl.AllGather(c->apx + (long long)c->rank * c->slot, c->apx, (size_t)c->slot, kNcclDouble,
+                        c->comm, c->stream));
+    return CGB_OK;
+}
+
+// the three vector kernels of one iteration; CSR contexts compute every scalar once per iteration
+int launch_vector_phase(cgb_ctx *c, const Mode &m)
+{
+    const VecArgs va = make_vec_args(c, m);
+    if (c->storage == 1) {
+        CK(launch_pap_alpha(va, c->stream));
+        CK(launch_update_xr_once(va, c->stream));
+        CK(launch_update_p_once(va, c->stream));
+    } else {
+        CK(launch_pap_partials(va, c->stream));                             // cg.cc:105
+        CK(launch_update_xr(va, c->stream));                                // cg.cc:106-117
+        CK(launch_update_p(va, c->stream));                                 // cg.cc:120-132
+    }
+    c->kernel_launches += 3;
+    return CGB_OK;
+}
+
+int launch_iteration(cgb_ctx *c, const Mode &m)
+{
+    int rc = launch_matvec(c, c->p, 1, c->variant, m);                     // cg.cc:100-102
+    if (rc) return rc;
+    if ((rc = launch_gather(c))) return rc;                                 // cg.cc:135-136 (moved)
+    return launch_vector_phase(c, m);
+}
+
+// ---- persistent schedule (persist.cu) ------------------------------------------------
+// The persistent kernel exists for the tile shapes listed in persist.cu; it needs one CTA per SM,
+// the fused exchange (or one rank), at most persist_max_chunks() vector chunks per CTA and the
+// scratch for the block / chunk partials next to the tile ring in shared memory.
+int persist_index(const cgb_ctx *c)
+{
+    const char *name = gemv_variant(c->variant).name;
+    for (int i = 0; i < persist_variant_count(); ++i)
+        if (strcmp(persist_variant(i).name, name) == 0) return i;
+    return -1;
+}
+
+void persist_scratch(const cgb_ctx *c, int *scr_n)
+{
+    const long long scr = c->nchunks > c->nblk ? c->nchunks : c->nblk; // chunk partials / per-CTA timings
+    *scr_n = (int)((scr + 1) & ~1LL);
+}
+
+// nullptr when the persistent schedule can run this context as configured, else the reason; `profile`:
+// "profile" is in force (a device solve runs as if it were 0)
+const char *persist_unusable(const cgb_ctx *c, bool profile)
+{
+    if (c->storage == 1) return "CSR storage";
+    if (c->opt_compat) return "compat mat-vec";
+    if (profile) return "profile mode (per-launch events)";
+    if (c->world > 1 && c->opt_exchange != 1) return "ncclAllGather exchange";
+    if (gemv_variant(c->variant).ctas_per_sm != 1) return "variant runs 2 CTAs per SM";
+    const int pi = persist_index(c);
+    if (pi < 0) return "no persistent instantiation of this tile shape";
+    if (c->nchunks > (long long)persist_max_chunks() * c->nblk) return "N too large for the per-CTA vector chunks";
+    int scr_n;
+    persist_scratch(c, &scr_n);
+    if (persist_variant(pi).smem_fixed() + (size_t)scr_n * 8 + 4096 > (size_t)c->smem_optin) // + static
+        return "tile ring + scratch exceed shared memory";
+    return nullptr;
+}
+
+int launch_persist(cgb_ctx *c, long long iters, const Mode &m)
+{
+    PersistArgs a;
+    memset(&a, 0, sizeof a);
+    a.A = c->A;
+    a.env = c->env;
+    a.x = c->x;
+    a.r = c->r;
+    a.p = c->p;
+    a.rrpart = c->rrpart;
+    peer_pointers(c, a.peer_ll);
+    a.ll = c->ll;
+    a.rr_ll = c->rr_ll;
+    a.rr_stride = c->aux_stride;
+    a.sync = c->psync;
+    a.st = c->run.st;
+    a.ctl = c->ctl;
+    a.hist = m.hist;
+    a.host_done = m.host_done;
+    a.ld = c->ld;
+    a.rows = c->rows;
+    a.row0 = c->row0;
+    a.n = c->n;
+    a.maxrows = c->maxrows;
+    a.n_loc = c->n_loc > 0 ? c->n_loc : 1;
+    a.loc_cap = loopback_cap(c);
+    a.slot = c->slot;
+    a.bufstride = c->bufstride;
+    a.slot_off = (long long)c->rank * c->slot;
+    a.nchunks = c->nchunks;
+    a.rank = c->rank;
+    a.world = c->world;
+    a.iters = (int)iters;
+    a.l2_prefetch = c->opt_l2_prefetch;
+    a.l2_ramp = c->opt_l2_ramp;
+    a.balance = c->opt_balance;
+    persist_scratch(c, &a.scr_n);
+    a.tol = c->run.tol;
+    a.spin_ns = (unsigned long long)c->spin_timeout_ms * 1000000ULL;
+    if (c->trace_cap > 0) a.trace = make_trace(c, 0, c->nblk);
+    CK(cudaMemsetAsync(c->psync, 0, sizeof(PersistSync), c->stream));
+    CK(persist_variant(persist_index(c)).launch(a, c->nblk, c->stream));
+    c->kernel_launches += 1;
+    c->persist_launches += 1;
+    return CGB_OK;
+}
+
+// ONE cooperative launch per 2^30 loop bodies (its count is an int); it leaves the loop on convergence by itself
+int launch_persist_bodies(cgb_ctx *c, long long todo, const Mode &m)
+{
+    while (todo > 0) {
+        const long long part = std::min<long long>(todo, 1 << 30);
+        const int rc = launch_persist(c, part, m);
+        if (rc) return rc;
+        todo -= part;
+    }
+    return CGB_OK;
+}
+
+bool exchange_configured(const cgb_ctx *c)
+{
+    return c->world == 1 || (c->opt_exchange == 1 ? c->p2p_ready : c->comm != nullptr);
+}
+
+// Hooks that read the gathered result with memcpys: in fused mode first consume the running
+// exchange into the plain buffer (this also advances the epoch, like every consumer kernel).
+int collect_for_host(cgb_ctx *c)
+{
+    const Gather g = make_gather(c);
+    if (g.p2p) {
+        CK(launch_exchange_collect(c->apx, g, c->stream));
+        c->kernel_launches += 1;
+    }
+    return CGB_OK;
+}
+
+// ---- the host loop (cgb_iterate) -------------------------------------------------------------
+// Ends cgb_iterate's timed window: ev1, the wait for it -- a device-side wait that timed out is
+// reported as such -- and the window's time added to the solve's
+int end_window(cgb_ctx *c, SolveRun &run, float *ms)
+{
+    CK(cudaEventRecord(c->ev1, c->stream));
+    cudaError_t e = cudaEventSynchronize(c->ev1);
+    if (e != cudaSuccess) {
+        const int code = *(volatile int *)c->h_done;
+        if (code < 0)
+            return fail(CGB_ERR_TIMEOUT, "a device-side wait (kind %d: 1 = an LL entry -- a peer rank's mat-vec rows or a chunk "
+                        "partial, 4 = p chunks, 5 = tile for the consumers, 6 / 9 = row partition hand-over, 7 = free "
+                        "pipeline stage, 8 = drain, 10 = column-window table) exceeded spin_timeout_ms = %lld: a rank is "
+                        "missing or stuck (%s) [cta %d thread %d: %d %d %d %d]", -code, c->spin_timeout_ms,
+                        cudaGetErrorString(e), c->h_done[1], c->h_done[2], c->h_done[3], c->h_done[4], c->h_done[5],
+                        c->h_done[6]);
+        CK(e);
+    }
+    float t = 0.f;
+    CK(cudaEventElapsedTime(&t, c->ev0, c->ev1));
+    run.loop_ms += t;
+    if (ms) *ms = t;
+    return CGB_OK;
+}
+
+// Up to `todo` loop bodies of the solve in progress on the graph schedule, timed.  `body()` enqueues
+// one body of `per_body` kernels.  Batches of poll_every bodies, each a replay of the cached graph `g`
+// (when `graph` and its L bodies fit the batch) or single bodies; the mapped flag is read between
+// batches, and the host keeps at most two batches in flight so that it never runs far ahead of it.
+template <class F>
+int host_loop(cgb_ctx *c, SolveRun &run, long long todo, bool graph, CachedGraph &g, int per_body, F body, float *ms)
+{
+    int rc;
+    const GraphKey key = graph_key(c, run.nrhs, run.tol, run.hist);
+    const bool replay = graph && todo >= key.len;
+    if (replay && !holds(g, key)) {
+        rc = rebuild(c, g, key, [&](cudaGraph_t gr) {
+            return capture_into(c, gr, nullptr, [&]() -> int {
+                int r = CGB_OK;
+                for (int u = 0; u < key.len && r == CGB_OK; ++u) r = body();
+                return r;
+            }, nullptr);
+        });
+        if (rc) return rc;
+    }
+    // ncclAllGather mode: the collectives of a batch run on every rank or on none, so all
+    // ranks must take the same stop decision -- wait for the batch just issued (the flag is
+    // then the same on every rank) instead of looking one batch back.  The fused exchange
+    // needs no such lockstep: launches after convergence communicate nothing.
+    const bool lockstep = c->world > 1 && c->opt_exchange == 0;
+    CK(cudaEventRecord(c->ev0, c->stream));
+    long long issued = 0;
+    int batch_idx = 0;
+    while (issued < todo) {
+        if (*(volatile int *)c->h_done) break; // converged: later launches would be no-ops
+        const long long batch = std::min<long long>(c->poll_every, todo - issued);
+        long long i = 0;
+        while (i < batch) {
+            if (replay && batch - i >= key.len) {
+                CK(cudaGraphLaunch(g.exec, c->stream));
+                c->kernel_launches += (long long)per_body * key.len;
+                c->graph_replays += 1;
+                i += key.len;
+            } else {
+                if ((rc = body())) return rc;
+                i += 1;
+            }
+        }
+        issued += batch;
+        CK(cudaEventRecord(c->ev_batch[batch_idx & 1], c->stream));
+        if (lockstep) CK(cudaEventSynchronize(c->ev_batch[batch_idx & 1]));
+        else if (batch_idx >= 1) CK(cudaEventSynchronize(c->ev_batch[(batch_idx - 1) & 1]));
+        ++batch_idx;
+    }
+    run.launched += issued;
+    return end_window(c, run, ms);
+}
+
+// cgb_solve_end / cgb_solve_block_end after the finalize kernel: the States, each column's executed
+// r'r history (to resid_hist + j * max_iter) and its cgb_solve_info
+int collect_solve(cgb_ctx *c, const SolveRun &run, double *resid_hist, cgb_solve_info *info)
+{
+    State s[kMaxRhs];
+    CK(cudaMemcpyAsync(s, run.st, (size_t)run.nrhs * sizeof(State), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    for (int j = 0; j < run.nrhs; ++j) {
+        const long long executed = s[j].done ? s[j].iter + 1 : s[j].iter;
+        if (resid_hist && executed > 0)
+            CK(cudaMemcpyAsync(resid_hist + (size_t)j * run.max_iter, run.hist + (size_t)j * run.hist_ld,
+                               (size_t)executed * 8, cudaMemcpyDeviceToHost, c->stream));
+        if (info) {
+            info[j].k = s[j].iter;
+            info[j].converged = s[j].done;
+            info[j].rsold = s[j].rsold;
+            info[j].rsnew = s[j].rsnew;
+            info[j].seconds = run.loop_ms * 1e-3;
+            info[j].iterations = executed;
+        }
+    }
+    CK(cudaStreamSynchronize(c->stream));
+    return CGB_OK;
+}
+
+// ---- block solve ---------------------------------------------------------------------------
+void free_block_vectors(cgb_ctx *c)
+{
+    BlockSolve &k = c->blk;
+    double *bufs[] = {k.x, k.r, k.p, k.b, k.ap, k.rrpart, k.papart};
+    for (double *p : bufs)
+        if (p) cudaFree(p);
+    if (k.run.st) cudaFree(k.run.st);
+    if (k.arrive) cudaFree(k.arrive);
+    k.x = k.r = k.p = k.b = k.ap = k.rrpart = k.papart = nullptr;
+    k.run.st = nullptr;
+    k.arrive = nullptr;
+    k.cap = 0;
+}
+
+// buffers for nrhs columns and, with a history, max(max_iter, 1) entries per column; grows only
+int size_block(cgb_ctx *c, int nrhs, long long max_iter, bool history)
+{
+    BlockSolve &k = c->blk;
+    auto alloc = [&](void **p, size_t bytes) -> int {
+        cudaError_t e = cudaMalloc(p, bytes);
+        if (e == cudaSuccess) e = cudaMemsetAsync(*p, 0, bytes, c->stream);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            return fail(e == cudaErrorMemoryAllocation ? CGB_ERR_NOMEM : CGB_ERR_CUDA, "block solve buffers: %s",
+                        cudaGetErrorString(e));
+        }
+        return CGB_OK;
+    };
+    int rc = CGB_OK;
+    const long long hist_need = max_iter > 0 ? max_iter : 1;
+    if (nrhs > k.cap) {
+        if (k.cap == 0) { // first block solve of this context
+            CK(preload_spmv_block_kernels());
+            CK(preload_vec_block_kernels());
+        }
+        c->graph_gen += 1; // the block graphs bake in the buffers
+        free_block_vectors(c);
+        const size_t vec = (size_t)nrhs * c->ld * sizeof(double);
+        const size_t part = (size_t)nrhs * c->nchunks * sizeof(double);
+        if ((rc = alloc((void **)&k.x, vec)) || (rc = alloc((void **)&k.r, vec)) || (rc = alloc((void **)&k.p, vec)) ||
+            (rc = alloc((void **)&k.b, vec)) || (rc = alloc((void **)&k.ap, (size_t)nrhs * c->slot_cap * sizeof(double))) ||
+            (rc = alloc((void **)&k.rrpart, part)) || (rc = alloc((void **)&k.papart, part)) ||
+            (rc = alloc((void **)&k.run.st, (size_t)nrhs * sizeof(State))) ||
+            (rc = alloc((void **)&k.arrive, (size_t)(2 * nrhs + 1) * sizeof(unsigned int)))) {
+            free_block_vectors(c);
+            return rc;
+        }
+        k.cap = nrhs;
+        if (k.hist_buf) cudaFree(k.hist_buf); // its column stride follows from the new capacity
+        k.hist_buf = nullptr;
+        k.hist_cap = 0;
+    }
+    if (history && hist_need > k.hist_cap) {
+        c->graph_gen += 1;
+        if (k.hist_buf) cudaFree(k.hist_buf);
+        k.hist_buf = nullptr;
+        k.hist_cap = 0;
+        if ((rc = alloc((void **)&k.hist_buf, (size_t)k.cap * hist_need * sizeof(double)))) return rc;
+        k.hist_cap = hist_need;
+    }
+    return CGB_OK;
+}
+
+// the block solve's run for nrhs columns, after size_block
+void start_block_run(cgb_ctx *c, int nrhs, long long max_iter, double tol, bool history)
+{
+    SolveRun &run = c->blk.run;
+    run.nrhs = nrhs;
+    run.max_iter = max_iter;
+    run.tol = tol;
+    run.launched = 0;
+    run.loop_ms = 0.0;
+    run.hist = history ? c->blk.hist_buf : nullptr;
+    run.hist_ld = c->blk.hist_cap;
+}
+
+BlockArgs make_block_args(const cgb_ctx *c, const double *v, int advance, const Mode &m)
+{
+    const BlockSolve &k = c->blk;
+    BlockArgs a;
+    memset(&a, 0, sizeof a);
+    a.rp = c->csr.rp;
+    a.col = c->csr.col;
+    a.val = c->csr.val;
+    a.v = v;
+    a.x = k.x;
+    a.r = k.r;
+    a.p = k.p;
+    a.b = k.b;
+    a.ap = k.ap;
+    a.rrpart = k.rrpart;
+    a.papart = k.papart;
+    a.st = k.run.st;
+    a.arrive = k.arrive;
+    a.ndone = k.arrive + 2 * k.cap;
+    a.host_done = m.host_done;
+    a.hist = m.hist;
+    a.n = c->n;
+    a.ld = c->ld;
+    a.rows = c->rows;
+    a.slot = c->slot_cap;
+    a.nchunks = c->nchunks;
+    a.hist_ld = k.run.hist_ld;
+    a.nrhs = k.run.nrhs;
+    a.advance = advance;
+    a.pdl = (advance && m.pdl) ? 1 : 0; // only inside the CG loop
+    a.tol = k.run.tol;
+    return a;
+}
+
+// mat-vec + the three vector kernels of one block iteration
+int launch_block_iteration(cgb_ctx *c, const Mode &m)
+{
+    const BlockArgs a = make_block_args(c, c->blk.p, 1, m);
+    CK(launch_spmv_block(a, c->sm_count, c->stream));
+    CK(launch_pap_alpha_block(a, c->stream));
+    CK(launch_update_xr_block(a, c->stream));
+    CK(launch_update_p_block(a, c->stream));
+    c->kernel_launches += 4;
+    return CGB_OK;
+}
+
+// ---- device solves -------------------------------------------------------------------------
+// Pointers a device solve takes: device memory of the context's GPU (or managed memory)
+int check_device_ptr(const cgb_ctx *c, const void *p, const char *what)
+{
+    if (!p) return fail(CGB_ERR_INVALID, "null %s", what);
+    cudaPointerAttributes a;
+    cudaError_t e = cudaPointerGetAttributes(&a, p);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(CGB_ERR_INVALID, "%s is not a pointer CUDA knows (%s)", what, cudaGetErrorString(e));
+    }
+    if (a.type == cudaMemoryTypeManaged) return CGB_OK;
+    if (a.type != cudaMemoryTypeDevice)
+        return fail(CGB_ERR_INVALID, "%s is host memory: a device solve takes device pointers", what);
+    if (a.device != c->device)
+        return fail(CGB_ERR_INVALID, "%s lives on device %d, the context on device %d", what, a.device, c->device);
+    return CGB_OK;
+}
+
+// The loop of a device solve as one graph (DESIGN 3.9), captured into `g`:
 //   head -> WHILE { len loop bodies ; ctl } -> mid -> WHILE { 1 loop body ; ctl }
 // head, mid and ctl are loop_ctl_kernel: each sets the condition of the WHILE node it precedes or
 // runs in -- the stop test has not fired and the bodies issued so far leave room for the next
 // body under max_iter.  So no loop body starts past max_iter, and the count of bodies issued is the
 // host loop's (whole graphs of `len`, then single iterations), short of the no-op bodies the host
-// issues after the stop test fired.  `body` enqueues one loop body on c->stream.
-int build_loop(cgb_ctx *c, DeviceLoop &d, int len, const int *done, const unsigned int *ndone, int nrhs,
-               int (*body)(cgb_ctx *))
+// issues after the stop test fired.  `body()` enqueues one loop body on c->stream.
+template <class F>
+int capture_loop(cgb_ctx *c, cudaGraph_t g, int len, const int *done, const unsigned int *ndone, int nrhs, F body)
 {
-    drop_loop(d);
-    CK(cudaGraphCreate(&d.graph, 0));
-    const long long before = c->kernel_launches;
     int rc = CGB_OK;
     cudaGraphNode_t tail = nullptr;
     for (int part = 0; part < 2 && rc == CGB_OK; ++part) {
         const int step = part == 0 ? len : 1;
         cudaGraphConditionalHandle h;
-        CK(cudaGraphConditionalHandleCreate(&h, d.graph, 0, cudaGraphCondAssignDefault));
+        CK(cudaGraphConditionalHandleCreate(&h, g, 0, cudaGraphCondAssignDefault));
         cudaGraphNode_t ctl = nullptr;
-        rc = capture_into(c, d.graph, tail, [&]() -> int {
+        rc = capture_into(c, g, tail, [&]() -> int {
             CK(launch_loop_ctl(c->loopctl, done, ndone, nrhs, h, 1, step, 0, part == 0 ? 1 : 0, c->stream));
             return CGB_OK;
         }, &ctl);
@@ -870,63 +890,44 @@ int build_loop(cgb_ctx *c, DeviceLoop &d, int len, const int *done, const unsign
         p.conditional.handle = h;
         p.conditional.type = cudaGraphCondTypeWhile;
         p.conditional.size = 1;
-        CK(cudaGraphAddNode(&tail, d.graph, &ctl, 1, &p));
+        CK(cudaGraphAddNode(&tail, g, &ctl, 1, &p));
         rc = capture_into(c, p.conditional.phGraph_out[0], nullptr, [&]() -> int {
             int r = CGB_OK;
-            for (int u = 0; u < step && r == CGB_OK; ++u) r = body(c);
+            for (int u = 0; u < step && r == CGB_OK; ++u) r = body();
             if (r == CGB_OK) CK(launch_loop_ctl(c->loopctl, done, ndone, nrhs, h, 1, step, step, 0, c->stream));
             return r;
         }, nullptr);
     }
-    c->kernel_launches = before; // capture launches nothing
-    if (rc) return rc;
-    CK(cudaGraphInstantiate(&d.exec, d.graph, 0));
-    d.len = len;
-    d.pdl = c->opt_pdl;
-    return CGB_OK;
+    return rc;
 }
 
-// The cached loop graph when its key still holds, else a new one.  The bodies are captured with
+// A device solve's loop on the graph schedule, launched: the cached loop graph `d` when its key still
+// holds, else a new capture.  The bodies (`body(mode)`, `per_body` kernels) are captured with
 // programmatic dependent launches when "pdl" asks for them; should the driver refuse them inside a
-// conditional body, they are captured without (DeviceLoop::pdl_used, option "device_loop_pdl").
-int ensure_loop(cgb_ctx *c, DeviceLoop &d, int len, int nrhs, double tol, const double *hist, long long gen,
-                const int *done, const unsigned int *ndone, int (*body)(cgb_ctx *))
+// conditional body, they are captured without (CachedGraph::pdl_used, option "device_loop_pdl").
+// Its kernels count as if the loop ran to max_iter: the host does not learn where it stops.
+template <class F>
+int launch_loop_graph(cgb_ctx *c, CachedGraph &d, const GraphKey &key, Mode m, const int *done,
+                      const unsigned int *ndone, int per_body, long long max_iter, F body)
 {
-    const void *m0 = c->storage == 1 ? (const void *)c->csr.col : (const void *)c->A;
-    const void *m1 = c->storage == 1 ? (const void *)c->csr.val : (const void *)c->env;
-    if (d.exec && d.len == len && d.nrhs == nrhs && d.tol == tol && d.hist == hist && d.gen == gen &&
-        d.pdl == c->opt_pdl && d.mat0 == m0 && d.mat1 == m1)
-        return CGB_OK;
-    const int want_pdl = c->opt_pdl;
-    int rc = build_loop(c, d, len, done, ndone, nrhs, body);
-    d.pdl_used = want_pdl;
-    if (rc && want_pdl) {
-        cudaGetLastError();
-        c->opt_pdl = 0; // DeviceLaunch restores it
-        rc = build_loop(c, d, len, done, ndone, nrhs, body);
-        d.pdl_used = 0;
+    if (!holds(d, key)) {
+        auto build = [&](cudaGraph_t g) {
+            return capture_loop(c, g, key.len, done, ndone, key.nrhs, [&]() { return body(m); });
+        };
+        int rc = rebuild(c, d, key, build);
+        d.pdl_used = m.pdl;
+        if (rc && m.pdl) {
+            cudaGetLastError();
+            m.pdl = 0;
+            rc = rebuild(c, d, key, build);
+            d.pdl_used = 0;
+        }
+        if (rc) return rc;
     }
-    if (rc) {
-        drop_loop(d);
-        return rc;
-    }
-    d.pdl = want_pdl;
-    d.nrhs = nrhs;
-    d.tol = tol;
-    d.hist = hist;
-    d.gen = gen;
-    d.mat0 = m0;
-    d.mat1 = m1;
+    CK(cudaGraphLaunch(d.exec, c->stream));
+    c->graph_replays += 1;
+    c->kernel_launches += per_body * max_iter + 2 + max_iter / key.len + max_iter % key.len;
     return CGB_OK;
-}
-
-int single_body(cgb_ctx *c) { return launch_iteration(c); }
-int block_body(cgb_ctx *c) { return launch_block_iteration(c); }
-
-// kernels of the loop graph when it runs to max_iter (the host does not learn where it stops)
-long long loop_kernels(long long max_iter, int len, int per_body)
-{
-    return per_body * max_iter + 2 + max_iter / len + max_iter % len;
 }
 
 } // namespace
@@ -1064,7 +1065,7 @@ static int create_ctx(int64_t n, int rank, int world, int device, int storage, c
     CKB(cudaMemsetAsync(c->papart, 0, (size_t)c->nchunks * sizeof(double), c->stream));
     CKB(cudaMalloc(&c->scratch, (size_t)(3 * c->nchunks + 8) * sizeof(double)));
     CKB(cudaMalloc(&c->sink, 64));
-    CKB(cudaMalloc(&c->st, sizeof(State)));
+    CKB(cudaMalloc(&c->run.st, sizeof(State)));
     CKB(cudaHostAlloc(&c->h_done, 8 * sizeof(int), cudaHostAllocMapped)); // [0] flag, [1..6] context of a timeout report
     CKB(cudaHostGetDevicePointer(&c->d_hdone, c->h_done, 0));
     CKB(cudaHostAlloc(&c->h_pin, 64 * sizeof(double), cudaHostAllocDefault));
@@ -1075,7 +1076,7 @@ static int create_ctx(int64_t n, int rank, int world, int device, int storage, c
     CKB(cudaMemsetAsync(c->b, 0, vec_bytes, c->stream));
     CKB(cudaMemsetAsync(c->apx, 0, (size_t)c->bufstride * sizeof(double), c->stream));
     CKB(cudaMemsetAsync(c->rrpart, 0, (size_t)c->nchunks * sizeof(double), c->stream));
-    CKB(cudaMemsetAsync(c->st, 0, sizeof(State), c->stream));
+    CKB(cudaMemsetAsync(c->run.st, 0, sizeof(State), c->stream));
     CKB(cudaStreamSynchronize(c->stream));
     CKB(preload_vec_kernels());
     if (storage == 1) {
@@ -1104,15 +1105,15 @@ extern "C" int cgb_destroy(cgb_ctx *c)
     if (!c) return CGB_OK;
     cudaSetDevice(c->device);
     if (c->stream) cudaStreamSynchronize(c->stream);
-    drop_graph(c);
+    drop_graphs(c);
     if (c->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(c->comm);
     for (cudaEvent_t e : c->prof_ev) cudaEventDestroy(e);
     for (void *p : c->ipc_opened)
         if (p) cudaIpcCloseMemHandle(p);
-    double *bufs[] = {c->A, c->p, c->r, c->x, c->b, c->apx, c->rrpart, c->papart, c->scratch, c->hist, c->sink};
+    double *bufs[] = {c->A, c->p, c->r, c->x, c->b, c->apx, c->rrpart, c->papart, c->scratch, c->run.hist, c->sink};
     for (double *p : bufs)
         if (p) cudaFree(p);
-    if (c->st) cudaFree(c->st);
+    if (c->run.st) cudaFree(c->run.st);
     if (c->env) cudaFree(c->env);
     if (c->csr.rp) cudaFree(c->csr.rp);
     if (c->csr.col) cudaFree(c->csr.col);
@@ -1126,8 +1127,8 @@ extern "C" int cgb_destroy(cgb_ctx *c)
     if (c->ctl) cudaFree(c->ctl);
     if (c->h_done) cudaFreeHost(c->h_done);
     if (c->h_pin) cudaFreeHost(c->h_pin);
-    free_block(c);
-    drop_loop(c->dloop);
+    free_block_vectors(c);
+    if (c->blk.hist_buf) cudaFree(c->blk.hist_buf);
     if (c->loopctl) cudaFree(c->loopctl);
     if (c->dev_hist) cudaFree(c->dev_hist);
     for (cudaEvent_t e : c->ev_dev)
@@ -1233,7 +1234,7 @@ extern "C" int cgb_exchange_import(cgb_ctx *c, const void *blobs)
     }
     c->p2p_ready = true;
     c->opt_exchange = 1;
-    drop_graph(c);
+    c->graph_gen += 1;
     return CGB_OK;
 }
 
@@ -1245,6 +1246,7 @@ extern "C" int cgb_generate_lap2d(cgb_ctx *c)
     if (c->in_solve) return fail(CGB_ERR_STATE, "solve in progress");
     if (c->storage == 1) {
         c->matrix_set = false;
+        c->graph_gen += 1; // the builders reallocate col / val, which the loop graphs bake in
         CK(csr_generate_lap2d(&c->csr, c->n, c->row0, c->rows, c->stream));
         c->kernel_launches += 3;
     } else {
@@ -1320,6 +1322,7 @@ extern "C" int cgb_set_matrix_coo(cgb_ctx *c, int64_t nz, const int32_t *irn, co
         }
         int bad = 0;
         c->matrix_set = false;
+        c->graph_gen += 1;
         CK(csr_from_coo(&c->csr, c->n, c->row0, c->rows, t.i, t.j, t.v, nz, symmetric ? 1 : 0, &bad, c->stream));
         if (bad) return fail(CGB_ERR_INVALID, "a COO entry lies outside %lld x %lld", (long long)c->n, (long long)c->n);
         c->matrix_set = true;
@@ -1420,7 +1423,7 @@ extern "C" int cgb_set_option(cgb_ctx *c, const char *key, int64_t value)
         if (value < 0 || value >= gemv_variant_count())
             return fail(CGB_ERR_INVALID, "gemv_variant %lld out of range", (long long)value);
         set_variant(c, (int)value);
-        drop_graph(c);
+        c->graph_gen += 1;
         if (use_device(c) == CGB_OK) {
             gemv_variant(c->variant).preload();
             if (persist_index(c) >= 0) persist_variant(persist_index(c)).preload();
@@ -1435,7 +1438,7 @@ extern "C" int cgb_set_option(cgb_ctx *c, const char *key, int64_t value)
     } else if (k == "graph_unroll") {
         if (value < 1 || value > 64) return fail(CGB_ERR_INVALID, "graph_unroll must be in [1, 64]");
         c->graph_unroll = (int)value;
-        drop_graph(c);
+        c->graph_gen += 1;
     } else if (k == "compat") {
         if (value != 0) {
             if (c->world != 1) return fail(CGB_ERR_INVALID, "compat mat-vec is single-GPU (like the reference CUDA program)");
@@ -1456,17 +1459,17 @@ extern "C" int cgb_set_option(cgb_ctx *c, const char *key, int64_t value)
             }
         }
         c->opt_compat = value != 0;
-        drop_graph(c);
+        c->graph_gen += 1;
     } else if (k == "pdl") {
         c->opt_pdl = value != 0;
-        drop_graph(c);
+        c->graph_gen += 1;
     } else if (k == "l2_ramp") {
         if (value < 0 || value > 64) return fail(CGB_ERR_INVALID, "l2_ramp must be in [0, 64] pipeline steps");
         c->opt_l2_ramp = (int)value;
     } else if (k == "l2_prefetch") {
         if (value < 0 || value > 64) return fail(CGB_ERR_INVALID, "l2_prefetch must be in [0, 64] pipeline steps");
         c->opt_l2_prefetch = (int)value;
-        drop_graph(c);
+        c->graph_gen += 1;
     } else if (k == "balance") {
         c->opt_balance = value != 0;
     } else if (k == "schedule") {
@@ -1482,7 +1485,7 @@ extern "C" int cgb_set_option(cgb_ctx *c, const char *key, int64_t value)
         if (rc) return rc;
         CK(cudaStreamSynchronize(c->stream));
         free_trace(c);
-        drop_graph(c);
+        c->graph_gen += 1;
         if (value > 0) {
             int max_cps = 1;
             for (int v = 0; v < gemv_variant_count(); ++v)
@@ -1514,7 +1517,7 @@ extern "C" int cgb_set_option(cgb_ctx *c, const char *key, int64_t value)
             c->p2p_ready = false;
             c->opt_exchange = 0;
         }
-        drop_graph(c);
+        c->graph_gen += 1;
     } else if (k == "exchange") {
         if (value != 0 && value != 1) return fail(CGB_ERR_INVALID, "exchange must be 0 (nccl) or 1 (fused p2p)");
         if (c->world > 1 && value == 1 && !c->p2p_ready)
@@ -1522,18 +1525,18 @@ extern "C" int cgb_set_option(cgb_ctx *c, const char *key, int64_t value)
         if (c->world > 1 && value == 0 && !c->comm)
             return fail(CGB_ERR_STATE, "exchange = 0 needs cgb_comm_init first");
         c->opt_exchange = (int)value;
-        drop_graph(c);
+        c->graph_gen += 1;
     } else if (k == "num_threads") {
         c->opt_num_threads = (int)value;
         c->opt_compat = 0; // re-enable with "compat" = 1 (re-validates, re-sizes the partial buffer)
-        drop_graph(c);
+        c->graph_gen += 1;
     } else if (k == "block_width") {
         c->opt_block_width = (int)value;
         c->opt_compat = 0;
-        drop_graph(c);
+        c->graph_gen += 1;
     } else if (k == "transposed") {
         c->opt_transposed = value != 0;
-        drop_graph(c);
+        c->graph_gen += 1;
     } else {
         return fail(CGB_ERR_INVALID, "unknown option '%s'", key);
     }
@@ -1550,7 +1553,7 @@ extern "C" int cgb_get_option(cgb_ctx *c, const char *key, int64_t *value)
     else if (k == "poll_every") *value = c->poll_every;
     else if (k == "graph_unroll") *value = c->graph_unroll;
     else if (k == "graph_replays") *value = c->graph_replays;
-    else if (k == "device_loop_pdl") *value = c->dloop.pdl_used >= 0 ? c->dloop.pdl_used : c->blk.dloop.pdl_used;
+    else if (k == "device_loop_pdl") *value = c->loop_single.pdl_used >= 0 ? c->loop_single.pdl_used : c->loop_block.pdl_used;
     else if (k == "compat") *value = c->opt_compat;
     else if (k == "pdl") *value = c->opt_pdl;
     else if (k == "l2_prefetch") *value = c->opt_l2_prefetch;
@@ -1559,7 +1562,7 @@ extern "C" int cgb_get_option(cgb_ctx *c, const char *key, int64_t *value)
     else if (k == "trace") *value = c->trace_cap;
     else if (k == "schedule") *value = c->opt_schedule;
     else if (k == "balance") *value = c->opt_balance;
-    else if (k == "schedule_in_use") *value = (c->opt_schedule == 1 && !persist_unusable(c)) ? 1 : 0;
+    else if (k == "schedule_in_use") *value = (c->opt_schedule == 1 && !persist_unusable(c, c->opt_profile)) ? 1 : 0;
     else if (k == "spin_timeout_ms") *value = c->spin_timeout_ms;
     else if (k == "loopback") *value = c->opt_loopback;
     else if (k == "num_threads") *value = c->opt_num_threads;
@@ -1610,41 +1613,39 @@ extern "C" int cgb_solve_begin(cgb_ctx *c, const double *x0_host, int64_t max_it
     if (max_iter < 0) return fail(CGB_ERR_INVALID, "max_iter < 0");
     if (!exchange_configured(c))
         return fail(CGB_ERR_STATE, "world > 1 but neither cgb_comm_init nor cgb_exchange_import was called");
-    c->max_iter = max_iter;
-    c->tol = tol;
-    if (c->graph_exec && c->graph_tol != tol) drop_graph(c);
-    c->launched = 0;
-    c->loop_ms = 0.0;
+    SolveRun &run = c->run;
+    run.max_iter = max_iter;
+    run.tol = tol;
+    run.launched = 0;
+    run.loop_ms = 0.0;
     c->prof_gemv_ms = 0.0;
     c->prof_gemv_n = 0;
     if (keep_history) {
         const long long need = max_iter > 0 ? max_iter : 1;
         if (need > c->hist_cap) {
-            if (c->hist) cudaFree(c->hist);
-            c->hist = nullptr;
+            if (run.hist) cudaFree(run.hist);
+            run.hist = nullptr;
             c->hist_cap = 0;
-            CK(cudaMalloc(&c->hist, (size_t)need * sizeof(double)));
+            CK(cudaMalloc(&run.hist, (size_t)need * sizeof(double)));
             c->hist_cap = need;
-            drop_graph(c); // the history pointer is baked into captured kernel arguments
+            c->graph_gen += 1;
         }
-        CK(cudaMemsetAsync(c->hist, 0, (size_t)c->hist_cap * sizeof(double), c->stream));
-    } else if (c->hist) {
-        cudaFree(c->hist);
-        c->hist = nullptr;
+        CK(cudaMemsetAsync(run.hist, 0, (size_t)c->hist_cap * sizeof(double), c->stream));
+    } else if (run.hist) {
+        cudaFree(run.hist);
+        run.hist = nullptr;
         c->hist_cap = 0;
-        drop_graph(c);
+        c->graph_gen += 1;
     }
-    State s0;
-    memset(&s0, 0, sizeof s0);
-    s0.iter = -1;
     *c->h_done = 0;
-    CK(cudaMemcpyAsync(c->st, &s0, sizeof s0, cudaMemcpyHostToDevice, c->stream));
+    if ((rc = reset_states(c, run.st, 1))) return rc;
     if (x0_host) CK(cudaMemcpyAsync(c->x, x0_host, (size_t)c->n * 8, cudaMemcpyHostToDevice, c->stream));
     else CK(cudaMemsetAsync(c->x, 0, (size_t)c->ld * 8, c->stream));
     // r = b - A x0 ; p = r ; partials of r.p                          cg.cc:77-92
-    if ((rc = launch_matvec(c, c->x, 0, c->variant))) return rc;
+    const Mode m = host_mode(c);
+    if ((rc = launch_matvec(c, c->x, 0, c->variant, m))) return rc;
     if ((rc = launch_gather(c))) return rc;
-    CK(launch_init_residual(make_vec_args(c), c->stream));
+    CK(launch_init_residual(make_vec_args(c, m), c->stream));
     c->kernel_launches += 1;
     CK(cudaStreamSynchronize(c->stream));
     c->in_solve = true;
@@ -1657,46 +1658,23 @@ extern "C" int cgb_iterate(cgb_ctx *c, int64_t iters, float *ms)
     if (rc) return rc;
     if (!c->in_solve) return fail(CGB_ERR_STATE, "cgb_solve_begin was not called");
     if (iters < 0) return fail(CGB_ERR_INVALID, "iters < 0");
-    if (c->blk.active) return block_iterate(c, iters, ms);
-    long long todo = std::min<long long>(iters, c->max_iter - c->launched);
+    SolveRun &run = c->blk.active ? c->blk.run : c->run;
+    long long todo = std::min<long long>(iters, run.max_iter - run.launched);
     if (todo < 0) todo = 0;
-    const bool profile = c->opt_profile != 0;
-    const bool graph = c->opt_graph != 0 && !profile;
-    const bool lockstep = c->world > 1 && c->opt_exchange == 0;
-    if (c->opt_schedule == 1 && !persist_unusable(c) && todo > 0) {
-        // ONE cooperative launch runs all `todo` loop bodies (it leaves the loop by itself on
-        // convergence): no graph, no per-iteration launch, no host polling
+    if (c->blk.active) {
+        const Mode m = {run.hist, c->d_hdone, c->opt_pdl};
+        return host_loop(c, run, todo, c->opt_graph != 0, c->graph_block, 4,
+                         [&]() { return launch_block_iteration(c, m); }, ms);
+    }
+    const Mode m = host_mode(c);
+    if (c->opt_schedule == 1 && !persist_unusable(c, c->opt_profile) && todo > 0) {
+        // no graph, no per-iteration launch, no host polling
         CK(cudaEventRecord(c->ev0, c->stream));
-        while (todo > 0) {
-            const long long part = std::min<long long>(todo, 1 << 30);
-            if ((rc = launch_persist(c, part))) return rc;
-            todo -= part;
-            c->launched += part;
-        }
-        CK(cudaEventRecord(c->ev1, c->stream));
-        cudaError_t e = cudaEventSynchronize(c->ev1);
-        if (e != cudaSuccess) {
-            const int code = *(volatile int *)c->h_done;
-            if (code < 0)
-                return fail(CGB_ERR_TIMEOUT, "a device-side wait (kind %d: 1 = an LL entry -- a peer rank's mat-vec rows or a chunk "
-                            "partial, 4 = p chunks, 5 = tile for the consumers, 6 / 9 = row partition hand-over, 7 = free "
-                            "pipeline stage, 8 = drain, 10 = column-window table) exceeded spin_timeout_ms = %lld: a rank is "
-                            "missing or stuck (%s) [cta %d thread %d: %d %d %d %d]", -code, c->spin_timeout_ms,
-                            cudaGetErrorString(e), c->h_done[1], c->h_done[2], c->h_done[3], c->h_done[4], c->h_done[5],
-                            c->h_done[6]);
-            CK(e);
-        }
-        float t = 0.f;
-        CK(cudaEventElapsedTime(&t, c->ev0, c->ev1));
-        c->loop_ms += t;
-        if (ms) *ms = t;
-        return CGB_OK;
+        if ((rc = launch_persist_bodies(c, todo, m))) return rc;
+        run.launched += todo;
+        return end_window(c, run, ms);
     }
-    const int want_len = c->graph_unroll < c->poll_every ? c->graph_unroll : c->poll_every;
-    if (graph && c->graph_exec && c->graph_len != want_len) drop_graph(c);
-    if (graph && !c->graph_exec && todo >= want_len) {
-        if ((rc = build_graph(c))) return rc;
-    }
+    const bool profile = c->opt_profile != 0;
     if (profile) {
         while ((long long)c->prof_ev.size() < 2 * todo) {
             cudaEvent_t e;
@@ -1704,64 +1682,24 @@ extern "C" int cgb_iterate(cgb_ctx *c, int64_t iters, float *ms)
             c->prof_ev.push_back(e);
         }
     }
-    CK(cudaEventRecord(c->ev0, c->stream));
-    long long issued = 0;
-    int batch_idx = 0;
-    while (issued < todo) {
-        if (*(volatile int *)c->h_done) break; // converged: later launches would be no-ops
-        const long long batch = std::min<long long>(c->poll_every, todo - issued);
-        long long i = 0;
-        while (i < batch) {
-            if (graph && c->graph_exec && batch - i >= c->graph_len) {
-                CK(cudaGraphLaunch(c->graph_exec, c->stream));
-                c->kernel_launches += (c->opt_compat ? 5LL : 4LL) * c->graph_len;
-                c->graph_replays += 1;
-                i += c->graph_len;
-            } else if (profile) {
-                const long long slot = 2 * (issued + i);
-                CK(cudaEventRecord(c->prof_ev[slot], c->stream));
-                if ((rc = launch_matvec(c, c->p, 1, c->variant))) return rc;
-                CK(cudaEventRecord(c->prof_ev[slot + 1], c->stream));
-                if ((rc = launch_gather(c))) return rc;
-                if ((rc = launch_vector_phase(c))) return rc;
-                i += 1;
-            } else {
-                if ((rc = launch_iteration(c))) return rc;
-                i += 1;
-            }
-        }
-        issued += batch;
-        // keep at most two batches in flight so the host never runs far ahead of the stop flag.
-        // ncclAllGather mode: the collectives of a batch run on every rank or on none, so all
-        // ranks must take the same stop decision -- wait for the batch just issued (the flag is
-        // then the same on every rank) instead of looking one batch back.  The fused exchange
-        // needs no such lockstep: launches after convergence communicate nothing.
-        CK(cudaEventRecord(c->ev_batch[batch_idx & 1], c->stream));
-        if (lockstep) CK(cudaEventSynchronize(c->ev_batch[batch_idx & 1]));
-        else if (batch_idx >= 1) CK(cudaEventSynchronize(c->ev_batch[(batch_idx - 1) & 1]));
-        ++batch_idx;
+    long long profiled = 0; // "profile": each body's mat-vec between two events
+    rc = host_loop(c, run, todo, c->opt_graph != 0 && !profile, c->graph_single, c->opt_compat ? 5 : 4, [&]() -> int {
+        if (!profile) return launch_iteration(c, m);
+        const long long slot = 2 * profiled++;
+        CK(cudaEventRecord(c->prof_ev[slot], c->stream));
+        int r = launch_matvec(c, c->p, 1, c->variant, m);
+        if (r) return r;
+        CK(cudaEventRecord(c->prof_ev[slot + 1], c->stream));
+        if ((r = launch_gather(c))) return r;
+        return launch_vector_phase(c, m);
+    }, ms);
+    if (rc) return rc;
+    for (long long k = 0; k < profiled; ++k) {
+        float g = 0.f;
+        CK(cudaEventElapsedTime(&g, c->prof_ev[2 * k], c->prof_ev[2 * k + 1]));
+        c->prof_gemv_ms += g;
     }
-    CK(cudaEventRecord(c->ev1, c->stream));
-    {
-        cudaError_t e = cudaEventSynchronize(c->ev1);
-        if (e != cudaSuccess && *(volatile int *)c->h_done < 0)
-            return fail(CGB_ERR_TIMEOUT, "a wait for a peer rank's mat-vec rows exceeded spin_timeout_ms = %lld: "
-                        "a rank is missing or stuck (%s)", c->spin_timeout_ms, cudaGetErrorString(e));
-        CK(e);
-    }
-    float t = 0.f;
-    CK(cudaEventElapsedTime(&t, c->ev0, c->ev1));
-    c->loop_ms += t;
-    c->launched += issued;
-    if (profile) {
-        for (long long k = 0; k < issued; ++k) {
-            float g = 0.f;
-            CK(cudaEventElapsedTime(&g, c->prof_ev[2 * k], c->prof_ev[2 * k + 1]));
-            c->prof_gemv_ms += g;
-        }
-        c->prof_gemv_n += issued;
-    }
-    if (ms) *ms = t;
+    c->prof_gemv_n += profiled;
     return CGB_OK;
 }
 
@@ -1771,26 +1709,11 @@ extern "C" int cgb_solve_end(cgb_ctx *c, double *x_host, double *resid_hist, cgb
     if (rc) return rc;
     if (!c->in_solve) return fail(CGB_ERR_STATE, "no solve in progress");
     if (c->blk.active) return fail(CGB_ERR_STATE, "a block solve is in progress (cgb_solve_block_end)");
-    CK(launch_finalize(make_vec_args(c), c->stream));
+    if (resid_hist && !c->run.hist) return fail(CGB_ERR_STATE, "history was not requested in cgb_solve_begin");
+    CK(launch_finalize(make_vec_args(c, host_mode(c)), c->stream));
     c->kernel_launches += 1;
-    State s;
-    if ((rc = read_state(c, &s))) return rc;
     if (x_host) CK(cudaMemcpyAsync(x_host, c->x, (size_t)c->n * 8, cudaMemcpyDeviceToHost, c->stream));
-    const long long executed = s.done ? s.iter + 1 : s.iter;
-    if (resid_hist) {
-        if (!c->hist) return fail(CGB_ERR_STATE, "history was not requested in cgb_solve_begin");
-        if (executed > 0)
-            CK(cudaMemcpyAsync(resid_hist, c->hist, (size_t)executed * 8, cudaMemcpyDeviceToHost, c->stream));
-    }
-    CK(cudaStreamSynchronize(c->stream));
-    if (info) {
-        info->k = s.iter;
-        info->converged = s.done;
-        info->rsold = s.rsold;
-        info->rsnew = s.rsnew;
-        info->seconds = c->loop_ms * 1e-3;
-        info->iterations = executed;
-    }
+    if ((rc = collect_solve(c, c->run, resid_hist, info))) return rc;
     c->in_solve = false;
     return CGB_OK;
 }
@@ -1839,25 +1762,17 @@ extern "C" int cgb_solve_block_begin(cgb_ctx *c, int nrhs, const double *b_host,
     if (c->in_solve) return fail(CGB_ERR_STATE, c->blk.active ? "block solve already in progress" : "a single solve is in progress");
     BlockSolve &k = c->blk;
     if ((rc = size_block(c, nrhs, max_iter, keep_history != 0))) return rc;
-    k.nrhs = nrhs;
-    k.max_iter = max_iter;
-    k.tol = tol;
-    k.keep_history = keep_history != 0;
-    k.launched = 0;
-    k.loop_ms = 0.0;
-    if (k.keep_history) CK(cudaMemsetAsync(k.hist, 0, (size_t)k.cap * k.hist_ld * sizeof(double), c->stream));
-    std::vector<State> s0((size_t)nrhs);
-    memset(s0.data(), 0, s0.size() * sizeof(State));
-    for (State &s : s0) s.iter = -1;
-    *k.h_done = 0;
-    CK(cudaMemcpyAsync(k.st, s0.data(), s0.size() * sizeof(State), cudaMemcpyHostToDevice, c->stream));
+    start_block_run(c, nrhs, max_iter, tol, keep_history != 0);
+    if (k.run.hist) CK(cudaMemsetAsync(k.run.hist, 0, (size_t)k.cap * k.hist_cap * sizeof(double), c->stream));
+    *c->h_done = 0;
+    if ((rc = reset_states(c, k.run.st, nrhs))) return rc;
     CK(cudaMemsetAsync(k.arrive, 0, (size_t)(2 * k.cap + 1) * sizeof(unsigned int), c->stream));
     const size_t row = (size_t)c->n * 8, pitch = (size_t)c->ld * 8;
     CK(cudaMemcpy2DAsync(k.b, pitch, b_host, row, row, (size_t)nrhs, cudaMemcpyHostToDevice, c->stream));
     if (x0_host) CK(cudaMemcpy2DAsync(k.x, pitch, x0_host, row, row, (size_t)nrhs, cudaMemcpyHostToDevice, c->stream));
     else CK(cudaMemsetAsync(k.x, 0, (size_t)nrhs * pitch, c->stream));
     // r = b - A x0 ; p = r ; partials of r.p, per column                cg.cc:77-92
-    const BlockArgs a = make_block_args(c, k.x, 0);
+    const BlockArgs a = make_block_args(c, k.x, 0, {k.run.hist, c->d_hdone, c->opt_pdl});
     CK(launch_spmv_block(a, c->sm_count, c->stream));
     CK(launch_init_residual_block(a, c->stream));
     c->kernel_launches += 2;
@@ -1874,30 +1789,12 @@ extern "C" int cgb_solve_block_end(cgb_ctx *c, double *x_host, double *resid_his
     if (rc) return rc;
     BlockSolve &k = c->blk;
     if (!k.active) return fail(CGB_ERR_STATE, "no block solve in progress");
-    if (resid_hist && !k.keep_history) return fail(CGB_ERR_STATE, "history was not requested in cgb_solve_block_begin");
-    const BlockArgs a = make_block_args(c, k.p, 0);
-    CK(launch_finalize_block(a, c->stream));
+    if (resid_hist && !k.run.hist) return fail(CGB_ERR_STATE, "history was not requested in cgb_solve_block_begin");
+    CK(launch_finalize_block(make_block_args(c, k.p, 0, {k.run.hist, c->d_hdone, c->opt_pdl}), c->stream));
     c->kernel_launches += 1;
-    std::vector<State> s((size_t)k.nrhs);
-    CK(cudaMemcpyAsync(s.data(), k.st, s.size() * sizeof(State), cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaStreamSynchronize(c->stream));
     const size_t row = (size_t)c->n * 8, pitch = (size_t)c->ld * 8;
-    if (x_host) CK(cudaMemcpy2DAsync(x_host, row, k.x, pitch, row, (size_t)k.nrhs, cudaMemcpyDeviceToHost, c->stream));
-    for (int j = 0; j < k.nrhs; ++j) {
-        const long long executed = s[j].done ? s[j].iter + 1 : s[j].iter;
-        if (resid_hist && executed > 0)
-            CK(cudaMemcpyAsync(resid_hist + (size_t)j * k.max_iter, k.hist + (size_t)j * k.hist_ld,
-                               (size_t)executed * 8, cudaMemcpyDeviceToHost, c->stream));
-        if (info) {
-            info[j].k = s[j].iter;
-            info[j].converged = s[j].done;
-            info[j].rsold = s[j].rsold;
-            info[j].rsnew = s[j].rsnew;
-            info[j].seconds = k.loop_ms * 1e-3;
-            info[j].iterations = executed;
-        }
-    }
-    CK(cudaStreamSynchronize(c->stream));
+    if (x_host) CK(cudaMemcpy2DAsync(x_host, row, k.x, pitch, row, (size_t)k.run.nrhs, cudaMemcpyDeviceToHost, c->stream));
+    if ((rc = collect_solve(c, k.run, resid_hist, info))) return rc;
     k.active = false;
     c->in_solve = false;
     return CGB_OK;
@@ -1920,28 +1817,55 @@ extern "C" int cgb_solve_block(cgb_ctx *c, int nrhs, const double *b_host, doubl
 }
 
 // ------------------------------------------------------------------ device solves
-// Refusals every device solve shares
-static int device_solve_state(cgb_ctx *c)
+// The refusals both device solves share, and what a context's first device solve allocates
+static int device_solve_check(cgb_ctx *c, const double *B, const double *X, const double *hist_dev,
+                              const cgb_solve_info *info, const char *bname, const char *xname)
 {
     if (c->world > 1)
         return fail(CGB_ERR_STATE, "device solves run on one rank: the exchange of a world > 1 needs the host in lockstep");
     if (c->in_solve)
         return fail(CGB_ERR_STATE, c->blk.active ? "a block solve is in progress" : "a single solve is in progress");
     if (!c->matrix_set) return fail(CGB_ERR_STATE, "matrix not set");
+    int rc;
+    if ((rc = check_device_ptr(c, B, bname)) || (rc = check_device_ptr(c, X, xname)) ||
+        (rc = check_device_ptr(c, info, "info")) || (hist_dev && (rc = check_device_ptr(c, hist_dev, "history"))))
+        return rc;
+    if (c->loopctl) return CGB_OK;
+    CK(preload_loop_kernels());
+    for (cudaEvent_t &e : c->ev_dev)
+        if (!e) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    CK(cudaMalloc(&c->loopctl, sizeof(LoopCtl)));
+    CK(cudaMemsetAsync(c->loopctl, 0, sizeof(LoopCtl), c->stream));
     return CGB_OK;
 }
 
-// caller's stream -> context stream: the solve sees everything enqueued on `us` before the call
-static int device_solve_enter(cgb_ctx *c, cudaStream_t us)
+// The start of both device solves: the caller's stream gates the context's (the solve sees everything
+// enqueued on `us` before the call), b and x0 go into the solve's ld-padded buffers, and device_begin
+// sets the States and the loop's body limit from kernel arguments
+static int device_solve_enter(cgb_ctx *c, cudaStream_t us, int nrhs, long long max_iter, const double *B,
+                              const double *X, double *b, double *x, State *st)
 {
     CK(cudaEventRecord(c->ev_dev[0], us));
     CK(cudaStreamWaitEvent(c->stream, c->ev_dev[0], 0));
+    const size_t row = (size_t)c->n * 8, pitch = (size_t)c->ld * 8;
+    CK(cudaMemcpy2DAsync(b, pitch, B, row, row, (size_t)nrhs, cudaMemcpyDeviceToDevice, c->stream));
+    CK(cudaMemcpy2DAsync(x, pitch, X, row, row, (size_t)nrhs, cudaMemcpyDeviceToDevice, c->stream));
+    CK(launch_device_begin(st, nrhs, c->loopctl, max_iter, c->stream));
+    c->kernel_launches += 1;
     return CGB_OK;
 }
 
-// ... and back: work enqueued on `us` after the call sees x, the history and the info
-static int device_solve_leave(cgb_ctx *c, cudaStream_t us)
+// ... and its end, after the finalize kernel: the info and the executed history into the caller's
+// memory, x back, and the context's stream gates the caller's (work enqueued on `us` after the call
+// sees them)
+static int device_solve_leave(cgb_ctx *c, cudaStream_t us, int nrhs, long long max_iter, const State *st,
+                              const double *hist, long long hist_ld, double *hist_dev, cgb_solve_info *info,
+                              const double *x, double *X)
 {
+    CK(launch_device_info(st, nrhs, c->loopctl, info, hist, hist_ld, hist_dev, max_iter, c->stream));
+    c->kernel_launches += 2; // and finalize
+    const size_t row = (size_t)c->n * 8, pitch = (size_t)c->ld * 8;
+    CK(cudaMemcpy2DAsync(X, row, x, pitch, row, (size_t)nrhs, cudaMemcpyDeviceToDevice, c->stream));
     CK(cudaEventRecord(c->ev_dev[1], c->stream));
     CK(cudaStreamWaitEvent(us, c->ev_dev[1], 0));
     return CGB_OK;
@@ -1953,12 +1877,8 @@ extern "C" int cgb_solve_device(cgb_ctx *c, const double *b_dev, double *x_dev, 
     if (!c) return null_context();
     int rc = use_device(c);
     if (rc) return rc;
-    if ((rc = device_solve_state(c))) return rc;
     if (max_iter < 0) return fail(CGB_ERR_INVALID, "max_iter < 0");
-    if ((rc = check_device_ptr(c, b_dev, "b")) || (rc = check_device_ptr(c, x_dev, "x")) ||
-        (rc = check_device_ptr(c, info_dev, "info")) || (hist_dev && (rc = check_device_ptr(c, hist_dev, "history"))))
-        return rc;
-    if ((rc = prepare_device_solve(c))) return rc;
+    if ((rc = device_solve_check(c, b_dev, x_dev, hist_dev, info_dev, "b", "x"))) return rc;
     const long long hist_need = max_iter > 0 ? max_iter : 1;
     if (hist_dev && hist_need > c->dev_hist_cap) { // grows only; the loop graph is keyed on the pointer
         CK(cudaStreamSynchronize(c->stream));
@@ -1969,42 +1889,26 @@ extern "C" int cgb_solve_device(cgb_ctx *c, const double *b_dev, double *x_dev, 
         c->dev_hist_cap = hist_need;
     }
     const cudaStream_t us = static_cast<cudaStream_t>(stream);
-    DeviceLaunch guard(c, hist_dev ? c->dev_hist : nullptr);
-    c->tol = tol;
-    const size_t bytes = (size_t)c->n * 8;
-    if ((rc = device_solve_enter(c, us))) return rc;
-    // cgb_set_rhs + cgb_solve_begin, stream-ordered: b, x0, State; r = b - A x0 ; p = r ; rsold = r.p
-    CK(cudaMemcpyAsync(c->b, b_dev, bytes, cudaMemcpyDeviceToDevice, c->stream));
-    CK(cudaMemcpyAsync(c->x, x_dev, bytes, cudaMemcpyDeviceToDevice, c->stream));
-    CK(launch_device_begin(c->st, 1, c->loopctl, max_iter, c->stream));
+    const Mode m = {hist_dev ? c->dev_hist : nullptr, nullptr, c->opt_pdl};
+    c->run.tol = tol;
+    if ((rc = device_solve_enter(c, us, 1, max_iter, b_dev, x_dev, c->b, c->x, c->run.st))) return rc;
+    // cgb_solve_begin's r = b - A x0 ; p = r ; rsold = r.p, then cgb_iterate's loop
+    if ((rc = launch_matvec(c, c->x, 0, c->variant, m))) return rc;
+    CK(launch_init_residual(make_vec_args(c, m), c->stream));
     c->kernel_launches += 1;
-    if ((rc = launch_matvec(c, c->x, 0, c->variant))) return rc;
-    CK(launch_init_residual(make_vec_args(c), c->stream));
-    c->kernel_launches += 1;
-    if (c->opt_schedule == 1 && !persist_unusable(c)) {
-        // cgb_iterate's persistent launch: it leaves the loop on convergence by itself
+    if (c->opt_schedule == 1 && !persist_unusable(c, false)) {
         if (max_iter > 0) {
             CK(launch_loop_ctl(c->loopctl, nullptr, nullptr, 0, 0, 0, 1, 0, 1, c->stream)); // start stamp
             c->kernel_launches += 1;
         }
-        for (long long todo = max_iter; todo > 0;) {
-            const long long part = std::min<long long>(todo, 1 << 30);
-            if ((rc = launch_persist(c, part))) return rc;
-            todo -= part;
-        }
+        if ((rc = launch_persist_bodies(c, max_iter, m))) return rc;
     } else {
-        const int len = c->graph_unroll < c->poll_every ? c->graph_unroll : c->poll_every;
-        if ((rc = ensure_loop(c, c->dloop, len, 1, tol, c->dloop_hist, c->graph_gen, &c->st->done, nullptr, single_body)))
-            return rc;
-        CK(cudaGraphLaunch(c->dloop.exec, c->stream));
-        c->graph_replays += 1;
-        c->kernel_launches += loop_kernels(max_iter, len, c->opt_compat ? 5 : 4);
+        rc = launch_loop_graph(c, c->loop_single, graph_key(c, 1, tol, m.hist), m, &c->run.st->done, nullptr,
+                               c->opt_compat ? 5 : 4, max_iter, [&](const Mode &bm) { return launch_iteration(c, bm); });
+        if (rc) return rc;
     }
-    CK(launch_finalize(make_vec_args(c), c->stream));
-    CK(launch_device_info(c->st, 1, c->loopctl, info_dev, c->dloop_hist, 0, hist_dev, 0, c->stream));
-    c->kernel_launches += 2;
-    CK(cudaMemcpyAsync(x_dev, c->x, bytes, cudaMemcpyDeviceToDevice, c->stream));
-    if ((rc = device_solve_leave(c, us))) return rc;
+    CK(launch_finalize(make_vec_args(c, m), c->stream));
+    if ((rc = device_solve_leave(c, us, 1, 0, c->run.st, m.hist, 0, hist_dev, info_dev, c->x, x_dev))) return rc;
     c->rhs_set = true;
     return CGB_OK;
 }
@@ -2019,41 +1923,24 @@ extern "C" int cgb_solve_block_device(cgb_ctx *c, int nrhs, const double *B_dev,
     if (rc) return rc;
     if (c->storage != 1)
         return fail(CGB_ERR_STATE, "block solves need CSR storage: the dense mat-vec streams one p per tile pipeline");
-    if ((rc = device_solve_state(c))) return rc;
-    if ((rc = check_device_ptr(c, B_dev, "B")) || (rc = check_device_ptr(c, X_dev, "X")) ||
-        (rc = check_device_ptr(c, info_dev, "info")) || (hist_dev && (rc = check_device_ptr(c, hist_dev, "history"))))
-        return rc;
-    if ((rc = prepare_device_solve(c))) return rc;
+    if ((rc = device_solve_check(c, B_dev, X_dev, hist_dev, info_dev, "B", "X"))) return rc;
     BlockSolve &k = c->blk;
     if ((rc = size_block(c, nrhs, max_iter, hist_dev != nullptr))) return rc;
-    k.nrhs = nrhs;
-    k.max_iter = max_iter;
-    k.tol = tol;
-    k.keep_history = hist_dev != nullptr;
+    start_block_run(c, nrhs, max_iter, tol, hist_dev != nullptr);
     const cudaStream_t us = static_cast<cudaStream_t>(stream);
-    DeviceLaunch guard(c, nullptr);
-    if ((rc = device_solve_enter(c, us))) return rc;
-    // cgb_solve_block_begin, stream-ordered
-    const size_t row = (size_t)c->n * 8, pitch = (size_t)c->ld * 8;
+    const Mode m = {k.run.hist, nullptr, c->opt_pdl};
+    if ((rc = device_solve_enter(c, us, nrhs, max_iter, B_dev, X_dev, k.b, k.x, k.run.st))) return rc;
+    // cgb_solve_block_begin's initial residuals, then cgb_iterate's loop
     CK(cudaMemsetAsync(k.arrive, 0, (size_t)(2 * k.cap + 1) * sizeof(unsigned int), c->stream));
-    CK(cudaMemcpy2DAsync(k.b, pitch, B_dev, row, row, (size_t)nrhs, cudaMemcpyDeviceToDevice, c->stream));
-    CK(cudaMemcpy2DAsync(k.x, pitch, X_dev, row, row, (size_t)nrhs, cudaMemcpyDeviceToDevice, c->stream));
-    CK(launch_device_begin(k.st, nrhs, c->loopctl, max_iter, c->stream));
-    const BlockArgs a = make_block_args(c, k.x, 0);
+    const BlockArgs a = make_block_args(c, k.x, 0, m);
     CK(launch_spmv_block(a, c->sm_count, c->stream));
     CK(launch_init_residual_block(a, c->stream));
-    c->kernel_launches += 3;
-    const int len = c->graph_unroll < c->poll_every ? c->graph_unroll : c->poll_every;
-    if ((rc = ensure_loop(c, k.dloop, len, nrhs, tol, a.hist, k.gen, nullptr, k.arrive + 2 * k.cap, block_body)))
-        return rc;
-    CK(cudaGraphLaunch(k.dloop.exec, c->stream));
-    c->graph_replays += 1;
-    c->kernel_launches += loop_kernels(max_iter, len, 4);
-    CK(launch_finalize_block(make_block_args(c, k.p, 0), c->stream));
-    CK(launch_device_info(k.st, nrhs, c->loopctl, info_dev, a.hist, k.hist_ld, hist_dev, max_iter, c->stream));
     c->kernel_launches += 2;
-    CK(cudaMemcpy2DAsync(X_dev, row, k.x, pitch, row, (size_t)nrhs, cudaMemcpyDeviceToDevice, c->stream));
-    return device_solve_leave(c, us);
+    rc = launch_loop_graph(c, c->loop_block, graph_key(c, nrhs, tol, m.hist), m, nullptr, k.arrive + 2 * k.cap, 4,
+                           max_iter, [&](const Mode &bm) { return launch_block_iteration(c, bm); });
+    if (rc) return rc;
+    CK(launch_finalize_block(make_block_args(c, k.p, 0, m), c->stream));
+    return device_solve_leave(c, us, nrhs, max_iter, k.run.st, m.hist, k.run.hist_ld, hist_dev, info_dev, k.x, X_dev);
 }
 
 extern "C" int cgb_residual_check(cgb_ctx *c, double *norm_x, double *rel_resid)
@@ -2063,11 +1950,12 @@ extern "C" int cgb_residual_check(cgb_ctx *c, double *norm_x, double *rel_resid)
     if (c->in_solve) return fail(CGB_ERR_STATE, "solve in progress");
     if (!c->matrix_set || !c->rhs_set) return fail(CGB_ERR_STATE, "matrix / right-hand side not set");
     // `done` may still be raised from the solve: the DEBUG mat-vec must run regardless
-    CK(cudaMemsetAsync(&c->st->done, 0, sizeof(int), c->stream));
-    if ((rc = launch_matvec(c, c->x, 0, c->variant))) return rc;   // cg.cc:146-147
+    CK(cudaMemsetAsync(&c->run.st->done, 0, sizeof(int), c->stream));
+    const Mode m = host_mode(c);
+    if ((rc = launch_matvec(c, c->x, 0, c->variant, m))) return rc;   // cg.cc:146-147
     if ((rc = launch_gather(c))) return rc;
     double *out = c->scratch + 3 * c->nchunks;
-    CK(launch_debug_norms(make_vec_args(c), c->scratch, out, c->stream));
+    CK(launch_debug_norms(make_vec_args(c, m), c->scratch, out, c->stream));
     c->kernel_launches += 2;
     CK(cudaMemcpyAsync(c->h_pin, out, 2 * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
@@ -2085,10 +1973,10 @@ extern "C" int cgb_gemv(cgb_ctx *c, const double *v_host, double *y_host, double
     if (c->in_solve) return fail(CGB_ERR_STATE, "solve in progress");
     if (!c->matrix_set) return fail(CGB_ERR_STATE, "matrix not set");
     if (!v_host) return fail(CGB_ERR_INVALID, "null v");
-    CK(cudaMemsetAsync(&c->st->done, 0, sizeof(int), c->stream));
+    CK(cudaMemsetAsync(&c->run.st->done, 0, sizeof(int), c->stream));
     CK(cudaMemcpyAsync(c->p, v_host, (size_t)c->n * 8, cudaMemcpyHostToDevice, c->stream));
     if (!exchange_configured(c)) return fail(CGB_ERR_STATE, "world > 1 but no exchange is configured");
-    if ((rc = launch_matvec(c, c->p, 0, c->variant))) return rc;
+    if ((rc = launch_matvec(c, c->p, 0, c->variant, host_mode(c)))) return rc;
     if ((rc = launch_gather(c))) return rc;
     if ((rc = collect_for_host(c))) return rc;
     const Gather gth = make_gather(c);
@@ -2137,14 +2025,15 @@ extern "C" int cgb_bench_gemv(cgb_ctx *c, int variant, int reps, float *ms_avg)
     const int keep_variant = c->variant;
     if (variant != keep_variant && c->storage == 0) {
         set_variant(c, variant);
-        drop_graph(c);
+        c->graph_gen += 1;
         CK(gemv_variant(variant).preload()); // loads the kernel and sets its shared-memory limit
     }
-    CK(cudaMemsetAsync(&c->st->done, 0, sizeof(int), c->stream));
-    if ((rc = launch_matvec(c, c->p, 0, variant))) return rc; // warm-up
+    CK(cudaMemsetAsync(&c->run.st->done, 0, sizeof(int), c->stream));
+    const Mode m = host_mode(c);
+    if ((rc = launch_matvec(c, c->p, 0, variant, m))) return rc; // warm-up
     CK(cudaEventRecord(c->ev0, c->stream));
     for (int i = 0; i < reps; ++i)
-        if ((rc = launch_matvec(c, c->p, 0, variant))) return rc;
+        if ((rc = launch_matvec(c, c->p, 0, variant, m))) return rc;
     CK(cudaEventRecord(c->ev1, c->stream));
     // fused mode: the launches above all carried the same tag; consume it so that the next
     // exchange starts from a fresh tag on every rank
@@ -2237,7 +2126,7 @@ extern "C" int cgb_autotune(cgb_ctx *c, int iters, int *chosen, float *us_per_it
     }
     const int keep_variant = c->variant, keep_loopback = c->opt_loopback, keep_exchange = c->opt_exchange;
     const bool keep_ready = c->p2p_ready;
-    const double keep_tol = c->tol;
+    const double keep_tol = c->run.tol;
     const bool want_persist = c->opt_schedule == 1 && !c->opt_compat && !(c->world > 1 && keep_exchange == 0 && c->comm);
     Ctl ctl0;
     CK(cudaMemcpy(&ctl0, c->ctl, sizeof ctl0, cudaMemcpyDeviceToHost));
@@ -2260,8 +2149,8 @@ extern "C" int cgb_autotune(cgb_ctx *c, int iters, int *chosen, float *us_per_it
         c->p2p_ready = true;
         c->opt_exchange = 1;
     }
-    c->tol = 0.0; // never converges
-    drop_graph(c);
+    c->run.tol = 0.0; // never converges
+    c->graph_gen += 1;
     int best = keep_variant;
     float best_us = -1.f, default_us = -1.f;
     // the timed runs; a lambda so that a failing CUDA call still reaches the restore below
@@ -2273,21 +2162,18 @@ extern "C" int cgb_autotune(cgb_ctx *c, int iters, int *chosen, float *us_per_it
         // only shapes with a persistent instantiation, on either schedule (DESIGN.md 3.3): the
         // choice stays a shape both schedules run when the schedule is switched after tuning
         if (persist_index(c) < 0) continue;
-        const bool persist = want_persist && !persist_unusable(c);
+        const bool persist = want_persist && !persist_unusable(c, c->opt_profile);
         if (want_persist && !persist) continue; // compare like with like
         if (gemv_variant(v).preload() != cudaSuccess) { cudaGetLastError(); continue; }
         if (persist && persist_variant(persist_index(c)).preload() != cudaSuccess) { cudaGetLastError(); continue; }
         float t_best = -1.f;
         for (int rep = 0; rep < 3 && rc == CGB_OK; ++rep) { // rep 0 warms up
-            State s0;
-            memset(&s0, 0, sizeof s0);
-            s0.iter = -1;
-            CK(cudaMemcpyAsync(c->st, &s0, sizeof s0, cudaMemcpyHostToDevice, c->stream));
+            if ((rc = reset_states(c, c->run.st, 1))) break;
             CK(cudaEventRecord(c->ev0, c->stream));
             if (persist) {
-                rc = launch_persist(c, iters);
+                rc = launch_persist(c, iters, host_mode(c));
             } else {
-                for (int i = 0; i < iters && rc == CGB_OK; ++i) rc = launch_iteration(c);
+                for (int i = 0; i < iters && rc == CGB_OK; ++i) rc = launch_iteration(c, host_mode(c));
             }
             if (rc) break;
             CK(cudaEventRecord(c->ev1, c->stream));
@@ -2320,14 +2206,14 @@ extern "C" int cgb_autotune(cgb_ctx *c, int iters, int *chosen, float *us_per_it
     c->opt_loopback = keep_loopback;
     c->p2p_ready = keep_ready;
     c->opt_exchange = keep_exchange;
-    c->tol = keep_tol;
+    c->run.tol = keep_tol;
     set_variant(c, best);
-    drop_graph(c);
+    c->graph_gen += 1;
     if (rc) return rc;
     gemv_variant(best).preload();
     if (persist_index(c) >= 0) persist_variant(persist_index(c)).preload();
     CK(cudaMemcpyAsync(c->ctl, &ctl0, sizeof ctl0, cudaMemcpyHostToDevice, c->stream));
-    CK(cudaMemsetAsync(c->st, 0, sizeof(State), c->stream));
+    CK(cudaMemsetAsync(c->run.st, 0, sizeof(State), c->stream));
     *c->h_done = 0;
     CK(cudaStreamSynchronize(c->stream));
     if (chosen) *chosen = best;

@@ -185,6 +185,44 @@ def test_dense_past_the_int_limit_vs_csr_oracle(cgb, O):
     _same_as_oracle(got, csr_oracle.solve_csr(csr_oracle.generate_lap2d_csr(n), b, max_iter=50))
 
 
+@pytest.mark.parametrize("form", ["solve", "solve_block"])
+def test_csr_graph_solve_after_matrix_reload(cgb, O, form):
+    """Every CSR build reallocates col / val, which the captured loop graphs bake in.  A second solve with
+    the same tol and history after loading a larger matrix must capture its graph anew: replaying the
+    first one would run the mat-vec on the freed arrays of lap2d."""
+    from test_gpu_block import _ragged_coo
+    n, max_iter = 3001, 200
+    irn, jcn, val, empty = _ragged_coo(n, 11)
+    m = csr_oracle.csr_from_coo(n, irn, jcn, val, False)
+    B = np.random.default_rng(12).standard_normal((3, n))
+    B[0] = O.init_source_term(n)
+    B[:, empty] = 0.0
+    with cgb.Context(n, storage="csr") as ctx:
+        assert max_iter >= min(ctx.get_option("graph_unroll"), ctx.get_option("poll_every"))
+
+        def run():
+            if form == "solve":
+                ctx.set_rhs(B[0])
+                x = np.zeros(n)
+                info, hist = ctx.solve(x, max_iter=max_iter, history=True)
+                return x[None], [info], hist[None]
+            return ctx.solve_block(B, None, max_iter=max_iter, history=True)
+
+        ctx.generate_lap2d()
+        lap_nnz = ctx.nnz()
+        run()
+        replays = ctx.get_option("graph_replays")
+        ctx.set_matrix_coo(irn, jcn, val, symmetric=False)
+        assert ctx.nnz() == m.col.size > lap_nnz
+        X, infos, hist = run()
+        assert ctx.get_option("graph_replays") > replays
+    for j in range(len(infos)):
+        ref = csr_oracle.solve_csr(m, B[j], np.zeros(n), max_iter=max_iter)
+        assert (infos[j].k, bool(infos[j].converged), infos[j].iterations) == (ref.k, ref.converged, len(ref.hist))
+        assert _eq(hist[j], ref.hist) and _eq(X[j], ref.x)
+        assert _eq([infos[j].rsold, infos[j].rsnew], [ref.rsold, ref.rsnew])
+
+
 # --------------------------------------------------------------------------- options
 def test_csr_options(cgb):
     n = 4096
