@@ -54,6 +54,8 @@ SIGNATURES = [
     ("cgb_generate_lap2d", C.c_int, [_CTX]),
     ("cgb_set_matrix_rows", C.c_int, [_CTX, _dp, C.c_int64, C.c_int64, C.c_int64]),
     ("cgb_set_matrix_coo", C.c_int, [_CTX, C.c_int64, _i32p, _i32p, _dp, C.c_int]),
+    ("cgb_set_matrix_csr", C.c_int, [_CTX, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    ("cgb_update_matrix_values", C.c_int, [_CTX, C.c_void_p, C.c_void_p]),
     ("cgb_get_matrix_rows", C.c_int, [_CTX, _dp, C.c_int64, C.c_int64, C.c_int64]),
     ("cgb_init_source_term", C.c_int, [C.c_int64, C.c_double, _dp]),
     ("cgb_set_rhs", C.c_int, [_CTX, _dp]),
@@ -264,6 +266,54 @@ class Context:
         val = np.ascontiguousarray(val, dtype=np.float64)
         _check(self._lib.cgb_set_matrix_coo(self._h, irn.size, irn.ctypes.data_as(_i32p),
                                             jcn.ctypes.data_as(_i32p), _p(val), int(bool(symmetric))))
+
+    def set_matrix_csr(self, A, stream=None):
+        """cgb_set_matrix_csr from the full n x n matrix on the GPU: a CUDA torch.sparse_csr_tensor of float64
+        or a (crow, col, val) tuple of CUDA tensors, crow and col both int32 or both int64.  This rank's rows
+        are passed on `stream` (default: the current torch stream); the call returns with the matrix built."""
+        import torch
+        if isinstance(A, torch.Tensor):
+            if A.layout != torch.sparse_csr:
+                raise TypeError("A must be a torch.sparse_csr_tensor or a (crow, col, val) tuple")
+            if tuple(A.shape) != (self.n, self.n):
+                raise ValueError(f"A is {tuple(A.shape)}, the context {self.n} x {self.n}")
+            crow, col, val = A.crow_indices(), A.col_indices(), A.values()
+        else:
+            crow, col, val = A
+        torch, dev, stream = self._device_args([("val", val)], stream)
+        for nm, t in (("crow", crow), ("col", col)):
+            if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype in (torch.int32, torch.int64)
+                    and t.is_contiguous()):
+                raise TypeError(f"{nm} must be a contiguous int32 or int64 CUDA tensor")
+            if t.device.index != dev:
+                raise ValueError(f"{nm} is on cuda:{t.device.index}, the context on cuda:{dev}")
+        if crow.dtype != col.dtype:
+            raise TypeError("crow and col must share one index dtype")
+        if crow.numel() != self.n + 1:
+            raise ValueError(f"crow has {crow.numel()} entries, the full matrix n + 1 = {self.n + 1}")
+        lay = self.layout()
+        with torch.cuda.stream(stream):
+            rp = crow[lay.row0:lay.row0 + lay.rows + 1].to(torch.int64)
+            base, end = (int(v) for v in rp[[0, -1]].cpu())   # a synchronisation: the call makes one anyway
+            if not 0 <= base <= end <= min(col.numel(), val.numel()):
+                raise ValueError(f"crow[{lay.row0}] = {base} and crow[{lay.row0 + lay.rows}] = {end} do not "
+                                 f"delimit this rank's entries of col / val")
+            cols = col[base:end]
+            if cols.dtype != torch.int32:
+                cols = cols.clamp(-1, self.n).to(torch.int32)   # a column out of range stays out of range
+            vals = val[base:end]
+            _check(self._lib.cgb_set_matrix_csr(self._h, rp.data_ptr(), cols.data_ptr(), vals.data_ptr(),
+                                                end - base, stream.cuda_stream))
+
+    def update_matrix_values(self, val, stream=None):
+        """cgb_update_matrix_values: new values (the first nnz() entries of the float64 CUDA tensor `val`, in
+        stored order) for this CSR context's matrix, enqueued on `stream`; returns at once."""
+        torch, dev, stream = self._device_args([("val", val)], stream)
+        nnz = self.nnz()
+        if val.numel() < nnz:
+            raise ValueError(f"val has {val.numel()} entries, the matrix {nnz}")
+        _check(self._lib.cgb_update_matrix_values(self._h, val.data_ptr(), stream.cuda_stream))
+        val.record_stream(stream)   # its memory is not handed out again before `stream` has passed the copy
 
     def get_matrix_rows(self, first_row: int, nrows: int) -> np.ndarray:
         out = np.empty((nrows, self.n), dtype=np.float64)

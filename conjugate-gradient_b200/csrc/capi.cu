@@ -160,6 +160,7 @@ struct cgb_ctx {
     size_t compat_part_cap = 0;
     int poll_every = 16, graph_unroll = 16, opt_pdl = 1, opt_l2_prefetch = 4, opt_l2_ramp = 2;
     long long graph_replays = 0;   // graph launches since creation ("graph_replays", read-only option)
+    long long graph_captures = 0;  // loop graphs captured and instantiated ("graph_captures", read-only option)
     int opt_balance = 1;           // persistent kernel: re-balance the rows between the CTAs from measured speeds
     long long aux_stride = 0;      // entries of one parity of the local LL side buffer
     int opt_schedule = 1;          // 1: persistent cooperative kernel (persist.cu) when usable, 0: CUDA graph of 4 kernels per iteration
@@ -450,6 +451,7 @@ int rebuild(cgb_ctx *c, CachedGraph &g, const GraphKey &key, F build)
         return rc;
     }
     g.key = key;
+    c->graph_captures += 1;
     return CGB_OK;
 }
 
@@ -858,9 +860,18 @@ int check_device_ptr(const cgb_ctx *c, const void *p, const char *what)
     }
     if (a.type == cudaMemoryTypeManaged) return CGB_OK;
     if (a.type != cudaMemoryTypeDevice)
-        return fail(CGB_ERR_INVALID, "%s is host memory: a device solve takes device pointers", what);
+        return fail(CGB_ERR_INVALID, "%s is host memory: this call takes device pointers", what);
     if (a.device != c->device)
         return fail(CGB_ERR_INVALID, "%s lives on device %d, the context on device %d", what, a.device, c->device);
+    return CGB_OK;
+}
+
+// The two events that order the context's stream after a caller's stream and back (device solves,
+// cgb_set_matrix_csr, cgb_update_matrix_values); created on first use
+int stream_events(cgb_ctx *c)
+{
+    for (cudaEvent_t &e : c->ev_dev)
+        if (!e) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     return CGB_OK;
 }
 
@@ -1370,7 +1381,7 @@ extern "C" int cgb_get_matrix_rows(cgb_ctx *c, double *rows_host, int64_t first_
     if (nrows > 0 && c->storage == 1) { // densified through a device buffer (a test hook)
         double *dense = nullptr;
         CK(cudaMalloc(&dense, (size_t)nrows * c->n * sizeof(double)));
-        cudaError_t e = csr_densify(c->csr, first_row - c->row0, nrows, c->n, dense, c->stream);
+        cudaError_t e = csr_densify(c->csr.rp, c->csr.col, c->csr.val, first_row - c->row0, nrows, c->n, dense, c->stream);
         if (e == cudaSuccess)
             e = cudaMemcpy2DAsync(rows_host, (size_t)ld_host * 8, dense, (size_t)c->n * 8, (size_t)c->n * 8,
                                   (size_t)nrows, cudaMemcpyDeviceToHost, c->stream);
@@ -1553,6 +1564,7 @@ extern "C" int cgb_get_option(cgb_ctx *c, const char *key, int64_t *value)
     else if (k == "poll_every") *value = c->poll_every;
     else if (k == "graph_unroll") *value = c->graph_unroll;
     else if (k == "graph_replays") *value = c->graph_replays;
+    else if (k == "graph_captures") *value = c->graph_captures;
     else if (k == "device_loop_pdl") *value = c->loop_single.pdl_used >= 0 ? c->loop_single.pdl_used : c->loop_block.pdl_used;
     else if (k == "compat") *value = c->opt_compat;
     else if (k == "pdl") *value = c->opt_pdl;
@@ -1832,8 +1844,7 @@ static int device_solve_check(cgb_ctx *c, const double *B, const double *X, cons
         return rc;
     if (c->loopctl) return CGB_OK;
     CK(preload_loop_kernels());
-    for (cudaEvent_t &e : c->ev_dev)
-        if (!e) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    if ((rc = stream_events(c))) return rc;
     CK(cudaMalloc(&c->loopctl, sizeof(LoopCtl)));
     CK(cudaMemsetAsync(c->loopctl, 0, sizeof(LoopCtl), c->stream));
     return CGB_OK;
@@ -1941,6 +1952,84 @@ extern "C" int cgb_solve_block_device(cgb_ctx *c, int nrhs, const double *B_dev,
     if (rc) return rc;
     CK(launch_finalize_block(make_block_args(c, k.p, 0, m), c->stream));
     return device_solve_leave(c, us, nrhs, max_iter, k.run.st, m.hist, k.run.hist_ld, hist_dev, info_dev, k.x, X_dev);
+}
+
+// ------------------------------------------------------------------ matrix from device memory (DESIGN 3.10)
+extern "C" int cgb_set_matrix_csr(cgb_ctx *c, const int64_t *rp_dev, const int32_t *col_dev, const double *val_dev,
+                                  int64_t nnz, void *stream)
+{
+    if (!c) return null_context();
+    int rc = use_device(c);
+    if (rc) return rc;
+    if (c->in_solve) return fail(CGB_ERR_STATE, c->blk.active ? "a block solve is in progress" : "a single solve is in progress");
+    if (nnz < 0) return fail(CGB_ERR_INVALID, "nnz < 0 (got %lld)", (long long)nnz);
+    if ((rc = check_device_ptr(c, rp_dev, "rp")) ||
+        (nnz > 0 && ((rc = check_device_ptr(c, col_dev, "col")) || (rc = check_device_ptr(c, val_dev, "val")))))
+        return rc;
+    if ((rc = stream_events(c))) return rc;
+    CK(cudaEventRecord(c->ev_dev[0], static_cast<cudaStream_t>(stream)));
+    CK(cudaStreamWaitEvent(c->stream, c->ev_dev[0], 0));
+    struct Tmp { // freed on every path
+        long long *rp = nullptr;
+        unsigned long long *err = nullptr;
+        ~Tmp()
+        {
+            cudaFree(rp);
+            cudaFree(err);
+        }
+    } t;
+    CK(cudaMalloc(&t.rp, (size_t)(c->rows + 1) * sizeof(long long)));
+    CK(cudaMalloc(&t.err, sizeof(unsigned long long)));
+    // nothing of the context is touched before the input has been checked
+    CK(launch_validate_csr(reinterpret_cast<const long long *>(rp_dev), col_dev, nnz, c->n, c->rows, t.rp, t.err,
+                           c->stream));
+    c->kernel_launches += 1;
+    CK(cudaMemcpyAsync(c->h_pin, t.err, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    unsigned long long err;
+    memcpy(&err, c->h_pin, sizeof err);
+    if (err != ~0ULL) {
+        static const char *const what[kCsrFaultKinds] = {
+            "rp[0] is negative", "rp decreases (row pointers must be monotone)",
+            "its entries reach past rp[0] + nnz", "a column lies outside [0, n)",
+            "columns are not strictly ascending (a duplicate or a descending pair)", "rp[rows] - rp[0] != nnz"};
+        return fail(CGB_ERR_INVALID, "CSR refused at local row %llu: %s (n %lld, rows %lld, nnz %lld)",
+                    err / kCsrFaultKinds, what[err % kCsrFaultKinds], c->n, c->rows, (long long)nnz);
+    }
+    if (c->storage == 1) {
+        c->matrix_set = false;
+        c->graph_gen += 1; // col / val are reallocated, and the loop graphs bake them in
+        CK(csr_from_device(&c->csr, t.rp, c->rows, col_dev, val_dev, nnz, c->stream));
+    } else {
+        // the shard cgb_set_matrix_coo builds from the same triples: zeros, the entries, the envelopes
+        CK(csr_densify(t.rp, col_dev, val_dev, 0, c->rows, c->ld, c->A, c->stream));
+        CK(launch_row_envelope(c->A, c->ld, 0, c->rows, c->env, c->stream));
+        c->kernel_launches += 2;
+        CK(cudaStreamSynchronize(c->stream));
+    }
+    c->matrix_set = true;
+    return CGB_OK;
+}
+
+extern "C" int cgb_update_matrix_values(cgb_ctx *c, const double *val_dev, void *stream)
+{
+    if (!c) return null_context();
+    int rc = use_device(c);
+    if (rc) return rc;
+    if (c->storage != 1) return fail(CGB_ERR_STATE, "values can only be updated on a CSR context: a dense shard keeps no pattern");
+    if (!c->matrix_set) return fail(CGB_ERR_STATE, "matrix not set");
+    if (c->in_solve) return fail(CGB_ERR_STATE, c->blk.active ? "a block solve is in progress" : "a single solve is in progress");
+    if (c->csr.nnz > 0 && (rc = check_device_ptr(c, val_dev, "val"))) return rc;
+    if ((rc = stream_events(c))) return rc;
+    // col / val stay where they are: every cached loop graph stays valid, no generation bump
+    const cudaStream_t us = static_cast<cudaStream_t>(stream);
+    CK(cudaEventRecord(c->ev_dev[0], us));
+    CK(cudaStreamWaitEvent(c->stream, c->ev_dev[0], 0));
+    if (c->csr.nnz > 0)
+        CK(cudaMemcpyAsync(c->csr.val, val_dev, (size_t)c->csr.nnz * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
+    CK(cudaEventRecord(c->ev_dev[1], c->stream));
+    CK(cudaStreamWaitEvent(us, c->ev_dev[1], 0));
+    return CGB_OK;
 }
 
 extern "C" int cgb_residual_check(cgb_ctx *c, double *norm_x, double *rel_resid)

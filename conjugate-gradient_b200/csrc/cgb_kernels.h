@@ -159,8 +159,19 @@ cudaError_t csr_generate_lap2d(CsrShard *m, long long n, long long row0, long lo
 // win); *bad_host = 1 (and the shard unchanged) when an entry lies outside n x n; synchronises
 cudaError_t csr_from_coo(CsrShard *m, long long n, long long row0, long long rows, const int *irn, const int *jcn,
                          const double *val, long long nz, int symmetric, int *bad_host, cudaStream_t s);
-// local rows [lr0, lr0 + nrows) as a dense nrows x n device buffer
-cudaError_t csr_densify(const CsrShard &m, long long lr0, long long nrows, long long n, double *dst, cudaStream_t s);
+// rows [lr0, lr0 + nrows) of a CSR (rp indexing col / val from 0) into a dense nrows x ld device buffer,
+// zeroed first
+cudaError_t csr_densify(const long long *rp, const int *col, const double *val, long long lr0, long long nrows,
+                        long long ld, double *dst, cudaStream_t s);
+// A caller's CSR of `rows` rows against the stored format (cgb_set_matrix_csr): rp[0] >= 0, rp monotone,
+// rp[rows] - rp[0] == nnz, columns in [0, n) and strictly ascending per row.  *err = ~0 when it holds,
+// else the first fault as row * kCsrFaultKinds + kind; rp_local[rows + 1] = rp - rp[0]
+enum { kCsrNegativeBase, kCsrNotMonotone, kCsrPastNnz, kCsrColumnRange, kCsrNotAscending, kCsrCount, kCsrFaultKinds };
+cudaError_t launch_validate_csr(const long long *rp, const int *col, long long nnz, long long n, long long rows,
+                                long long *rp_local, unsigned long long *err, cudaStream_t s);
+// the shard replaced by validated device arrays (rp_local rebased to 0); synchronises
+cudaError_t csr_from_device(CsrShard *m, const long long *rp_local, long long rows, const int *col, const double *val,
+                            long long nnz, cudaStream_t s);
 // streams the three CSR arrays once (the read ceiling of the CSR mat-vec)
 cudaError_t launch_read_csr(const CsrShard &m, long long rows, double *sink, int sm_count, cudaStream_t s);
 

@@ -392,13 +392,52 @@ __global__ void csr_cols_kernel(const unsigned long long *key, long long nnz, in
     if (k < nnz) col[k] = (int)(key[k] & 0xffffffffULL);
 }
 
-// rows [lr0, lr0 + nrows) of the shard into a dense nrows x n buffer (zeroed by the caller)
+// rows [lr0, lr0 + nrows) of a CSR into a dense nrows x ld buffer (zeroed by the caller)
 __global__ void csr_densify_kernel(const long long *rp, const int *col, const double *val, long long lr0,
-                                   long long nrows, long long n, double *dst)
+                                   long long nrows, long long ld, double *dst)
 {
     const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= nrows) return;
-    for (long long k = rp[lr0 + r]; k < rp[lr0 + r + 1]; ++k) dst[r * n + col[k]] = val[k];
+    for (long long k = rp[lr0 + r]; k < rp[lr0 + r + 1]; ++k) dst[r * ld + col[k]] = val[k];
+}
+
+// A caller's CSR (cgb_set_matrix_csr) checked against the stored format, one warp per row.  The row's
+// rp pair is checked first, and its columns are read only when the pair lies inside [rp[0], rp[0] + nnz]:
+// a bad rp is refused and never leads to a read outside the caller's nnz entries.  Then the lanes stride
+// over the row's entries for the range and the strict ascent.  The first fault lands in *err as
+// row * kCsrFaultKinds + kind (atomicMin: the smallest row, and the first failed check of that row);
+// rp_local receives rp - rp[0].
+__global__ void __launch_bounds__(256) validate_csr_kernel(const long long *rp, const int *col, long long nnz,
+                                                            long long n, long long rows, long long *rp_local,
+                                                            unsigned long long *err)
+{
+    const long long row = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (row >= rows) return;
+    const long long base = rp[0], beg = rp[row], end = rp[row + 1]; // warp-uniform
+    const unsigned long long here = (unsigned long long)row * kCsrFaultKinds;
+    int kind = -1;
+    if (base < 0) kind = kCsrNegativeBase;
+    else if (end < beg) kind = kCsrNotMonotone;
+    else if (beg < base || end - base > nnz) kind = kCsrPastNnz;
+    if (kind >= 0) {
+        if (lane == 0) atomicMin(err, here + kind);
+        return;
+    }
+    bool range = false, order = false;
+    for (long long k = beg - base + lane; k < end - base; k += 32) {
+        const int c = col[k];
+        if (c < 0 || c >= n) range = true;
+        else if (k > beg - base && col[k - 1] >= c) order = true;
+    }
+    range = __any_sync(0xffffffffu, range);
+    order = __any_sync(0xffffffffu, order);
+    if (lane != 0) return;
+    if (range) atomicMin(err, here + kCsrColumnRange);
+    else if (order) atomicMin(err, here + kCsrNotAscending);
+    else if (row == rows - 1 && end - base != nnz) atomicMin(err, here + kCsrCount);
+    rp_local[row + 1] = end - base;
+    if (row == 0) rp_local[0] = 0;
 }
 
 inline unsigned blocks_for(long long n, int t) { return (unsigned)((n + t - 1) / t > 0 ? (n + t - 1) / t : 1); }
@@ -567,11 +606,32 @@ cudaError_t csr_from_coo(CsrShard *m, long long n, long long row0, long long row
     return cudaStreamSynchronize(s);
 }
 
-cudaError_t csr_densify(const CsrShard &m, long long lr0, long long nrows, long long n, double *dst, cudaStream_t s)
+cudaError_t csr_densify(const long long *rp, const int *col, const double *val, long long lr0, long long nrows,
+                        long long ld, double *dst, cudaStream_t s)
 {
-    CU(cudaMemsetAsync(dst, 0, (size_t)nrows * n * sizeof(double), s));
-    csr_densify_kernel<<<blocks_for(nrows, 256), 256, 0, s>>>(m.rp, m.col, m.val, lr0, nrows, n, dst);
+    CU(cudaMemsetAsync(dst, 0, (size_t)nrows * ld * sizeof(double), s));
+    csr_densify_kernel<<<blocks_for(nrows, 256), 256, 0, s>>>(rp, col, val, lr0, nrows, ld, dst);
     return cudaGetLastError();
+}
+
+cudaError_t launch_validate_csr(const long long *rp, const int *col, long long nnz, long long n, long long rows,
+                                long long *rp_local, unsigned long long *err, cudaStream_t s)
+{
+    CU(cudaMemsetAsync(err, 0xff, sizeof *err, s));
+    validate_csr_kernel<<<blocks_for(rows, 8), 256, 0, s>>>(rp, col, nnz, n, rows, rp_local, err);
+    return cudaGetLastError();
+}
+
+cudaError_t csr_from_device(CsrShard *m, const long long *rp_local, long long rows, const int *col, const double *val,
+                            long long nnz, cudaStream_t s)
+{
+    CU(csr_resize(m, nnz));
+    CU(cudaMemcpyAsync(m->rp, rp_local, (size_t)(rows + 1) * sizeof(long long), cudaMemcpyDeviceToDevice, s));
+    if (nnz > 0) {
+        CU(cudaMemcpyAsync(m->col, col, (size_t)nnz * sizeof(int), cudaMemcpyDeviceToDevice, s));
+        CU(cudaMemcpyAsync(m->val, val, (size_t)nnz * sizeof(double), cudaMemcpyDeviceToDevice, s));
+    }
+    return cudaStreamSynchronize(s);
 }
 
 cudaError_t launch_read_csr(const CsrShard &m, long long rows, double *sink, int sm_count, cudaStream_t s)

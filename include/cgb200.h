@@ -59,7 +59,8 @@ int cgb_create(int64_t n, int rank, int world, int device, cgb_ctx **out);
 /* The same rank with the shard held in CSR storage: no dense shard is allocated, so the system
  * size is bounded by the non-zeros, not by n^2 (n <= INT32_MAX: column indices are int32_t,
  * global; row pointers int64_t; values double; columns ascending and unique within a row).
- * The matrix comes from cgb_generate_lap2d or cgb_set_matrix_coo (built on the device);
+ * The matrix comes from cgb_generate_lap2d, cgb_set_matrix_coo or cgb_set_matrix_csr (built on the
+ * device), its values may be refreshed with cgb_update_matrix_values;
  * cgb_set_matrix_rows returns CGB_ERR_STATE.  Vectors, exchange wiring and cgb_get_layout are
  * those of cgb_create; the solve runs on the graph schedule ("schedule_in_use" reads 0).
  * Exactness: the CSR mat-vec keeps the lane order of the dense one over the stored entries, and
@@ -112,6 +113,38 @@ int cgb_set_matrix_rows(cgb_ctx *ctx, const double *rows_host, int64_t first_row
 int cgb_set_matrix_coo(cgb_ctx *ctx, int64_t nz, const int32_t *irn, const int32_t *jcn,
                        const double *val, int symmetric);
 
+/* This rank's rows [row0, row0 + rows) from a CSR matrix in device memory of the context's GPU:
+ *   rp_dev   rows + 1 row pointers; local row i holds the entries rp[i] - rp[0] .. rp[i+1] - rp[0]
+ *   col_dev  nnz = rp[rows] - rp[0] global columns, in [0, n) and strictly ascending within a row
+ *   val_dev  nnz values (explicit zeros are stored, as by cgb_set_matrix_coo); empty rows are allowed
+ * So a rank of a larger CSR passes rp + row0 and col / val + rp[row0], with nothing rebased.  col_dev and
+ * val_dev may be null when nnz == 0.  The reads are ordered after the work enqueued on `stream` (a
+ * cudaStream_t as void *, NULL = the legacy default stream) by an event; the call synchronises, like every
+ * builder, and returns with the matrix built: the caller may overwrite its arrays afterwards.
+ * The input is checked on the device before anything of the context is touched -- rp[0] >= 0, rp
+ * monotone, rp[rows] - rp[0] == nnz, every column in range and strictly ascending; a row's columns are read
+ * only after its rp pair has been checked.  A refusal returns CGB_ERR_INVALID with a message naming the
+ * first offending local row, and the previous matrix stays as it was.
+ * CSR context: the shard takes copies of the arrays (col / val are reallocated, so the next solve captures
+ * its loop graph anew).  Dense context: the shard cgb_set_matrix_coo builds from the same triples.
+ * CGB_ERR_STATE: a single or block solve between begin and end.  CGB_ERR_INVALID: nnz < 0, a null
+ * pointer, a host pointer or one on another device.  Its kernels count in cgb_launch_count. */
+int cgb_set_matrix_csr(cgb_ctx *ctx, const int64_t *rp_dev, const int32_t *col_dev, const double *val_dev,
+                       int64_t nnz, void *stream);
+
+/* New values for the matrix of a CSR context, its pattern kept: val_dev holds the context's "nnz" values
+ * in stored order (rows ascending, columns ascending within a row -- cgb_set_matrix_csr's input order,
+ * defined as well for a matrix from cgb_generate_lap2d or cgb_set_matrix_coo), in device memory of the
+ * context's GPU (null allowed when nnz == 0).  Fully asynchronous: an event orders the copy after the work
+ * enqueued on `stream` and after every solve already enqueued on the context from any stream, and work
+ * enqueued on `stream` after the call sees the new values.  No host synchronisation, no allocation (the
+ * first call of a context that has run no device solve creates two events), and the values array does
+ * not move, so every cached loop graph stays valid: the next device solve is one graph launch, nothing
+ * captured ("graph_captures" does not change).
+ * CGB_ERR_STATE: a dense context (a dense shard keeps no pattern), the matrix not set, a single or block
+ * solve between begin and end.  CGB_ERR_INVALID: a null pointer, a host pointer or one on another device. */
+int cgb_update_matrix_values(cgb_ctx *ctx, const double *val_dev, void *stream);
+
 /* Read rows of the shard back (tests); a CSR shard is densified. */
 int cgb_get_matrix_rows(cgb_ctx *ctx, double *rows_host, int64_t first_row, int64_t nrows,
                         int64_t ld_host);
@@ -133,7 +166,8 @@ int cgb_set_rhs(cgb_ctx *ctx, const double *b_host);
  * column-tile width of the mat-vec; "graph": 0/1 CUDA-graph replay of the iteration;
  * "poll_every" / "graph_unroll": graph schedule only -- iterations between two looks at the stop flag and
  * iterations per graph (the instantiated graph holds min of the two; "graph_replays", read-only,
- * counts its launches, and those of the block solve's graph);
+ * counts its launches, and those of the block solve's graph; "graph_captures", read-only, counts the
+ * loop graphs -- host and device loops, single and block -- this context has captured and instantiated);
  * "pdl": 0/1 programmatic dependent launch between the kernels of the iteration (the next
  * mat-vec prefetches A while the vector updates still run); "l2_prefetch": pipeline steps of A
  * the mat-vec additionally pulls into L2 before that wait (0 = off); "l2_ramp": persistent
