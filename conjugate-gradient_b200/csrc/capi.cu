@@ -1250,24 +1250,64 @@ extern "C" int cgb_exchange_import(cgb_ctx *c, const void *blobs)
 }
 
 // ------------------------------------------------------------------ inputs
+namespace {
+
+// A local CSR a builder stages for install_matrix.  What it holds when it goes out of scope is freed: the
+// staged arrays after a refusal or an error, the context's previous ones after an install that adopted it.
+struct StagedCsr : CsrShard {
+    ~StagedCsr()
+    {
+        cudaFree(rp);
+        cudaFree(col);
+        cudaFree(val);
+    }
+};
+
+// The one place a built matrix becomes the context's.  `m` is this rank's validated local CSR in device
+// memory: rp rebased to 0, columns ascending and unique per row, explicit zeros kept.  A CSR context adopts
+// it: a builder's staging (`staged`) is swapped in, a caller's arrays are copied.  The loop graphs bake in
+// col / val, which move, so the generation is bumped.  A dense context densifies it into A (the whole
+// rows x ld block is zeroed first) and rebuilds every row's envelope; its graphs bake in A and env, which
+// stay where they are, so its generation is not bumped.
+int install_matrix(cgb_ctx *c, CsrShard &m, bool staged)
+{
+    c->matrix_set = false; // until the install completes
+    if (c->storage == 1) {
+        StagedCsr copy;
+        if (!staged) {
+            CK(cudaMalloc(&copy.rp, (size_t)(c->rows + 1) * sizeof(long long)));
+            CK(csr_alloc_entries(&copy, m.nnz));
+            CK(cudaMemcpyAsync(copy.rp, m.rp, (size_t)(c->rows + 1) * sizeof(long long), cudaMemcpyDeviceToDevice,
+                               c->stream));
+            if (m.nnz > 0) {
+                CK(cudaMemcpyAsync(copy.col, m.col, (size_t)m.nnz * sizeof(int), cudaMemcpyDeviceToDevice, c->stream));
+                CK(cudaMemcpyAsync(copy.val, m.val, (size_t)m.nnz * sizeof(double), cudaMemcpyDeviceToDevice,
+                                   c->stream));
+            }
+        }
+        std::swap(c->csr, staged ? m : copy);
+        c->graph_gen += 1;
+    } else {
+        CK(csr_densify(m.rp, m.col, m.val, 0, c->rows, c->ld, c->A, c->stream));
+        CK(launch_row_envelope(c->A, c->ld, 0, c->rows, c->env, c->stream));
+        c->kernel_launches += 2;
+    }
+    CK(cudaStreamSynchronize(c->stream));
+    c->matrix_set = true;
+    return CGB_OK;
+}
+
+} // namespace
+
 extern "C" int cgb_generate_lap2d(cgb_ctx *c)
 {
     int rc = use_device(c);
     if (rc) return rc;
     if (c->in_solve) return fail(CGB_ERR_STATE, "solve in progress");
-    if (c->storage == 1) {
-        c->matrix_set = false;
-        c->graph_gen += 1; // the builders reallocate col / val, which the loop graphs bake in
-        CK(csr_generate_lap2d(&c->csr, c->n, c->row0, c->rows, c->stream));
-        c->kernel_launches += 3;
-    } else {
-        CK(launch_generate_lap2d(c->A, c->n, c->ld, c->row0, c->rows, c->stream));
-        CK(launch_row_envelope(c->A, c->ld, 0, c->rows, c->env, c->stream));
-        c->kernel_launches += 2;
-        CK(cudaStreamSynchronize(c->stream));
-    }
-    c->matrix_set = true;
-    return CGB_OK;
+    StagedCsr m;
+    CK(csr_generate_lap2d(&m, c->n, c->row0, c->rows, c->stream));
+    c->kernel_launches += 3;
+    return install_matrix(c, m, true);
 }
 
 extern "C" int cgb_set_matrix_rows(cgb_ctx *c, const double *rows_host, int64_t first_row,
@@ -1301,72 +1341,23 @@ extern "C" int cgb_set_matrix_coo(cgb_ctx *c, int64_t nz, const int32_t *irn, co
     if (rc) return rc;
     if (c->in_solve) return fail(CGB_ERR_STATE, "solve in progress");
     if (nz < 0 || (nz > 0 && (!irn || !jcn || !val))) return fail(CGB_ERR_INVALID, "bad COO arguments");
-    // Sequential "later entries overwrite" semantics (matrix.cc:12-21) under a parallel scatter,
-    // resolved ON THE DEVICE: (1) every entry raises the cells it writes (inside this shard) to its
-    // own index + 1 with atomicMax, the shard's 8-byte cells serving as the index array; (2) an
-    // entry whose index survived in a cell is that cell's last writer; (3) the winners store
-    // their values.  Untouched cells keep the zero bits of step 0.  The host only copies the triples.
-    struct Tmp { // freed on every path
-        int *i = nullptr, *j = nullptr;
-        double *v = nullptr;
-        unsigned char *win = nullptr;
-        int *bad = nullptr;
-        ~Tmp()
-        {
-            cudaFree(i);
-            cudaFree(j);
-            cudaFree(v);
-            cudaFree(win);
-            cudaFree(bad);
-        }
-    } t;
-    if (c->storage == 1) {
-        // CSR: the writes as sequence 2z (direct) / 2z+1 (mirror), stable-sorted by (row, column),
-        // the last of every run kept (spmv.cu)
-        if (nz > 0) {
-            CK(cudaMalloc(&t.i, (size_t)nz * sizeof(int)));
-            CK(cudaMalloc(&t.j, (size_t)nz * sizeof(int)));
-            CK(cudaMalloc(&t.v, (size_t)nz * sizeof(double)));
-            CK(cudaMemcpyAsync(t.i, irn, (size_t)nz * sizeof(int), cudaMemcpyHostToDevice, c->stream));
-            CK(cudaMemcpyAsync(t.j, jcn, (size_t)nz * sizeof(int), cudaMemcpyHostToDevice, c->stream));
-            CK(cudaMemcpyAsync(t.v, val, (size_t)nz * sizeof(double), cudaMemcpyHostToDevice, c->stream));
-        }
-        int bad = 0;
-        c->matrix_set = false;
-        c->graph_gen += 1;
-        CK(csr_from_coo(&c->csr, c->n, c->row0, c->rows, t.i, t.j, t.v, nz, symmetric ? 1 : 0, &bad, c->stream));
-        if (bad) return fail(CGB_ERR_INVALID, "a COO entry lies outside %lld x %lld", (long long)c->n, (long long)c->n);
-        c->matrix_set = true;
-        return CGB_OK;
-    }
-    CK(cudaMemsetAsync(c->A, 0, (size_t)c->rows * c->ld * sizeof(double), c->stream));
+    // Matrix::read's sequential "later entries overwrite" (matrix.cc:12-21) on the device: the writes as
+    // sequence 2z (direct) / 2z+1 (mirror), stable-sorted by (row, column), the last of every run kept (spmv.cu)
+    DevBuf i, j, v;
+    CK(i.alloc((size_t)nz * sizeof(int)));
+    CK(j.alloc((size_t)nz * sizeof(int)));
+    CK(v.alloc((size_t)nz * sizeof(double)));
     if (nz > 0) {
-        CK(cudaMalloc(&t.i, (size_t)nz * sizeof(int)));
-        CK(cudaMalloc(&t.j, (size_t)nz * sizeof(int)));
-        CK(cudaMalloc(&t.v, (size_t)nz * sizeof(double)));
-        CK(cudaMalloc(&t.win, (size_t)nz));
-        CK(cudaMalloc(&t.bad, sizeof(int)));
-        CK(cudaMemsetAsync(t.bad, 0, sizeof(int), c->stream));
-        CK(cudaMemcpyAsync(t.i, irn, (size_t)nz * sizeof(int), cudaMemcpyHostToDevice, c->stream));
-        CK(cudaMemcpyAsync(t.j, jcn, (size_t)nz * sizeof(int), cudaMemcpyHostToDevice, c->stream));
-        CK(cudaMemcpyAsync(t.v, val, (size_t)nz * sizeof(double), cudaMemcpyHostToDevice, c->stream));
-        CK(launch_scatter_coo(c->A, c->n, c->ld, c->row0, c->rows, t.i, t.j, t.v, nz, symmetric ? 1 : 0, t.win,
-                              t.bad, c->stream));
-        CK(launch_row_envelope(c->A, c->ld, 0, c->rows, c->env, c->stream));
-        c->kernel_launches += 4;
-        int bad = 0;
-        CK(cudaMemcpyAsync(&bad, t.bad, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-        CK(cudaStreamSynchronize(c->stream));
-        if (bad) {
-            c->matrix_set = false;
-            return fail(CGB_ERR_INVALID, "a COO entry lies outside %lld x %lld", (long long)c->n, (long long)c->n);
-        }
-    } else {
-        CK(cudaMemsetAsync(c->env, 0, (size_t)c->rows * sizeof(int2), c->stream)); // the zeroed shard: every row empty
-        CK(cudaStreamSynchronize(c->stream));
+        CK(cudaMemcpyAsync(i.p, irn, (size_t)nz * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+        CK(cudaMemcpyAsync(j.p, jcn, (size_t)nz * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+        CK(cudaMemcpyAsync(v.p, val, (size_t)nz * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     }
-    c->matrix_set = true;
-    return CGB_OK;
+    StagedCsr m;
+    int bad = 0;
+    CK(csr_from_coo(&m, c->n, c->row0, c->rows, i.as<int>(), j.as<int>(), v.as<double>(), nz, symmetric ? 1 : 0, &bad,
+                    c->stream));
+    if (bad) return fail(CGB_ERR_INVALID, "a COO entry lies outside %lld x %lld", (long long)c->n, (long long)c->n);
+    return install_matrix(c, m, true);
 }
 
 extern "C" int cgb_get_matrix_rows(cgb_ctx *c, double *rows_host, int64_t first_row, int64_t nrows,
@@ -1969,22 +1960,14 @@ extern "C" int cgb_set_matrix_csr(cgb_ctx *c, const int64_t *rp_dev, const int32
     if ((rc = stream_events(c))) return rc;
     CK(cudaEventRecord(c->ev_dev[0], static_cast<cudaStream_t>(stream)));
     CK(cudaStreamWaitEvent(c->stream, c->ev_dev[0], 0));
-    struct Tmp { // freed on every path
-        long long *rp = nullptr;
-        unsigned long long *err = nullptr;
-        ~Tmp()
-        {
-            cudaFree(rp);
-            cudaFree(err);
-        }
-    } t;
-    CK(cudaMalloc(&t.rp, (size_t)(c->rows + 1) * sizeof(long long)));
-    CK(cudaMalloc(&t.err, sizeof(unsigned long long)));
+    DevBuf rp, err_dev;
+    CK(rp.alloc((size_t)(c->rows + 1) * sizeof(long long)));
+    CK(err_dev.alloc(sizeof(unsigned long long)));
     // nothing of the context is touched before the input has been checked
-    CK(launch_validate_csr(reinterpret_cast<const long long *>(rp_dev), col_dev, nnz, c->n, c->rows, t.rp, t.err,
-                           c->stream));
+    CK(launch_validate_csr(reinterpret_cast<const long long *>(rp_dev), col_dev, nnz, c->n, c->rows,
+                           rp.as<long long>(), err_dev.as<unsigned long long>(), c->stream));
     c->kernel_launches += 1;
-    CK(cudaMemcpyAsync(c->h_pin, t.err, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(c->h_pin, err_dev.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
     unsigned long long err;
     memcpy(&err, c->h_pin, sizeof err);
@@ -1996,19 +1979,8 @@ extern "C" int cgb_set_matrix_csr(cgb_ctx *c, const int64_t *rp_dev, const int32
         return fail(CGB_ERR_INVALID, "CSR refused at local row %llu: %s (n %lld, rows %lld, nnz %lld)",
                     err / kCsrFaultKinds, what[err % kCsrFaultKinds], c->n, c->rows, (long long)nnz);
     }
-    if (c->storage == 1) {
-        c->matrix_set = false;
-        c->graph_gen += 1; // col / val are reallocated, and the loop graphs bake them in
-        CK(csr_from_device(&c->csr, t.rp, c->rows, col_dev, val_dev, nnz, c->stream));
-    } else {
-        // the shard cgb_set_matrix_coo builds from the same triples: zeros, the entries, the envelopes
-        CK(csr_densify(t.rp, col_dev, val_dev, 0, c->rows, c->ld, c->A, c->stream));
-        CK(launch_row_envelope(c->A, c->ld, 0, c->rows, c->env, c->stream));
-        c->kernel_launches += 2;
-        CK(cudaStreamSynchronize(c->stream));
-    }
-    c->matrix_set = true;
-    return CGB_OK;
+    CsrShard m{rp.as<long long>(), const_cast<int *>(col_dev), const_cast<double *>(val_dev), nnz};
+    return install_matrix(c, m, false);
 }
 
 extern "C" int cgb_update_matrix_values(cgb_ctx *c, const double *val_dev, void *stream)

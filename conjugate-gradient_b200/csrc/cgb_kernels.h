@@ -129,21 +129,24 @@ cudaError_t launch_update_p_once(const VecArgs &a, cudaStream_t s);
 // (the kernels of the iteration read the LL entries directly)
 cudaError_t launch_exchange_collect(double *apx, const Gather &g, cudaStream_t s);
 
-// ---- matrix construction (vec.cu) --------------------------------------------------
-// generate_lap2d_matrix (cg.cc:159-188) into the shard
-cudaError_t launch_generate_lap2d(double *A, long long n, long long ld, long long row0,
-                                  long long rows, cudaStream_t s);
-// non-zero envelope of local rows [lr0, lr0 + nrows) of the shard into env (see block_window)
+// ---- matrix construction ------------------------------------------------------------
+// Every builder of a shard, dense or CSR, makes this rank's local CSR on the device (spmv.cu: lap2d_row
+// is the one statement of generate_lap2d_matrix's stencil, csr_from_coo the one of Matrix::read), and
+// capi.cu installs it: a CSR context adopts it, a dense one densifies it and rebuilds the envelopes.
+
+// device scratch freed on every path
+struct DevBuf {
+    void *p = nullptr;
+    ~DevBuf() { cudaFree(p); }
+    cudaError_t alloc(size_t bytes) { return cudaMalloc(&p, bytes > 0 ? bytes : 1); }
+    template <class T> T *as() const { return static_cast<T *>(p); }
+};
+// non-zero envelope of local rows [lr0, lr0 + nrows) of the dense shard into env (see block_window; vec.cu)
 cudaError_t launch_row_envelope(const double *A, long long ld, long long lr0, long long nrows, int2 *env,
                                 cudaStream_t s);
-// Matrix::read's densification (matrix.cc:12-21) on the device, "later entries overwrite" resolved
-// with an atomicMax of the entry index per cell (win: nz bytes of scratch, bad: 1 int, both device)
-cudaError_t launch_scatter_coo(double *A, long long n, long long ld, long long row0, long long rows,
-                               const int *irn, const int *jcn, const double *val, long long nz,
-                               int symmetric, unsigned char *win, int *bad, cudaStream_t s);
 
 // ---- CSR storage (spmv.cu) ----------------------------------------------------------
-// The shard: rp[rows + 1] (allocated with the context), col[nnz] / val[nnz] (sized by the builders)
+// The shard: rp[rows + 1] (rebased to 0), col[nnz] (ascending and unique per row) / val[nnz]
 struct CsrShard {
     long long *rp = nullptr;
     int *col = nullptr;
@@ -153,14 +156,18 @@ struct CsrShard {
 cudaError_t preload_spmv_kernels();
 // the CSR mat-vec, lane order (bitwise the dense mat-vec); a.csr_* set
 cudaError_t launch_spmv(const GemvArgs &a, int sm_count, cudaStream_t s);
-// generate_lap2d_matrix's non-zeros of rows [row0, row0 + rows); synchronises
+// The builders fill an empty shard `m` (all of its arrays allocated here, freed by the caller on every
+// path) and synchronise.
+// generate_lap2d_matrix's non-zeros of rows [row0, row0 + rows)
 cudaError_t csr_generate_lap2d(CsrShard *m, long long n, long long row0, long long rows, cudaStream_t s);
 // Matrix::read semantics from device COO triples (file order, mirror when symmetric, later writes
-// win); *bad_host = 1 (and the shard unchanged) when an entry lies outside n x n; synchronises
+// win, explicit zeros stored); *bad_host = 1 (and `m` left empty) when an entry lies outside n x n
 cudaError_t csr_from_coo(CsrShard *m, long long n, long long row0, long long rows, const int *irn, const int *jcn,
                          const double *val, long long nz, int symmetric, int *bad_host, cudaStream_t s);
+// col / val of `nnz` entries for a shard without them
+cudaError_t csr_alloc_entries(CsrShard *m, long long nnz);
 // rows [lr0, lr0 + nrows) of a CSR (rp indexing col / val from 0) into a dense nrows x ld device buffer,
-// zeroed first
+// zeroed first (padding columns included)
 cudaError_t csr_densify(const long long *rp, const int *col, const double *val, long long lr0, long long nrows,
                         long long ld, double *dst, cudaStream_t s);
 // A caller's CSR of `rows` rows against the stored format (cgb_set_matrix_csr): rp[0] >= 0, rp monotone,
@@ -169,9 +176,6 @@ cudaError_t csr_densify(const long long *rp, const int *col, const double *val, 
 enum { kCsrNegativeBase, kCsrNotMonotone, kCsrPastNnz, kCsrColumnRange, kCsrNotAscending, kCsrCount, kCsrFaultKinds };
 cudaError_t launch_validate_csr(const long long *rp, const int *col, long long nnz, long long n, long long rows,
                                 long long *rp_local, unsigned long long *err, cudaStream_t s);
-// the shard replaced by validated device arrays (rp_local rebased to 0); synchronises
-cudaError_t csr_from_device(CsrShard *m, const long long *rp_local, long long rows, const int *col, const double *val,
-                            long long nnz, cudaStream_t s);
 // streams the three CSR arrays once (the read ceiling of the CSR mat-vec)
 cudaError_t launch_read_csr(const CsrShard &m, long long rows, double *sink, int sm_count, cudaStream_t s);
 

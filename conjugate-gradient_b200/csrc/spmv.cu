@@ -307,8 +307,9 @@ __global__ void __launch_bounds__(kSpmvThreads) spmv_csr_block_kernel(const Bloc
 }
 
 // ---- builders ---------------------------------------------------------------------------
-// generate_lap2d_matrix (cg.cc:159-188): the non-zeros of generate_lap2d_kernel, per row in
-// ascending column order: i-1-inc, i-1, i, i+1, i+1+inc; emit(column, value) for each
+// generate_lap2d_matrix (cg.cc:159-188), the one statement of the stencil (dense shards are densified
+// from it): the non-zeros of row i in ascending column order i-1-inc, i-1, i, i+1, i+1+inc;
+// emit(column, value) for each
 template <class Emit>
 __device__ __forceinline__ void lap2d_row(long long n, long long inc, long long i, Emit emit)
 {
@@ -442,35 +443,21 @@ __global__ void __launch_bounds__(256) validate_csr_kernel(const long long *rp, 
 
 inline unsigned blocks_for(long long n, int t) { return (unsigned)((n + t - 1) / t > 0 ? (n + t - 1) / t : 1); }
 
-// device scratch freed on every path
-struct DevBuf {
-    void *p = nullptr;
-    ~DevBuf() { cudaFree(p); }
-    cudaError_t alloc(size_t bytes) { return cudaMalloc(&p, bytes > 0 ? bytes : 1); }
-    template <class T> T *as() const { return static_cast<T *>(p); }
-};
-
 #define CU(call)                                                                                   \
     do {                                                                                           \
         cudaError_t e_ = (call);                                                                   \
         if (e_ != cudaSuccess) return e_;                                                          \
     } while (0)
 
-// replace the value / column arrays of the shard by fresh ones of `nnz` entries
-cudaError_t csr_resize(CsrShard *m, long long nnz)
+} // namespace
+
+cudaError_t csr_alloc_entries(CsrShard *m, long long nnz)
 {
-    cudaFree(m->col);
-    cudaFree(m->val);
-    m->col = nullptr;
-    m->val = nullptr;
-    m->nnz = 0;
     CU(cudaMalloc(&m->col, (size_t)(nnz > 0 ? nnz : 1) * sizeof(int)));
     CU(cudaMalloc(&m->val, (size_t)(nnz > 0 ? nnz : 1) * sizeof(double)));
     m->nnz = nnz;
     return cudaSuccess;
 }
-
-} // namespace
 
 cudaError_t preload_spmv_kernels()
 {
@@ -535,6 +522,7 @@ cudaError_t csr_generate_lap2d(CsrShard *m, long long n, long long row0, long lo
 {
     const long long inc = (long long)floor(sqrt((double)n)); // cg.cc:175
     DevBuf cnt, tmp;
+    CU(cudaMalloc(&m->rp, (size_t)(rows + 1) * sizeof(long long)));
     CU(cnt.alloc((size_t)rows * sizeof(long long)));
     lap2d_count_kernel<<<blocks_for(rows, 256), 256, 0, s>>>(n, inc, row0, rows, cnt.as<long long>());
     CU(cudaGetLastError());
@@ -546,7 +534,7 @@ cudaError_t csr_generate_lap2d(CsrShard *m, long long n, long long row0, long lo
     long long nnz = 0;
     CU(cudaMemcpyAsync(&nnz, m->rp + rows, sizeof nnz, cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
-    CU(csr_resize(m, nnz));
+    CU(csr_alloc_entries(m, nnz));
     lap2d_fill_kernel<<<blocks_for(rows, 256), 256, 0, s>>>(n, inc, row0, rows, m->rp, m->col, m->val);
     CU(cudaGetLastError());
     return cudaStreamSynchronize(s);
@@ -557,14 +545,14 @@ cudaError_t csr_from_coo(CsrShard *m, long long n, long long row0, long long row
 {
     *bad_host = 0;
     const long long m2 = 2 * nz;
-    DevBuf key, kval, key_s, kval_s, keep, key_k, kval_k, nsel, bad, tmp;
+    // 66 B per triple: 2 writes x (8 B key + 8 B value) x (unsorted, sorted) + 2 flag bytes.  key / kval
+    // are dead after the sort and receive the writes kept.
+    DevBuf key, kval, key_s, kval_s, keep, nsel, bad, tmp;
     CU(key.alloc((size_t)m2 * 8));
     CU(kval.alloc((size_t)m2 * 8));
     CU(key_s.alloc((size_t)m2 * 8));
     CU(kval_s.alloc((size_t)m2 * 8));
     CU(keep.alloc((size_t)m2));
-    CU(key_k.alloc((size_t)m2 * 8));
-    CU(kval_k.alloc((size_t)m2 * 8));
     CU(nsel.alloc(sizeof(long long)));
     CU(bad.alloc(sizeof(int)));
     CU(cudaMemsetAsync(bad.p, 0, sizeof(int), s));
@@ -578,9 +566,9 @@ cudaError_t csr_from_coo(CsrShard *m, long long n, long long row0, long long row
         CU(cub::DeviceRadixSort::SortPairs(nullptr, b_sort, key.as<unsigned long long>(), key_s.as<unsigned long long>(),
                                            kval.as<double>(), kval_s.as<double>(), m2, 0, 64, s));
         CU(cub::DeviceSelect::Flagged(nullptr, b_sel, key_s.as<unsigned long long>(), keep.as<unsigned char>(),
-                                      key_k.as<unsigned long long>(), nsel.as<long long>(), m2, s));
+                                      key.as<unsigned long long>(), nsel.as<long long>(), m2, s));
         CU(cub::DeviceSelect::Flagged(nullptr, b_sel2, kval_s.as<double>(), keep.as<unsigned char>(),
-                                      kval_k.as<double>(), nsel.as<long long>(), m2, s));
+                                      kval.as<double>(), nsel.as<long long>(), m2, s));
         size_t b = b_sort > b_sel ? b_sort : b_sel;
         if (b_sel2 > b) b = b_sel2;
         CU(tmp.alloc(b));
@@ -589,20 +577,21 @@ cudaError_t csr_from_coo(CsrShard *m, long long n, long long row0, long long row
         coo_last_kernel<<<blocks_for(m2, 256), 256, 0, s>>>(key_s.as<unsigned long long>(), m2, keep.as<unsigned char>());
         CU(cudaGetLastError());
         CU(cub::DeviceSelect::Flagged(tmp.p, b_sel, key_s.as<unsigned long long>(), keep.as<unsigned char>(),
-                                      key_k.as<unsigned long long>(), nsel.as<long long>(), m2, s));
+                                      key.as<unsigned long long>(), nsel.as<long long>(), m2, s));
         CU(cub::DeviceSelect::Flagged(tmp.p, b_sel2, kval_s.as<double>(), keep.as<unsigned char>(),
-                                      kval_k.as<double>(), nsel.as<long long>(), m2, s));
+                                      kval.as<double>(), nsel.as<long long>(), m2, s));
     }
     long long nnz = 0;
     CU(cudaMemcpyAsync(&nnz, nsel.p, sizeof nnz, cudaMemcpyDeviceToHost, s));
     CU(cudaMemcpyAsync(bad_host, bad.p, sizeof(int), cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
     if (*bad_host) return cudaSuccess;
-    CU(csr_resize(m, nnz));
-    csr_rows_kernel<<<blocks_for(rows + 1, 256), 256, 0, s>>>(key_k.as<unsigned long long>(), nnz, rows, m->rp);
-    csr_cols_kernel<<<blocks_for(nnz, 256), 256, 0, s>>>(key_k.as<unsigned long long>(), nnz, m->col);
+    CU(cudaMalloc(&m->rp, (size_t)(rows + 1) * sizeof(long long)));
+    CU(csr_alloc_entries(m, nnz));
+    csr_rows_kernel<<<blocks_for(rows + 1, 256), 256, 0, s>>>(key.as<unsigned long long>(), nnz, rows, m->rp);
+    csr_cols_kernel<<<blocks_for(nnz, 256), 256, 0, s>>>(key.as<unsigned long long>(), nnz, m->col);
     CU(cudaGetLastError());
-    if (nnz > 0) CU(cudaMemcpyAsync(m->val, kval_k.p, (size_t)nnz * 8, cudaMemcpyDeviceToDevice, s));
+    if (nnz > 0) CU(cudaMemcpyAsync(m->val, kval.p, (size_t)nnz * 8, cudaMemcpyDeviceToDevice, s));
     return cudaStreamSynchronize(s);
 }
 
@@ -620,18 +609,6 @@ cudaError_t launch_validate_csr(const long long *rp, const int *col, long long n
     CU(cudaMemsetAsync(err, 0xff, sizeof *err, s));
     validate_csr_kernel<<<blocks_for(rows, 8), 256, 0, s>>>(rp, col, nnz, n, rows, rp_local, err);
     return cudaGetLastError();
-}
-
-cudaError_t csr_from_device(CsrShard *m, const long long *rp_local, long long rows, const int *col, const double *val,
-                            long long nnz, cudaStream_t s)
-{
-    CU(csr_resize(m, nnz));
-    CU(cudaMemcpyAsync(m->rp, rp_local, (size_t)(rows + 1) * sizeof(long long), cudaMemcpyDeviceToDevice, s));
-    if (nnz > 0) {
-        CU(cudaMemcpyAsync(m->col, col, (size_t)nnz * sizeof(int), cudaMemcpyDeviceToDevice, s));
-        CU(cudaMemcpyAsync(m->val, val, (size_t)nnz * sizeof(double), cudaMemcpyDeviceToDevice, s));
-    }
-    return cudaStreamSynchronize(s);
 }
 
 cudaError_t launch_read_csr(const CsrShard &m, long long rows, double *sink, int sm_count, cudaStream_t s)

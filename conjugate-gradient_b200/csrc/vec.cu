@@ -453,37 +453,6 @@ __global__ void __launch_bounds__(kChunk) exchange_collect_kernel(double *apx, c
     exchange_consumed(g, tid);
 }
 
-// generate_lap2d_matrix (cg.cc:159-188): every element of the shard is written once, two
-// columns per thread (128-bit stores); padding columns [n, ld) are zero.
-__global__ void __launch_bounds__(256) generate_lap2d_kernel(double *A, long long n, long long ld,
-                                                              long long row0, long long rows,
-                                                              long long inc)
-{
-    const long long half = ld >> 1;
-    const long long total = rows * half;
-    const long long stride = (long long)gridDim.x * blockDim.x;
-    for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += stride) {
-        const long long li = e / half;
-        const long long j0 = (e - li * half) * 2;
-        const long long i = row0 + li;
-        double v[2];
-#pragma unroll
-        for (int u = 0; u < 2; ++u) {
-            const long long j = j0 + u;
-            double val = 0.0;
-            if (j < n) {
-                if (i > inc && j == i - 1 - inc) val = -1.0;
-                if (i > 0 && j == i - 1) val = -1.0;
-                if (j == i) val = 4.0;
-                if (i < n - 1 && j == i + 1) val = -1.0;
-                if (i < n - 1 - inc && j == i + 1 + inc) val = -1.0;
-            }
-            v[u] = val;
-        }
-        *reinterpret_cast<double2 *>(A + li * ld + j0) = make_double2(v[0], v[1]);
-    }
-}
-
 // Envelope of every row of [lr0, lr0 + nrows) (see block_window): one warp per row, 128-bit loads,
 // lane l sees the columns 2(l + 32 i), +1; "non-zero" is any bit pattern but +-0 (NaN and Inf count).
 __global__ void __launch_bounds__(256) row_envelope_kernel(const double *A, long long ld, long long lr0,
@@ -517,56 +486,6 @@ __global__ void __launch_bounds__(256) row_envelope_kernel(const double *A, long
     first = __reduce_min_sync(0xffffffffu, first);
     last = __reduce_max_sync(0xffffffffu, last);
     if (lane == 0) env[lr0 + row] = last >= 0 ? make_int2(first, last + 1) : make_int2(0, 0);
-}
-
-// Matrix::read's densification (matrix.cc:12-21: A(i,j) = a, and A(j,i) = a when symmetric, in file
-// order, later entries overwriting) as three parallel passes.  The shard's own 8-byte cells hold
-// "index of the last writer + 1" between pass 1 and pass 3 (0 = untouched = the value 0.0).
-__device__ __forceinline__ unsigned long long *coo_cell(double *A, long long ld, long long row0, long long rows,
-                                                         long long i, long long j)
-{
-    return (i >= row0 && i < row0 + rows) ? reinterpret_cast<unsigned long long *>(A + (i - row0) * ld + j) : nullptr;
-}
-__global__ void __launch_bounds__(256) coo_claim_kernel(double *A, long long n, long long ld, long long row0,
-                                                         long long rows, const int *irn, const int *jcn,
-                                                         long long nz, int symmetric, int *bad)
-{
-    const long long z = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (z >= nz) return;
-    const long long i = irn[z], j = jcn[z];
-    if (i < 0 || j < 0 || i >= n || j >= n) {
-        *bad = 1;
-        return;
-    }
-    if (unsigned long long *cell = coo_cell(A, ld, row0, rows, i, j)) atomicMax(cell, (unsigned long long)z + 1ULL);
-    if (symmetric)
-        if (unsigned long long *cell = coo_cell(A, ld, row0, rows, j, i)) atomicMax(cell, (unsigned long long)z + 1ULL);
-}
-__global__ void __launch_bounds__(256) coo_winner_kernel(double *A, long long n, long long ld, long long row0,
-                                                          long long rows, const int *irn, const int *jcn,
-                                                          long long nz, int symmetric, unsigned char *win)
-{
-    const long long z = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (z >= nz) return;
-    const long long i = irn[z], j = jcn[z];
-    unsigned char w = 0;
-    if (i >= 0 && j >= 0 && i < n && j < n) {
-        if (unsigned long long *cell = coo_cell(A, ld, row0, rows, i, j)) w |= (*cell == (unsigned long long)z + 1ULL) ? 1 : 0;
-        if (symmetric)
-            if (unsigned long long *cell = coo_cell(A, ld, row0, rows, j, i)) w |= (*cell == (unsigned long long)z + 1ULL) ? 2 : 0;
-    }
-    win[z] = w;
-}
-__global__ void __launch_bounds__(256) coo_store_kernel(double *A, long long ld, long long row0, const int *irn,
-                                                         const int *jcn, const double *val, long long nz,
-                                                         const unsigned char *win)
-{
-    const long long z = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (z >= nz) return;
-    const unsigned char w = win[z];
-    const long long i = irn[z], j = jcn[z];
-    if (w & 1) A[(i - row0) * ld + j] = val[z];                                     // matrix.cc:17
-    if (w & 2) A[(j - row0) * ld + i] = val[z];                                     // matrix.cc:18-20
 }
 
 inline int grid_for(long long n) { return (int)((n + kChunk - 1) / kChunk); }
@@ -714,30 +633,6 @@ cudaError_t launch_exchange_collect(double *apx, const Gather &g, cudaStream_t s
     long long blocks = (total + kChunk - 1) / kChunk;
     if (blocks > 296) blocks = 296;
     exchange_collect_kernel<<<(int)blocks, kChunk, 0, s>>>(apx, g);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_generate_lap2d(double *A, long long n, long long ld, long long row0,
-                                  long long rows, cudaStream_t s)
-{
-    const long long inc = (long long)floor(sqrt((double)n)); // cg.cc:175
-    const long long total = rows * (ld >> 1);
-    long long blocks = (total + 255) / 256;
-    if (blocks > 148LL * 32) blocks = 148LL * 32;
-    if (blocks < 1) blocks = 1;
-    generate_lap2d_kernel<<<(int)blocks, 256, 0, s>>>(A, n, ld, row0, rows, inc);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_scatter_coo(double *A, long long n, long long ld, long long row0, long long rows,
-                               const int *irn, const int *jcn, const double *val, long long nz,
-                               int symmetric, unsigned char *win, int *bad, cudaStream_t s)
-{
-    if (nz <= 0) return cudaSuccess;
-    const int grid = (int)((nz + 255) / 256);
-    coo_claim_kernel<<<grid, 256, 0, s>>>(A, n, ld, row0, rows, irn, jcn, nz, symmetric, bad);
-    coo_winner_kernel<<<grid, 256, 0, s>>>(A, n, ld, row0, rows, irn, jcn, nz, symmetric, win);
-    coo_store_kernel<<<grid, 256, 0, s>>>(A, ld, row0, irn, jcn, val, nz, win);
     return cudaGetLastError();
 }
 

@@ -97,8 +97,9 @@ int cgb_exchange_export(cgb_ctx *ctx, void *blob_out);
 int cgb_exchange_import(cgb_ctx *ctx, const void *blobs);
 
 /* ---- inputs -------------------------------------------------------------------------- */
-/* CGSolver::generate_lap2d_matrix (code/MPI/cg.cc:159-188), written straight into this
- * rank's device shard (values exactly 0, -1, 4; inc = floor(sqrt(n))). */
+/* CGSolver::generate_lap2d_matrix (code/MPI/cg.cc:159-188), this rank's rows built on the device
+ * (values exactly 0, -1, 4; inc = floor(sqrt(n))): staged as CSR (5 non-zeros per row), then taken
+ * over by a CSR context or densified into a dense one, padding columns zeroed. */
 int cgb_generate_lap2d(cgb_ctx *ctx);
 
 /* Dense rows from the host (what Matrix::read, matrix.cc:6-22, produces): `nrows` rows
@@ -107,9 +108,15 @@ int cgb_generate_lap2d(cgb_ctx *ctx);
 int cgb_set_matrix_rows(cgb_ctx *ctx, const double *rows_host, int64_t first_row, int64_t nrows,
                         int64_t ld_host);
 
-/* Matrix::read's densification (matrix.cc:12-21) done on the device: zero the shard, then
- * scatter the COO triples (0-based) in file order, mirroring (j,i) when `symmetric`.
- * Later duplicates win, as in the reference. */
+/* Matrix::read's densification (matrix.cc:12-21) done on the device: the COO triples (0-based)
+ * in file order, mirroring (j,i) when `symmetric`; later duplicates win, as in the reference, and
+ * explicit zeros are stored.  The triples are uploaded once and this rank's rows staged as CSR (a
+ * stable sort of the writes by row and column, the last of each run kept), which a CSR context takes
+ * over and a dense one densifies, padding columns zeroed.  The staging takes about 82 bytes of device
+ * memory per triple besides the shard and the sort's scratch, so a dense context loaded from a very
+ * large COO (around 10^9 triples: some 82 GB) needs that much free next to its shard.  An entry
+ * outside n x n returns CGB_ERR_INVALID before anything of the context is touched: the previous
+ * matrix stays, and stays set. */
 int cgb_set_matrix_coo(cgb_ctx *ctx, int64_t nz, const int32_t *irn, const int32_t *jcn,
                        const double *val, int symmetric);
 

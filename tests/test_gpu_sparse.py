@@ -66,21 +66,45 @@ def test_generate_lap2d_csr_rows(cgb, O, n):
 
 
 @pytest.mark.parametrize("symmetric", [False, True])
-def test_csr_from_coo_million_duplicates_is_the_dense_scatter(cgb, symmetric):
+def test_coo_million_duplicates_dense_and_csr_are_the_oracle(cgb, symmetric):
     n, nz = 1500, 1_000_000
     rng = np.random.default_rng(31 + int(symmetric))
     irn = rng.integers(0, n, nz, dtype=np.int32)
     jcn = rng.integers(0, n, nz, dtype=np.int32)
     val = rng.standard_normal(nz)
     val[::1000] = 0.0
+    want = csr_oracle.csr_from_coo(n, irn, jcn, val, symmetric).dense()
     with cgb.Context(n) as d, cgb.Context(n, storage="csr") as c:
         d.set_matrix_coo(irn, jcn, val, symmetric=symmetric)
         c.set_matrix_coo(irn, jcn, val, symmetric=symmetric)
-        assert np.array_equal(_bits(c.get_matrix_rows(0, n)), _bits(d.get_matrix_rows(0, n)))
+        assert _eq(d.get_matrix_rows(0, n), want)
+        assert _eq(c.get_matrix_rows(0, n), want)
         with pytest.raises(cgb.CgbError) as ei:
             c.set_matrix_coo(np.array([0, n], dtype=np.int32), np.array([0, 0], dtype=np.int32),
                              np.array([1.0, 2.0]), symmetric=False)
         assert ei.value.code == 1
+
+
+@pytest.mark.parametrize("storage", ["dense", "csr"])
+def test_refused_coo_keeps_the_previous_matrix(cgb, O, storage):
+    """A COO load with an entry outside n x n is refused before the context is touched: the previous
+    matrix stays, bit for bit, and still solves."""
+    n = 1000
+    b = O.init_source_term(n)
+    x_ref, info_ref, hist_ref, _, _ = _solve(cgb, n, storage, _lap2d(b), n)
+    with cgb.Context(n, storage=storage) as ctx:
+        ctx.generate_lap2d()
+        ctx.set_rhs(b)
+        A = ctx.get_matrix_rows(0, n)
+        with pytest.raises(cgb.CgbError) as ei:
+            ctx.set_matrix_coo(np.array([0, n], dtype=np.int32), np.array([0, 0], dtype=np.int32),
+                               np.array([1.0, 2.0]), symmetric=False)
+        assert ei.value.code == 1 and "outside" in str(ei.value)
+        assert _eq(ctx.get_matrix_rows(0, n), A)
+        x = np.zeros(n)
+        info, hist = ctx.solve(x, max_iter=n, history=True)
+    assert (info.k, info.converged) == (info_ref.k, info_ref.converged)
+    assert _eq(hist, hist_ref) and _eq(x, x_ref)
 
 
 # --------------------------------------------------------------------------- mat-vec
