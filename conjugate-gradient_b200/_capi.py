@@ -56,6 +56,8 @@ SIGNATURES = [
     ("cgb_set_matrix_coo", C.c_int, [_CTX, C.c_int64, _i32p, _i32p, _dp, C.c_int]),
     ("cgb_set_matrix_csr", C.c_int, [_CTX, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     ("cgb_update_matrix_values", C.c_int, [_CTX, C.c_void_p, C.c_void_p]),
+    ("cgb_assemble_coo", C.c_int, [_CTX, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    ("cgb_assemble_values", C.c_int, [_CTX, C.c_void_p, C.c_void_p]),
     ("cgb_get_matrix_rows", C.c_int, [_CTX, _dp, C.c_int64, C.c_int64, C.c_int64]),
     ("cgb_init_source_term", C.c_int, [C.c_int64, C.c_double, _dp]),
     ("cgb_set_rhs", C.c_int, [_CTX, _dp]),
@@ -314,6 +316,50 @@ class Context:
             raise ValueError(f"val has {val.numel()} entries, the matrix {nnz}")
         _check(self._lib.cgb_update_matrix_values(self._h, val.data_ptr(), stream.cuda_stream))
         val.record_stream(stream)   # its memory is not handed out again before `stream` has passed the copy
+
+    def assemble_coo(self, coo, symmetric: bool = False, stream=None):
+        """cgb_assemble_coo: the matrix as the sum of COO contributions on the GPU -- an uncoalesced CUDA
+        torch.sparse_coo_tensor of float64 (its entries read in stored order; it is never coalesced, which would
+        reorder them) or a (rows, cols, vals) tuple of CUDA tensors, indices int32 or int64.  Duplicates are
+        added in entry order (see include/cgb200.h).  Runs on `stream` (default: the current torch stream) and
+        returns with the matrix built."""
+        import torch
+        if isinstance(coo, torch.Tensor):
+            if coo.layout != torch.sparse_coo:
+                raise TypeError("coo must be a torch.sparse_coo_tensor or a (rows, cols, vals) tuple")
+            if tuple(coo.shape) != (self.n, self.n):
+                raise ValueError(f"coo is {tuple(coo.shape)}, the context {self.n} x {self.n}")
+            idx = coo._indices()
+            rows, cols, vals = idx[0], idx[1], coo._values()
+        else:
+            rows, cols, vals = coo
+        torch, dev, stream = self._device_args([("vals", vals)], stream)
+        nz = vals.numel()
+        for nm, t in (("rows", rows), ("cols", cols)):
+            if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype in (torch.int32, torch.int64)):
+                raise TypeError(f"{nm} must be an int32 or int64 CUDA tensor")
+            if t.device.index != dev:
+                raise ValueError(f"{nm} is on cuda:{t.device.index}, the context on cuda:{dev}")
+            if t.numel() != nz:
+                raise ValueError(f"{nm} has {t.numel()} entries, vals {nz}")
+        with torch.cuda.stream(stream):
+            # an index out of range stays out of range, and is refused by the library
+            irn, jcn = (t.contiguous() if t.dtype == torch.int32 else t.clamp(-1, self.n).to(torch.int32)
+                        for t in (rows, cols))
+            _check(self._lib.cgb_assemble_coo(self._h, nz, irn.data_ptr(), jcn.data_ptr(), vals.data_ptr(),
+                                              int(bool(symmetric)), stream.cuda_stream))
+        self._assembled_nz = nz
+
+    def assemble_values(self, vals, stream=None):
+        """cgb_assemble_values: new contributions (the float64 CUDA tensor `vals`, in the entry order of the last
+        assemble_coo) folded into the matrix with its pattern and fold order, enqueued on `stream`; returns at
+        once."""
+        torch, dev, stream = self._device_args([("vals", vals)], stream)
+        nz = getattr(self, "_assembled_nz", 0)
+        if vals.numel() < nz:
+            raise ValueError(f"vals has {vals.numel()} entries, the assembly {nz}")
+        _check(self._lib.cgb_assemble_values(self._h, vals.data_ptr(), stream.cuda_stream))
+        vals.record_stream(stream)   # its memory is not handed out again before `stream` has passed the fold
 
     def get_matrix_rows(self, first_row: int, nrows: int) -> np.ndarray:
         out = np.empty((nrows, self.n), dtype=np.float64)

@@ -178,6 +178,7 @@ struct cgb_ctx {
 
     int storage = 0;               // 0: dense rows x ld shard `A`, 1: CSR shard `csr` (cgb_create_csr)
     CsrShard csr;
+    AsmPlan plan;                  // the last cgb_assemble_coo's, while its matrix is the context's (start: null)
     unsigned int *arrive = nullptr; // CSR: arrival counters of the once-per-iteration vector phase
     double *A = nullptr, *p = nullptr, *r = nullptr, *x = nullptr, *b = nullptr;
     int2 *env = nullptr;           // dense: [first, last + 1) of the non-zero columns of every local row,
@@ -1129,6 +1130,7 @@ extern "C" int cgb_destroy(cgb_ctx *c)
     if (c->csr.rp) cudaFree(c->csr.rp);
     if (c->csr.col) cudaFree(c->csr.col);
     if (c->csr.val) cudaFree(c->csr.val);
+    asm_plan_free(&c->plan);
     if (c->arrive) cudaFree(c->arrive);
     if (c->compat_part) cudaFree(c->compat_part);
     free_trace(c);
@@ -1263,15 +1265,22 @@ struct StagedCsr : CsrShard {
     }
 };
 
+// cgb_assemble_coo's plan until install_matrix adopts it
+struct StagedPlan : AsmPlan {
+    ~StagedPlan() { asm_plan_free(this); }
+};
+
 // The one place a built matrix becomes the context's.  `m` is this rank's validated local CSR in device
 // memory: rp rebased to 0, columns ascending and unique per row, explicit zeros kept.  A CSR context adopts
 // it: a builder's staging (`staged`) is swapped in, a caller's arrays are copied.  The loop graphs bake in
 // col / val, which move, so the generation is bumped.  A dense context densifies it into A (the whole
 // rows x ld block is zeroed first) and rebuilds every row's envelope; its graphs bake in A and env, which
-// stay where they are, so its generation is not bumped.
-int install_matrix(cgb_ctx *c, CsrShard &m, bool staged)
+// stay where they are, so its generation is not bumped.  The previous matrix's assembly plan goes; `plan`
+// (cgb_assemble_coo's, of `m`) becomes the context's, on a dense context with m's rp / col to find A's cells.
+int install_matrix(cgb_ctx *c, CsrShard &m, bool staged, AsmPlan *plan = nullptr)
 {
     c->matrix_set = false; // until the install completes
+    asm_plan_free(&c->plan);
     if (c->storage == 1) {
         StagedCsr copy;
         if (!staged) {
@@ -1293,6 +1302,13 @@ int install_matrix(cgb_ctx *c, CsrShard &m, bool staged)
         c->kernel_launches += 2;
     }
     CK(cudaStreamSynchronize(c->stream));
+    if (plan) {
+        if (c->storage == 0) {
+            std::swap(plan->rp, m.rp);
+            std::swap(plan->col, m.col);
+        }
+        std::swap(c->plan, *plan);
+    }
     c->matrix_set = true;
     return CGB_OK;
 }
@@ -1322,6 +1338,7 @@ extern "C" int cgb_set_matrix_rows(cgb_ctx *c, const double *rows_host, int64_t 
                     (long long)nrows, (long long)ld_host);
     const long long lo = std::max<long long>(first_row, c->row0);
     const long long hi = std::min<long long>(first_row + nrows, c->row0 + c->rows);
+    asm_plan_free(&c->plan); // the rows may overwrite assembled cells
     if (hi > lo) {
         CK(cudaMemcpy2DAsync(c->A + (lo - c->row0) * c->ld, (size_t)c->ld * 8,
                              rows_host + (lo - first_row) * ld_host, (size_t)ld_host * 8,
@@ -1999,6 +2016,60 @@ extern "C" int cgb_update_matrix_values(cgb_ctx *c, const double *val_dev, void 
     CK(cudaStreamWaitEvent(c->stream, c->ev_dev[0], 0));
     if (c->csr.nnz > 0)
         CK(cudaMemcpyAsync(c->csr.val, val_dev, (size_t)c->csr.nnz * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
+    CK(cudaEventRecord(c->ev_dev[1], c->stream));
+    CK(cudaStreamWaitEvent(us, c->ev_dev[1], 0));
+    return CGB_OK;
+}
+
+// ------------------------------------------------------------------ sum-assembly from device COO (DESIGN 3.11)
+extern "C" int cgb_assemble_coo(cgb_ctx *c, int64_t nz, const int32_t *irn_dev, const int32_t *jcn_dev,
+                                const double *val_dev, int symmetric, void *stream)
+{
+    if (!c) return null_context();
+    int rc = use_device(c);
+    if (rc) return rc;
+    if (c->in_solve) return fail(CGB_ERR_STATE, c->blk.active ? "a block solve is in progress" : "a single solve is in progress");
+    if (nz < 0) return fail(CGB_ERR_INVALID, "nz < 0 (got %lld)", (long long)nz);
+    if (nz > 0 && ((rc = check_device_ptr(c, irn_dev, "irn")) || (rc = check_device_ptr(c, jcn_dev, "jcn")) ||
+                   (rc = check_device_ptr(c, val_dev, "val"))))
+        return rc;
+    if ((rc = stream_events(c))) return rc;
+    CK(cudaEventRecord(c->ev_dev[0], static_cast<cudaStream_t>(stream)));
+    CK(cudaStreamWaitEvent(c->stream, c->ev_dev[0], 0));
+    StagedCsr m;
+    StagedPlan plan;
+    int bad = 0;
+    CK(csr_assemble_coo(&m, &plan, c->n, c->row0, c->rows, irn_dev, jcn_dev, val_dev, nz, symmetric ? 1 : 0, &bad,
+                        c->stream));
+    c->kernel_launches += nz > 0 ? 5 : 2; // keys, runs, rows, cols, fold (CUB's sort and selects not counted)
+    // nothing of the context, its matrix or its plan, is touched before every triple has been checked
+    if (bad) return fail(CGB_ERR_INVALID, "a COO entry lies outside %lld x %lld", (long long)c->n, (long long)c->n);
+    return install_matrix(c, m, true, &plan);
+}
+
+extern "C" int cgb_assemble_values(cgb_ctx *c, const double *val_dev, void *stream)
+{
+    if (!c) return null_context();
+    int rc = use_device(c);
+    if (rc) return rc;
+    if (!c->plan.start || !c->matrix_set)
+        return fail(CGB_ERR_STATE, "no assembly plan: the matrix was not built by cgb_assemble_coo, or another builder replaced it");
+    if (c->in_solve) return fail(CGB_ERR_STATE, c->blk.active ? "a block solve is in progress" : "a single solve is in progress");
+    if (c->plan.nz > 0 && (rc = check_device_ptr(c, val_dev, "val"))) return rc;
+    if ((rc = stream_events(c))) return rc;
+    // the values are written where they are (CSR: csr.val, dense: A): every cached loop graph stays valid
+    const cudaStream_t us = static_cast<cudaStream_t>(stream);
+    CK(cudaEventRecord(c->ev_dev[0], us));
+    CK(cudaStreamWaitEvent(c->stream, c->ev_dev[0], 0));
+    if (c->storage == 1) {
+        CK(launch_assemble_csr(c->plan, val_dev, c->csr.val, c->stream));
+        c->kernel_launches += 1;
+    } else {
+        // a cell stored as 0 at assembly lies outside its row's envelope and may have become non-zero
+        CK(launch_assemble_dense(c->plan, val_dev, c->ld, c->A, c->stream));
+        CK(launch_row_envelope(c->A, c->ld, 0, c->rows, c->env, c->stream));
+        c->kernel_launches += 2;
+    }
     CK(cudaEventRecord(c->ev_dev[1], c->stream));
     CK(cudaStreamWaitEvent(us, c->ev_dev[1], 0));
     return CGB_OK;

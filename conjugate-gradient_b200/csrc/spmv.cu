@@ -1,5 +1,5 @@
 // spmv.cu -- CSR storage of the row shard: the mat-vec in lane order and the builders of the shard
-// (generate_lap2d_matrix, Matrix::read's COO semantics) on the device.
+// (generate_lap2d_matrix, Matrix::read's COO semantics, sum-assembly of COO contributions) on the device.
 //
 // Exactness.  The dense mat-vec (gemv.cu, oracle/cg_oracle.h "lane order") keeps 64 accumulators
 // acc[c % 64] = fma(A[i][c], p[c], acc[c % 64]) over ascending c from +0, adds acc[2l] + acc[2l+1]
@@ -22,6 +22,7 @@
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 #include <cub/device/device_select.cuh>
+#include <thrust/iterator/counting_iterator.h>
 
 namespace cgb {
 
@@ -373,6 +374,67 @@ __global__ void coo_last_kernel(const unsigned long long *key, long long m, unsi
     keep[k] = (key[k] != kNoKey && (k == m - 1 || key[k + 1] != key[k])) ? 1 : 0;
 }
 
+// Sum-assembly (cgb_assemble_coo): coo_keys_kernel's write sequence, except that a diagonal triple is not
+// mirrored (in a sum it would count twice) and the sort payload is the write id, so that the sorted order
+// doubles as the plan every later re-assembly gathers by
+__global__ void asm_keys_kernel(long long n, long long row0, long long rows, const int *irn, const int *jcn,
+                                long long nz, int symmetric, unsigned long long *key, long long *wid, int *bad)
+{
+    const long long z = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (z >= nz) return;
+    const long long i = irn[z], j = jcn[z];
+    unsigned long long k0 = kNoKey, k1 = kNoKey;
+    if (i < 0 || j < 0 || i >= n || j >= n) {
+        *bad = 1;
+    } else {
+        if (i >= row0 && i < row0 + rows) k0 = ((unsigned long long)(i - row0) << 32) | (unsigned long long)j;
+        if (symmetric && i != j && j >= row0 && j < row0 + rows)
+            k1 = ((unsigned long long)(j - row0) << 32) | (unsigned long long)i;
+    }
+    key[2 * z] = k0;
+    key[2 * z + 1] = k1;
+    wid[2 * z] = 2 * z;
+    wid[2 * z + 1] = 2 * z + 1;
+}
+
+// after the stable sort: flag the first write of every (row, column) run; *nw = the writes this shard keeps
+__global__ void asm_runs_kernel(const unsigned long long *key, long long m, unsigned char *first, long long *nw)
+{
+    const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= m) return;
+    const bool kept = key[k] != kNoKey;
+    first[k] = (kept && (k == 0 || key[k - 1] != key[k])) ? 1 : 0;
+    if (kept && (k == m - 1 || key[k + 1] == kNoKey)) *nw = k + 1;
+}
+
+// The one statement of the fold: stored entry e is its run of writes folded left in write order, starting
+// from the first write (not from +0, which would turn a lone -0 into +0).  Serial per cell by definition.
+__device__ __forceinline__ double fold_run(const AsmPlan &p, const double *val, long long e)
+{
+    const long long end = p.start[e + 1];
+    long long k = p.start[e];
+    double v = val[p.wid[k] >> 1];
+    for (++k; k < end; ++k) v = __dadd_rn(v, val[p.wid[k] >> 1]);
+    return v;
+}
+
+// CSR shard: the values in stored order, one thread per entry
+__global__ void assemble_csr_kernel(const AsmPlan p, const double *val, double *out)
+{
+    const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e < p.nnz) out[e] = fold_run(p, val, e);
+}
+
+// dense shard: one warp per row (its row from the plan's rp), lanes striding over the row's entries
+__global__ void __launch_bounds__(256) assemble_dense_kernel(const AsmPlan p, const double *val, long long ld,
+                                                              double *A)
+{
+    const long long row = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (row >= p.rows) return;
+    const long long end = p.rp[row + 1];
+    for (long long e = p.rp[row] + (threadIdx.x & 31); e < end; e += 32) A[row * ld + p.col[e]] = fold_run(p, val, e);
+}
+
 // row pointers and columns from the surviving keys (sorted by row, then column)
 __global__ void csr_rows_kernel(const unsigned long long *key, long long nnz, long long rows, long long *rp)
 {
@@ -593,6 +655,97 @@ cudaError_t csr_from_coo(CsrShard *m, long long n, long long row0, long long row
     CU(cudaGetLastError());
     if (nnz > 0) CU(cudaMemcpyAsync(m->val, kval.p, (size_t)nnz * 8, cudaMemcpyDeviceToDevice, s));
     return cudaStreamSynchronize(s);
+}
+
+void asm_plan_free(AsmPlan *p)
+{
+    cudaFree(p->wid);
+    cudaFree(p->start);
+    cudaFree(p->rp);
+    cudaFree(p->col);
+    *p = AsmPlan();
+}
+
+cudaError_t csr_assemble_coo(CsrShard *m, AsmPlan *p, long long n, long long row0, long long rows, const int *irn,
+                             const int *jcn, const double *val, long long nz, int symmetric, int *bad_host,
+                             cudaStream_t s)
+{
+    *bad_host = 0;
+    const long long m2 = 2 * nz;
+    // 66 B per triple: 2 writes x (8 B key + 8 B write id) x (unsorted, sorted) + 2 flag bytes.  key / wid are
+    // dead after the sort and receive the unique keys and the run starts.  cnt: [0] entries, [1] writes kept.
+    DevBuf key, wid, key_s, wid_s, first, cnt, bad, tmp;
+    CU(key.alloc((size_t)m2 * 8));
+    CU(wid.alloc((size_t)m2 * 8));
+    CU(key_s.alloc((size_t)m2 * 8));
+    CU(wid_s.alloc((size_t)m2 * 8));
+    CU(first.alloc((size_t)m2));
+    CU(cnt.alloc(2 * sizeof(long long)));
+    CU(bad.alloc(sizeof(int)));
+    CU(cudaMemsetAsync(bad.p, 0, sizeof(int), s));
+    CU(cudaMemsetAsync(cnt.p, 0, 2 * sizeof(long long), s));
+    if (nz > 0) {
+        asm_keys_kernel<<<blocks_for(nz, 256), 256, 0, s>>>(n, row0, rows, irn, jcn, nz, symmetric,
+                                                            key.as<unsigned long long>(), wid.as<long long>(), bad.as<int>());
+        CU(cudaGetLastError());
+        // radix sort is stable: equal (row, column) keys keep their write order
+        const thrust::counting_iterator<long long> pos(0);
+        size_t b_sort = 0, b_sel = 0, b_sel2 = 0;
+        CU(cub::DeviceRadixSort::SortPairs(nullptr, b_sort, key.as<unsigned long long>(), key_s.as<unsigned long long>(),
+                                           wid.as<long long>(), wid_s.as<long long>(), m2, 0, 64, s));
+        CU(cub::DeviceSelect::Flagged(nullptr, b_sel, key_s.as<unsigned long long>(), first.as<unsigned char>(),
+                                      key.as<unsigned long long>(), cnt.as<long long>(), m2, s));
+        CU(cub::DeviceSelect::Flagged(nullptr, b_sel2, pos, first.as<unsigned char>(), wid.as<long long>(),
+                                      cnt.as<long long>(), m2, s));
+        size_t b = b_sort > b_sel ? b_sort : b_sel;
+        if (b_sel2 > b) b = b_sel2;
+        CU(tmp.alloc(b));
+        CU(cub::DeviceRadixSort::SortPairs(tmp.p, b_sort, key.as<unsigned long long>(), key_s.as<unsigned long long>(),
+                                           wid.as<long long>(), wid_s.as<long long>(), m2, 0, 64, s));
+        asm_runs_kernel<<<blocks_for(m2, 256), 256, 0, s>>>(key_s.as<unsigned long long>(), m2, first.as<unsigned char>(),
+                                                            cnt.as<long long>() + 1);
+        CU(cudaGetLastError());
+        CU(cub::DeviceSelect::Flagged(tmp.p, b_sel, key_s.as<unsigned long long>(), first.as<unsigned char>(),
+                                      key.as<unsigned long long>(), cnt.as<long long>(), m2, s));
+        CU(cub::DeviceSelect::Flagged(tmp.p, b_sel2, pos, first.as<unsigned char>(), wid.as<long long>(),
+                                      cnt.as<long long>(), m2, s));
+    }
+    long long counts[2] = {0, 0};
+    CU(cudaMemcpyAsync(counts, cnt.p, sizeof counts, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpyAsync(bad_host, bad.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    if (*bad_host) return cudaSuccess;
+    const long long nnz = counts[0], nw = counts[1];
+    CU(cudaMalloc(&m->rp, (size_t)(rows + 1) * sizeof(long long)));
+    CU(csr_alloc_entries(m, nnz));
+    CU(cudaMalloc(&p->wid, (size_t)(nw > 0 ? nw : 1) * sizeof(long long)));
+    CU(cudaMalloc(&p->start, (size_t)(nnz + 1) * sizeof(long long)));
+    p->nz = nz;
+    p->nnz = nnz;
+    p->nwrites = nw;
+    p->rows = rows;
+    csr_rows_kernel<<<blocks_for(rows + 1, 256), 256, 0, s>>>(key.as<unsigned long long>(), nnz, rows, m->rp);
+    csr_cols_kernel<<<blocks_for(nnz, 256), 256, 0, s>>>(key.as<unsigned long long>(), nnz, m->col);
+    CU(cudaGetLastError());
+    if (nw > 0) CU(cudaMemcpyAsync(p->wid, wid_s.p, (size_t)nw * 8, cudaMemcpyDeviceToDevice, s));
+    if (nnz > 0) CU(cudaMemcpyAsync(p->start, wid.p, (size_t)nnz * 8, cudaMemcpyDeviceToDevice, s));
+    CU(cudaMemcpyAsync(p->start + nnz, cnt.as<long long>() + 1, sizeof(long long), cudaMemcpyDeviceToDevice, s));
+    CU(launch_assemble_csr(*p, val, m->val, s));
+    return cudaStreamSynchronize(s);
+}
+
+cudaError_t launch_assemble_csr(const AsmPlan &p, const double *val, double *out, cudaStream_t s)
+{
+    if (p.nnz == 0) return cudaSuccess;
+    assemble_csr_kernel<<<blocks_for(p.nnz, 256), 256, 0, s>>>(p, val, out);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_assemble_dense(const AsmPlan &p, const double *val, long long ld, double *A, cudaStream_t s)
+{
+    if (p.nnz == 0) return cudaSuccess;
+    assemble_dense_kernel<<<blocks_for(p.rows, 8), 256, 0, s>>>(p, val, ld, A);
+    return cudaGetLastError();
 }
 
 cudaError_t csr_densify(const long long *rp, const int *col, const double *val, long long lr0, long long nrows,

@@ -59,8 +59,8 @@ int cgb_create(int64_t n, int rank, int world, int device, cgb_ctx **out);
 /* The same rank with the shard held in CSR storage: no dense shard is allocated, so the system
  * size is bounded by the non-zeros, not by n^2 (n <= INT32_MAX: column indices are int32_t,
  * global; row pointers int64_t; values double; columns ascending and unique within a row).
- * The matrix comes from cgb_generate_lap2d, cgb_set_matrix_coo or cgb_set_matrix_csr (built on the
- * device), its values may be refreshed with cgb_update_matrix_values;
+ * The matrix comes from cgb_generate_lap2d, cgb_set_matrix_coo, cgb_set_matrix_csr or cgb_assemble_coo
+ * (built on the device), its values may be refreshed with cgb_update_matrix_values or cgb_assemble_values;
  * cgb_set_matrix_rows returns CGB_ERR_STATE.  Vectors, exchange wiring and cgb_get_layout are
  * those of cgb_create; the solve runs on the graph schedule ("schedule_in_use" reads 0).
  * Exactness: the CSR mat-vec keeps the lane order of the dense one over the stored entries, and
@@ -151,6 +151,48 @@ int cgb_set_matrix_csr(cgb_ctx *ctx, const int64_t *rp_dev, const int32_t *col_d
  * CGB_ERR_STATE: a dense context (a dense shard keeps no pattern), the matrix not set, a single or block
  * solve between begin and end.  CGB_ERR_INVALID: a null pointer, a host pointer or one on another device. */
 int cgb_update_matrix_values(cgb_ctx *ctx, const double *val_dev, void *stream);
+
+/* Sum-assembly of COO contributions held in device memory of the context's GPU (finite-element or
+ * finite-volume assembly: duplicates are added, as by scipy's coo_matrix.tocsr() or PETSc's ADD_VALUES).
+ *   irn_dev, jcn_dev  nz 0-based global (row, column) pairs;  val_dev  nz values
+ * Triple z makes write 2z at (i, j) and, with `symmetric` and i != j, write 2z+1 at (j, i).  A diagonal
+ * triple is NOT mirrored -- in a sum that would double the diagonal.  This is the one deliberate difference
+ * from the mirroring of cgb_set_matrix_coo (Matrix::read), which keeps the last write instead of adding.
+ * Only writes whose row lies in this rank's shard are kept.  The value of a cell is the sequential left fold
+ * of its writes in ascending write order, starting from the first write:
+ *   v = w0;  v = v + w1;  v = v + w2; ...   (each + one IEEE double addition, rounded to nearest even)
+ * This order is the contract: it makes the result reproducible and checkable bit for bit, and starting from
+ * w0 rather than +0 keeps a lone -0 as -0.  The fold is serial per cell, so a cell that receives 10^5
+ * writes is correct but slow; assembly gives a handful per cell.  Every cell that receives at least one
+ * write is stored, explicit zeros and sums that cancel to zero included, so the pattern depends only on
+ * (irn, jcn, symmetric), never on the values.  Dense and CSR contexts both work: this rank's rows are staged
+ * as CSR and installed like cgb_set_matrix_csr's.  The reads are ordered after the work enqueued on `stream`
+ * by an event; the call synchronises, like every builder.  Staging takes about 66 bytes of device memory per
+ * triple besides the shard, the plan and the sort's scratch.
+ * The call keeps an assembly plan in the context for cgb_assemble_values: 8 bytes per write kept in this
+ * shard and 8 bytes per stored entry (+ 8), and on a dense context also the staged row pointers and columns
+ * (8 bytes per row + 8, 4 bytes per stored entry).  Any other builder (cgb_generate_lap2d,
+ * cgb_set_matrix_coo, cgb_set_matrix_csr, cgb_set_matrix_rows) frees it; cgb_update_matrix_values leaves it.
+ * CGB_ERR_INVALID: nz < 0, a null, host or other-device pointer (nz > 0), or an entry outside n x n.  The
+ * entries are checked on the device before anything of the context is touched, so after a refusal the
+ * previous matrix and its plan stay.  CGB_ERR_STATE: a single or block solve between begin and end.
+ * Its kernels count in cgb_launch_count. */
+int cgb_assemble_coo(cgb_ctx *ctx, int64_t nz, const int32_t *irn_dev, const int32_t *jcn_dev,
+                     const double *val_dev, int symmetric, void *stream);
+
+/* Re-assembly: val_dev holds nz new values for the SAME triples as the last cgb_assemble_coo (same irn, jcn,
+ * symmetric, nz; only the values differ), in device memory of the context's GPU (null allowed when nz == 0).
+ * It writes the matrix cgb_assemble_coo would build from them, bit for bit, with the same fold order, by one
+ * gather-and-fold kernel over the plan.  Fully asynchronous, like cgb_update_matrix_values: an event orders
+ * it after the work enqueued on `stream` and after every solve already enqueued on the context, and work
+ * enqueued on `stream` after the call sees the new matrix.  No host synchronisation, no allocation.  A CSR
+ * context's values are written in place, so every cached loop graph stays valid ("graph_captures" does not
+ * change).  A dense context's cells are written in A and then every row's envelope is rebuilt: a cell that
+ * was an explicit zero at assembly may now be non-zero.
+ * CGB_ERR_STATE: no plan (no cgb_assemble_coo yet, or another builder replaced its matrix), a single or
+ * block solve between begin and end.  CGB_ERR_INVALID: a null pointer, a host pointer or one on another
+ * device. */
+int cgb_assemble_values(cgb_ctx *ctx, const double *val_dev, void *stream);
 
 /* Read rows of the shard back (tests); a CSR shard is densified. */
 int cgb_get_matrix_rows(cgb_ctx *ctx, double *rows_host, int64_t first_row, int64_t nrows,
