@@ -1313,6 +1313,23 @@ int install_matrix(cgb_ctx *c, CsrShard &m, bool staged, AsmPlan *plan = nullptr
     return CGB_OK;
 }
 
+// Stages this rank's rows of COO triples in device memory, each cell's writes folded by `fold`, and installs
+// them.  Nothing of the context, its matrix or its plan, is touched before every triple has been checked.  A
+// non-null `plan` (cgb_assemble_coo's) receives the assembly plan, which becomes the context's.
+int install_coo(cgb_ctx *c, int64_t nz, const int32_t *irn, const int32_t *jcn, const double *val, int symmetric,
+                AsmFold fold, AsmPlan *plan)
+{
+    StagedCsr m;
+    int bad = 0;
+    CK(csr_assemble_coo(&m, plan, fold, c->n, c->row0, c->rows, irn, jcn, val, nz, symmetric ? 1 : 0, &bad,
+                        c->stream));
+    // keys, runs, rows, cols, fold (CUB's sort and selects not counted); of the two COO builders only
+    // cgb_assemble_coo promises its kernels to cgb_launch_count
+    if (plan) c->kernel_launches += nz > 0 ? 5 : 2;
+    if (bad) return fail(CGB_ERR_INVALID, "a COO entry lies outside %lld x %lld", (long long)c->n, (long long)c->n);
+    return install_matrix(c, m, true, plan);
+}
+
 } // namespace
 
 extern "C" int cgb_generate_lap2d(cgb_ctx *c)
@@ -1369,12 +1386,7 @@ extern "C" int cgb_set_matrix_coo(cgb_ctx *c, int64_t nz, const int32_t *irn, co
         CK(cudaMemcpyAsync(j.p, jcn, (size_t)nz * sizeof(int), cudaMemcpyHostToDevice, c->stream));
         CK(cudaMemcpyAsync(v.p, val, (size_t)nz * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     }
-    StagedCsr m;
-    int bad = 0;
-    CK(csr_from_coo(&m, c->n, c->row0, c->rows, i.as<int>(), j.as<int>(), v.as<double>(), nz, symmetric ? 1 : 0, &bad,
-                    c->stream));
-    if (bad) return fail(CGB_ERR_INVALID, "a COO entry lies outside %lld x %lld", (long long)c->n, (long long)c->n);
-    return install_matrix(c, m, true);
+    return install_coo(c, nz, i.as<int32_t>(), j.as<int32_t>(), v.as<double>(), symmetric, kFoldLast, nullptr);
 }
 
 extern "C" int cgb_get_matrix_rows(cgb_ctx *c, double *rows_host, int64_t first_row, int64_t nrows,
@@ -2036,15 +2048,8 @@ extern "C" int cgb_assemble_coo(cgb_ctx *c, int64_t nz, const int32_t *irn_dev, 
     if ((rc = stream_events(c))) return rc;
     CK(cudaEventRecord(c->ev_dev[0], static_cast<cudaStream_t>(stream)));
     CK(cudaStreamWaitEvent(c->stream, c->ev_dev[0], 0));
-    StagedCsr m;
     StagedPlan plan;
-    int bad = 0;
-    CK(csr_assemble_coo(&m, &plan, c->n, c->row0, c->rows, irn_dev, jcn_dev, val_dev, nz, symmetric ? 1 : 0, &bad,
-                        c->stream));
-    c->kernel_launches += nz > 0 ? 5 : 2; // keys, runs, rows, cols, fold (CUB's sort and selects not counted)
-    // nothing of the context, its matrix or its plan, is touched before every triple has been checked
-    if (bad) return fail(CGB_ERR_INVALID, "a COO entry lies outside %lld x %lld", (long long)c->n, (long long)c->n);
-    return install_matrix(c, m, true, &plan);
+    return install_coo(c, nz, irn_dev, jcn_dev, val_dev, symmetric, kFoldSum, &plan);
 }
 
 extern "C" int cgb_assemble_values(cgb_ctx *c, const double *val_dev, void *stream)
@@ -2062,7 +2067,7 @@ extern "C" int cgb_assemble_values(cgb_ctx *c, const double *val_dev, void *stre
     CK(cudaEventRecord(c->ev_dev[0], us));
     CK(cudaStreamWaitEvent(c->stream, c->ev_dev[0], 0));
     if (c->storage == 1) {
-        CK(launch_assemble_csr(c->plan, val_dev, c->csr.val, c->stream));
+        CK(launch_assemble_csr(c->plan, kFoldSum, val_dev, c->csr.val, c->stream));
         c->kernel_launches += 1;
     } else {
         // a cell stored as 0 at assembly lies outside its row's envelope and may have become non-zero

@@ -131,9 +131,9 @@ cudaError_t launch_exchange_collect(double *apx, const Gather &g, cudaStream_t s
 
 // ---- matrix construction ------------------------------------------------------------
 // Every builder of a shard, dense or CSR, makes this rank's local CSR on the device (spmv.cu: lap2d_row
-// is the one statement of generate_lap2d_matrix's stencil, csr_from_coo the one of Matrix::read, fold_run
-// the one of a sum-assembly), and
-// capi.cu installs it: a CSR context adopts it, a dense one densifies it and rebuilds the envelopes.
+// is the one statement of generate_lap2d_matrix's stencil, csr_assemble_coo the one staging of COO triples,
+// fold_run the one statement of how a cell's writes become its value: Matrix::read's last write or a sum),
+// and capi.cu installs it: a CSR context adopts it, a dense one densifies it and rebuilds the envelopes.
 
 // device scratch freed on every path
 struct DevBuf {
@@ -161,13 +161,11 @@ cudaError_t launch_spmv(const GemvArgs &a, int sm_count, cudaStream_t s);
 // path) and synchronise.
 // generate_lap2d_matrix's non-zeros of rows [row0, row0 + rows)
 cudaError_t csr_generate_lap2d(CsrShard *m, long long n, long long row0, long long rows, cudaStream_t s);
-// Matrix::read semantics from device COO triples (file order, mirror when symmetric, later writes
-// win, explicit zeros stored); *bad_host = 1 (and `m` left empty) when an entry lies outside n x n
-cudaError_t csr_from_coo(CsrShard *m, long long n, long long row0, long long rows, const int *irn, const int *jcn,
-                         const double *val, long long nz, int symmetric, int *bad_host, cudaStream_t s);
-// Sum-assembly (cgb_assemble_coo, DESIGN 3.11).  Triple z makes write 2z at (irn[z], jcn[z]) and, symmetric
-// and off the diagonal, write 2z+1 at (jcn[z], irn[z]); a stored entry is the left fold of its writes in
-// write order.  The plan lets every later set of values for the same triples be folded without a sort.
+// COO triples in device memory (DESIGN 3.6, 3.11).  Triple z makes write 2z at (irn[z], jcn[z]) and, symmetric
+// and off the diagonal, write 2z+1 at (jcn[z], irn[z]).  A stored entry folds its writes in write order: to the
+// last (cgb_set_matrix_coo, Matrix::read) or to their left-fold sum (cgb_assemble_coo).  The plan lets every
+// later set of values for the same triples be folded without a sort.
+enum AsmFold { kFoldSum, kFoldLast };
 struct AsmPlan {
     long long *wid = nullptr;   // [nwrites] the writes this shard keeps, sorted by (row, column, write id)
     long long *start = nullptr; // [nnz + 1] entry e (stored order) folds wid[start[e] .. start[e+1])
@@ -176,14 +174,14 @@ struct AsmPlan {
     long long nz = 0, nnz = 0, nwrites = 0, rows = 0;
 };
 void asm_plan_free(AsmPlan *p);
-// this rank's rows of the sum of the triples into an empty shard `m` and plan `p` (wid / start; rp / col are
-// left null), synchronised; *bad_host = 1 (and `m`, `p` left empty) when an entry lies outside n x n
-cudaError_t csr_assemble_coo(CsrShard *m, AsmPlan *p, long long n, long long row0, long long rows, const int *irn,
-                             const int *jcn, const double *val, long long nz, int symmetric, int *bad_host,
-                             cudaStream_t s);
-// the plan's fold of nz values: into a CSR shard's values (stored order), or into the cells of the dense
+// this rank's rows of the triples into an empty shard `m` and, if `p` is not null, plan `p` (wid / start; rp /
+// col are left null), synchronised; *bad_host = 1 (and `m`, `p` left empty) when an entry lies outside n x n
+cudaError_t csr_assemble_coo(CsrShard *m, AsmPlan *p, AsmFold fold, long long n, long long row0, long long rows,
+                             const int *irn, const int *jcn, const double *val, long long nz, int symmetric,
+                             int *bad_host, cudaStream_t s);
+// the plan's fold of nz values: into a CSR shard's values (stored order), or by sum into the cells of the dense
 // rows x ld shard A (p.rp / p.col set)
-cudaError_t launch_assemble_csr(const AsmPlan &p, const double *val, double *out, cudaStream_t s);
+cudaError_t launch_assemble_csr(const AsmPlan &p, AsmFold fold, const double *val, double *out, cudaStream_t s);
 cudaError_t launch_assemble_dense(const AsmPlan &p, const double *val, long long ld, double *A, cudaStream_t s);
 // col / val of `nnz` entries for a shard without them
 cudaError_t csr_alloc_entries(CsrShard *m, long long nnz);

@@ -1,5 +1,5 @@
 // spmv.cu -- CSR storage of the row shard: the mat-vec in lane order and the builders of the shard
-// (generate_lap2d_matrix, Matrix::read's COO semantics, sum-assembly of COO contributions) on the device.
+// (generate_lap2d_matrix, COO writes folded by Matrix::read's last write or summed) on the device.
 //
 // Exactness.  The dense mat-vec (gemv.cu, oracle/cg_oracle.h "lane order") keeps 64 accumulators
 // acc[c % 64] = fma(A[i][c], p[c], acc[c % 64]) over ascending c from +0, adds acc[2l] + acc[2l+1]
@@ -342,43 +342,14 @@ __global__ void lap2d_fill_kernel(long long n, long long inc, long long row0, lo
     });
 }
 
-// Matrix::read (matrix.cc:12-21) as write sequence 2z (A(i,j)) and 2z+1 (A(j,i), symmetric only);
-// a write outside this shard's rows gets the key that sorts last
+// COO triples as a write sequence: triple z makes write 2z at (i, j) and, symmetric and off the diagonal, write
+// 2z+1 at (j, i).  A mirrored diagonal would count twice in a sum; under Matrix::read's "later entries
+// overwrite" it would only repeat write 2z's value in the same cell.  So neither fold needs it.  A write
+// outside this shard's rows gets the key that sorts last.  The sort payload is the write id, so that the
+// sorted order doubles as the plan every fold gathers by.
 constexpr unsigned long long kNoKey = ~0ULL;
-__global__ void coo_keys_kernel(long long n, long long row0, long long rows, const int *irn, const int *jcn,
-                                const double *val, long long nz, int symmetric, unsigned long long *key,
-                                double *kval, int *bad)
-{
-    const long long z = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (z >= nz) return;
-    const long long i = irn[z], j = jcn[z];
-    const double a = val[z];
-    unsigned long long k0 = kNoKey, k1 = kNoKey;
-    if (i < 0 || j < 0 || i >= n || j >= n) {
-        *bad = 1;
-    } else {
-        if (i >= row0 && i < row0 + rows) k0 = ((unsigned long long)(i - row0) << 32) | (unsigned long long)j;
-        if (symmetric && j >= row0 && j < row0 + rows) k1 = ((unsigned long long)(j - row0) << 32) | (unsigned long long)i;
-    }
-    key[2 * z] = k0;
-    key[2 * z + 1] = k1;
-    kval[2 * z] = a;
-    kval[2 * z + 1] = a;
-}
-
-// after the stable sort: the last write of every (row, column) run survives
-__global__ void coo_last_kernel(const unsigned long long *key, long long m, unsigned char *keep)
-{
-    const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= m) return;
-    keep[k] = (key[k] != kNoKey && (k == m - 1 || key[k + 1] != key[k])) ? 1 : 0;
-}
-
-// Sum-assembly (cgb_assemble_coo): coo_keys_kernel's write sequence, except that a diagonal triple is not
-// mirrored (in a sum it would count twice) and the sort payload is the write id, so that the sorted order
-// doubles as the plan every later re-assembly gathers by
 __global__ void asm_keys_kernel(long long n, long long row0, long long rows, const int *irn, const int *jcn,
-                                long long nz, int symmetric, unsigned long long *key, long long *wid, int *bad)
+                                long long nz, int symmetric, unsigned long long *key, long long *wid, long long *bad)
 {
     const long long z = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (z >= nz) return;
@@ -407,11 +378,14 @@ __global__ void asm_runs_kernel(const unsigned long long *key, long long m, unsi
     if (kept && (k == m - 1 || key[k + 1] == kNoKey)) *nw = k + 1;
 }
 
-// The one statement of the fold: stored entry e is its run of writes folded left in write order, starting
-// from the first write (not from +0, which would turn a lone -0 into +0).  Serial per cell by definition.
-__device__ __forceinline__ double fold_run(const AsmPlan &p, const double *val, long long e)
+// The one statement of the fold: stored entry e is its run of writes in write order, folded by F.
+//   kFoldSum   left fold from the first write (not from +0, which would turn a lone -0 into +0), serial per
+//              cell by definition;
+//   kFoldLast  the run's last write, verbatim (Matrix::read, matrix.cc:12-21: later entries overwrite).
+template <AsmFold F> __device__ __forceinline__ double fold_run(const AsmPlan &p, const double *val, long long e)
 {
     const long long end = p.start[e + 1];
+    if (F == kFoldLast) return val[p.wid[end - 1] >> 1];
     long long k = p.start[e];
     double v = val[p.wid[k] >> 1];
     for (++k; k < end; ++k) v = __dadd_rn(v, val[p.wid[k] >> 1]);
@@ -419,20 +393,22 @@ __device__ __forceinline__ double fold_run(const AsmPlan &p, const double *val, 
 }
 
 // CSR shard: the values in stored order, one thread per entry
-__global__ void assemble_csr_kernel(const AsmPlan p, const double *val, double *out)
+template <AsmFold F> __global__ void assemble_csr_kernel(const AsmPlan p, const double *val, double *out)
 {
     const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e < p.nnz) out[e] = fold_run(p, val, e);
+    if (e < p.nnz) out[e] = fold_run<F>(p, val, e);
 }
 
-// dense shard: one warp per row (its row from the plan's rp), lanes striding over the row's entries
+// dense shard (re-assembly, a sum): one warp per row (its row from the plan's rp), lanes striding over the row's
+// entries
 __global__ void __launch_bounds__(256) assemble_dense_kernel(const AsmPlan p, const double *val, long long ld,
                                                               double *A)
 {
     const long long row = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
     if (row >= p.rows) return;
     const long long end = p.rp[row + 1];
-    for (long long e = p.rp[row] + (threadIdx.x & 31); e < end; e += 32) A[row * ld + p.col[e]] = fold_run(p, val, e);
+    for (long long e = p.rp[row] + (threadIdx.x & 31); e < end; e += 32)
+        A[row * ld + p.col[e]] = fold_run<kFoldSum>(p, val, e);
 }
 
 // row pointers and columns from the surviving keys (sorted by row, then column)
@@ -602,61 +578,6 @@ cudaError_t csr_generate_lap2d(CsrShard *m, long long n, long long row0, long lo
     return cudaStreamSynchronize(s);
 }
 
-cudaError_t csr_from_coo(CsrShard *m, long long n, long long row0, long long rows, const int *irn, const int *jcn,
-                         const double *val, long long nz, int symmetric, int *bad_host, cudaStream_t s)
-{
-    *bad_host = 0;
-    const long long m2 = 2 * nz;
-    // 66 B per triple: 2 writes x (8 B key + 8 B value) x (unsorted, sorted) + 2 flag bytes.  key / kval
-    // are dead after the sort and receive the writes kept.
-    DevBuf key, kval, key_s, kval_s, keep, nsel, bad, tmp;
-    CU(key.alloc((size_t)m2 * 8));
-    CU(kval.alloc((size_t)m2 * 8));
-    CU(key_s.alloc((size_t)m2 * 8));
-    CU(kval_s.alloc((size_t)m2 * 8));
-    CU(keep.alloc((size_t)m2));
-    CU(nsel.alloc(sizeof(long long)));
-    CU(bad.alloc(sizeof(int)));
-    CU(cudaMemsetAsync(bad.p, 0, sizeof(int), s));
-    CU(cudaMemsetAsync(nsel.p, 0, sizeof(long long), s));
-    if (nz > 0) {
-        coo_keys_kernel<<<blocks_for(nz, 256), 256, 0, s>>>(n, row0, rows, irn, jcn, val, nz, symmetric,
-                                                            key.as<unsigned long long>(), kval.as<double>(), bad.as<int>());
-        CU(cudaGetLastError());
-        // radix sort is stable: equal (row, column) keys keep their write order
-        size_t b_sort = 0, b_sel = 0, b_sel2 = 0;
-        CU(cub::DeviceRadixSort::SortPairs(nullptr, b_sort, key.as<unsigned long long>(), key_s.as<unsigned long long>(),
-                                           kval.as<double>(), kval_s.as<double>(), m2, 0, 64, s));
-        CU(cub::DeviceSelect::Flagged(nullptr, b_sel, key_s.as<unsigned long long>(), keep.as<unsigned char>(),
-                                      key.as<unsigned long long>(), nsel.as<long long>(), m2, s));
-        CU(cub::DeviceSelect::Flagged(nullptr, b_sel2, kval_s.as<double>(), keep.as<unsigned char>(),
-                                      kval.as<double>(), nsel.as<long long>(), m2, s));
-        size_t b = b_sort > b_sel ? b_sort : b_sel;
-        if (b_sel2 > b) b = b_sel2;
-        CU(tmp.alloc(b));
-        CU(cub::DeviceRadixSort::SortPairs(tmp.p, b_sort, key.as<unsigned long long>(), key_s.as<unsigned long long>(),
-                                           kval.as<double>(), kval_s.as<double>(), m2, 0, 64, s));
-        coo_last_kernel<<<blocks_for(m2, 256), 256, 0, s>>>(key_s.as<unsigned long long>(), m2, keep.as<unsigned char>());
-        CU(cudaGetLastError());
-        CU(cub::DeviceSelect::Flagged(tmp.p, b_sel, key_s.as<unsigned long long>(), keep.as<unsigned char>(),
-                                      key.as<unsigned long long>(), nsel.as<long long>(), m2, s));
-        CU(cub::DeviceSelect::Flagged(tmp.p, b_sel2, kval_s.as<double>(), keep.as<unsigned char>(),
-                                      kval.as<double>(), nsel.as<long long>(), m2, s));
-    }
-    long long nnz = 0;
-    CU(cudaMemcpyAsync(&nnz, nsel.p, sizeof nnz, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(bad_host, bad.p, sizeof(int), cudaMemcpyDeviceToHost, s));
-    CU(cudaStreamSynchronize(s));
-    if (*bad_host) return cudaSuccess;
-    CU(cudaMalloc(&m->rp, (size_t)(rows + 1) * sizeof(long long)));
-    CU(csr_alloc_entries(m, nnz));
-    csr_rows_kernel<<<blocks_for(rows + 1, 256), 256, 0, s>>>(key.as<unsigned long long>(), nnz, rows, m->rp);
-    csr_cols_kernel<<<blocks_for(nnz, 256), 256, 0, s>>>(key.as<unsigned long long>(), nnz, m->col);
-    CU(cudaGetLastError());
-    if (nnz > 0) CU(cudaMemcpyAsync(m->val, kval.p, (size_t)nnz * 8, cudaMemcpyDeviceToDevice, s));
-    return cudaStreamSynchronize(s);
-}
-
 void asm_plan_free(AsmPlan *p)
 {
     cudaFree(p->wid);
@@ -666,27 +587,26 @@ void asm_plan_free(AsmPlan *p)
     *p = AsmPlan();
 }
 
-cudaError_t csr_assemble_coo(CsrShard *m, AsmPlan *p, long long n, long long row0, long long rows, const int *irn,
-                             const int *jcn, const double *val, long long nz, int symmetric, int *bad_host,
-                             cudaStream_t s)
+cudaError_t csr_assemble_coo(CsrShard *m, AsmPlan *p, AsmFold fold, long long n, long long row0, long long rows,
+                             const int *irn, const int *jcn, const double *val, long long nz, int symmetric,
+                             int *bad_host, cudaStream_t s)
 {
     *bad_host = 0;
     const long long m2 = 2 * nz;
     // 66 B per triple: 2 writes x (8 B key + 8 B write id) x (unsorted, sorted) + 2 flag bytes.  key / wid are
-    // dead after the sort and receive the unique keys and the run starts.  cnt: [0] entries, [1] writes kept.
-    DevBuf key, wid, key_s, wid_s, first, cnt, bad, tmp;
+    // dead after the sort and receive the unique keys and the run starts (wid one longer, for the sentinel
+    // start[nnz]).  cnt: [0] entries, [1] writes kept, [2] non-zero when an entry lies outside n x n.
+    DevBuf key, wid, key_s, wid_s, first, cnt, tmp;
     CU(key.alloc((size_t)m2 * 8));
-    CU(wid.alloc((size_t)m2 * 8));
+    CU(wid.alloc((size_t)(m2 + 1) * 8));
     CU(key_s.alloc((size_t)m2 * 8));
     CU(wid_s.alloc((size_t)m2 * 8));
     CU(first.alloc((size_t)m2));
-    CU(cnt.alloc(2 * sizeof(long long)));
-    CU(bad.alloc(sizeof(int)));
-    CU(cudaMemsetAsync(bad.p, 0, sizeof(int), s));
-    CU(cudaMemsetAsync(cnt.p, 0, 2 * sizeof(long long), s));
+    CU(cnt.alloc(3 * sizeof(long long)));
+    CU(cudaMemsetAsync(cnt.p, 0, 3 * sizeof(long long), s));
     if (nz > 0) {
-        asm_keys_kernel<<<blocks_for(nz, 256), 256, 0, s>>>(n, row0, rows, irn, jcn, nz, symmetric,
-                                                            key.as<unsigned long long>(), wid.as<long long>(), bad.as<int>());
+        asm_keys_kernel<<<blocks_for(nz, 256), 256, 0, s>>>(n, row0, rows, irn, jcn, nz, symmetric, key.as<unsigned long long>(),
+                                                            wid.as<long long>(), cnt.as<long long>() + 2);
         CU(cudaGetLastError());
         // radix sort is stable: equal (row, column) keys keep their write order
         const thrust::counting_iterator<long long> pos(0);
@@ -710,34 +630,39 @@ cudaError_t csr_assemble_coo(CsrShard *m, AsmPlan *p, long long n, long long row
         CU(cub::DeviceSelect::Flagged(tmp.p, b_sel2, pos, first.as<unsigned char>(), wid.as<long long>(),
                                       cnt.as<long long>(), m2, s));
     }
-    long long counts[2] = {0, 0};
+    long long counts[3] = {0, 0, 0};
     CU(cudaMemcpyAsync(counts, cnt.p, sizeof counts, cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(bad_host, bad.p, sizeof(int), cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
+    *bad_host = counts[2] != 0;
     if (*bad_host) return cudaSuccess;
     const long long nnz = counts[0], nw = counts[1];
+    // the staging buffers as a plan: the sorted write ids and the run starts where the selects left them
+    const AsmPlan run{wid_s.as<long long>(), wid.as<long long>(), nullptr, nullptr, nz, nnz, nw, rows};
+    CU(cudaMemcpyAsync(run.start + nnz, cnt.as<long long>() + 1, sizeof(long long), cudaMemcpyDeviceToDevice, s));
     CU(cudaMalloc(&m->rp, (size_t)(rows + 1) * sizeof(long long)));
     CU(csr_alloc_entries(m, nnz));
-    CU(cudaMalloc(&p->wid, (size_t)(nw > 0 ? nw : 1) * sizeof(long long)));
-    CU(cudaMalloc(&p->start, (size_t)(nnz + 1) * sizeof(long long)));
-    p->nz = nz;
-    p->nnz = nnz;
-    p->nwrites = nw;
-    p->rows = rows;
+    if (p) {
+        CU(cudaMalloc(&p->wid, (size_t)(nw > 0 ? nw : 1) * sizeof(long long)));
+        CU(cudaMalloc(&p->start, (size_t)(nnz + 1) * sizeof(long long)));
+        p->nz = nz;
+        p->nnz = nnz;
+        p->nwrites = nw;
+        p->rows = rows;
+        if (nw > 0) CU(cudaMemcpyAsync(p->wid, run.wid, (size_t)nw * 8, cudaMemcpyDeviceToDevice, s));
+        CU(cudaMemcpyAsync(p->start, run.start, (size_t)(nnz + 1) * 8, cudaMemcpyDeviceToDevice, s));
+    }
     csr_rows_kernel<<<blocks_for(rows + 1, 256), 256, 0, s>>>(key.as<unsigned long long>(), nnz, rows, m->rp);
     csr_cols_kernel<<<blocks_for(nnz, 256), 256, 0, s>>>(key.as<unsigned long long>(), nnz, m->col);
     CU(cudaGetLastError());
-    if (nw > 0) CU(cudaMemcpyAsync(p->wid, wid_s.p, (size_t)nw * 8, cudaMemcpyDeviceToDevice, s));
-    if (nnz > 0) CU(cudaMemcpyAsync(p->start, wid.p, (size_t)nnz * 8, cudaMemcpyDeviceToDevice, s));
-    CU(cudaMemcpyAsync(p->start + nnz, cnt.as<long long>() + 1, sizeof(long long), cudaMemcpyDeviceToDevice, s));
-    CU(launch_assemble_csr(*p, val, m->val, s));
+    CU(launch_assemble_csr(run, fold, val, m->val, s));
     return cudaStreamSynchronize(s);
 }
 
-cudaError_t launch_assemble_csr(const AsmPlan &p, const double *val, double *out, cudaStream_t s)
+cudaError_t launch_assemble_csr(const AsmPlan &p, AsmFold fold, const double *val, double *out, cudaStream_t s)
 {
     if (p.nnz == 0) return cudaSuccess;
-    assemble_csr_kernel<<<blocks_for(p.nnz, 256), 256, 0, s>>>(p, val, out);
+    if (fold == kFoldLast) assemble_csr_kernel<kFoldLast><<<blocks_for(p.nnz, 256), 256, 0, s>>>(p, val, out);
+    else assemble_csr_kernel<kFoldSum><<<blocks_for(p.nnz, 256), 256, 0, s>>>(p, val, out);
     return cudaGetLastError();
 }
 

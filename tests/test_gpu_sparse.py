@@ -73,12 +73,26 @@ def test_coo_million_duplicates_dense_and_csr_are_the_oracle(cgb, symmetric):
     jcn = rng.integers(0, n, nz, dtype=np.int32)
     val = rng.standard_normal(nz)
     val[::1000] = 0.0
-    want = csr_oracle.csr_from_coo(n, irn, jcn, val, symmetric).dense()
+    val[500::1000] = -0.0
+    ref = csr_oracle.csr_from_coo(n, irn, jcn, val, symmetric)
+    zero = ref.val == 0
+    assert np.signbit(ref.val[zero]).any() and not np.signbit(ref.val[zero]).all()  # -0 and +0 last writers
+    want = ref.dense()
     with cgb.Context(n) as d, cgb.Context(n, storage="csr") as c:
         d.set_matrix_coo(irn, jcn, val, symmetric=symmetric)
         c.set_matrix_coo(irn, jcn, val, symmetric=symmetric)
         assert _eq(d.get_matrix_rows(0, n), want)
         assert _eq(c.get_matrix_rows(0, n), want)
+        assert c.nnz() == ref.col.size   # explicit zeros stored
+        s, cnt = cgb.partition(n, 3)
+        for r in range(3):   # every shard of a 3-way split
+            part = csr_oracle.csr_from_coo(n, irn, jcn, val, symmetric, s[r], cnt[r])
+            for storage in ("dense", "csr"):
+                with cgb.Context(n, r, 3, 0, storage=storage) as ctx:
+                    ctx.set_matrix_coo(irn, jcn, val, symmetric=symmetric)
+                    assert _eq(ctx.get_matrix_rows(s[r], cnt[r]), part.dense())
+                    if storage == "csr":
+                        assert ctx.nnz() == part.col.size
         with pytest.raises(cgb.CgbError) as ei:
             c.set_matrix_coo(np.array([0, n], dtype=np.int32), np.array([0, 0], dtype=np.int32),
                              np.array([1.0, 2.0]), symmetric=False)
